@@ -77,7 +77,7 @@ WORKLOADS = {
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="env-steps in every timed section (headline, variants, end to end)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="40x40", choices=sorted(WORKLOADS))
@@ -98,7 +98,11 @@ def parse():
                          "default (compute_tar_psf=True, rlSupervisor.py:944-947); without the flag the figure is still "
                          "reported as a variant beside the headline")
     ap.add_argument("--no-variants", action="store_true", help="skip the extra sections (Strehl variant, learner, reset timing)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step left for its caller to DIR/<name>.npy (see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.denoise and a.workload == "40x40":
         a.workload = "40x40_d0_noise"          # config 4 runs on its own parameter file
     return a
@@ -313,7 +317,7 @@ def measure_variants(args, sim, t, rl, E, dist, barrier, ev):
     learn_*     config 5: one batched SAC update of all agents per env-step, gradients all-reduced over NCCL"""
     import torch
     out = {}
-    k = max(2, min(args.steps, 5))
+    k = args.steps
     if not args.strehl:
         sim.step_with_strehl(True, 1.65)
         for _ in range(2):
@@ -419,6 +423,32 @@ def format_variants(v, args, E, world, ms):
     return out
 
 
+DUMP_MAX_ENVS = 512
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, sim, t, rl, E, args):
+    """Writes what the last timed step left for its caller -- state, rewards, actions, slopes and commands, plus the
+    Strehl figures / geometric commands when the step computes them -- as float32 `path/<name>.npy`, [n, width] rows of
+    a fixed seeded sample of n <= 512 environments (their indices in env_index.npy), at most 64 MB in all.  The inputs
+    of a run depend only on its arguments, so two builds run with the same arguments can be compared file for file."""
+    import torch
+    outs = [("state", "STATE", rl.state_dim), ("reward", "REWARD", rl.n_agents), ("action", "ACTION", rl.action_dim),
+            ("slopes", "SLOPES", t.nslopes), ("commands", "COM", t.nactu)]
+    if args.strehl:
+        outs.append(("strehl", "STREHL", 4))
+    if args.geo:
+        outs.append(("geo_commands", "GEO_COM", t.nactu))
+    per_env = 8 + 4 * sum(width for _, _, width in outs)
+    n = min(E, DUMP_MAX_ENVS, DUMP_MAX_BYTES // per_env)
+    idx = np.sort(np.random.default_rng(0).choice(E, n, replace=False))
+    sel = torch.as_tensor(idx, device="cuda")
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "env_index.npy"), idx.astype(np.float64))
+    for name, buf, width in outs:
+        np.save(os.path.join(path, name + ".npy"), sim.rows(buf, width).index_select(0, sel).cpu().numpy())
+
+
 def run_ours(args):
     import torch
     rank = int(os.environ.get("RANK", "0"))
@@ -498,6 +528,8 @@ def run_ours(args):
     ms = e0.elapsed_time(e1)
     wfs_ms, _ = sim.wfs_time_ms()
     sim.time_wfs(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sim, t, rl, E, args)
 
     variants = {}
     if not args.no_variants:
@@ -521,7 +553,7 @@ def run_ours(args):
     snap_copied = [ev() for _ in range(2)]
     main = torch.cuda.current_stream()
     act_h.copy_(act_d)
-    k_e2e = max(2, args.steps)                    # the same K as the device-timed loop
+    k_e2e = args.steps                            # the same K as the device-timed loop
     barrier()
     f0, f1 = ev(enable_timing=True), ev(enable_timing=True)
     f0.record()

@@ -1,6 +1,6 @@
 """Development probe: device time of the denoiser (row a-6) per 40x40 frame: fused kernel vs cuDNN through torch."""
 import sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, ".")
 import numpy as np
 import torch
 from ao_marl_b200 import tables

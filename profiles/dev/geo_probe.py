@@ -1,6 +1,6 @@
 """Development probe: where does the CUDA geometric projection differ from the float64 host pipeline (40x40)?"""
 import sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, ".")
 import numpy as np
 import torch
 from ao_marl_b200 import tables

@@ -1,6 +1,6 @@
 """Development probe: device time of the geometric controller at the bench size (E = 4096, 40x40, 3 layers)."""
 import sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, ".")
 import numpy as np
 import torch
 from ao_marl_b200 import tables

@@ -1,6 +1,6 @@
 """Development probe: the literal BASELINE config-3 agent layout (14 x 90 modes + tip-tilt) through the fused step."""
 import sys, time
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, ".")
 import numpy as np
 import torch
 from ao_marl_b200.system import build_system

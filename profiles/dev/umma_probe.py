@@ -1,11 +1,11 @@
 """Development probe: wfs_frame_umma_kernel against the float32 FFT kernel (10x10 and 40x40), for both readings of
 the MN-major descriptor (AOM_UMMA_SWAP=0/1), each in its own process (an expired wait traps the context)."""
 import os, subprocess, sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, ".")
 
 CHILD = r'''
 import sys, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, ".")
 from ao_marl_b200 import tables
 from ao_marl_b200.config import load_config_from_file
 from ao_marl_b200.lib import Simulator
