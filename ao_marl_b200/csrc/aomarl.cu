@@ -2,6 +2,7 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdarg.h>
+#include <algorithm>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -39,6 +40,18 @@ struct aom_ctx {
   uint32_t* ext_count[AOM_MAX_LAYERS];
   float* amp_env[AOM_MAX_LAYERS];     // optional per-environment innovation amplitude (aom_set_layer_amp)
   double accx[AOM_MAX_LAYERS], accy[AOM_MAX_LAYERS];
+  // per-environment winds (aom_set_layer_wind).  While wind_pe is set every layer keeps one accumulator per environment
+  // on the device (wind_state_kernel) and in a host mirror that only sizes the extrusion passes; the extrusion and
+  // sampling kernels run their per-environment instantiations.  Otherwise accx / accy above hold the state.
+  float *wind_dx[AOM_MAX_LAYERS], *wind_dy[AOM_MAX_LAYERS];     // device [E] steps of layers with their own winds, else null
+  float *wind_hdx[AOM_MAX_LAYERS], *wind_hdy[AOM_MAX_LAYERS];   // host copies
+  bool wind_pe;
+  double* wind_acc;            // device [L][2][E] accumulators (x, y)
+  int* wind_steps;             // device [L][2][E] whole-pixel counts of the last frame (x, y)
+  WindRec* wind_rec;           // device [L][E] offsets for the samplers
+  double* wind_hacc;           // host mirror of wind_acc
+  int wind_passes[AOM_MAX_LAYERS][2];   // extrusion passes of the last frame: max over the batch of |count| (x, y)
+  int wind_box[AOM_MAX_LAYERS][4];      // min / max over the batch of ix, then of iy (pupil footprint check)
   uint32_t *k0, *k1;
   float *Z, *zref, *newcol;
   int ldz_max, ldn_max;
@@ -259,6 +272,8 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   CU(cudaFuncSetAttribute(gemm_tc_kernel<1, GTC_BN_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES_T(GTC_BN_WIDE)));
   CU(cudaFuncSetAttribute(wfs_frame_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
   CU(cudaFuncSetAttribute(wfs_frame_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
+  CU(cudaFuncSetAttribute(wfs_frame_kernel<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
+  CU(cudaFuncSetAttribute(wfs_frame_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
   return AOM_OK;
 }
 
@@ -269,7 +284,9 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
   for (int l = 0; l < AOM_MAX_LAYERS; ++l) {
     cudaFree(ctx->screen[l]); cudaFree(ctx->ox[l]); cudaFree(ctx->oy[l]); cudaFree(ctx->ext_count[l]);
     cudaFree(ctx->amp_env[l]);
+    cudaFree(ctx->wind_dx[l]); cudaFree(ctx->wind_dy[l]); free(ctx->wind_hdx[l]); free(ctx->wind_hdy[l]);
   }
+  cudaFree(ctx->wind_acc); cudaFree(ctx->wind_steps); cudaFree(ctx->wind_rec); free(ctx->wind_hacc);
   void* bufs[] = {ctx->k0, ctx->k1, ctx->Z, ctx->zref, ctx->newcol, ctx->slopes_frame, ctx->slopes, ctx->err_v,
                   ctx->com, ctx->com1, ctx->volts, ctx->com_before, ctx->bincube, ctx->phase, ctx->modes,
                   ctx->modes_before, ctx->modes_res, ctx->state, ctx->hist, ctx->reward, ctx->action,
@@ -453,12 +470,12 @@ static int sweep_prepare(aom_ctx* ctx, cudaStream_t st) {
   return AOM_OK;
 }
 
-template <int NL, int MODE>
+template <int NL, int MODE, bool PE>
 static int sweep_launch_t(aom_ctx* ctx, const SweepParams& P, cudaStream_t st) {
-  const size_t smem = psw_smem_bytes(NL);
-  CU(cudaFuncSetAttribute(pupil_sweep_kernel<NL, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const size_t smem = psw_smem_bytes(NL, PE);
+  CU(cudaFuncSetAttribute(pupil_sweep_kernel<NL, MODE, PE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   dim3 grid((P.n_strips * P.nb + PSW_WARPS - 1) / PSW_WARPS, P.w.E);
-  pupil_sweep_kernel<NL, MODE><<<grid, PSW_WARPS * 32, smem, st>>>(P);
+  pupil_sweep_kernel<NL, MODE, PE><<<grid, PSW_WARPS * 32, smem, st>>>(P);
   KCHECK();
   return AOM_OK;
 }
@@ -476,11 +493,19 @@ static int sweep_launch(aom_ctx* ctx, const WfsParams& w, float* Tp, double* mom
   P.nb = ctx->sweep_nb;
   P.n_strips = (c.n + PSW_STRIP - 1) / PSW_STRIP;
   P.err = ctx->d_err;
+  if (w.wind) {          // per-environment winds
+    switch (w.n_layers) {
+      case 1: return sweep_launch_t<1, MODE, true>(ctx, P, st);
+      case 2: return sweep_launch_t<2, MODE, true>(ctx, P, st);
+      case 3: return sweep_launch_t<3, MODE, true>(ctx, P, st);
+      default: return sweep_launch_t<4, MODE, true>(ctx, P, st);
+    }
+  }
   switch (w.n_layers) {
-    case 0: case 1: return sweep_launch_t<1, MODE>(ctx, P, st);
-    case 2: return sweep_launch_t<2, MODE>(ctx, P, st);
-    case 3: return sweep_launch_t<3, MODE>(ctx, P, st);
-    default: return sweep_launch_t<4, MODE>(ctx, P, st);
+    case 0: case 1: return sweep_launch_t<1, MODE, false>(ctx, P, st);
+    case 2: return sweep_launch_t<2, MODE, false>(ctx, P, st);
+    case 3: return sweep_launch_t<3, MODE, false>(ctx, P, st);
+    default: return sweep_launch_t<4, MODE, false>(ctx, P, st);
   }
 }
 
@@ -647,7 +672,8 @@ extern "C" int aom_gemm_tn(aom_ctx* ctx, const float* A, int lda, const float* B
 }
 
 // ---------------------------------------------------------------------------------------------
-static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st) {
+// steps != null: per-environment winds -- pass `pass` of the signed counts steps [E] of this axis (`sign` unused)
+static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st, const int* steps = nullptr, int pass = 0) {
   const aom_config& c = ctx->cfg;
   NEED(AOM_T_AB, l);
   NEED(AOM_T_STENCIL, l);
@@ -657,6 +683,7 @@ static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st
   p.N = c.screen_dim[l]; p.S = c.stencil_size[l]; p.E = c.n_env; p.layer = l; p.axis = axis; p.sign = sign;
   p.amp = c.amp[l]; p.amp_env = ctx->amp_env[l];
   p.ldz = AOM_LD(p.S + p.N); p.Z = ctx->Z; p.zref = ctx->zref; p.ldn = AOM_LD(p.N); p.newcol = ctx->newcol;
+  p.steps = steps; p.pass = pass;
   if (ctx->opt[AOM_OPT_EXTRUDE_PATH] == AOM_EXTRUDE_I8) {
     // exact integer contraction on tcgen05 (extrude_i8.cuh): digits of the inputs, 13 int8 digit-pair products with
     // int32 accumulators, one rounding to float32 after adding the reference pixel
@@ -675,6 +702,7 @@ static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st
     g.screen = p.screen; g.ox = p.ox; g.oy = p.oy; g.count = p.count; g.k0 = p.k0; g.k1 = p.k1; g.stencil = p.stencil;
     g.zref = p.zref; g.ev = ev; g.Zs = zs; g.N = p.N; g.S = p.S; g.E = p.E; g.KB = KB; g.layer = l;
     g.axis = axis; g.sign = sign; g.amp = p.amp; g.amp_env = ctx->amp_env[l];
+    g.steps = steps; g.pass = pass;
     OzGemmParams m;
     m.Zs = zs; m.ABs = ctx->oz_ab[l]; m.ev = ev; m.ea = ctx->oz_ea[l]; m.zref = p.zref;
     m.out = p.newcol; m.ldo = p.ldn; m.E = p.E; m.N = p.N; m.KB = KB; m.err = ctx->d_err;
@@ -683,14 +711,133 @@ static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st
     ctx->launches += 2;
     p.zref = nullptr;                                  // the reference pixel is already in the new column
   } else {
-    extrude_gather_kernel<<<c.n_env, 256, 0, st>>>(p);
+    if (steps) extrude_gather_kernel<true><<<c.n_env, 256, 0, st>>>(p);
+    else extrude_gather_kernel<false><<<c.n_env, 256, 0, st>>>(p);
     KCHECK();
     int rc = launch_gemm(ctx, 0, ctx->Z, p.ldz, 0, (const float*)ctx->tab[AOM_T_AB][l], p.ldz, 0, ctx->newcol, p.ldn, 0,
                          c.n_env, p.N, p.S + p.N, nullptr, 0, 0, 1, st, nullptr, 0, true);
     if (rc) return rc;
   }
-  extrude_scatter_kernel<<<c.n_env, EXTRUDE_SCATTER_THREADS, 0, st>>>(p);
+  if (steps) extrude_scatter_kernel<true><<<c.n_env, EXTRUDE_SCATTER_THREADS, 0, st>>>(p);
+  else extrude_scatter_kernel<false><<<c.n_env, EXTRUDE_SCATTER_THREADS, 0, st>>>(p);
   KCHECK();
+  return AOM_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// per-environment winds
+static bool wind_any_env(const aom_ctx* ctx) {
+  for (int l = 0; l < ctx->cfg.n_layers; ++l)
+    if (ctx->wind_dx[l]) return true;
+  return false;
+}
+
+// One transition of the wind state of every layer and environment (WIND_STEP / WIND_INIT / WIND_RESET, atmos_kernels.cuh)
+// on the device, asynchronously on `st`, and the same on the host mirror: passes per layer and offset bounds.
+static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st) {
+  const aom_config& c = ctx->cfg;
+  const int E = c.n_env, L = c.n_layers;
+  if (L == 0) return AOM_OK;
+  WindStateParams P;
+  memset(&P, 0, sizeof(P));
+  for (int l = 0; l < L; ++l) {
+    WindLayerParams& W = P.layer[l];
+    W.dx = ctx->wind_dx[l]; W.dy = ctx->wind_dy[l]; W.cdx = c.deltax[l]; W.cdy = c.deltay[l];
+    W.ax0 = ctx->accx[l]; W.ay0 = ctx->accy[l]; W.xoff = c.wfs_xoff[l]; W.yoff = c.wfs_yoff[l]; W.n2 = 2 * c.screen_dim[l];
+  }
+  P.acc = ctx->wind_acc; P.steps = ctx->wind_steps; P.rec = ctx->wind_rec; P.E = E; P.n_layers = L; P.mode = mode;
+  wind_state_kernel<<<(L * E + 255) / 256, 256, 0, st>>>(P);
+  KCHECK();
+  for (int l = 0; l < L; ++l) {
+    const WindLayerParams& W = P.layer[l];
+    double* ax = ctx->wind_hacc + (size_t)2 * l * E;
+    double* ay = ax + E;
+    int px = 0, py = 0;
+    int* box = ctx->wind_box[l];
+    for (int e = 0; e < E; ++e) {
+      const float dx = ctx->wind_hdx[l] ? ctx->wind_hdx[l][e] : W.cdx, dy = ctx->wind_hdy[l] ? ctx->wind_hdy[l][e] : W.cdy;
+      if (mode == WIND_STEP) {
+        const int nx = wind_advance(ax[e], dx), ny = wind_advance(ay[e], dy);
+        px = std::max(px, abs(nx)); py = std::max(py, abs(ny));
+      } else if (mode == WIND_INIT) {
+        ax[e] = W.ax0; ay[e] = W.ay0;
+      } else {
+        ax[e] = ay[e] = 0.0;
+        py = W.n2;
+      }
+      const WindRec r = wind_record(W.xoff, W.yoff, ax[e], ay[e]);
+      if (e == 0 || r.ix < box[0]) box[0] = r.ix;
+      if (e == 0 || r.ix > box[1]) box[1] = r.ix;
+      if (e == 0 || r.iy < box[2]) box[2] = r.iy;
+      if (e == 0 || r.iy > box[3]) box[3] = r.iy;
+    }
+    ctx->wind_passes[l][0] = px; ctx->wind_passes[l][1] = py;
+  }
+  return AOM_OK;
+}
+
+// Back to the common accumulators once no layer has winds of its own and every layer's accumulators agree over the batch
+// (at the latest after the next aom_reset, which zeroes them): the uniform kernels then run again.
+static void wind_try_uniform(aom_ctx* ctx) {
+  if (!ctx->wind_pe || wind_any_env(ctx)) return;
+  const int E = ctx->cfg.n_env;
+  for (int l = 0; l < ctx->cfg.n_layers; ++l) {
+    const double* a = ctx->wind_hacc + (size_t)2 * l * E;
+    for (int e = 1; e < E; ++e)
+      if (a[e] != a[0] || a[E + e] != a[E]) return;
+  }
+  for (int l = 0; l < ctx->cfg.n_layers; ++l) {
+    ctx->accx[l] = ctx->wind_hacc[(size_t)2 * l * E];
+    ctx->accy[l] = ctx->wind_hacc[(size_t)(2 * l + 1) * E];
+  }
+  ctx->wind_pe = false;
+}
+
+extern "C" int aom_set_layer_wind(aom_ctx* ctx, int layer, const float* deltax_host, const float* deltay_host) {
+  if (!ctx) return AOM_ERR_INVALID;
+  const aom_config& c = ctx->cfg;
+  if (layer < 0 || layer >= c.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
+  if (!deltax_host != !deltay_host) return fail(ctx, AOM_ERR_INVALID, "per-environment winds need both components (or neither)");
+  const size_t E = c.n_env;
+  CU(cudaDeviceSynchronize());                       // an extrusion in flight may still read the old steps
+  if (!deltax_host) {
+    cudaFree(ctx->wind_dx[layer]); cudaFree(ctx->wind_dy[layer]); free(ctx->wind_hdx[layer]); free(ctx->wind_hdy[layer]);
+    ctx->wind_dx[layer] = ctx->wind_dy[layer] = ctx->wind_hdx[layer] = ctx->wind_hdy[layer] = nullptr;
+    wind_try_uniform(ctx);
+    return AOM_OK;
+  }
+  for (size_t e = 0; e < E; ++e)
+    if (!isfinite(deltax_host[e]) || !isfinite(deltay_host[e]))
+      return fail(ctx, AOM_ERR_INVALID, "layer %d: wind of environment %zu is not finite", layer, e);
+  if (!ctx->wind_hdx[layer]) {
+    ctx->wind_hdx[layer] = (float*)malloc(E * sizeof(float));
+    ctx->wind_hdy[layer] = (float*)malloc(E * sizeof(float));
+    if (!ctx->wind_hdx[layer] || !ctx->wind_hdy[layer]) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+    CU(cudaMalloc((void**)&ctx->wind_dx[layer], E * sizeof(float)));
+    CU(cudaMalloc((void**)&ctx->wind_dy[layer], E * sizeof(float)));
+  }
+  memcpy(ctx->wind_hdx[layer], deltax_host, E * sizeof(float));
+  memcpy(ctx->wind_hdy[layer], deltay_host, E * sizeof(float));
+  CU(cudaMemcpy(ctx->wind_dx[layer], deltax_host, E * sizeof(float), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(ctx->wind_dy[layer], deltay_host, E * sizeof(float), cudaMemcpyHostToDevice));
+  if (!ctx->wind_pe) {
+    // every environment continues from the common accumulators: the screens do not jump
+    const size_t LE = (size_t)c.n_layers * E;
+    if (!ctx->wind_acc) {
+      CU(dalloc(&ctx->wind_acc, 2 * LE));
+      CU(dalloc(&ctx->wind_steps, 2 * LE));
+      CU(cudaMalloc((void**)&ctx->wind_rec, LE * sizeof(WindRec)));
+      ctx->wind_hacc = (double*)calloc(2 * LE, sizeof(double));
+      if (!ctx->wind_hacc) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+    }
+    int rc = wind_update(ctx, WIND_INIT, 0);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(0));                    // the legacy stream: the state is read next on any stream
+    ctx->wind_pe = true;
+  }
+  const int* b = ctx->wind_box[layer];
+  if (b[0] < 0 || b[2] < 0 || b[1] + c.n + 1 > c.screen_dim[layer] || b[3] + c.n + 1 > c.screen_dim[layer])
+    return fail(ctx, AOM_ERR_UNSUPPORTED, "layer %d: pupil footprint leaves the screen", layer);
   return AOM_OK;
 }
 
@@ -699,6 +846,21 @@ extern "C" int aom_move_atmos(aom_ctx* ctx, void* stream) {
   if (!ctx->seeded) return fail(ctx, AOM_ERR_STATE, "aom_reset must be called before aom_move_atmos");
   cudaStream_t st = (cudaStream_t)stream;
   const aom_config& c = ctx->cfg;
+  if (ctx->wind_pe) {
+    // per-environment winds: counts and offsets on the device, passes sized by the host mirror (x then y, as below);
+    // an environment takes part in the first |count| passes of each axis
+    int rc = wind_update(ctx, WIND_STEP, st);
+    if (rc) return rc;
+    const size_t E = c.n_env;
+    for (int l = 0; l < c.n_layers; ++l)
+      for (int a = 0; a < 2; ++a)
+        for (int i = 0; i < ctx->wind_passes[l][a]; ++i) {
+          rc = extrude_once(ctx, l, a, 1, st, ctx->wind_steps + (2 * l + a) * E, i);
+          if (rc) return rc;
+        }
+    wind_try_uniform(ctx);
+    return AOM_OK;
+  }
   for (int l = 0; l < c.n_layers; ++l) {
     ctx->accx[l] += (double)c.deltax[l];
     ctx->accy[l] += (double)c.deltay[l];
@@ -761,6 +923,13 @@ extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
   ctx->step = 0;
   int rc = clear_loop_state(ctx, st);
   if (rc) return rc;
+  for (int l = 0; l < c.n_layers; ++l) ctx->accx[l] = ctx->accy[l] = 0.0;
+  if (ctx->wind_pe && !wind_any_env(ctx)) ctx->wind_pe = false;      // every accumulator restarts from 0: common again
+  if (ctx->wind_pe) {
+    // per-environment winds: accumulators 0, start-up counts 2N along y signed like each environment's x wind
+    rc = wind_update(ctx, WIND_RESET, st);
+    if (rc) return rc;
+  }
   // (The layers' start-up chains are independent, but running them on separate streams with private scratch gained
   // nothing -- 1.35 s either way at 4096 environments: every extrusion kernel fills the GPU by itself.)
   for (int l = 0; l < c.n_layers; ++l) {
@@ -769,15 +938,15 @@ extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
     CU(cudaMemsetAsync(ctx->ox[l], 0, E * 4, st));
     CU(cudaMemsetAsync(ctx->oy[l], 0, E * 4, st));
     CU(cudaMemsetAsync(ctx->ext_count[l], 0, E * 4, st));
-    ctx->accx[l] = ctx->accy[l] = 0.0;
     int sign = c.deltax[l] < 0 ? -1 : 1;
+    const int* steps = ctx->wind_pe ? ctx->wind_steps + (2 * l + 1) * E : nullptr;
     // The reference starts a screen with 2N extrusions along x (columns: 648 pixels in 648 different DRAM rows per
     // environment, the expensive direction of the [y][x] layout -- 0.32 ms per extrusion at 4096 environments against
     // 0.19 ms along y).  From a zero screen with zero ring offsets the recursion along y produces exactly the transpose
     // (same stencil, same operator, same innovation counters; every index expression of the gather / scatter swaps its
     // roles, atmos_kernels.cuh / extrude_i8.cuh), and 2N extrusions bring the ring origin back to zero: so the start-up
     // runs along y and the screens are transposed in place once at the end -- bit-identical pixels, 1.29 -> 0.8 s.
-    for (size_t i = 0; i < 2 * N; ++i) { rc = extrude_once(ctx, l, 1, sign, st); if (rc) return rc; }
+    for (size_t i = 0; i < 2 * N; ++i) { rc = extrude_once(ctx, l, 1, sign, st, steps, (int)i); if (rc) return rc; }
     {
       const int T = (int)((N + 31) / 32);
       transpose_screens_kernel<<<dim3((unsigned)(T * (T + 1) / 2), (unsigned)E), dim3(32, 8), 0, st>>>(ctx->screen[l], (int)N);
@@ -1185,14 +1354,14 @@ static int fill_wfs_params(aom_ctx* ctx, WfsParams& p, int flags, float noise) {
   for (int l = 0; l < p.n_layers; ++l) {
     WfsLayer& L = p.layer[l];
     L.screen = ctx->screen[l]; L.ox = ctx->ox[l]; L.oy = ctx->oy[l]; L.N = c.screen_dim[l];
-    double px = (double)c.wfs_xoff[l] + ctx->accx[l], py = (double)c.wfs_yoff[l] + ctx->accy[l];
-    L.ix = (int)floor(px); L.iy = (int)floor(py);
-    L.fx = (float)(px - L.ix); L.fy = (float)(py - L.iy);
-    L.w00 = (1.f - L.fx) * (1.f - L.fy); L.w01 = L.fx * (1.f - L.fy);
-    L.w10 = (1.f - L.fx) * L.fy;         L.w11 = L.fx * L.fy;
-    if (L.ix < 0 || L.iy < 0 || L.ix + c.n + 1 > L.N || L.iy + c.n + 1 > L.N)
+    const WindRec r = wind_record(c.wfs_xoff[l], c.wfs_yoff[l], ctx->accx[l], ctx->accy[l]);
+    L.ix = r.ix; L.iy = r.iy; L.fx = r.fx; L.fy = r.fy; L.w00 = r.w00; L.w01 = r.w01; L.w10 = r.w10; L.w11 = r.w11;
+    int box[4] = {L.ix, L.ix, L.iy, L.iy};          // with per-environment winds: the extremes over the batch
+    if (ctx->wind_pe) memcpy(box, ctx->wind_box[l], sizeof(box));
+    if (box[0] < 0 || box[2] < 0 || box[1] + c.n + 1 > L.N || box[3] + c.n + 1 > L.N)
       return fail(ctx, AOM_ERR_UNSUPPORTED, "layer %d: pupil footprint leaves the screen", l);
   }
+  p.wind = (ctx->wind_pe && p.n_layers > 0) ? ctx->wind_rec : nullptr;
   p.use_dm = (flags & 2) ? 1 : 0;
   if (p.use_dm) {
     NEED(AOM_T_STAMP1D, 0); NEED(AOM_T_ACT_MAP, 0); NEED(AOM_T_TT_PLANES, 0);
@@ -1250,6 +1419,9 @@ extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* st
     cudaError_t le = wfs_umma_launch(p, ctx->umma, ctx->num_sms, !fast, path == AOM_WFS_UMMA_WS && p.noise < 0.f && p.bincube == nullptr, st);
     if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "wfs_umma_launch: %s", cudaGetErrorString(le));
   }
+  else if (c.nfft == 64 && path != AOM_WFS_SIMT && p.wind)
+    return fail(ctx, AOM_ERR_UNSUPPORTED, "per-environment wind is not implemented in the round-1 sensor kernels "
+                "(wfs_frame_tma_kernel, wfs_frame_mma_kernel): use the umma, umma_ws or simt path");
   else if (c.nfft == 64 && staged && ctx->fast_state == 1) {
     rc = wfs_fast_launch(ctx, p, !fast, st);
     if (rc) return rc;
@@ -1265,7 +1437,9 @@ extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* st
     }
 #undef WFM_LAUNCH
   }
+  else if (c.nfft == 64 && p.wind) wfs_frame_kernel<4, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
   else if (c.nfft == 64) wfs_frame_kernel<4><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
+  else if (p.wind) wfs_frame_kernel<8, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<8>(), st>>>(p);
   else wfs_frame_kernel<8><<<grid, WFS_WARPS * 32, wfs_smem_bytes<8>(), st>>>(p);
   KCHECK();
   if (timed) {
@@ -1321,7 +1495,8 @@ extern "C" int aom_raytrace_wfs(aom_ctx* ctx, int flags, void* stream) {
   }
   if (!ctx->phase) CU(dalloc(&ctx->phase, (size_t)c.n_env * c.n * c.n));
   dim3 blk(32, 8), grid((c.n + 31) / 32, (c.n + 7) / 8, c.n_env);
-  wfs_phase_kernel<<<grid, blk, 0, st>>>(p, ctx->phase);
+  if (p.wind) wfs_phase_kernel<true><<<grid, blk, 0, st>>>(p, ctx->phase);
+  else wfs_phase_kernel<false><<<grid, blk, 0, st>>>(p, ctx->phase);
   KCHECK();
   return AOM_OK;
 }
@@ -1372,7 +1547,8 @@ extern "C" int aom_comp_strehl(aom_ctx* ctx, int flags, float lambda_um, int acc
       if (rc) return rc;
     } else {
       dim3 blk(32, 8), grid((c.n + 31) / 32, (c.n + 7) / 8, c.n_env);
-      target_moments_kernel<<<grid, blk, 0, st>>>(p, mom, k2t, peak ? PSW_MOM2 : 5, peak ? 1.f / (float)nfft : 0.f);
+      if (p.wind) target_moments_kernel<true><<<grid, blk, 0, st>>>(p, mom, k2t, peak ? PSW_MOM2 : 5, peak ? 1.f / (float)nfft : 0.f);
+      else target_moments_kernel<false><<<grid, blk, 0, st>>>(p, mom, k2t, peak ? PSW_MOM2 : 5, peak ? 1.f / (float)nfft : 0.f);
       KCHECK();
     }
     if (flags & AOM_TAR_TRACE) return AOM_OK;        // sums pending until AOM_TAR_PUBLISH
@@ -1407,7 +1583,8 @@ extern "C" int aom_do_control_geo(aom_ctx* ctx, void* stream) {
   } else {
     const size_t smem = (size_t)GEO_ROW_WARPS * (c.n + (c.n >> 4) + 2) * sizeof(float);
     dim3 grid((c.n + GEO_ROW_WARPS - 1) / GEO_ROW_WARPS, c.n_env);
-    geo_rows_kernel<<<grid, GEO_ROW_WARPS * 32, smem, st>>>(p, ctx->geo_T, ctx->geo_gp, ctx->geo_mom);
+    if (p.wind) geo_rows_kernel<true><<<grid, GEO_ROW_WARPS * 32, smem, st>>>(p, ctx->geo_T, ctx->geo_gp, ctx->geo_mom);
+    else geo_rows_kernel<false><<<grid, GEO_ROW_WARPS * 32, smem, st>>>(p, ctx->geo_T, ctx->geo_gp, ctx->geo_mom);
     KCHECK();
   }
   geo_cols_kernel<<<c.n_env, 256, 0, st>>>(p, ctx->geo_T, ctx->geo_gp, nb, ctx->geo_mom,

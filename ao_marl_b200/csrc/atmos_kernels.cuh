@@ -11,7 +11,9 @@
 // One extrusion of all E environments = gather Z [E][S+N] -> GEMM with [A|B] -> scatter N pixels.
 #pragma once
 #include <cuda_runtime.h>
+#include "../../include/aomarl.h"
 #include "rng.cuh"
+#include "wind_host.h"
 
 struct ExtrudeParams {
   float* screen;          // [E][N][N]
@@ -25,7 +27,21 @@ struct ExtrudeParams {
   int N, S, E, layer, axis, sign;
   float amp;
   const float* amp_env;   // [E] per-environment amplitude, or null
+  // per-environment winds (the PE instantiations): signed whole-pixel counts of this axis for this frame [E]; pass
+  // `pass` extrudes environment e iff pass < |steps[e]|, with the sign of steps[e] (`sign` is not read).  An environment
+  // that sits out a pass is not touched: no gather, no store, no RNG counter increment.
+  const int* steps;
+  int pass;
 };
+
+// the direction of this pass for environment e; false: e sits it out
+template <bool PE>
+__device__ __forceinline__ bool extr_active(const int* steps, int pass, int e, int& sign) {
+  if (!PE) return true;
+  const int n = steps[e];
+  sign = n < 0 ? -1 : 1;
+  return pass < (n < 0 ? -n : n);
+}
 
 __device__ __forceinline__ void extr_logical(int r, int c, int N, int axis, int sign, int& lr, int& lc) {
   if (axis == 0) { lr = r; lc = c; } else { lr = c; lc = r; }
@@ -40,21 +56,24 @@ __device__ __forceinline__ int wrapN(int v, int N) { return v >= N ? v - N : v; 
 // dependent chain (stencil index -> screen pixel) is pipelined over ~5 iterations per thread instead of being paid
 // once per 256-thread block (32 k tiny blocks per launch were block-latency bound: 75 us per launch), and one
 // Philox block yields its four innovations instead of one.
+template <bool PE = false>
 __global__ void __launch_bounds__(256) extrude_gather_kernel(ExtrudeParams p) {
   const int e = blockIdx.x;
+  int sign = p.sign;
+  if (!extr_active<PE>(p.steps, p.pass, e, sign)) return;
   const int N = p.N;
   const float* scr = p.screen + (size_t)e * N * N;
   const int ox = p.ox[e], oy = p.oy[e];
   // reference pixel: p'[0, N-1] of the rotated/transposed screen
   int rr, rc;
-  extr_logical(0, N - 1, N, p.axis, p.sign, rr, rc);
+  extr_logical(0, N - 1, N, p.axis, sign, rr, rc);
   const float zr = scr[(size_t)wrapN(rr + oy, N) * N + wrapN(rc + ox, N)];
   if (threadIdx.x == 0) p.zref[e] = zr;
   float* Z = p.Z + (size_t)e * p.ldz;
   for (int k = threadIdx.x; k < p.S; k += blockDim.x) {
     const int idx = p.stencil[k];
     int lr, lc;
-    extr_logical(idx / N, idx % N, N, p.axis, p.sign, lr, lc);
+    extr_logical(idx / N, idx % N, N, p.axis, sign, lr, lc);
     Z[k] = scr[(size_t)wrapN(lr + oy, N) * N + wrapN(lc + ox, N)] - zr;
   }
   const uint32_t cnt = p.count[e], k0 = p.k0[e], k1 = p.k1[e];
@@ -78,15 +97,18 @@ __global__ void __launch_bounds__(256) extrude_gather_kernel(ExtrudeParams p) {
 // 81 MB written for 10.6 MB of pixels -- and stays at 117 us however many stores are in flight (120 us before): it is
 // bound by DRAM row activations (profiles/r02_extrude_kernels_metrics.csv), the price of storing every layer [y][x].
 #define EXTRUDE_SCATTER_THREADS 128
+template <bool PE = false>
 __global__ void __launch_bounds__(EXTRUDE_SCATTER_THREADS) extrude_scatter_kernel(ExtrudeParams p) {
   const int e = blockIdx.x;
+  int sign = p.sign;
+  if (!extr_active<PE>(p.steps, p.pass, e, sign)) return;
   const int N = p.N;
   float* scr = p.screen + (size_t)e * N * N;
   const int ox = p.ox[e], oy = p.oy[e];
   const float zr = p.zref ? p.zref[e] : 0.f;           // null: the GEMM already added the reference pixel
   int nox = ox, noy = oy;
-  if (p.axis == 0) nox = (p.sign > 0) ? wrapN(ox + 1, N) : (ox == 0 ? N - 1 : ox - 1);
-  else             noy = (p.sign > 0) ? wrapN(oy + 1, N) : (oy == 0 ? N - 1 : oy - 1);
+  if (p.axis == 0) nox = (sign > 0) ? wrapN(ox + 1, N) : (ox == 0 ? N - 1 : ox - 1);
+  else             noy = (sign > 0) ? wrapN(oy + 1, N) : (oy == 0 ? N - 1 : oy - 1);
   const float* col = p.newcol + (size_t)e * p.ldn;
   constexpr int PER = 8;                                    // pixels per thread and pass (N <= 1024 in one pass)
   for (int j0 = threadIdx.x; j0 < N; j0 += PER * EXTRUDE_SCATTER_THREADS) {
@@ -102,12 +124,12 @@ __global__ void __launch_bounds__(EXTRUDE_SCATTER_THREADS) extrude_scatter_kerne
       if (j < N) {
         size_t addr;
         if (p.axis == 0) {
-          const int pc = (p.sign > 0) ? ox : nox;                 // new logical column N-1 (or 0)
-          const int lr = (p.sign > 0) ? j : N - 1 - j;
+          const int pc = (sign > 0) ? ox : nox;                 // new logical column N-1 (or 0)
+          const int lr = (sign > 0) ? j : N - 1 - j;
           addr = (size_t)wrapN(lr + oy, N) * N + pc;
         } else {
-          const int pr = (p.sign > 0) ? oy : noy;                 // new logical row N-1 (or 0)
-          const int lc = (p.sign > 0) ? j : N - 1 - j;
+          const int pr = (sign > 0) ? oy : noy;                 // new logical row N-1 (or 0)
+          const int lc = (sign > 0) ? j : N - 1 - j;
           addr = (size_t)pr * N + wrapN(lc + ox, N);
         }
         scr[addr] = v[i];
@@ -152,4 +174,49 @@ __global__ void __launch_bounds__(256) transpose_screens_kernel(float* __restric
 // grid-stride fill helpers
 __global__ void fill_i32_kernel(int* p, int v, size_t n) {
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = v;
+}
+
+// Wind state of every layer and environment when the environments have their own winds: accumulators acc [L][2][E]
+// (x, y), whole-pixel counts of the frame steps [L][2][E] (x, y) and the samplers' offsets rec [L][E].  One thread per
+// (layer, environment), the arithmetic of wind_host.h (the host keeps a mirror of the accumulators with the same
+// functions to know how many extrusion passes to launch).
+#define WIND_STEP 0      // one frame of wind: acc += delta, counts = whole pixels
+#define WIND_INIT 1      // accumulators <- the layer's common ones (ax0, ay0), no extrusion
+#define WIND_RESET 2     // accumulators <- 0; counts of the start-up: 2N along y, signed like the environment's x wind
+struct WindLayerParams {
+  const float* dx; const float* dy;      // [E] steps in pixels per frame, or null: the common cdx / cdy
+  float cdx, cdy;
+  double ax0, ay0;                       // WIND_INIT
+  float xoff, yoff;                      // sensor offsets of the layer (aom_config.wfs_xoff / wfs_yoff)
+  int n2;                                // WIND_RESET: 2 N
+};
+struct WindStateParams {
+  WindLayerParams layer[AOM_MAX_LAYERS];
+  double* acc; int* steps; WindRec* rec;
+  int E, n_layers, mode;
+};
+
+__global__ void wind_state_kernel(const __grid_constant__ WindStateParams P) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.n_layers * P.E) return;
+  const int l = i / P.E, e = i - l * P.E;
+  const WindLayerParams& L = P.layer[l];
+  const float dx = L.dx ? L.dx[e] : L.cdx, dy = L.dy ? L.dy[e] : L.cdy;
+  double* ax = P.acc + (size_t)2 * l * P.E + e;
+  double* ay = ax + P.E;
+  double x = 0.0, y = 0.0;
+  int nx = 0, ny = 0;
+  if (P.mode == WIND_STEP) {
+    x = *ax; y = *ay;
+    nx = wind_advance(x, dx);
+    ny = wind_advance(y, dy);
+  } else if (P.mode == WIND_INIT) {
+    x = L.ax0; y = L.ay0;
+  } else {
+    ny = dx < 0.f ? -L.n2 : L.n2;
+  }
+  *ax = x; *ay = y;
+  P.steps[(size_t)2 * l * P.E + e] = nx;
+  P.steps[(size_t)(2 * l + 1) * P.E + e] = ny;
+  P.rec[(size_t)l * P.E + e] = wind_record(L.xoff, L.yoff, x, y);
 }

@@ -17,7 +17,8 @@ static cudaError_t oz_attrs() {
 cudaError_t oz_extrude_launch(const OzGatherParams& g, const OzGemmParams& m, int MT, int NT, cudaStream_t st) {
   cudaError_t e = oz_attrs();
   if (e != cudaSuccess) return e;
-  oz_gather_slice_kernel<<<g.E, 256, (size_t)g.KB * OZ_BK * sizeof(double), st>>>(g);
+  if (g.steps) oz_gather_slice_kernel<true><<<g.E, 256, (size_t)g.KB * OZ_BK * sizeof(double), st>>>(g);
+  else oz_gather_slice_kernel<false><<<g.E, 256, (size_t)g.KB * OZ_BK * sizeof(double), st>>>(g);
   e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   oz_gemm_kernel<0, OZ_LEVELS><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);

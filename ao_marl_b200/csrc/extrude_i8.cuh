@@ -61,6 +61,8 @@ struct OzGatherParams {
   int N, S, E, KB, layer, axis, sign;
   float amp;
   const float* amp_env;     // [E] per-environment amplitude, or null
+  const int* steps;         // per-environment winds: signed counts of this axis [E] (see ExtrudeParams), or null
+  int pass;
 };
 
 struct OzGemmParams {
@@ -132,14 +134,23 @@ __device__ __forceinline__ int oz_wrap(int v, int N) { return v >= N ? v - N : v
 // grid: E blocks of 256 threads; dynamic shared memory: KB * 32 doubles.
 // Gathers the stencil pixels (minus the reference pixel) and the scaled innovations of one environment, finds the row
 // scale, cuts the row into digit planes and stores them in the tile layout the tensor core reads.
+// PE: per-environment winds -- environment e takes part in pass p.pass of the axis iff p.pass < |steps[e]|, in the
+// direction of steps[e]; otherwise it stores nothing (the GEMM's row of e is computed from stale digits and not scattered).
+template <bool PE = false>
 __global__ void __launch_bounds__(256) oz_gather_slice_kernel(OzGatherParams p) {
   extern __shared__ double oz_v[];
   __shared__ double s_red[8];
   const int e = blockIdx.x, N = p.N, Kp = p.KB * OZ_BK;
+  int sign = p.sign;
+  if (PE) {
+    const int n = p.steps[e];
+    if (p.pass >= (n < 0 ? -n : n)) return;
+    sign = n < 0 ? -1 : 1;
+  }
   const float* scr = p.screen + (size_t)e * N * N;
   const int ox = p.ox[e], oy = p.oy[e];
   int rr, rc;
-  oz_logical(0, N - 1, N, p.axis, p.sign, rr, rc);
+  oz_logical(0, N - 1, N, p.axis, sign, rr, rc);
   const float zr = scr[(size_t)oz_wrap(rr + oy, N) * N + oz_wrap(rc + ox, N)];
   // differences and products in float64, i.e. exactly: what the oracle (and a float64 reading of iterkolmo.py:281-284) does
   double amax = 0.0;
@@ -148,7 +159,7 @@ __global__ void __launch_bounds__(256) oz_gather_slice_kernel(OzGatherParams p) 
     const int idx = p.stencil[k];
     const int sr = (int)__umulhi((uint32_t)idx, magic), sc = idx - sr * N;
     int lr, lc;
-    oz_logical(sr, sc, N, p.axis, p.sign, lr, lc);
+    oz_logical(sr, sc, N, p.axis, sign, lr, lc);
     const double v = (double)scr[(size_t)oz_wrap(lr + oy, N) * N + oz_wrap(lc + ox, N)] - (double)zr;
     oz_v[k] = v;
     amax = fmax(amax, fabs(v));

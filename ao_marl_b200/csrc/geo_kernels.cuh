@@ -19,6 +19,7 @@
 
 #define GEO_ROW_WARPS 4
 
+template <bool PE = false>      // PE: per-environment winds (layer offsets from p.wind)
 __global__ void __launch_bounds__(GEO_ROW_WARPS * 32) geo_rows_kernel(WfsParams p, float* __restrict__ T, int gp,
                                                                        double* __restrict__ mom) {
   extern __shared__ float s_rows[];
@@ -39,14 +40,15 @@ __global__ void __launch_bounds__(GEO_ROW_WARPS * 32) geo_rows_kernel(WfsParams 
         const int N = L.N;
         const float* scr = L.screen + (size_t)e * N * N;
         const int ox = L.ox[e], oy = L.oy[e];
+        const WindRec w = wind_of<PE>(p, l, e);
         // footprint inside the screen (checked on the host) and 0 <= ox, oy < N: one conditional subtract wraps
-        int pc0 = x + L.ix + ox; pc0 -= (pc0 >= N) ? N : 0;
+        int pc0 = x + w.ix + ox; pc0 -= (pc0 >= N) ? N : 0;
         int pc1 = pc0 + 1;       pc1 -= (pc1 >= N) ? N : 0;
-        int pr0 = y + L.iy + oy; pr0 -= (pr0 >= N) ? N : 0;
+        int pr0 = y + w.iy + oy; pr0 -= (pr0 >= N) ? N : 0;
         int pr1 = pr0 + 1;       pr1 -= (pr1 >= N) ? N : 0;
-        float top = wfs_layer_row(scr, N, pr0, pc0, pc1, L.fx);
-        float bot = wfs_layer_row(scr, N, pr1, pc0, pc1, L.fx);
-        v += top + L.fy * (bot - top);
+        float top = wfs_layer_row(scr, N, pr0, pc0, pc1, w.fx);
+        float bot = wfs_layer_row(scr, N, pr1, pc0, pc1, w.fx);
+        v += top + w.fy * (bot - top);
       }
       s1 += v;
       sx = fmaf(v, __ldg(ttx + x), sx);

@@ -60,7 +60,9 @@ struct SweepParams {
 __host__ __device__ inline size_t psw_warp_floats(int NL) {
   return (size_t)PSW_SLOTS * NL * PSW_BW + 160 + 32 + 48 + 16 + 8;   // ring, out row, Q, volt window, R row, barriers
 }
-__host__ __device__ inline size_t psw_smem_bytes(int NL) { return (PSW_WARPS * psw_warp_floats(NL) + 64) * sizeof(float); }
+__host__ __device__ inline size_t psw_smem_bytes(int NL, bool pe = false) {
+  return (PSW_WARPS * psw_warp_floats(NL) + 64) * sizeof(float) + (pe ? (size_t)NL * sizeof(WindRec) : 0);
+}
 
 // mask / tip-tilt planes in the lattice frame; grid (n), block 128
 __global__ void sweep_tables_kernel(WfsParams p, uint32_t* maskw, float* ttp, int nb) {
@@ -91,8 +93,8 @@ __device__ __forceinline__ void psw_bulk(uint32_t dst, const float* src, uint32_
 
 // four pixels of one layer from the staged upper / lower screen rows (16-byte aligned pointers, wanted columns start
 // D floats in)
-template <int D>
-__device__ __forceinline__ void psw_layer(const float* __restrict__ up, const float* __restrict__ lo, const WfsLayer& L,
+template <int D, class Wt>      // Wt: WfsLayer (common offset) or WindRec (the environment's own)
+__device__ __forceinline__ void psw_layer(const float* __restrict__ up, const float* __restrict__ lo, const Wt& L,
                                           float (&ph)[4]) {
   float a[8], b[8];
   const float4 a0 = *reinterpret_cast<const float4*>(up), b0 = *reinterpret_cast<const float4*>(lo);
@@ -117,7 +119,8 @@ __device__ __forceinline__ void psw_layer(const float* __restrict__ up, const fl
   }
 }
 
-template <int NL, int MODE>
+// PE: per-environment winds -- the block's environment reads its layer offsets from P.w.wind once, into shared memory
+template <int NL, int MODE, bool PE = false>
 __global__ void __launch_bounds__(PSW_WARPS * 32, MODE == 2 ? 3 : 4) pupil_sweep_kernel(const __grid_constant__ SweepParams P) {
   extern __shared__ __align__(128) float psw_smem[];
   const WfsParams& p = P.w;
@@ -134,8 +137,12 @@ __global__ void __launch_bounds__(PSW_WARPS * 32, MODE == 2 ? 3 : 4) pupil_sweep
   float* s_v = s_q + 32;                                    // [4][12]   MODE 1: volts of the four lattice rows in reach
   float* s_r = s_v + 48;                                    // [16]      MODE 1: R_y[g], g = 8 cb - 3 + index
   unsigned long long* s_bar = reinterpret_cast<unsigned long long*>(s_r + 16);   // [PSW_SLOTS]
+  WindRec* s_wr = reinterpret_cast<WindRec*>(psw_smem + 64 + PSW_WARPS * psw_warp_floats(NL));   // PE: [NL] this environment's offsets
 
   for (int i = threadIdx.x; i < 64; i += blockDim.x) s_f[i] = i < p.ss ? p.stamp1d[i] : 0.f;
+  if (PE && threadIdx.x < 8 * nl)
+    reinterpret_cast<uint32_t*>(s_wr)[threadIdx.x] =
+        __ldg(reinterpret_cast<const uint32_t*>(p.wind + (size_t)(threadIdx.x >> 3) * p.E + e) + (threadIdx.x & 7));
   if (lane < 16) s_r[lane] = 0.f;
   if (lane < PSW_SLOTS)
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(wft_smem_u32(s_bar + lane)) : "memory");
@@ -160,8 +167,9 @@ __global__ void __launch_bounds__(PSW_WARPS * 32, MODE == 2 ? 3 : 4) pupil_sweep
       const WfsLayer& L = p.layer[l];
       const int N = L.N;
       const int oy = __shfl_sync(0xffffffffu, __ldg(L.oy + e), 0), ox = __shfl_sync(0xffffffffu, __ldg(L.ox + e), 0);
-      int r = yb + L.iy + oy; r -= (r >= N) ? N : 0;
-      int c = (128 * cb + xs0 + L.ix + ox) % N;           // column of the block's first pixel (x may lie outside the frame)
+      const int ix = PE ? s_wr[l].ix : L.ix, iy = PE ? s_wr[l].iy : L.iy;
+      int r = yb + iy + oy; r -= (r >= N) ? N : 0;
+      int c = (128 * cb + xs0 + ix + ox) % N;             // column of the block's first pixel (x may lie outside the frame)
       c += (c < 0) ? N : 0;
       dd[l] = c & 3; c &= ~3;
       src[l] = L.screen + (size_t)e * N * N + c + (size_t)r * N;
@@ -281,11 +289,20 @@ __global__ void __launch_bounds__(PSW_WARPS * 32, MODE == 2 ? 3 : 4) pupil_sweep
 #pragma unroll
       for (int l = 0; l < NL; ++l) {
         if (l < nl) {
-          switch (dd[l]) {
-            case 0: psw_layer<0>(up + l * PSW_BW, lo + l * PSW_BW, p.layer[l], ph); break;
-            case 1: psw_layer<1>(up + l * PSW_BW, lo + l * PSW_BW, p.layer[l], ph); break;
-            case 2: psw_layer<2>(up + l * PSW_BW, lo + l * PSW_BW, p.layer[l], ph); break;
-            default: psw_layer<3>(up + l * PSW_BW, lo + l * PSW_BW, p.layer[l], ph); break;
+          if (PE) {
+            switch (dd[l]) {
+              case 0: psw_layer<0>(up + l * PSW_BW, lo + l * PSW_BW, s_wr[l], ph); break;
+              case 1: psw_layer<1>(up + l * PSW_BW, lo + l * PSW_BW, s_wr[l], ph); break;
+              case 2: psw_layer<2>(up + l * PSW_BW, lo + l * PSW_BW, s_wr[l], ph); break;
+              default: psw_layer<3>(up + l * PSW_BW, lo + l * PSW_BW, s_wr[l], ph); break;
+            }
+          } else {
+            switch (dd[l]) {
+              case 0: psw_layer<0>(up + l * PSW_BW, lo + l * PSW_BW, p.layer[l], ph); break;
+              case 1: psw_layer<1>(up + l * PSW_BW, lo + l * PSW_BW, p.layer[l], ph); break;
+              case 2: psw_layer<2>(up + l * PSW_BW, lo + l * PSW_BW, p.layer[l], ph); break;
+              default: psw_layer<3>(up + l * PSW_BW, lo + l * PSW_BW, p.layer[l], ph); break;
+            }
           }
         }
       }

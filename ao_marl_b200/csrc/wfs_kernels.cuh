@@ -26,7 +26,8 @@ __device__ __forceinline__ float wfs_layer_row(const float* scr, int N, int prow
   return a + fx * (b - a);
 }
 
-template <int R>
+// PE: per-environment winds (the layer offsets come from p.wind)
+template <int R, bool PE = false>
 __global__ void __launch_bounds__(WFS_WARPS * 32, 2) wfs_frame_kernel(WfsParams p) {
   constexpr int NFFT = 16 * R;
   constexpr int H = 4 * R;            // half width of the kept spectrum
@@ -78,15 +79,16 @@ __global__ void __launch_bounds__(WFS_WARPS * 32, 2) wfs_frame_kernel(WfsParams 
       const int N = L.N;
       const float* scr = L.screen + (size_t)e * N * N;
       const int ox = L.ox[e], oy = L.oy[e];
-      int pc0 = x0 + hx + L.ix + ox;  pc0 -= (pc0 >= N) ? N : 0;  pc0 -= (pc0 >= N) ? N : 0;
+      const WindRec w = wind_of<PE>(p, l, e);
+      int pc0 = x0 + hx + w.ix + ox;  pc0 -= (pc0 >= N) ? N : 0;  pc0 -= (pc0 >= N) ? N : 0;
       int pc1 = pc0 + 1;              pc1 -= (pc1 >= N) ? N : 0;
-      int pr = y0 + hy + L.iy + oy;   pr -= (pr >= N) ? N : 0;    pr -= (pr >= N) ? N : 0;
-      float prev = wfs_layer_row(scr, N, pr, pc0, pc1, L.fx);
+      int pr = y0 + hy + w.iy + oy;   pr -= (pr >= N) ? N : 0;    pr -= (pr >= N) ? N : 0;
+      float prev = wfs_layer_row(scr, N, pr, pc0, pc1, w.fx);
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
         pr += 1; pr -= (pr >= N) ? N : 0;
-        float cur = wfs_layer_row(scr, N, pr, pc0, pc1, L.fx);
-        ph[i] += prev + L.fy * (cur - prev);
+        float cur = wfs_layer_row(scr, N, pr, pc0, pc1, w.fx);
+        ph[i] += prev + w.fy * (cur - prev);
         prev = cur;
       }
     }
@@ -257,6 +259,7 @@ constexpr size_t wfs_smem_bytes() {
 
 // Materialised pupil phase (wfs.get_wfs_phase): one thread per pixel, same arithmetic as above but
 // with the mirror surface evaluated through the lattice directly.
+template <bool PE = false>
 __global__ void wfs_phase_kernel(WfsParams p, float* phase) {
   const int e = blockIdx.z;
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
@@ -268,11 +271,12 @@ __global__ void wfs_phase_kernel(WfsParams p, float* phase) {
     const int N = L.N;
     const float* scr = L.screen + (size_t)e * N * N;
     const int ox = L.ox[e], oy = L.oy[e];
-    int pc0 = (x + L.ix + ox) % N, pc1 = (pc0 + 1) % N;
-    int pr0 = (y + L.iy + oy) % N, pr1 = (pr0 + 1) % N;
-    float top = wfs_layer_row(scr, N, pr0, pc0, pc1, L.fx);
-    float bot = wfs_layer_row(scr, N, pr1, pc0, pc1, L.fx);
-    acc += top + L.fy * (bot - top);
+    const WindRec w = wind_of<PE>(p, l, e);
+    int pc0 = (x + w.ix + ox) % N, pc1 = (pc0 + 1) % N;
+    int pr0 = (y + w.iy + oy) % N, pr1 = (pr0 + 1) % N;
+    float top = wfs_layer_row(scr, N, pr0, pc0, pc1, w.fx);
+    float bot = wfs_layer_row(scr, N, pr1, pc0, pc1, w.fx);
+    acc += top + w.fy * (bot - top);
   }
   if (p.use_dm) {
     const float* volts = p.volts + (size_t)e * p.ldv;
@@ -303,6 +307,7 @@ __global__ void wfs_phase_kernel(WfsParams p, float* phase) {
 // sum m sin(k phi) per environment (double atomics) -- instead of materialising [E][n][n].
 // grid (ceil(n/32), ceil(n/8), E), block (32, 8).  (Per-pixel cross-check form of pupil_sweep.cuh MODE 1.)
 #define TAR_ACC 12   // floats per environment of the long-exposure accumulators: SE sum, variance sum, 9 core pixels
+template <bool PE = false>
 __global__ void target_moments_kernel(WfsParams p, double* mom, float k2t, int stride, float core_step) {
   const int e = blockIdx.z;
   const int x = blockIdx.x * blockDim.x + threadIdx.x;
@@ -315,11 +320,12 @@ __global__ void target_moments_kernel(WfsParams p, double* mom, float k2t, int s
       const int N = L.N;
       const float* scr = L.screen + (size_t)e * N * N;
       const int ox = L.ox[e], oy = L.oy[e];
-      int pc0 = (x + L.ix + ox) % N, pc1 = (pc0 + 1) % N;
-      int pr0 = (y + L.iy + oy) % N, pr1 = (pr0 + 1) % N;
-      float top = wfs_layer_row(scr, N, pr0, pc0, pc1, L.fx);
-      float bot = wfs_layer_row(scr, N, pr1, pc0, pc1, L.fx);
-      acc += top + L.fy * (bot - top);
+      const WindRec w = wind_of<PE>(p, l, e);
+      int pc0 = (x + w.ix + ox) % N, pc1 = (pc0 + 1) % N;
+      int pr0 = (y + w.iy + oy) % N, pr1 = (pr0 + 1) % N;
+      float top = wfs_layer_row(scr, N, pr0, pc0, pc1, w.fx);
+      float bot = wfs_layer_row(scr, N, pr1, pc0, pc1, w.fx);
+      acc += top + w.fy * (bot - top);
     }
     if (p.use_dm) {
       const float* volts = p.volts + (size_t)e * p.ldv;

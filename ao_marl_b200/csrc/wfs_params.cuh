@@ -3,6 +3,7 @@
 #pragma once
 #include <stdint.h>
 #include "../../include/aomarl.h"
+#include "wind_host.h"
 
 struct WfsLayer {
   const float* screen;   // [E][N][N]
@@ -35,5 +36,18 @@ struct WfsParams {
   // outputs
   float* slopes; int lds;              // [E][lds]: x slopes then y slopes
   float* bincube;                      // [E][nvalid][256] or null
+  // per-environment winds: offsets of every layer and environment [n_layers][E], read by the kernels' per-environment
+  // instantiations in place of layer[l].ix .. w11 (null while every layer moves all environments alike)
+  const WindRec* wind;
 };
+
+// raytrace offset of layer l for environment e: the layer's common one, or its record when PE (per-environment winds)
+template <bool PE>
+__device__ __forceinline__ WindRec wind_of(const WfsParams& p, int l, int e) {
+  if (PE) return p.wind[(size_t)l * p.E + e];
+  const WfsLayer& L = p.layer[l];
+  WindRec r;
+  r.ix = L.ix; r.iy = L.iy; r.fx = L.fx; r.fy = L.fy; r.w00 = L.w00; r.w01 = L.w01; r.w10 = L.w10; r.w11 = L.w11;
+  return r;
+}
 

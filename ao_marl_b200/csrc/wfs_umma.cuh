@@ -73,11 +73,13 @@ struct WfsUmmaParams {
 };
 
 #define WU_AUX_BYTES 288                   // per warp and parity: 32 pupil words, 32 volts, one subaperture record (+ pad)
+// per-environment winds: the item's layer offsets (WindRec [WU_MAX_LAYERS], one word per lane) follow in the slot
+#define WU_AUX_BYTES_PE (WU_AUX_BYTES + WU_MAX_LAYERS * 32)
 
-template <int NL>
+template <int NL, bool PE = false>
 constexpr size_t wu_smem_bytes(int gw) {
   return (size_t)2 * WU_A_BYTES + 4 * WU_A_BYTES + 4 * WU_B_BYTES + (size_t)WU_WARPS * (NL > 0 ? NL : 1) * WU_TILE_STRIDE +
-         128 + 2 * WU_NG * 16 * 4 + WU_WARPS * 2 * WU_AUX_BYTES + (((size_t)gw * gw * 2 + 15) & ~(size_t)15);
+         128 + 2 * WU_NG * 16 * 4 + WU_WARPS * 2 * (PE ? WU_AUX_BYTES_PE : WU_AUX_BYTES) + (((size_t)gw * gw * 2 + 15) & ~(size_t)15);
 }
 
 __device__ __forceinline__ uint32_t wu_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -238,8 +240,8 @@ struct WuPhase {
 // start address of a box must be 16-byte aligned: profiles/dev/tma_probe.cu), so the wanted columns begin
 // D = origin & 3 floats into the row; pixel c, tap b reads v[D + c + b].  The aligned register pairs (v[2k], v[2k+1])
 // serve the X pairing for the taps with D + b even and the Y pairing for the others.
-template <int D>
-__device__ __forceinline__ void wu_layer(const float* __restrict__ t, const WfsLayer& L, WuPhase& a) {
+template <int D, class Wt>      // Wt: WfsLayer (common offset) or WindRec (the item's environment's own)
+__device__ __forceinline__ void wu_layer(const float* __restrict__ t, const Wt& L, WuPhase& a) {
   float v[2][12];
 #pragma unroll
   for (int r = 0; r < 2; ++r) {
@@ -277,12 +279,15 @@ __device__ __forceinline__ void wu_layer(const float* __restrict__ t, const WfsL
 
 // FULL = 1: three fp16 products in both stages (fp32-grade slopes).  0: the stage-1 result goes to stage 2 as a single
 // rounded fp16 (slopes ~3e-5 relative).
-template <int NL, int FULL>
+// PE: per-environment winds (layer offsets from p.wind: the ring origin per environment, the weights per item through
+// the aux slot)
+template <int NL, int FULL, bool PE = false>
 __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const __grid_constant__ WfsUmmaParams P) {
   const WfsParams& p = P.p;
   const WfsUmmaTables& f = P.f;
   extern __shared__ __align__(1024) unsigned char wu_smem_raw[];
   constexpr int NLS = NL > 0 ? NL : 1;
+  constexpr int AUXB = PE ? WU_AUX_BYTES_PE : WU_AUX_BYTES;
   unsigned char* s_a1 = wu_smem_raw;                                   // [hi, lo][WU_A_BYTES]
   unsigned char* s_a2 = s_a1 + 2 * WU_A_BYTES;                         // [tile][hi, lo][WU_A_BYTES]
   unsigned char* s_b1 = s_a2 + 4 * WU_A_BYTES;                         // [hi, lo][WU_B_BYTES]
@@ -292,8 +297,8 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
   uint32_t* s_cnt = (uint32_t*)(s_bar + 12);                           // [2] TMEM slot   (s_bar[10], [11]: stage-1 / stage-2 arrivals of the 8 warps)
   float* s_fx = (float*)((unsigned char*)s_bar + 128);                 // [NG][16]
   float* s_fyT = s_fx + WU_NG * 16;                                    // [16][NG]
-  unsigned char* s_aux = (unsigned char*)(s_fyT + 16 * WU_NG);         // [warp][parity][WU_AUX_BYTES]
-  short* s_amap = (short*)(s_aux + WU_WARPS * 2 * WU_AUX_BYTES);
+  unsigned char* s_aux = (unsigned char*)(s_fyT + 16 * WU_NG);         // [warp][parity][AUXB]
+  short* s_amap = (short*)(s_aux + WU_WARPS * 2 * AUXB);
 
   // lane through a volatile read: the compiler otherwise re-derives it from S2R SR_TID.X at ~25 places of the loop body
   // and each of those reads stalls its warp (5 % of the stall samples in profiles/r02_wfs_umma_v5)
@@ -328,7 +333,7 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
   const uint32_t my_tiles_u32 = wu_smem_u32(my_tiles);
   const uint32_t my_bar_u32 = wu_smem_u32(s_bar + warp);
   const uint32_t mma1_bar = wu_smem_u32(s_bar + 8), mma2_bar = wu_smem_u32(s_bar + 9);
-  unsigned char* my_aux = s_aux + (size_t)warp * 2 * WU_AUX_BYTES;     // per parity: pm[32] | volts[32] | record
+  unsigned char* my_aux = s_aux + (size_t)warp * 2 * AUXB;     // per parity: pm[32] | volts[32] | record
   const uint32_t my_aux_u32 = wu_smem_u32(my_aux);
   const int lane_off = y * WU_TILE_W + 8 * h;                          // floats, inside a tile
   const int amap_lane = (lane >> 2) * f.GW + (lane & 3);
@@ -388,8 +393,8 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
 #pragma unroll
       for (int l = 0; l < NL; ++l) {
         const int N = p.layer[l].N;
-        int a = p.layer[l].ix + p.layer[l].ox[pe];  a -= (a >= N) ? N : 0;
-        int b = p.layer[l].iy + p.layer[l].oy[pe];  b -= (b >= N) ? N : 0;
+        int a = (PE ? __ldg(&p.wind[(size_t)l * p.E + pe].ix) : p.layer[l].ix) + p.layer[l].ox[pe];  a -= (a >= N) ? N : 0;
+        int b = (PE ? __ldg(&p.wind[(size_t)l * p.E + pe].iy) : p.layer[l].iy) + p.layer[l].oy[pe];  b -= (b >= N) ? N : 0;
         rx[l] = a; ry[l] = b;
       }
       ring_e = pe;
@@ -447,14 +452,17 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
   // ---- per-lane inputs of one work item into the parity slot: pupil word, neighbourhood volts (cp.async: no register
   //      waits for them), and the record of the item after it ----
   auto issue_aux = [&](int pe, int pk, uint2 sb, int slot, int k_after, bool has_after) {
-    const uint32_t dst = my_aux_u32 + (uint32_t)slot * WU_AUX_BYTES;
+    const uint32_t dst = my_aux_u32 + (uint32_t)slot * AUXB;
     wu_cp_async4(dst + 4u * lane, f.pmask + (size_t)pk * 32 + lane);
     if (p.use_dm && lane < 18) {
       const int idx = (lane < 16) ? (int)s_amap[(int)(sb.y & 0x7fffffffu) + amap_lane] : p.pzt_nact + lane - 16;
       if (idx >= 0) wu_cp_async4(dst + 128u + 4u * lane, p.volts + (size_t)pe * p.ldv + idx);
-      else *reinterpret_cast<float*>(my_aux + slot * WU_AUX_BYTES + 128 + 4 * lane) = 0.f;
+      else *reinterpret_cast<float*>(my_aux + slot * AUXB + 128 + 4 * lane) = 0.f;
     }
-    if (has_after && lane == 0) wu_cp_async8(my_aux_u32 + (uint32_t)(slot ^ 1) * WU_AUX_BYTES + 256u, f.sub + k_after);
+    if (has_after && lane == 0) wu_cp_async8(my_aux_u32 + (uint32_t)(slot ^ 1) * AUXB + 256u, f.sub + k_after);
+    if (PE && lane < 8 * NL)      // the layer offsets of this item's environment, one word per lane
+      wu_cp_async4(dst + (uint32_t)WU_AUX_BYTES + 4u * lane,
+                   reinterpret_cast<const uint32_t*>(p.wind + (size_t)(lane >> 3) * p.E + pe) + (lane & 7));
     asm volatile("cp.async.commit_group;" ::: "memory");
   };
 
@@ -631,8 +639,8 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
     wu_f2 P[4];
     uint32_t c_pm = 0u;
     if (c_valid) {
-      c_pm = *reinterpret_cast<const uint32_t*>(my_aux + s * WU_AUX_BYTES + 4 * lane);
-      const float* V = reinterpret_cast<const float*>(my_aux + s * WU_AUX_BYTES + 128);
+      c_pm = *reinterpret_cast<const uint32_t*>(my_aux + s * AUXB + 4 * lane);
+      const float* V = reinterpret_cast<const float*>(my_aux + s * AUXB + 128);
       // this item's mirror inputs are requested before the bookkeeping of the next item (which is full of memory-
       // clobbering copies the compiler cannot move loads across), so that their latency is covered by it
       float4 v0 = make_float4(0.f, 0.f, 0.f, 0.f), v1r = v0, v2r = v0, v3 = v0;
@@ -648,7 +656,7 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
       //      tiles as soon as the current ones are sampled ----
       uint2 sb1 = make_uint2(0u, 0u);
       if (nx_valid) {
-        sb1 = *reinterpret_cast<const uint2*>(my_aux + (s ^ 1) * WU_AUX_BYTES + 256);
+        sb1 = *reinterpret_cast<const uint2*>(my_aux + (s ^ 1) * AUXB + 256);
         sb1.x = __shfl_sync(0xffffffffu, sb1.x, 0); sb1.y = __shfl_sync(0xffffffffu, sb1.y, 0);
         k += WU_WARPS;
         if (k >= p.nvalid) { k -= p.nvalid; e += 1; }
@@ -707,11 +715,21 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
 #pragma unroll
         for (int l = 0; l < NL; ++l) {
           const float* t = reinterpret_cast<const float*>(my_tiles + l * WU_TILE_STRIDE) + lane_off;
-          switch ((c_d >> (2 * l)) & 3u) {
-            case 0: wu_layer<0>(t, p.layer[l], acc); break;
-            case 1: wu_layer<1>(t, p.layer[l], acc); break;
-            case 2: wu_layer<2>(t, p.layer[l], acc); break;
-            default: wu_layer<3>(t, p.layer[l], acc); break;
+          if (PE) {
+            const WindRec* wr = reinterpret_cast<const WindRec*>(my_aux + s * AUXB + WU_AUX_BYTES);
+            switch ((c_d >> (2 * l)) & 3u) {
+              case 0: wu_layer<0>(t, wr[l], acc); break;
+              case 1: wu_layer<1>(t, wr[l], acc); break;
+              case 2: wu_layer<2>(t, wr[l], acc); break;
+              default: wu_layer<3>(t, wr[l], acc); break;
+            }
+          } else {
+            switch ((c_d >> (2 * l)) & 3u) {
+              case 0: wu_layer<0>(t, p.layer[l], acc); break;
+              case 1: wu_layer<1>(t, p.layer[l], acc); break;
+              case 2: wu_layer<2>(t, p.layer[l], acc); break;
+              default: wu_layer<3>(t, p.layer[l], acc); break;
+            }
           }
           asm volatile("" ::: "memory");                // one layer's window in registers at a time
         }

@@ -22,12 +22,13 @@
 #define WS_THREADS 384
 #define WS_MIN_BLOCKS 2                    // two CTAs per SM: 80 registers per thread
 
-template <int NL, int FULL>
+template <int NL, int FULL, bool PE = false>     // PE: per-environment winds, as in wfs_frame_umma_kernel
 __global__ void __launch_bounds__(WS_THREADS, WS_MIN_BLOCKS) wfs_frame_ws_kernel(const __grid_constant__ WfsUmmaParams P) {
   const WfsParams& p = P.p;
   const WfsUmmaTables& f = P.f;
   extern __shared__ __align__(1024) unsigned char wu_smem_raw[];
   constexpr int NLS = NL > 0 ? NL : 1;
+  constexpr int AUXB = PE ? WU_AUX_BYTES_PE : WU_AUX_BYTES;
   unsigned char* s_a1 = wu_smem_raw;                                   // [hi, lo][WU_A_BYTES]
   unsigned char* s_a2 = s_a1 + 2 * WU_A_BYTES;                         // [tile][hi, lo][WU_A_BYTES]
   unsigned char* s_b1 = s_a2 + 4 * WU_A_BYTES;                         // [hi, lo][WU_B_BYTES]
@@ -39,8 +40,8 @@ __global__ void __launch_bounds__(WS_THREADS, WS_MIN_BLOCKS) wfs_frame_ws_kernel
   uint32_t* s_cnt = (uint32_t*)(s_bar + 15) - 2;                       // [2] TMEM slot (the last 4 bytes before byte 128)
   float* s_fx = (float*)((unsigned char*)s_bar + 128);                 // [NG][16]
   float* s_fyT = s_fx + WU_NG * 16;                                    // [16][NG]
-  unsigned char* s_aux = (unsigned char*)(s_fyT + 16 * WU_NG);         // [warp][parity][WU_AUX_BYTES]
-  short* s_amap = (short*)(s_aux + WU_WARPS * 2 * WU_AUX_BYTES);
+  unsigned char* s_aux = (unsigned char*)(s_fyT + 16 * WU_NG);         // [warp][parity][AUXB]
+  short* s_amap = (short*)(s_aux + WU_WARPS * 2 * AUXB);
 
   // lane through a volatile read: the compiler otherwise re-derives it from S2R SR_TID.X at ~25 places of the loop body
   // and each of those reads stalls its warp (5 % of the stall samples in profiles/r02_wfs_umma_v5)
@@ -91,7 +92,7 @@ __global__ void __launch_bounds__(WS_THREADS, WS_MIN_BLOCKS) wfs_frame_ws_kernel
     unsigned char* my_tiles = s_tiles + (size_t)warp * NLS * WU_TILE_STRIDE;
     const uint32_t my_tiles_u32 = wu_smem_u32(my_tiles);
     const uint32_t my_bar_u32 = wu_smem_u32(s_bar + warp);
-    unsigned char* my_aux = s_aux + (size_t)warp * 2 * WU_AUX_BYTES;     // per parity: pm[32] | volts[32] | record
+    unsigned char* my_aux = s_aux + (size_t)warp * 2 * AUXB;     // per parity: pm[32] | volts[32] | record
     const uint32_t my_aux_u32 = wu_smem_u32(my_aux);
     const int lane_off = y * WU_TILE_W + 8 * h;                          // floats, inside a tile
     const int amap_lane = (lane >> 2) * f.GW + (lane & 3);
@@ -137,8 +138,8 @@ __global__ void __launch_bounds__(WS_THREADS, WS_MIN_BLOCKS) wfs_frame_ws_kernel
   #pragma unroll
         for (int l = 0; l < NL; ++l) {
           const int N = p.layer[l].N;
-          int a = p.layer[l].ix + p.layer[l].ox[pe];  a -= (a >= N) ? N : 0;
-          int b = p.layer[l].iy + p.layer[l].oy[pe];  b -= (b >= N) ? N : 0;
+          int a = (PE ? __ldg(&p.wind[(size_t)l * p.E + pe].ix) : p.layer[l].ix) + p.layer[l].ox[pe];  a -= (a >= N) ? N : 0;
+          int b = (PE ? __ldg(&p.wind[(size_t)l * p.E + pe].iy) : p.layer[l].iy) + p.layer[l].oy[pe];  b -= (b >= N) ? N : 0;
           rx[l] = a; ry[l] = b;
         }
         ring_e = pe;
@@ -196,14 +197,17 @@ __global__ void __launch_bounds__(WS_THREADS, WS_MIN_BLOCKS) wfs_frame_ws_kernel
     // ---- per-lane inputs of one work item into the parity slot: pupil word, neighbourhood volts (cp.async: no register
     //      waits for them), and the record of the item after it ----
     auto issue_aux = [&](int pe, int pk, uint2 sb, int slot, int k_after, bool has_after) {
-      const uint32_t dst = my_aux_u32 + (uint32_t)slot * WU_AUX_BYTES;
+      const uint32_t dst = my_aux_u32 + (uint32_t)slot * AUXB;
       wu_cp_async4(dst + 4u * lane, f.pmask + (size_t)pk * 32 + lane);
       if (p.use_dm && lane < 18) {
         const int idx = (lane < 16) ? (int)s_amap[(int)(sb.y & 0x7fffffffu) + amap_lane] : p.pzt_nact + lane - 16;
         if (idx >= 0) wu_cp_async4(dst + 128u + 4u * lane, p.volts + (size_t)pe * p.ldv + idx);
-        else *reinterpret_cast<float*>(my_aux + slot * WU_AUX_BYTES + 128 + 4 * lane) = 0.f;
+        else *reinterpret_cast<float*>(my_aux + slot * AUXB + 128 + 4 * lane) = 0.f;
       }
-      if (has_after && lane == 0) wu_cp_async8(my_aux_u32 + (uint32_t)(slot ^ 1) * WU_AUX_BYTES + 256u, f.sub + k_after);
+      if (has_after && lane == 0) wu_cp_async8(my_aux_u32 + (uint32_t)(slot ^ 1) * AUXB + 256u, f.sub + k_after);
+      if (PE && lane < 8 * NL)      // the layer offsets of this item's environment, one word per lane
+        wu_cp_async4(dst + (uint32_t)WU_AUX_BYTES + 4u * lane,
+                     reinterpret_cast<const uint32_t*>(p.wind + (size_t)(lane >> 3) * p.E + pe) + (lane & 7));
       asm volatile("cp.async.commit_group;" ::: "memory");
     };
 
@@ -232,8 +236,8 @@ __global__ void __launch_bounds__(WS_THREADS, WS_MIN_BLOCKS) wfs_frame_ws_kernel
       wu_f2 P[4];
       uint32_t c_pm = 0u;
       if (c_valid) {
-        c_pm = *reinterpret_cast<const uint32_t*>(my_aux + s * WU_AUX_BYTES + 4 * lane);
-        const float* V = reinterpret_cast<const float*>(my_aux + s * WU_AUX_BYTES + 128);
+        c_pm = *reinterpret_cast<const uint32_t*>(my_aux + s * AUXB + 4 * lane);
+        const float* V = reinterpret_cast<const float*>(my_aux + s * AUXB + 128);
         // this item's mirror inputs are requested before the bookkeeping of the next item (which is full of memory-
         // clobbering copies the compiler cannot move loads across), so that their latency is covered by it
         float4 v0 = make_float4(0.f, 0.f, 0.f, 0.f), v1r = v0, v2r = v0, v3 = v0;
@@ -249,7 +253,7 @@ __global__ void __launch_bounds__(WS_THREADS, WS_MIN_BLOCKS) wfs_frame_ws_kernel
         //      tiles as soon as the current ones are sampled ----
         uint2 sb1 = make_uint2(0u, 0u);
         if (nx_valid) {
-          sb1 = *reinterpret_cast<const uint2*>(my_aux + (s ^ 1) * WU_AUX_BYTES + 256);
+          sb1 = *reinterpret_cast<const uint2*>(my_aux + (s ^ 1) * AUXB + 256);
           sb1.x = __shfl_sync(0xffffffffu, sb1.x, 0); sb1.y = __shfl_sync(0xffffffffu, sb1.y, 0);
           k += WU_WARPS;
           if (k >= p.nvalid) { k -= p.nvalid; e += 1; }
@@ -308,11 +312,21 @@ __global__ void __launch_bounds__(WS_THREADS, WS_MIN_BLOCKS) wfs_frame_ws_kernel
   #pragma unroll
           for (int l = 0; l < NL; ++l) {
             const float* t = reinterpret_cast<const float*>(my_tiles + l * WU_TILE_STRIDE) + lane_off;
-            switch ((c_d >> (2 * l)) & 3u) {
-              case 0: wu_layer<0>(t, p.layer[l], acc); break;
-              case 1: wu_layer<1>(t, p.layer[l], acc); break;
-              case 2: wu_layer<2>(t, p.layer[l], acc); break;
-              default: wu_layer<3>(t, p.layer[l], acc); break;
+            if (PE) {
+              const WindRec* wr = reinterpret_cast<const WindRec*>(my_aux + s * AUXB + WU_AUX_BYTES);
+              switch ((c_d >> (2 * l)) & 3u) {
+                case 0: wu_layer<0>(t, wr[l], acc); break;
+                case 1: wu_layer<1>(t, wr[l], acc); break;
+                case 2: wu_layer<2>(t, wr[l], acc); break;
+                default: wu_layer<3>(t, wr[l], acc); break;
+              }
+            } else {
+              switch ((c_d >> (2 * l)) & 3u) {
+                case 0: wu_layer<0>(t, p.layer[l], acc); break;
+                case 1: wu_layer<1>(t, p.layer[l], acc); break;
+                case 2: wu_layer<2>(t, p.layer[l], acc); break;
+                default: wu_layer<3>(t, p.layer[l], acc); break;
+              }
             }
             asm volatile("" ::: "memory");                // one layer's window in registers at a time
           }

@@ -51,7 +51,7 @@ OPTIONS = ["WFS_PATH", "GEMM_PATH", "TIME_WFS", "GEO", "DENOISE", "PUPIL_PATH", 
 O = {name: i for i, name in enumerate(OPTIONS)}
 
 EXPORTS = ["aom_config_size", "aom_create", "aom_destroy", "aom_last_error", "aom_set_table", "aom_get_buffer",
-           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_comp_wfs_image", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
+           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
            "aom_comp_strehl", "aom_reset_strehl", "aom_do_control_geo", "aom_apply_control_geo", "aom_denoise", "aom_set_bincube", "aom_do_centroids", "aom_do_centroids_geom", "aom_do_control", "aom_set_command", "aom_apply_control",
            "aom_set_gain", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
            "aom_state_begin", "aom_state_end", "aom_reward", "aom_actor_forward", "aom_step", "aom_gemm_tn",
@@ -90,6 +90,7 @@ def load_library():
     lib.aom_move_atmos.argtypes = [vp, vp]
     lib.aom_set_layer.argtypes = [vp, i32, f32, f32, f32]
     lib.aom_set_layer_amp.argtypes = [vp, i32, vp]
+    lib.aom_set_layer_wind.argtypes = [vp, i32, vp, vp]
     lib.aom_comp_wfs_image.argtypes = [vp, i32, f32, vp]
     lib.aom_raytrace_wfs.argtypes = [vp, i32, vp]
     lib.aom_wfs_time_ms.argtypes = [vp, ctypes.POINTER(f32), ctypes.POINTER(i32)]
@@ -379,6 +380,17 @@ class Simulator:
     def set_layer(self, layer, deltax, deltay, amp):
         self._check(self.lib.aom_set_layer(self._ctx, int(layer), float(deltax), float(deltay), float(amp)),
                     "aom_set_layer")
+
+    def set_layer_wind(self, layer, deltax, deltay):
+        """Wind step of one layer per environment (pixels / frame, float [E] each; a scalar broadcasts); None, None
+        returns the layer to its common wind (set_layer).  Accumulators continue from the common one."""
+        if deltax is None and deltay is None:
+            self._check(self.lib.aom_set_layer_wind(self._ctx, int(layer), None, None), "aom_set_layer_wind")
+            return
+        dx = np.ascontiguousarray(np.broadcast_to(np.asarray(deltax, dtype=np.float32), (self.n_env,)))
+        dy = np.ascontiguousarray(np.broadcast_to(np.asarray(deltay, dtype=np.float32), (self.n_env,)))
+        self._check(self.lib.aom_set_layer_wind(self._ctx, int(layer), dx.ctypes.data_as(ctypes.c_void_p),
+                                                dy.ctypes.data_as(ctypes.c_void_p)), "aom_set_layer_wind")
 
     def set_layer_amp(self, layer, amp):
         """Innovation amplitude of one layer per environment (float [E]); None restores the common amplitude."""

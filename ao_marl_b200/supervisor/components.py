@@ -69,19 +69,42 @@ class AtmosB200(_Base):
             seed = np.random.randint(int(1e4)) if reset_seed == 0 else reset_seed
             self._sim.reset(self._sim.env_seeds(1234 + seed))
 
-    def set_wind(self, screen_index, *, windspeed=None, winddir=None):
+    def _wind_step(self, windspeed, winddir):
+        """(deltax, deltay) in pixels per frame of one wind speed (m/s) and direction (degrees)."""
         c = self._config
-        a = c.p_atmos
-        if windspeed is not None:
-            a.windspeed[screen_index] = windspeed
-        if winddir is not None:
-            a.winddir[screen_index] = winddir
-        lin = c.p_geom.pupdiam / c.p_tel.diam * a.windspeed[screen_index] * np.cos(DEG2RAD * c.p_geom.zenithangle) \
-            * c.p_loop.ittime
-        a._deltax[screen_index] = lin * np.sin(DEG2RAD * a.winddir[screen_index] + np.pi)
-        a._deltay[screen_index] = lin * np.cos(DEG2RAD * a.winddir[screen_index] + np.pi)
-        # a change of sign needs no new stencil here: mirroring is index arithmetic in the kernels
-        self._sim.set_layer(screen_index, a._deltax[screen_index], a._deltay[screen_index], self._amp(screen_index))
+        lin = c.p_geom.pupdiam / c.p_tel.diam * windspeed * np.cos(DEG2RAD * c.p_geom.zenithangle) * c.p_loop.ittime
+        return lin * np.sin(DEG2RAD * winddir + np.pi), lin * np.cos(DEG2RAD * winddir + np.pi)
+
+    def set_wind(self, screen_index, *, windspeed=None, winddir=None):
+        """atmosCompass.py:79-135.  `windspeed` and `winddir` may each be a scalar or an array [E] (one wind per
+        environment of the batch; a scalar broadcasts against the other, an omitted one is the layer's current value).
+        Both scalar: the layer's common wind, recorded in p_atmos as in the reference, and any per-environment wind of
+        the layer is dropped.  Otherwise the winds go to the environments only (p_atmos keeps the common wind); every
+        environment continues from the layer's current sub-pixel position."""
+        a = self._config.p_atmos
+        l = screen_index
+        if np.ndim(windspeed) == 0 and np.ndim(winddir) == 0:
+            if windspeed is not None:
+                a.windspeed[l] = windspeed
+            if winddir is not None:
+                a.winddir[l] = winddir
+            a._deltax[l], a._deltay[l] = self._wind_step(a.windspeed[l], a.winddir[l])
+            # a change of sign needs no new stencil here: mirroring is index arithmetic in the kernels
+            self._sim.set_layer(l, a._deltax[l], a._deltay[l], self._amp(l))
+            self._sim.set_layer_wind(l, None, None)
+            return
+        E = self._sim.n_env
+        speed = np.asarray(a.windspeed[l] if windspeed is None else windspeed, dtype=np.float64)
+        direction = np.asarray(a.winddir[l] if winddir is None else winddir, dtype=np.float64)
+        for v in (speed, direction):
+            if v.ndim != 0 and v.shape != (E,):
+                raise ValueError("Dimension mismatch")
+        speed, direction = np.broadcast_to(speed, (E,)), np.broadcast_to(direction, (E,))
+        # element by element with the scalar formula on values of p_atmos' own types (float32 in the parameter files):
+        # the same operations as a common wind of that value, so each environment moves exactly as such a batch would
+        ts, td = np.asarray(a.windspeed).dtype.type, np.asarray(a.winddir).dtype.type
+        steps = [self._wind_step(ts(speed[e]), td(direction[e])) for e in range(E)]
+        self._sim.set_layer_wind(l, np.array([d[0] for d in steps], np.float32), np.array([d[1] for d in steps], np.float32))
 
     def get_atmos_layer(self, indx):
         """Logical (un-rotated) screen(s) of layer `indx`."""

@@ -237,8 +237,25 @@ int aom_set_layer(aom_ctx* ctx, int layer, float deltax, float deltay, float amp
 
 /* AtmosCompass.set_r0 per environment (the reference changes r0 of its single simulator at run time,
  * train_rpc.py:429-449; a batch can hold one condition per environment): innovation amplitude of `layer` for every
- * environment, host float [E] (NULL: back to the layer's common amplitude).  The wind stays common to the batch. */
+ * environment, host float [E] (NULL: back to the layer's common amplitude).  The wind is set per environment by
+ * aom_set_layer_wind. */
 int aom_set_layer_amp(aom_ctx* ctx, int layer, const float* amp_host);
+
+/* AtmosCompass.set_wind per environment (atmosCompass.py:79-135; the reference changes the wind of its single simulator
+ * at run time, train_rpc.py:429-449): wind step (pixels / frame) of `layer` for every environment, host float [E] each
+ * (NULL, NULL: back to the layer's common wind of aom_config.deltax / deltay and aom_set_layer).
+ * - Setting per-environment winds starts every environment's accumulator from the layer's current common one: the
+ *   screens do not jump mid-episode.  Every environment then sees exactly the extrusions, innovations and raytrace
+ *   offsets it would see in a batch where every environment had its wind.
+ * - aom_set_layer changes the common wind (and the amplitude) and leaves per-environment winds in force.
+ * - Back on the common wind, the library returns to its uniform kernels as soon as every layer's accumulators agree
+ *   over the batch, at the latest after the next aom_reset (whose start-up extrudes each environment in the direction
+ *   of its own x wind).
+ * - AOM_ERR_UNSUPPORTED when the pupil footprint of an environment leaves the screen.  The round-1 sensor kernels (wfs
+ *   paths tensor_reg / tensor / tensor_fast) have no per-environment form: their frames return AOM_ERR_UNSUPPORTED
+ *   ("per-environment wind is not implemented in the round-1 sensor kernels ...") while such winds are in force.
+ * Waits for the device; not for the step path. */
+int aom_set_layer_wind(aom_ctx* ctx, int layer, const float* deltax_host, const float* deltay_host);
 
 /* WfsCompass.raytrace + compute_wfs_image fused (wfsCompass.py:334-343, sourceCompass.py:54-85).
  * flags: bit0 atmosphere, bit1 mirrors, bit2 keep image (writes AOM_B_BINCUBE), bit3 do not advance the frame counter
