@@ -106,6 +106,17 @@ struct aom_ctx {
   float *aX, *aH1, *aH2, *aHO;
   int ld_ain, ld_ah, ld_aho;
   bool seeded;
+  // staggered environments (aom_reset_envs): from the first partial reset until the next aom_reset every environment
+  // counts its noise frames, actor decisions and long-exposure frames from its own reset, and an environment whose
+  // first step is pending (first[e]) takes no action and accumulates no Strehl in its next rl half-step
+  bool staggered;
+  bool first_any;              // some first[e] may be set (cleared by aom_state_end)
+  int* rs_envs;                // device [E] environments of the last aom_reset_envs
+  uint32_t* rs_seeds;          // device [2][E] their seeds (low, high words)
+  uint32_t* frame0;            // device [E] global noise frame of each environment's first frame
+  uint32_t* step_env;          // device [E] actor decision counters
+  int* le_n;                   // device [2][E] long-exposure counts (main target, geometric target)
+  int* first;                  // device [E] first step pending
   // TMA-staged Shack-Hartmann kernel (wfs_tma.cuh): host copies of the tables it derives from, derived tables
   void* htab[AOM_T_COUNT];
   size_t htab_bytes[AOM_T_COUNT];
@@ -292,7 +303,8 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
                   ctx->modes_before, ctx->modes_res, ctx->state, ctx->hist, ctx->reward, ctx->action,
                   ctx->action_mean, ctx->strehl, ctx->tar_mom, ctx->tar_acc, ctx->aX, ctx->aH1, ctx->aH2, ctx->aHO, ctx->d_err,
                   ctx->geo_com, ctx->geo_volts, ctx->geo_b, ctx->geo_T, ctx->strehl_geo, ctx->geo_acc, ctx->geo_mom,
-                  ctx->sweep_mask, ctx->sweep_ttp};
+                  ctx->sweep_mask, ctx->sweep_ttp, ctx->rs_envs, ctx->rs_seeds, ctx->frame0, ctx->step_env,
+                  ctx->le_n, ctx->first};
   for (void* b : bufs) cudaFree(b);
   for (int l = 0; l < AOM_MAX_LAYERS; ++l) { cudaFree(ctx->oz_ab[l]); cudaFree(ctx->oz_ea[l]); }
   for (int t = 0; t < AOM_T_COUNT; ++t) { cudaFree(ctx->ozop[t]); cudaFree(ctx->ozop_ea[t]); }
@@ -549,6 +561,9 @@ extern "C" int aom_get_buffer(aom_ctx* ctx, int buffer, int index, void** dptr, 
     case AOM_B_RING_OY:
       if (index < 0 || index >= c.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
       p = ctx->oy[index]; n = E; break;
+    case AOM_B_EXT_COUNT:
+      if (index < 0 || index >= c.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
+      p = ctx->ext_count[index]; n = E; break;
     case AOM_B_SLOPES: p = ctx->slopes; n = E * ctx->lds; break;
     case AOM_B_ERR: p = ctx->err_v; n = E * ctx->lda; break;
     case AOM_B_COM: p = ctx->com; n = E * ctx->lda; break;
@@ -672,9 +687,13 @@ extern "C" int aom_gemm_tn(aom_ctx* ctx, const float* A, int lda, const float* B
 }
 
 // ---------------------------------------------------------------------------------------------
-// steps != null: per-environment winds -- pass `pass` of the signed counts steps [E] of this axis (`sign` unused)
-static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st, const int* steps = nullptr, int pass = 0) {
+// steps != null: per-environment winds -- pass `pass` of the signed counts steps [E] of this axis (`sign` unused).
+// envs != null: only the K environments envs[0..K) (device), compacted into the first K rows of the scratch and the
+// contraction (the start-up of aom_reset_envs).
+static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st, const int* steps = nullptr, int pass = 0,
+                        const int* envs = nullptr, int K = 0) {
   const aom_config& c = ctx->cfg;
+  const int rows = envs ? K : c.n_env;
   NEED(AOM_T_AB, l);
   NEED(AOM_T_STENCIL, l);
   ExtrudeParams p;
@@ -683,11 +702,11 @@ static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st
   p.N = c.screen_dim[l]; p.S = c.stencil_size[l]; p.E = c.n_env; p.layer = l; p.axis = axis; p.sign = sign;
   p.amp = c.amp[l]; p.amp_env = ctx->amp_env[l];
   p.ldz = AOM_LD(p.S + p.N); p.Z = ctx->Z; p.zref = ctx->zref; p.ldn = AOM_LD(p.N); p.newcol = ctx->newcol;
-  p.steps = steps; p.pass = pass;
+  p.steps = steps; p.pass = pass; p.envs = envs;
   if (ctx->opt[AOM_OPT_EXTRUDE_PATH] == AOM_EXTRUDE_I8) {
     // exact integer contraction on tcgen05 (extrude_i8.cuh): digits of the inputs, 13 int8 digit-pair products with
     // int32 accumulators, one rounding to float32 after adding the reference pixel
-    const int KB = ctx->oz_kb[l], NT = ctx->oz_nt[l], MT = (c.n_env + OZ_BM - 1) / OZ_BM;
+    const int KB = ctx->oz_kb[l], NT = ctx->oz_nt[l], MT = (rows + OZ_BM - 1) / OZ_BM;
     const size_t need = (size_t)MT * KB * OZ_SLICES * OZ_A_TILE;
     if (need > ctx->oz_zs_bytes) {
       cudaFree(ctx->oz_zs); ctx->oz_zs = nullptr; ctx->oz_zs_bytes = 0;
@@ -700,26 +719,26 @@ static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st
     int* ev = ctx->oz_ev;
     OzGatherParams g;
     g.screen = p.screen; g.ox = p.ox; g.oy = p.oy; g.count = p.count; g.k0 = p.k0; g.k1 = p.k1; g.stencil = p.stencil;
-    g.zref = p.zref; g.ev = ev; g.Zs = zs; g.N = p.N; g.S = p.S; g.E = p.E; g.KB = KB; g.layer = l;
+    g.zref = p.zref; g.ev = ev; g.Zs = zs; g.N = p.N; g.S = p.S; g.E = rows; g.KB = KB; g.layer = l;
     g.axis = axis; g.sign = sign; g.amp = p.amp; g.amp_env = ctx->amp_env[l];
-    g.steps = steps; g.pass = pass;
+    g.steps = steps; g.pass = pass; g.envs = envs;
     OzGemmParams m;
     m.Zs = zs; m.ABs = ctx->oz_ab[l]; m.ev = ev; m.ea = ctx->oz_ea[l]; m.zref = p.zref;
-    m.out = p.newcol; m.ldo = p.ldn; m.E = p.E; m.N = p.N; m.KB = KB; m.err = ctx->d_err;
+    m.out = p.newcol; m.ldo = p.ldn; m.E = rows; m.N = p.N; m.KB = KB; m.err = ctx->d_err;
     cudaError_t le = oz_extrude_launch(g, m, MT, NT, st);
     if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "oz_extrude_launch: %s", cudaGetErrorString(le));
     ctx->launches += 2;
     p.zref = nullptr;                                  // the reference pixel is already in the new column
   } else {
-    if (steps) extrude_gather_kernel<true><<<c.n_env, 256, 0, st>>>(p);
-    else extrude_gather_kernel<false><<<c.n_env, 256, 0, st>>>(p);
+    if (steps) extrude_gather_kernel<true><<<rows, 256, 0, st>>>(p);
+    else extrude_gather_kernel<false><<<rows, 256, 0, st>>>(p);
     KCHECK();
     int rc = launch_gemm(ctx, 0, ctx->Z, p.ldz, 0, (const float*)ctx->tab[AOM_T_AB][l], p.ldz, 0, ctx->newcol, p.ldn, 0,
-                         c.n_env, p.N, p.S + p.N, nullptr, 0, 0, 1, st, nullptr, 0, true);
+                         rows, p.N, p.S + p.N, nullptr, 0, 0, 1, st, nullptr, 0, true);
     if (rc) return rc;
   }
-  if (steps) extrude_scatter_kernel<true><<<c.n_env, EXTRUDE_SCATTER_THREADS, 0, st>>>(p);
-  else extrude_scatter_kernel<false><<<c.n_env, EXTRUDE_SCATTER_THREADS, 0, st>>>(p);
+  if (steps) extrude_scatter_kernel<true><<<rows, EXTRUDE_SCATTER_THREADS, 0, st>>>(p);
+  else extrude_scatter_kernel<false><<<rows, EXTRUDE_SCATTER_THREADS, 0, st>>>(p);
   KCHECK();
   return AOM_OK;
 }
@@ -734,7 +753,9 @@ static bool wind_any_env(const aom_ctx* ctx) {
 
 // One transition of the wind state of every layer and environment (WIND_STEP / WIND_INIT / WIND_RESET, atmos_kernels.cuh)
 // on the device, asynchronously on `st`, and the same on the host mirror: passes per layer and offset bounds.
-static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st) {
+// WIND_RESET_ENVS: WIND_RESET of the K environments listed in envs_d (device) / envs_h (host) only.
+static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st, const int* envs_d = nullptr, const int* envs_h = nullptr,
+                       int K = 0) {
   const aom_config& c = ctx->cfg;
   const int E = c.n_env, L = c.n_layers;
   if (L == 0) return AOM_OK;
@@ -746,7 +767,9 @@ static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st) {
     W.ax0 = ctx->accx[l]; W.ay0 = ctx->accy[l]; W.xoff = c.wfs_xoff[l]; W.yoff = c.wfs_yoff[l]; W.n2 = 2 * c.screen_dim[l];
   }
   P.acc = ctx->wind_acc; P.steps = ctx->wind_steps; P.rec = ctx->wind_rec; P.E = E; P.n_layers = L; P.mode = mode;
-  wind_state_kernel<<<(L * E + 255) / 256, 256, 0, st>>>(P);
+  P.envs = envs_d; P.K = K;
+  const int n = mode == WIND_RESET_ENVS ? K : E;
+  wind_state_kernel<<<(L * n + 255) / 256, 256, 0, st>>>(P);
   KCHECK();
   for (int l = 0; l < L; ++l) {
     const WindLayerParams& W = P.layer[l];
@@ -754,6 +777,10 @@ static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st) {
     double* ay = ax + E;
     int px = 0, py = 0;
     int* box = ctx->wind_box[l];
+    if (mode == WIND_RESET_ENVS) {
+      for (int k = 0; k < K; ++k) ax[envs_h[k]] = ay[envs_h[k]] = 0.0;
+      py = W.n2;
+    }
     for (int e = 0; e < E; ++e) {
       const float dx = ctx->wind_hdx[l] ? ctx->wind_hdx[l][e] : W.cdx, dy = ctx->wind_hdy[l] ? ctx->wind_hdy[l][e] : W.cdy;
       if (mode == WIND_STEP) {
@@ -761,7 +788,7 @@ static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st) {
         px = std::max(px, abs(nx)); py = std::max(py, abs(ny));
       } else if (mode == WIND_INIT) {
         ax[e] = W.ax0; ay[e] = W.ay0;
-      } else {
+      } else if (mode == WIND_RESET) {
         ax[e] = ay[e] = 0.0;
         py = W.n2;
       }
@@ -793,6 +820,23 @@ static void wind_try_uniform(aom_ctx* ctx) {
   ctx->wind_pe = false;
 }
 
+// Per-environment wind state from the common one (WIND_INIT on `st`): every environment continues from the layer's
+// common accumulators.
+static int wind_begin_pe(aom_ctx* ctx, cudaStream_t st) {
+  const size_t LE = (size_t)ctx->cfg.n_layers * ctx->cfg.n_env;
+  if (!ctx->wind_acc) {
+    CU(dalloc(&ctx->wind_acc, 2 * LE));
+    CU(dalloc(&ctx->wind_steps, 2 * LE));
+    CU(cudaMalloc((void**)&ctx->wind_rec, LE * sizeof(WindRec)));
+    ctx->wind_hacc = (double*)calloc(2 * LE, sizeof(double));
+    if (!ctx->wind_hacc) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+  }
+  int rc = wind_update(ctx, WIND_INIT, st);
+  if (rc) return rc;
+  ctx->wind_pe = true;
+  return AOM_OK;
+}
+
 extern "C" int aom_set_layer_wind(aom_ctx* ctx, int layer, const float* deltax_host, const float* deltay_host) {
   if (!ctx) return AOM_ERR_INVALID;
   const aom_config& c = ctx->cfg;
@@ -822,18 +866,9 @@ extern "C" int aom_set_layer_wind(aom_ctx* ctx, int layer, const float* deltax_h
   CU(cudaMemcpy(ctx->wind_dy[layer], deltay_host, E * sizeof(float), cudaMemcpyHostToDevice));
   if (!ctx->wind_pe) {
     // every environment continues from the common accumulators: the screens do not jump
-    const size_t LE = (size_t)c.n_layers * E;
-    if (!ctx->wind_acc) {
-      CU(dalloc(&ctx->wind_acc, 2 * LE));
-      CU(dalloc(&ctx->wind_steps, 2 * LE));
-      CU(cudaMalloc((void**)&ctx->wind_rec, LE * sizeof(WindRec)));
-      ctx->wind_hacc = (double*)calloc(2 * LE, sizeof(double));
-      if (!ctx->wind_hacc) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
-    }
-    int rc = wind_update(ctx, WIND_INIT, 0);
+    int rc = wind_begin_pe(ctx, 0);
     if (rc) return rc;
     CU(cudaStreamSynchronize(0));                    // the legacy stream: the state is read next on any stream
-    ctx->wind_pe = true;
   }
   const int* b = ctx->wind_box[layer];
   if (b[0] < 0 || b[2] < 0 || b[1] + c.n + 1 > c.screen_dim[layer] || b[3] + c.n + 1 > c.screen_dim[layer])
@@ -902,6 +937,8 @@ static int clear_loop_state(aom_ctx* ctx, cudaStream_t st) {
   return AOM_OK;
 }
 
+static int start_screens(aom_ctx* ctx, const int* envs, int K, cudaStream_t st);
+
 extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
   if (!ctx || !seeds) return fail(ctx, AOM_ERR_INVALID, "null argument");
   cudaStream_t st = (cudaStream_t)stream;
@@ -923,6 +960,14 @@ extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
   ctx->step = 0;
   int rc = clear_loop_state(ctx, st);
   if (rc) return rc;
+  ctx->staggered = false;                                                // every environment in lockstep again
+  ctx->first_any = false;
+  if (ctx->first) {
+    CU(cudaMemsetAsync(ctx->frame0, 0, E * sizeof(uint32_t), st));
+    CU(cudaMemsetAsync(ctx->step_env, 0, E * sizeof(uint32_t), st));
+    CU(cudaMemsetAsync(ctx->le_n, 0, 2 * E * sizeof(int), st));
+    CU(cudaMemsetAsync(ctx->first, 0, E * sizeof(int), st));
+  }
   for (int l = 0; l < c.n_layers; ++l) ctx->accx[l] = ctx->accy[l] = 0.0;
   if (ctx->wind_pe && !wind_any_env(ctx)) ctx->wind_pe = false;      // every accumulator restarts from 0: common again
   if (ctx->wind_pe) {
@@ -930,14 +975,27 @@ extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
     rc = wind_update(ctx, WIND_RESET, st);
     if (rc) return rc;
   }
-  // (The layers' start-up chains are independent, but running them on separate streams with private scratch gained
-  // nothing -- 1.35 s either way at 4096 environments: every extrusion kernel fills the GPU by itself.)
   for (int l = 0; l < c.n_layers; ++l) {
     size_t N = c.screen_dim[l];
     CU(cudaMemsetAsync(ctx->screen[l], 0, E * N * N * 4, st));
     CU(cudaMemsetAsync(ctx->ox[l], 0, E * 4, st));
     CU(cudaMemsetAsync(ctx->oy[l], 0, E * 4, st));
     CU(cudaMemsetAsync(ctx->ext_count[l], 0, E * 4, st));
+  }
+  return start_screens(ctx, nullptr, 0, st);
+}
+
+// Start-up of the screens of every environment (envs null) or of the K environments envs[0..K) (device list, compacted
+// extrusions): zero screens, ring origins and counters are expected, and the wind state of WIND_RESET (WIND_RESET_ENVS).
+// (The layers' start-up chains are independent, but running them on separate streams with private scratch gained
+// nothing for the whole batch -- 1.35 s either way at 4096 environments: every extrusion kernel fills the GPU by itself.)
+static int start_screens(aom_ctx* ctx, const int* envs, int K, cudaStream_t st) {
+  const aom_config& c = ctx->cfg;
+  const size_t E = c.n_env;
+  const unsigned rows = envs ? (unsigned)K : (unsigned)E;
+  int rc;
+  for (int l = 0; l < c.n_layers; ++l) {
+    size_t N = c.screen_dim[l];
     int sign = c.deltax[l] < 0 ? -1 : 1;
     const int* steps = ctx->wind_pe ? ctx->wind_steps + (2 * l + 1) * E : nullptr;
     // The reference starts a screen with 2N extrusions along x (columns: 648 pixels in 648 different DRAM rows per
@@ -946,15 +1004,99 @@ extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
     // (same stencil, same operator, same innovation counters; every index expression of the gather / scatter swaps its
     // roles, atmos_kernels.cuh / extrude_i8.cuh), and 2N extrusions bring the ring origin back to zero: so the start-up
     // runs along y and the screens are transposed in place once at the end -- bit-identical pixels, 1.29 -> 0.8 s.
-    for (size_t i = 0; i < 2 * N; ++i) { rc = extrude_once(ctx, l, 1, sign, st, steps, (int)i); if (rc) return rc; }
+    for (size_t i = 0; i < 2 * N; ++i) { rc = extrude_once(ctx, l, 1, sign, st, steps, (int)i, envs, K); if (rc) return rc; }
     {
       const int T = (int)((N + 31) / 32);
-      transpose_screens_kernel<<<dim3((unsigned)(T * (T + 1) / 2), (unsigned)E), dim3(32, 8), 0, st>>>(ctx->screen[l], (int)N);
+      transpose_screens_kernel<<<dim3((unsigned)(T * (T + 1) / 2), rows), dim3(32, 8), 0, st>>>(ctx->screen[l], (int)N, envs);
       KCHECK();
       // ring origin: 2N steps along y leave oy = 0 as 2N steps along x leave ox = 0 (2N mod N); nothing to swap
     }
   }
   return AOM_OK;
+}
+
+extern "C" int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const int64_t* seeds, void* stream) {
+  if (!ctx) return AOM_ERR_INVALID;
+  const aom_config& c = ctx->cfg;
+  const int E = c.n_env;
+  if (n < 0) return fail(ctx, AOM_ERR_INVALID, "aom_reset_envs: negative environment count %d", n);
+  if (n > 0 && (!envs || !seeds)) return fail(ctx, AOM_ERR_INVALID, "null argument");
+  if (n > E) return fail(ctx, AOM_ERR_INVALID, "aom_reset_envs: %d environments listed, the batch has %d", n, E);
+  {
+    char* seen = (char*)calloc((size_t)E, 1);
+    if (!seen) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+    for (int k = 0; k < n; ++k) {
+      const int e = envs[k];
+      if (e < 0 || e >= E) { free(seen); return fail(ctx, AOM_ERR_INVALID, "aom_reset_envs: environment %d out of range [0, %d)", e, E); }
+      if (seen[e]) { free(seen); return fail(ctx, AOM_ERR_INVALID, "aom_reset_envs: environment %d listed twice", e); }
+      seen[e] = 1;
+    }
+    free(seen);
+  }
+  if (!ctx->seeded) return fail(ctx, AOM_ERR_STATE, "aom_reset must be called before aom_reset_envs");
+  if (n == 0) return AOM_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  CU(cudaStreamSynchronize(st));                     // the wind mirror and the staging buffers are updated from the host
+  if (!ctx->first) {
+    CU(dalloc(&ctx->rs_envs, (size_t)E));
+    CU(dalloc(&ctx->rs_seeds, 2 * (size_t)E));
+    CU(dalloc(&ctx->frame0, (size_t)E));
+    CU(dalloc(&ctx->step_env, (size_t)E));
+    CU(dalloc(&ctx->le_n, 2 * (size_t)E));
+    CU(dalloc(&ctx->first, (size_t)E));
+  }
+  if (!ctx->staggered) {
+    // the batch leaves lockstep: every environment's counters start at the batch's
+    stagger_counters_kernel<<<(E + 255) / 256, 256, 0, st>>>(ctx->frame0, ctx->step_env, ctx->le_n, ctx->first, E, ctx->step,
+                                                             ctx->tar_n, ctx->geo_tar_n);
+    KCHECK();
+    ctx->staggered = true;
+  }
+  {
+    uint32_t* h = (uint32_t*)malloc(2 * (size_t)n * sizeof(uint32_t));
+    if (!h) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+    for (int k = 0; k < n; ++k) {
+      const uint64_t sd = (uint64_t)seeds[k];
+      h[k] = (uint32_t)(sd & 0xffffffffu);
+      h[n + k] = (uint32_t)(sd >> 32);
+    }
+    cudaError_t e1 = cudaMemcpyAsync(ctx->rs_envs, envs, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, st);
+    cudaError_t e2 = cudaMemcpyAsync(ctx->rs_seeds, h, 2 * (size_t)n * sizeof(uint32_t), cudaMemcpyHostToDevice, st);
+    cudaError_t e3 = cudaStreamSynchronize(st);
+    free(h);
+    CU(e1); CU(e2); CU(e3);
+  }
+  // every per-environment row aom_reset clears, the listed environments' screens and ring state, keys and counters
+  ResetEnvsParams P;
+  memset(&P, 0, sizeof(P));
+  auto add = [&](void* b, long long ld, int slots = 1, long long slot_stride = 0) {
+    if (!b || P.nbuf == RESET_MAX_BUFS) return;
+    P.buf[P.nbuf] = (uint32_t*)b; P.ld[P.nbuf] = ld; P.slots[P.nbuf] = slots; P.slot_stride[P.nbuf] = slot_stride;
+    P.nbuf++;
+  };
+  add(ctx->slopes, ctx->lds); add(ctx->slopes_frame, ctx->lds); add(ctx->err_v, ctx->lda); add(ctx->com, ctx->lda);
+  add(ctx->com1, ctx->lda); add(ctx->volts, ctx->lda); add(ctx->com_before, ctx->lda); add(ctx->modes_res, ctx->ldm);
+  add(ctx->state, ctx->ldst); add(ctx->action, ctx->ldact); add(ctx->tar_acc, TAR_ACC); add(ctx->strehl, 4);
+  if (ctx->hist) add(ctx->hist, c.state_modes, c.n_hist, (long long)E * c.state_modes);   // every slot of the ring
+  add(ctx->geo_com, ctx->lda); add(ctx->geo_volts, ctx->lda); add(ctx->geo_acc, TAR_ACC); add(ctx->strehl_geo, 4);
+  for (int l = 0; l < c.n_layers; ++l) {
+    add(ctx->screen[l], (long long)c.screen_dim[l] * c.screen_dim[l]);
+    add(ctx->ox[l], 1); add(ctx->oy[l], 1); add(ctx->ext_count[l], 1);
+  }
+  P.envs = ctx->rs_envs; P.seeds = ctx->rs_seeds; P.K = n; P.E = E;
+  P.k0 = ctx->k0; P.k1 = ctx->k1; P.frame0 = ctx->frame0; P.step_env = ctx->step_env; P.le_n = ctx->le_n;
+  P.first = ctx->first; P.frame = ctx->frame;
+  reset_envs_kernel<<<dim3((unsigned)n, (unsigned)P.nbuf + 1), 256, 0, st>>>(P);
+  KCHECK();
+  ctx->first_any = true;
+  if (c.n_layers == 0) return AOM_OK;
+  // The listed environments' accumulators restart from 0 while the others keep theirs: the per-environment wind state
+  // (common winds included) until they agree again (wind_try_uniform)
+  int rc;
+  if (!ctx->wind_pe) { rc = wind_begin_pe(ctx, st); if (rc) return rc; }
+  rc = wind_update(ctx, WIND_RESET_ENVS, st, ctx->rs_envs, envs, n);
+  if (rc) return rc;
+  return start_screens(ctx, ctx->rs_envs, n, st);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1381,6 +1523,7 @@ static int fill_wfs_params(aom_ctx* ctx, WfsParams& p, int flags, float noise) {
   p.k2 = (float)(2.0 * M_PI / (double)c.lambda_um);
   p.nphotons = c.nphotons; p.noise = noise; p.cog_offset = c.cog_offset; p.pixsize = c.pixsize;
   p.frame = ctx->frame; p.wfs_index = (uint32_t)c.wfs_index; p.k0 = ctx->k0; p.k1 = ctx->k1;
+  p.frame0 = ctx->staggered ? ctx->frame0 : nullptr;
   p.slopes = ctx->slopes_frame; p.lds = ctx->lds;
   return AOM_OK;
 }
@@ -1419,6 +1562,9 @@ extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* st
     cudaError_t le = wfs_umma_launch(p, ctx->umma, ctx->num_sms, !fast, path == AOM_WFS_UMMA_WS && p.noise < 0.f && p.bincube == nullptr, st);
     if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "wfs_umma_launch: %s", cudaGetErrorString(le));
   }
+  else if (c.nfft == 64 && path != AOM_WFS_SIMT && p.frame0)
+    return fail(ctx, AOM_ERR_UNSUPPORTED, "staggered environments (aom_reset_envs) are not implemented in the round-1 sensor "
+                "kernels (wfs_frame_tma_kernel, wfs_frame_mma_kernel) until the next aom_reset: use the umma, umma_ws or simt path");
   else if (c.nfft == 64 && path != AOM_WFS_SIMT && p.wind)
     return fail(ctx, AOM_ERR_UNSUPPORTED, "per-environment wind is not implemented in the round-1 sensor kernels "
                 "(wfs_frame_tma_kernel, wfs_frame_mma_kernel): use the umma, umma_ws or simt path");
@@ -1556,8 +1702,10 @@ extern "C" int aom_comp_strehl(aom_ctx* ctx, int flags, float lambda_um, int acc
   if (accumulate) n_le += 1;
   float* out = geo ? ctx->strehl_geo : ctx->strehl;
   float* acc = geo ? ctx->geo_acc : ctx->tar_acc;
-  if (peak) target_strehl_core_kernel<<<(c.n_env + 127) / 128, 128, 0, st>>>(mom, out, acc, c.n_env, accumulate ? n_le : 0);
-  else target_strehl_kernel<<<(c.n_env + 127) / 128, 128, 0, st>>>(mom, 5, out, acc, c.n_env, accumulate ? n_le : 0);
+  // staggered environments: their own long-exposure counts; one whose first step is pending is skipped
+  int* le_n = ctx->staggered ? ctx->le_n + (geo ? c.n_env : 0) : nullptr;
+  if (peak) target_strehl_core_kernel<<<(c.n_env + 127) / 128, 128, 0, st>>>(mom, out, acc, c.n_env, accumulate ? n_le : 0, le_n, ctx->first);
+  else target_strehl_kernel<<<(c.n_env + 127) / 128, 128, 0, st>>>(mom, 5, out, acc, c.n_env, accumulate ? n_le : 0, le_n, ctx->first);
   KCHECK();
   return AOM_OK;
 }
@@ -1609,10 +1757,12 @@ extern "C" int aom_apply_control_geo(aom_ctx* ctx, void* stream) {
 extern "C" int aom_reset_strehl(aom_ctx* ctx, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
   ctx->tar_n = 0;
+  if (ctx->le_n) CU(cudaMemsetAsync(ctx->le_n, 0, (size_t)ctx->cfg.n_env * sizeof(int), (cudaStream_t)stream));
   CU(cudaMemsetAsync(ctx->tar_acc, 0, (size_t)ctx->cfg.n_env * TAR_ACC * sizeof(float), (cudaStream_t)stream));
   CU(cudaMemsetAsync(ctx->strehl, 0, (size_t)ctx->cfg.n_env * 4 * sizeof(float), (cudaStream_t)stream));
   if (ctx->geo_com) {
     ctx->geo_tar_n = 0;
+    if (ctx->le_n) CU(cudaMemsetAsync(ctx->le_n + ctx->cfg.n_env, 0, (size_t)ctx->cfg.n_env * sizeof(int), (cudaStream_t)stream));
     CU(cudaMemsetAsync(ctx->geo_acc, 0, (size_t)ctx->cfg.n_env * TAR_ACC * sizeof(float), (cudaStream_t)stream));
     CU(cudaMemsetAsync(ctx->strehl_geo, 0, (size_t)ctx->cfg.n_env * 4 * sizeof(float), (cudaStream_t)stream));
   }
@@ -1813,7 +1963,7 @@ extern "C" int aom_rl_control(aom_ctx* ctx, const float* daction, void* stream) 
   dim3 grid((c.action_dim + 127) / 128, c.n_env);
   inject_action_kernel<<<grid, 128, 0, st>>>(ctx->modes, ctx->ldm, act, ctx->ldact, (const int*)ctx->tab[AOM_T_ACTION_MAP][0],
                                              (const float*)ctx->tab[AOM_T_FREEDOM][0], c.action_dim, c.n_env,
-                                             c.env_act_scale, c.env_act_bias);
+                                             c.env_act_scale, c.env_act_bias, ctx->first_any ? ctx->first : nullptr);
   KCHECK();
   if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_M2V])
     return launch_oz_product(ctx, AOM_T_M2V, ctx->modes, ctx->ldm, c.nmodes, ctx->com, ctx->lda, c.nactu, 0, nullptr, 0, st);
@@ -1825,6 +1975,14 @@ extern "C" int aom_state_begin(aom_ctx* ctx, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
   CU(cudaMemcpyAsync(ctx->com_before, ctx->com, (size_t)ctx->cfg.n_env * ctx->lda * 4, cudaMemcpyDeviceToDevice,
                      (cudaStream_t)stream));
+  return AOM_OK;
+}
+
+// The linear half-step of environments restarted by aom_reset_envs is done: their next rl half-step is an ordinary one.
+static int end_first_steps(aom_ctx* ctx, cudaStream_t st) {
+  if (!ctx->first_any) return AOM_OK;
+  CU(cudaMemsetAsync(ctx->first, 0, (size_t)ctx->cfg.n_env * sizeof(int), st));
+  ctx->first_any = false;
   return AOM_OK;
 }
 
@@ -1847,7 +2005,7 @@ extern "C" int aom_state_end(aom_ctx* ctx, void* stream) {
                                            c.n_env);
   KCHECK();
   if (c.n_hist > 0) ctx->hist_head = (ctx->hist_head + 1) % c.n_hist;
-  return AOM_OK;
+  return end_first_steps(ctx, st);
 }
 
 extern "C" int aom_reward(aom_ctx* ctx, float factor, void* stream) {
@@ -1891,7 +2049,8 @@ extern "C" int aom_actor_forward(aom_ctx* ctx, int eval_mode, void* stream) {
   if (rc) return rc;
   actor_sample_kernel<<<E, 256, 0, st>>>(ctx->aHO, ctx->ld_aho, c.actor_out, (const int*)ctx->tab[AOM_T_AGENT_ACT][0], E, A,
                                          c.log_sig_min, c.log_sig_max, c.pol_act_scale, c.pol_act_bias, eval_mode, ctx->step,
-                                         ctx->k0, ctx->k1, ctx->action, ctx->action_mean, ctx->ldact);
+                                         ctx->k0, ctx->k1, ctx->action, ctx->action_mean, ctx->ldact,
+                                         ctx->staggered ? ctx->step_env : nullptr, ctx->first);
   KCHECK();
   ctx->step++;      // one decision per call: the exploration-noise counter (oracle/rng.py TAG_ACTOR)
   return AOM_OK;
@@ -1949,6 +2108,7 @@ extern "C" int aom_step(aom_ctx* ctx, int mode, int eval_mode, void* stream) {
   rc = aom_do_centroids(ctx, stream); if (rc) return rc;
   rc = aom_do_control(ctx, stream); if (rc) return rc;
   if (ctx->state) { rc = aom_state_end(ctx, stream); if (rc) return rc; }
+  else { rc = end_first_steps(ctx, st); if (rc) return rc; }
   if (geo && fork) CU(cudaStreamWaitEvent(st, ctx->ev_geo, 0));
   return AOM_OK;
 }

@@ -32,6 +32,8 @@ struct ExtrudeParams {
   // that sits out a pass is not touched: no gather, no store, no RNG counter increment.
   const int* steps;
   int pass;
+  // compacted start-up (aom_reset_envs): row k of Z / zref / newcol belongs to environment envs[k]; null: row e = environment e
+  const int* envs;
 };
 
 // the direction of this pass for environment e; false: e sits it out
@@ -58,7 +60,7 @@ __device__ __forceinline__ int wrapN(int v, int N) { return v >= N ? v - N : v; 
 // Philox block yields its four innovations instead of one.
 template <bool PE = false>
 __global__ void __launch_bounds__(256) extrude_gather_kernel(ExtrudeParams p) {
-  const int e = blockIdx.x;
+  const int row = blockIdx.x, e = p.envs ? p.envs[row] : row;
   int sign = p.sign;
   if (!extr_active<PE>(p.steps, p.pass, e, sign)) return;
   const int N = p.N;
@@ -68,8 +70,8 @@ __global__ void __launch_bounds__(256) extrude_gather_kernel(ExtrudeParams p) {
   int rr, rc;
   extr_logical(0, N - 1, N, p.axis, sign, rr, rc);
   const float zr = scr[(size_t)wrapN(rr + oy, N) * N + wrapN(rc + ox, N)];
-  if (threadIdx.x == 0) p.zref[e] = zr;
-  float* Z = p.Z + (size_t)e * p.ldz;
+  if (threadIdx.x == 0) p.zref[row] = zr;
+  float* Z = p.Z + (size_t)row * p.ldz;
   for (int k = threadIdx.x; k < p.S; k += blockDim.x) {
     const int idx = p.stencil[k];
     int lr, lc;
@@ -90,7 +92,7 @@ __global__ void __launch_bounds__(256) extrude_gather_kernel(ExtrudeParams p) {
   for (int k = p.S + N + threadIdx.x; k < p.ldz; k += blockDim.x) Z[k] = 0.f;
 }
 
-// grid: E blocks of EXTRUDE_SCATTER_THREADS threads, one block per environment, every thread holds its (up to 8) pixels
+// grid: E (or K compacted) blocks of EXTRUDE_SCATTER_THREADS threads, one block per environment, every thread holds its (up to 8) pixels
 // of the new column in registers before it stores them.  A row-direction extrusion (contiguous) takes 9 us per 4096
 // environments (15 us with one warp per environment and a load -> store loop).  A column-direction extrusion is 648
 // four-byte stores into 648 different DRAM rows per environment -- a read-modify-write of a sector each, 91 MB read +
@@ -99,17 +101,17 @@ __global__ void __launch_bounds__(256) extrude_gather_kernel(ExtrudeParams p) {
 #define EXTRUDE_SCATTER_THREADS 128
 template <bool PE = false>
 __global__ void __launch_bounds__(EXTRUDE_SCATTER_THREADS) extrude_scatter_kernel(ExtrudeParams p) {
-  const int e = blockIdx.x;
+  const int row = blockIdx.x, e = p.envs ? p.envs[row] : row;
   int sign = p.sign;
   if (!extr_active<PE>(p.steps, p.pass, e, sign)) return;
   const int N = p.N;
   float* scr = p.screen + (size_t)e * N * N;
   const int ox = p.ox[e], oy = p.oy[e];
-  const float zr = p.zref ? p.zref[e] : 0.f;           // null: the GEMM already added the reference pixel
+  const float zr = p.zref ? p.zref[row] : 0.f;         // null: the GEMM already added the reference pixel
   int nox = ox, noy = oy;
   if (p.axis == 0) nox = (sign > 0) ? wrapN(ox + 1, N) : (ox == 0 ? N - 1 : ox - 1);
   else             noy = (sign > 0) ? wrapN(oy + 1, N) : (oy == 0 ? N - 1 : oy - 1);
-  const float* col = p.newcol + (size_t)e * p.ldn;
+  const float* col = p.newcol + (size_t)row * p.ldn;
   constexpr int PER = 8;                                    // pixels per thread and pass (N <= 1024 in one pass)
   for (int j0 = threadIdx.x; j0 < N; j0 += PER * EXTRUDE_SCATTER_THREADS) {
     float v[PER];
@@ -145,16 +147,17 @@ __global__ void __launch_bounds__(EXTRUDE_SCATTER_THREADS) extrude_scatter_kerne
 }
 
 // In-place transpose of E square screens [N][N].  grid (T (T + 1) / 2, E) with T = ceil(N / 32): every block swaps one pair
-// of 32 x 32 tiles (bi <= bj) through shared memory; block (32, 8).  Used by aom_reset, which runs its 2N start-up
-// extrusions along the contiguous axis of a transposed screen (see there).
-__global__ void __launch_bounds__(256) transpose_screens_kernel(float* __restrict__ screens, int N) {
+// of 32 x 32 tiles (bi <= bj) through shared memory; block (32, 8).  Used by the start-up of aom_reset / aom_reset_envs,
+// which runs its 2N extrusions along the contiguous axis of a transposed screen (see there).  envs: grid.y = K and
+// block row k transposes the screen of environment envs[k]; null: environment blockIdx.y.
+__global__ void __launch_bounds__(256) transpose_screens_kernel(float* __restrict__ screens, int N, const int* __restrict__ envs) {
   __shared__ float ta[32][33], tb[32][33];
   const int T = (N + 31) / 32;
   // tile pair index -> (bi, bj), bi <= bj
   int t = blockIdx.x, bi = 0;
   while (t >= T - bi) { t -= T - bi; ++bi; }
   const int bj = bi + t;
-  float* scr = screens + (size_t)blockIdx.y * N * N;
+  float* scr = screens + (size_t)(envs ? envs[blockIdx.y] : (int)blockIdx.y) * N * N;
   const int tx = threadIdx.x, ty = threadIdx.y;
   for (int r = ty; r < 32; r += 8) {
     const int ya = bi * 32 + r, xa = bj * 32 + tx;            // tile A = (rows of bi, columns of bj)
@@ -183,6 +186,7 @@ __global__ void fill_i32_kernel(int* p, int v, size_t n) {
 #define WIND_STEP 0      // one frame of wind: acc += delta, counts = whole pixels
 #define WIND_INIT 1      // accumulators <- the layer's common ones (ax0, ay0), no extrusion
 #define WIND_RESET 2     // accumulators <- 0; counts of the start-up: 2N along y, signed like the environment's x wind
+#define WIND_RESET_ENVS 3  // WIND_RESET of the listed environments envs[0..K) only (aom_reset_envs); the others keep their state
 struct WindLayerParams {
   const float* dx; const float* dy;      // [E] steps in pixels per frame, or null: the common cdx / cdy
   float cdx, cdy;
@@ -194,12 +198,16 @@ struct WindStateParams {
   WindLayerParams layer[AOM_MAX_LAYERS];
   double* acc; int* steps; WindRec* rec;
   int E, n_layers, mode;
+  const int* envs; int K;                // WIND_RESET_ENVS
 };
 
+// grid: one thread per (layer, environment), or per (layer, listed environment) with WIND_RESET_ENVS.
 __global__ void wind_state_kernel(const __grid_constant__ WindStateParams P) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= P.n_layers * P.E) return;
-  const int l = i / P.E, e = i - l * P.E;
+  const int n = P.mode == WIND_RESET_ENVS ? P.K : P.E;
+  if (i >= P.n_layers * n) return;
+  const int l = i / n, k = i - l * n;
+  const int e = P.mode == WIND_RESET_ENVS ? P.envs[k] : k;
   const WindLayerParams& L = P.layer[l];
   const float dx = L.dx ? L.dx[e] : L.cdx, dy = L.dy ? L.dy[e] : L.cdy;
   double* ax = P.acc + (size_t)2 * l * P.E + e;

@@ -63,6 +63,7 @@ struct OzGatherParams {
   const float* amp_env;     // [E] per-environment amplitude, or null
   const int* steps;         // per-environment winds: signed counts of this axis [E] (see ExtrudeParams), or null
   int pass;
+  const int* envs;          // compacted start-up: digit row k (and zref / ev [k]) belongs to environment envs[k], or null
 };
 
 struct OzGemmParams {
@@ -131,7 +132,8 @@ __device__ __forceinline__ void oz_logical(int r, int c, int N, int axis, int si
 }
 __device__ __forceinline__ int oz_wrap(int v, int N) { return v >= N ? v - N : v; }
 
-// grid: E blocks of 256 threads; dynamic shared memory: KB * 32 doubles.
+// grid: E blocks of 256 threads (K with p.envs: block k serves environment envs[k] and writes row k); dynamic shared
+// memory: KB * 32 doubles.
 // Gathers the stencil pixels (minus the reference pixel) and the scaled innovations of one environment, finds the row
 // scale, cuts the row into digit planes and stores them in the tile layout the tensor core reads.
 // PE: per-environment winds -- environment e takes part in pass p.pass of the axis iff p.pass < |steps[e]|, in the
@@ -140,7 +142,7 @@ template <bool PE = false>
 __global__ void __launch_bounds__(256) oz_gather_slice_kernel(OzGatherParams p) {
   extern __shared__ double oz_v[];
   __shared__ double s_red[8];
-  const int e = blockIdx.x, N = p.N, Kp = p.KB * OZ_BK;
+  const int row = blockIdx.x, e = p.envs ? p.envs[row] : row, N = p.N, Kp = p.KB * OZ_BK;
   int sign = p.sign;
   if (PE) {
     const int n = p.steps[e];
@@ -188,9 +190,9 @@ __global__ void __launch_bounds__(256) oz_gather_slice_kernel(OzGatherParams p) 
 #pragma unroll
   for (int i = 1; i < 8; ++i) amax = fmax(amax, s_red[i]);
   const int ex = oz_exponent(amax);
-  if (threadIdx.x == 0) { p.zref[e] = zr; p.ev[e] = ex; }
+  if (threadIdx.x == 0) { p.zref[row] = zr; p.ev[row] = ex; }
   const double scale = __longlong_as_double((long long)(1023 - ex) << 52);      // 2^-ex
-  const int mt = e >> 7, r = e & 127;
+  const int mt = row >> 7, r = row & 127;
   // eight values per thread and pass: the 1984 values of a 648-pixel layer keep 248 of the 256 threads busy in one pass
   for (int j = threadIdx.x; j < Kp / 8; j += blockDim.x) {
     uint32_t w[OZ_SLICES][2];

@@ -479,9 +479,15 @@ __host__ __device__ inline double psw_core_peak(const double (&I)[3][3]) {
 
 // Strehl figures from the MODE 2 sums: SE = fitted peak of this frame's core, LE = fitted peak of the accumulated core
 // (the reference takes the maximum of the long-exposure image, not the mean of the short-exposure maxima).
-__global__ void target_strehl_core_kernel(const double* mom, float* strehl, float* acc, int E, int n_le) {
+// le_n / first: per-environment counts of staggered environments, as target_strehl_kernel.
+__global__ void target_strehl_core_kernel(const double* mom, float* strehl, float* acc, int E, int n_le, int* le_n,
+                                          const int* first) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= E) return;
+  if (le_n) {
+    if (first[e]) return;
+    n_le = n_le > 0 ? ++le_n[e] : 0;
+  }
   const double* m = mom + (size_t)e * PSW_MOM2;
   const double s0 = m[0];
   double I[3][3];

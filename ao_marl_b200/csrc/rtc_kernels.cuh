@@ -19,11 +19,14 @@ __global__ void apply_control_kernel(const float* com, float* com1, float* volts
 
 // RlSupervisor.correction_modal_basis step 2 (rlSupervisor.py:799-813):
 // modes[action_map[i]] += (a[i] * act_scale + act_bias) * freedom[action_map[i]]
+// first [E] (or null): environments restarted by aom_reset_envs whose first step is pending take no action.
 __global__ void inject_action_kernel(float* modes, int ldm, const float* action, int lda, const int* action_map,
-                                     const float* freedom, int action_dim, int E, float act_scale, float act_bias) {
+                                     const float* freedom, int action_dim, int E, float act_scale, float act_bias,
+                                     const int* first) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   int e = blockIdx.y;
   if (i >= action_dim || e >= E) return;
+  if (first && first[e]) return;
   int m = action_map[i];
   float a = action[(size_t)e * lda + i] * act_scale + act_bias;
   modes[(size_t)e * ldm + m] += a * freedom[m];
@@ -94,14 +97,18 @@ __global__ void __launch_bounds__(256) actor_gather_kernel(const float* __restri
 // GaussianPolicy.sample(only_choosing_action=True) + TrainerRPC.report_action
 // (model_rpc.py:131-144, train_rpc.py:667-675).  heads[a][e][0:out] = mean, [out:2 out] = log std.
 // grid: E blocks of 256 threads, every block loops over (agent, output).
+// step_env [E] (or null: `step` for every environment): each environment's own decision counter, advanced here except
+// for an environment whose first step after aom_reset_envs is pending (first[e]): that step's action is not used.
 __global__ void __launch_bounds__(256) actor_sample_kernel(const float* __restrict__ heads, int ldh, int actor_out,
                                                            const int* __restrict__ act_slot, int E, int n_agents,
                                                            float log_sig_min, float log_sig_max, float act_scale,
                                                            float act_bias, int eval_mode, uint32_t step,
                                                            const uint32_t* k0, const uint32_t* k1, float* action,
-                                                           float* action_mean, int lda) {
+                                                           float* action_mean, int lda, uint32_t* step_env,
+                                                           const int* first) {
   const int e = blockIdx.x;
   const uint32_t key0 = k0[e], key1 = k1[e];
+  if (step_env) step = step_env[e];
   const int total = n_agents * actor_out;
   for (int t = threadIdx.x; t < total; t += blockDim.x) {
     const int a = t / actor_out, j = t - a * actor_out;
@@ -117,6 +124,10 @@ __global__ void __launch_bounds__(256) actor_sample_kernel(const float* __restri
     action[(size_t)e * lda + slot] = eval_mode ? mean : act;
     action_mean[(size_t)e * lda + slot] = mean;
   }
+  if (step_env) {
+    __syncthreads();                                  // every thread has read the counter
+    if (threadIdx.x == 0 && !first[e]) step_env[e] = step + 1;
+  }
 }
 
 __global__ void pixel_noise_kernel(const float* lam, float* out, long long n, float noise, uint32_t k0,
@@ -131,4 +142,57 @@ __global__ void copy_rows_kernel(const float* src, int lds_, float* dst, int ldd
   int e = blockIdx.y;
   if (i >= ldd || e >= E) return;
   dst[(size_t)e * ldd + i] = (i < n) ? src[(size_t)e * lds_ + i] : 0.f;
+}
+
+// ---------------------------------------------------------------------------------------------
+// aom_reset_envs: restart listed environments while the others run on.
+#define RESET_MAX_BUFS (17 + 4 * AOM_MAX_LAYERS)    // controller, state and Strehl rows + screen and ring state per layer
+struct ResetEnvsParams {
+  // per-environment buffers whose rows are zeroed: word (s * slot_stride + e * ld + i), s < slots, i < ld
+  uint32_t* buf[RESET_MAX_BUFS];
+  long long ld[RESET_MAX_BUFS], slot_stride[RESET_MAX_BUFS];
+  int slots[RESET_MAX_BUFS];
+  int nbuf;
+  const int* envs;              // [K] environments to restart
+  const uint32_t* seeds;        // [2][K] low, high words of their new seeds
+  int K, E;
+  uint32_t *k0, *k1;            // [E] Philox keys
+  uint32_t* frame0;             // [E] noise frame of the environment's first sensor frame
+  uint32_t* step_env;           // [E] actor decision counters
+  int* le_n;                    // [2][E] long-exposure counts (main target, geometric target)
+  int* first;                   // [E] first step pending
+  uint32_t frame;
+};
+
+// grid (K, nbuf + 1): block (k, b < nbuf) zeroes the rows of buffer b of environment envs[k]; block (k, nbuf) sets its
+// keys and counters.
+__global__ void __launch_bounds__(256) reset_envs_kernel(const __grid_constant__ ResetEnvsParams P) {
+  const int k = blockIdx.x, b = blockIdx.y, e = P.envs[k];
+  if (b < P.nbuf) {
+    uint32_t* base = P.buf[b] + (size_t)e * P.ld[b];
+    for (int s = 0; s < P.slots[b]; ++s)
+      for (long long i = threadIdx.x; i < P.ld[b]; i += blockDim.x) base[s * P.slot_stride[b] + i] = 0u;
+    return;
+  }
+  if (threadIdx.x == 0) {
+    P.k0[e] = P.seeds[k];
+    P.k1[e] = P.seeds[P.K + k];
+    P.frame0[e] = P.frame;
+    P.step_env[e] = 0u;
+    P.le_n[e] = 0;
+    P.le_n[P.E + e] = 0;
+    P.first[e] = 1;
+  }
+}
+
+// The per-environment counters when the batch stops running in lockstep: every environment at the batch's counts.
+__global__ void stagger_counters_kernel(uint32_t* frame0, uint32_t* step_env, int* le_n, int* first, int E, uint32_t step,
+                                        int n_main, int n_geo) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= E) return;
+  frame0[e] = 0u;
+  step_env[e] = step;
+  le_n[e] = n_main;
+  le_n[E + e] = n_geo;
+  first[e] = 0;
 }

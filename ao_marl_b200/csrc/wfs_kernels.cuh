@@ -217,13 +217,13 @@ __global__ void __launch_bounds__(WFS_WARPS * 32, 2) wfs_frame_kernel(WfsParams 
 #pragma unroll
     for (int sft = 16; sft > 0; sft >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, sft);
     const float scale = p.nphotons * p.flux[k] / tot;
-    const uint32_t k0 = p.k0[e], k1 = p.k1[e];
+    const uint32_t k0 = p.k0[e], k1 = p.k1[e], fr = noise_frame(p, e);
     float s0 = 0.f, sy = 0.f;
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const int pidx = lane + 32 * j;
       float v = px[j] * scale;
-      v = aom_pixel_noise(v, p.noise, (uint32_t)(k * 256 + pidx), p.frame, p.wfs_index, k0, k1);
+      v = aom_pixel_noise(v, p.noise, (uint32_t)(k * 256 + pidx), fr, p.wfs_index, k0, k1);
       px[j] = v;
       s0 += v;
       sy += v * (float)(pidx >> 4);
@@ -392,9 +392,16 @@ __global__ void target_moments_kernel(WfsParams p, double* mom, float k2t, int s
 // and stays meaningful in open loop where that underflows.  The long-exposure PSF is the mean of the short ones, so
 // its peak is the running mean.  acc [E][2] running sums of SE and var, n_le the number of accumulated frames
 // including this one (0: no accumulation).
-__global__ void target_strehl_kernel(const double* mom, int stride, float* strehl, float* acc, int E, int n_le) {
+// le_n [E] (or null): per-environment counts once environments are staggered (aom_reset_envs), advanced here when n_le > 0;
+// an environment whose first step is pending (first[e]) is left untouched.
+__global__ void target_strehl_kernel(const double* mom, int stride, float* strehl, float* acc, int E, int n_le, int* le_n,
+                                     const int* first) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= E) return;
+  if (le_n) {
+    if (first[e]) return;
+    n_le = n_le > 0 ? ++le_n[e] : 0;
+  }
   const double* m = mom + (size_t)e * stride;
   const double s0 = m[0], s1 = m[1], s2 = m[2], sc = m[3], ss = m[4];
   float var = 0.f, se = 1.f;

@@ -33,6 +33,7 @@ struct WfsParams {
   float cog_offset, pixsize;
   uint32_t frame, wfs_index;
   const uint32_t* k0; const uint32_t* k1;
+  const uint32_t* frame0;              // [E] or null: environment e's noise frame is frame - frame0[e] (aom_reset_envs)
   // outputs
   float* slopes; int lds;              // [E][lds]: x slopes then y slopes
   float* bincube;                      // [E][nvalid][256] or null
@@ -49,5 +50,10 @@ __device__ __forceinline__ WindRec wind_of(const WfsParams& p, int l, int e) {
   WindRec r;
   r.ix = L.ix; r.iy = L.iy; r.fx = L.fx; r.fy = L.fy; r.w00 = L.w00; r.w01 = L.w01; r.w10 = L.w10; r.w11 = L.w11;
   return r;
+}
+
+// noise frame of environment e: its frames count from its own reset once environments are staggered
+__device__ __forceinline__ uint32_t noise_frame(const WfsParams& p, int e) {
+  return p.frame0 ? p.frame - p.frame0[e] : p.frame;
 }
 

@@ -584,14 +584,14 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
 #pragma unroll
       for (int sft = 16; sft > 0; sft >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, sft);
       const float scale = p.nphotons * p.flux[ik] / tot;
-      const uint32_t k0 = p.k0[ie], k1 = p.k1[ie];
+      const uint32_t k0 = p.k0[ie], k1 = p.k1[ie], fr = noise_frame(p, ie);
       float* cube = p.bincube ? p.bincube + ((size_t)ie * p.nvalid + ik) * 256 : nullptr;
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         const int py = py0 + j;
         const int pidx = py * 16 + px;
         float v = mine[j] * scale;
-        v = aom_pixel_noise(v, p.noise, (uint32_t)(ik * 256 + pidx), p.frame, p.wfs_index, k0, k1);
+        v = aom_pixel_noise(v, p.noise, (uint32_t)(ik * 256 + pidx), fr, p.wfs_index, k0, k1);
         if (cube) cube[pidx] = v;
         s0 += v;
         sx = fmaf(v, (float)px, sx);

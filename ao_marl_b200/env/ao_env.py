@@ -69,6 +69,12 @@ class AoEnv:
             return None
         return self.linear_step(return_dict, geometric_do_control, geometric_apply_control)
 
+    def reset_envs(self, envs, seeds):
+        """Autoreset of the environments `envs` with `seeds` (RlSupervisor.reset_envs): their next rl_step is ignored
+        (reward 0) and their next linear_step returns their s0, while every other environment runs on.  Set the new
+        episode's conditions (set_r0 / set_wind with [E] arrays) before the call."""
+        self.supervisor.reset_envs(envs, seeds)
+
     def state(self):
         return self.sim.rows("STATE", self.state_size)
 

@@ -115,6 +115,17 @@ class StepLearner:
         self.stream = torch.cuda.Stream()
         self.E = sim.n_env
         self._s = sim.rows("STATE", rl.state_dim).clone()
+        # env-steps so far, and per environment the step that returned its s0 (0: the state at construction); a
+        # transition of environment e is pushed only when the whole window lies after that step
+        self._t = 0
+        self._first = np.zeros(self.E, dtype=np.int64)
+
+    def reset_envs(self, envs, seeds):
+        """Autoreset of the environments `envs` with `seeds` (Simulator.reset_envs): their next step returns their s0, and
+        from then on they push exactly what a StepLearner started after a full reset and linear step pushes.  No
+        transition spans two episodes.  Set the new episode's conditions before the call."""
+        self.sim.reset_envs(envs, seeds)
+        self._first[np.asarray(envs, dtype=np.int64)] = self._t + 1
 
     def states_per_agent(self, state):
         return state[:, self._idx].permute(1, 0, 2) * self._idx_ok[:, None, :]
@@ -134,6 +145,7 @@ class StepLearner:
             with torch.cuda.stream(self.stream):
                 L.update()
         sim.step(mode=0)
+        self._t += 1
         a = sim.rows("ACTION", rl.action_dim).clone()
         r = sim.buffer("REWARD").view(self.E, rl.n_agents).clone()
         s_next = sim.rows("STATE", rl.state_dim).clone()
@@ -143,7 +155,12 @@ class StepLearner:
             main.wait_stream(self.stream)          # the replay is written below; the new actors are uploaded by the caller
         if self.mdp.check_update_possibility():
             s0, a0, s2 = self.mdp.credit_assignment()
-            L.memory.push(self.states_per_agent(s0), self.actions_per_agent(a0), r.t().contiguous(),
-                          self.states_per_agent(s2), torch.ones_like(r.t()))
+            ok = self._first <= self._t - self.mdp.depth - 1        # the oldest state of the window is the episode's
+            if not ok.all():
+                i = torch.as_tensor(np.flatnonzero(ok), device=r.device)
+                s0, a0, s2, r = s0[i], a0[i], s2[i], r[i]
+            if ok.any():
+                L.memory.push(self.states_per_agent(s0), self.actions_per_agent(a0), r.t().contiguous(),
+                              self.states_per_agent(s2), torch.ones_like(r.t()))
         self.mdp.save(self._s, a, s_next)
         self._s = s_next

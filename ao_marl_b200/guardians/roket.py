@@ -54,6 +54,10 @@ class Roket(RlSupervisor):
             raise ValueError("ROKET needs the geometric controller of the parameter file (p_controllers[1].type == 'geo')")
         self.iter_number = 0
 
+    def reset_envs(self, envs, seeds):
+        """Not available: the error-breakdown buffers ([N_total, E, .]) hold one run of the whole batch."""
+        raise NotImplementedError("ROKET's breakdown buffers are whole-batch: use reset()")
+
     # -- buffers ----------------------------------------------------------------------------------------------------------
     def init_config_roket(self, N_total=3000, N_preloop=1000, agent=None, nfiltered=None, gamma=1.0, include_tip_tilt=True,
                           n_zernike_start=None, n_zernike_end=None):

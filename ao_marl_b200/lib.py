@@ -44,14 +44,15 @@ TABLES = ["AB", "STENCIL", "MPUPIL", "HALFXY", "SUB_X0", "SUB_Y0", "FLUX", "STAM
           "ACTOR_W2", "ACTOR_B2", "ACTOR_WH", "ACTOR_BH", "GEO_PROJ", "GEO_SIFN", "DENOISER", "DENOISER_TC"]
 T = {name: i for i, name in enumerate(TABLES)}
 BUFFERS = ["SCREEN", "RING_OX", "RING_OY", "SLOPES", "ERR", "COM", "VOLTS", "BINCUBE", "PHASE", "MODES",
-           "RES_MODES", "STATE", "REWARD", "ACTION", "ACTION_MEAN", "STREHL", "GEO_COM", "GEO_VOLTS", "STREHL_GEO", "GEO_PROJ"]
+           "RES_MODES", "STATE", "REWARD", "ACTION", "ACTION_MEAN", "STREHL", "GEO_COM", "GEO_VOLTS", "STREHL_GEO", "GEO_PROJ",
+           "EXT_COUNT"]
 B = {name: i for i, name in enumerate(BUFFERS)}
-_INT_BUFFERS = {"RING_OX", "RING_OY"}
+_INT_BUFFERS = {"RING_OX", "RING_OY", "EXT_COUNT"}
 OPTIONS = ["WFS_PATH", "GEMM_PATH", "TIME_WFS", "GEO", "DENOISE", "PUPIL_PATH", "KEEP_IMAGE", "STREHL", "STREHL_LAMBDA_NM", "EXTRUDE_PATH", "STREHL_PEAK", "PSF_NFFT", "DENOISE_PATH"]
 O = {name: i for i, name in enumerate(OPTIONS)}
 
 EXPORTS = ["aom_config_size", "aom_create", "aom_destroy", "aom_last_error", "aom_set_table", "aom_get_buffer",
-           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
+           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_reset_envs", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
            "aom_comp_strehl", "aom_reset_strehl", "aom_do_control_geo", "aom_apply_control_geo", "aom_denoise", "aom_set_bincube", "aom_do_centroids", "aom_do_centroids_geom", "aom_do_control", "aom_set_command", "aom_apply_control",
            "aom_set_gain", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
            "aom_state_begin", "aom_state_end", "aom_reward", "aom_actor_forward", "aom_step", "aom_gemm_tn",
@@ -87,6 +88,7 @@ def load_library():
     lib.aom_set_option.argtypes = [vp, i32, i32]
     lib.aom_check_device.argtypes = [vp]
     lib.aom_reset.argtypes = [vp, vp, vp]
+    lib.aom_reset_envs.argtypes = [vp, i32, vp, vp, vp]
     lib.aom_move_atmos.argtypes = [vp, vp]
     lib.aom_set_layer.argtypes = [vp, i32, f32, f32, f32]
     lib.aom_set_layer_amp.argtypes = [vp, i32, vp]
@@ -373,6 +375,25 @@ class Simulator:
     def reset(self, seeds):
         seeds = np.ascontiguousarray(np.broadcast_to(np.asarray(seeds, dtype=np.int64), (self.n_env,)))
         self._check(self.lib.aom_reset(self._ctx, seeds.ctypes.data_as(ctypes.c_void_p), self.stream), "aom_reset")
+
+    def reset_envs(self, envs, seeds):
+        """Restart the environments `envs` (distinct indices, int [n]) with `seeds` (int [n]) while the others run on
+        (aom_reset_envs).  Their next step acts as the linear step after a reset: its rl half-step is ignored, its reward
+        is 0 and the state it leaves is their s0.  Set the new episode's conditions first (set_layer_amp / set_layer_wind
+        with [E] arrays): the start-up of the screens already uses them."""
+        envs, seeds = np.asarray(envs), np.asarray(seeds)
+        if envs.ndim != 1 or seeds.shape != envs.shape:
+            raise ValueError("reset_envs: envs and seeds must be 1-D arrays of the same length")
+        if envs.size and (envs.dtype.kind not in "iu" or seeds.dtype.kind not in "iu"):
+            raise TypeError("reset_envs: envs and seeds must be integer arrays")
+        if envs.size and (envs.min() < 0 or envs.max() >= self.n_env):
+            raise ValueError("reset_envs: environment index out of range [0, %d)" % self.n_env)
+        if np.unique(envs).size != envs.size:
+            raise ValueError("reset_envs: duplicate environment index")
+        envs = np.ascontiguousarray(envs, dtype=np.int32)
+        seeds = np.ascontiguousarray(seeds, dtype=np.int64)
+        self._check(self.lib.aom_reset_envs(self._ctx, int(envs.size), envs.ctypes.data_as(ctypes.c_void_p),
+                                            seeds.ctypes.data_as(ctypes.c_void_p), self.stream), "aom_reset_envs")
 
     def move_atmos(self):
         self._check(self.lib.aom_move_atmos(self._ctx, self.stream), "aom_move_atmos")

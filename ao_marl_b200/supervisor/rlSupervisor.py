@@ -121,6 +121,13 @@ class RlSupervisor:
             self.target.reset_strehl(tar_index)
         self.rtc.close_loop()
 
+    def reset_envs(self, envs, seeds):
+        """Restart the environments `envs` with `seeds` while the others run on (aom_reset_envs): everything reset() does,
+        for those environments only.  Their next next_part_two is ignored (no action, no Strehl) and their next
+        next_part_one + state leave their s0.  Conditions of the new episode (atmos.set_r0 / set_wind with [E] arrays)
+        must be set before the call, so that the start-up of their screens uses them."""
+        self.sim.reset_envs(envs, seeds)
+
     def get_m_pupil(self):
         return self.config.p_geom._mpupil
 

@@ -147,6 +147,7 @@ typedef enum aom_buffer {
   AOM_B_GEO_VOLTS,     /* float [E][ld(nactu)]     voltages on the mirrors it drives      */
   AOM_B_STREHL_GEO,    /* float [E][4]  as AOM_B_STREHL, for the target behind those mirrors */
   AOM_B_GEO_PROJ,      /* float [E][ld(nactu)]     IF (phi - <phi>): the phase projected on the influence functions */
+  AOM_B_EXT_COUNT,     /* uint32 [E] extrusions since the environment's reset (its screen RNG counter), index = layer */
   AOM_B_COUNT
 } aom_buffer;
 
@@ -227,6 +228,25 @@ int aom_check_device(aom_ctx* ctx);
 /* RlSupervisor.reset (rlSupervisor.py:236-246): reseed + regenerate turbulence (2N extrusions per layer),
  * clear mirrors / integrator / delay line / histories.  seeds: host int64 [E]. */
 int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream);
+
+/* Per-environment reset (the "autoreset" of vectorised environments): restart environments envs[0..n) (host int32,
+ * distinct, 0 <= e < E) with seeds[0..n) (host int64) while the others run on.
+ * - Each listed environment gets at once what aom_reset gives it: screens regenerated from its new seed (2N start-up
+ *   extrusions per layer with its current amplitude and the sign of its current x wind, common or per-environment), ring
+ *   origins, extrusion counters and wind accumulators at 0, and its rows of slopes, err, com, com1, volts, com_before,
+ *   residual modes, every history slot, state, Strehl accumulators / figures and geometric controller buffers cleared.
+ *   Set the new episode's conditions (aom_set_layer_amp / aom_set_layer_wind) before the call.
+ * - Its next aom_step acts as the linear step that follows an aom_reset: its rl half-step is ignored (no action is
+ *   injected, com stays 0, no Strehl is accumulated, reward 0) and the state it leaves is the s0 of a fresh episode
+ *   (Gymnasium's next-step autoreset).  Called half-step by half-step: aom_rl_control skips the injection,
+ *   aom_comp_strehl skips the environment and aom_state_end ends the status.
+ * - Noise frames, actor decisions (exploration noise) and long-exposure counts of each environment count from its own
+ *   reset.  From the call on, a listed environment computes bit for bit what it computes in a batch that was aom_reset
+ *   with its new seed and given one linear step; every other environment computes what it would have without the call.
+ * - AOM_ERR_INVALID: n < 0, an index out of range or listed twice.  AOM_ERR_STATE: no aom_reset yet.  n = 0: nothing.
+ *   The round-1 sensor kernels (tensor_reg / tensor / tensor_fast) return AOM_ERR_UNSUPPORTED while environments are
+ *   staggered, until the next aom_reset.  Waits for `stream`; cost about that of aom_reset for n = E, less for fewer. */
+int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const int64_t* seeds, void* stream);
 
 /* AtmosCompass.move_atmos (atmosCompass.py:158-161) */
 int aom_move_atmos(aom_ctx* ctx, void* stream);
