@@ -94,6 +94,12 @@ struct aom_ctx {
   float gain;
   int closed;
   uint32_t frame;
+  // sensor noise / photon count / integrator gain: common values (aom_set_wfs_noise, aom_set_gain) and optional
+  // per-environment ones (aom_set_wfs_noise_env, aom_set_gain_env): device [E] arrays while in force, else null, with
+  // host copies that route the frames without a device read
+  float noise_c, nph_c;
+  float *noise_env, *nph_env, *gain_env;
+  float *noise_henv, *nph_henv, *gain_henv;
   int opt[AOM_OPT_COUNT];
   long long* dn_dbg;
   float dn_prm[DT_NPARAM];    // float parameters of the tensor-core denoiser (head of AOM_T_DENOISER_TC)
@@ -198,6 +204,8 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   memset(ctx, 0, sizeof(aom_ctx));
   ctx->cfg = *cfg;
   ctx->gain = cfg->gain;
+  ctx->noise_c = cfg->noise;
+  ctx->nph_c = cfg->nphotons;
   ctx->closed = 1;
   ctx->opt[AOM_OPT_WFS_PATH] = AOM_WFS_UMMA_WS;
   {
@@ -281,10 +289,16 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   CU(cudaFuncSetAttribute(gemm_tc_kernel<1, GTC_BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES));
   CU(cudaFuncSetAttribute(gemm_tc_kernel<0, GTC_BN_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES_T(GTC_BN_WIDE)));
   CU(cudaFuncSetAttribute(gemm_tc_kernel<1, GTC_BN_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES_T(GTC_BN_WIDE)));
+  CU(cudaFuncSetAttribute(gemm_tc_kernel<2, GTC_BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES));
+  CU(cudaFuncSetAttribute(gemm_tc_kernel<2, GTC_BN_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES_T(GTC_BN_WIDE)));
   CU(cudaFuncSetAttribute(wfs_frame_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
   CU(cudaFuncSetAttribute(wfs_frame_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
   CU(cudaFuncSetAttribute(wfs_frame_kernel<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
   CU(cudaFuncSetAttribute(wfs_frame_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
+  CU(cudaFuncSetAttribute(wfs_frame_kernel<4, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
+  CU(cudaFuncSetAttribute(wfs_frame_kernel<8, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
+  CU(cudaFuncSetAttribute(wfs_frame_kernel<4, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
+  CU(cudaFuncSetAttribute(wfs_frame_kernel<8, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
   return AOM_OK;
 }
 
@@ -298,6 +312,8 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
     cudaFree(ctx->wind_dx[l]); cudaFree(ctx->wind_dy[l]); free(ctx->wind_hdx[l]); free(ctx->wind_hdy[l]);
   }
   cudaFree(ctx->wind_acc); cudaFree(ctx->wind_steps); cudaFree(ctx->wind_rec); free(ctx->wind_hacc);
+  cudaFree(ctx->noise_env); cudaFree(ctx->nph_env); cudaFree(ctx->gain_env);
+  free(ctx->noise_henv); free(ctx->nph_henv); free(ctx->gain_henv);
   void* bufs[] = {ctx->k0, ctx->k1, ctx->Z, ctx->zref, ctx->newcol, ctx->slopes_frame, ctx->slopes, ctx->err_v,
                   ctx->com, ctx->com1, ctx->volts, ctx->com_before, ctx->bincube, ctx->phase, ctx->modes,
                   ctx->modes_before, ctx->modes_res, ctx->state, ctx->hist, ctx->reward, ctx->action,
@@ -611,6 +627,7 @@ static int launch_gemm(aom_ctx* ctx, int epi, const float* A, int lda, long long
   p.sA = sA; p.sB = sB; p.sC = sC; p.sBias = sBias; p.relu = relu;
   p.com = com; p.ldcom = ldcom; p.gain = ctx->gain; p.closed = ctx->closed;
   p.Bt = Bt; p.sBt = sBt;
+  if (epi == 1 && ctx->gain_env) { epi = 2; p.gain_env = ctx->gain_env; }   // integrator with one gain per environment
   // `exact`: float32 FFMA accumulation with round-to-nearest (the recursive screen extrusion needs it: the
   // tensor core truncates its float32 accumulator, a ~1e-5 systematic shrink that an autoregression integrates)
   if (!exact && ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT) {
@@ -620,11 +637,13 @@ static int launch_gemm(aom_ctx* ctx, int epi, const float* A, int lda, long long
     if (!Bt && waves(GTC_BN_WIDE) < waves(GTC_BN)) {
       dim3 grid((ldc + GTC_BN_WIDE - 1) / GTC_BN_WIDE, (unsigned)rows, batch);
       if (epi == 0) gemm_tc_kernel<0, GTC_BN_WIDE><<<grid, GTC_THREADS, GTC_SMEM_BYTES_T(GTC_BN_WIDE), st>>>(p, ctx->d_err);
-      else gemm_tc_kernel<1, GTC_BN_WIDE><<<grid, GTC_THREADS, GTC_SMEM_BYTES_T(GTC_BN_WIDE), st>>>(p, ctx->d_err);
+      else if (epi == 1) gemm_tc_kernel<1, GTC_BN_WIDE><<<grid, GTC_THREADS, GTC_SMEM_BYTES_T(GTC_BN_WIDE), st>>>(p, ctx->d_err);
+      else gemm_tc_kernel<2, GTC_BN_WIDE><<<grid, GTC_THREADS, GTC_SMEM_BYTES_T(GTC_BN_WIDE), st>>>(p, ctx->d_err);
     } else {
       dim3 grid((ldc + GTC_BN - 1) / GTC_BN, (unsigned)rows, batch);
       if (epi == 0) gemm_tc_kernel<0, GTC_BN><<<grid, GTC_THREADS, GTC_SMEM_BYTES, st>>>(p, ctx->d_err);
-      else gemm_tc_kernel<1, GTC_BN><<<grid, GTC_THREADS, GTC_SMEM_BYTES, st>>>(p, ctx->d_err);
+      else if (epi == 1) gemm_tc_kernel<1, GTC_BN><<<grid, GTC_THREADS, GTC_SMEM_BYTES, st>>>(p, ctx->d_err);
+      else gemm_tc_kernel<2, GTC_BN><<<grid, GTC_THREADS, GTC_SMEM_BYTES, st>>>(p, ctx->d_err);
     }
   } else if (exact && epi == 0 && batch == 1 && !bias && !relu && ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT) {
     // shaped exact kernel: column tile 8 CN with the least padding.  Only columns < N are consumed by the
@@ -648,7 +667,8 @@ static int launch_gemm(aom_ctx* ctx, int epi, const float* A, int lda, long long
   } else {
     dim3 grid((ldc + GEMM_BN - 1) / GEMM_BN, (M + GEMM_BM - 1) / GEMM_BM, batch);
     if (epi == 0) gemm_tn_kernel<0><<<grid, 256, 0, st>>>(p);
-    else gemm_tn_kernel<1><<<grid, 256, 0, st>>>(p);
+    else if (epi == 1) gemm_tn_kernel<1><<<grid, 256, 0, st>>>(p);
+    else gemm_tn_kernel<2><<<grid, 256, 0, st>>>(p);
   }
   KCHECK();
   return AOM_OK;
@@ -674,6 +694,7 @@ static int launch_oz_product(aom_ctx* ctx, int op, const float* X, int ldx, int 
   memset(&m, 0, sizeof(m));
   m.Zs = ctx->oz_xs; m.ABs = ctx->ozop[op]; m.ev = ctx->oz_xev; m.ea = ctx->ozop_ea[op]; m.out = out; m.ldo = ldo;
   m.E = c.n_env; m.N = N; m.KB = KB; m.com = com; m.ldcom = ldcom; m.gain = ctx->gain; m.closed = ctx->closed; m.err = ctx->d_err;
+  m.gain_env = integrator ? ctx->gain_env : nullptr;
   cudaError_t le = oz_product_launch(sl, m, integrator, MT, NT, st);
   if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "oz_product_launch: %s", cudaGetErrorString(le));
   ctx->launches += 2;
@@ -1521,7 +1542,11 @@ static int fill_wfs_params(aom_ctx* ctx, WfsParams& p, int flags, float noise) {
   p.pzt_off = c.pzt_off; p.pzt_nact = c.pzt_nact;
   p.tt_planes = (const float*)ctx->tab[AOM_T_TT_PLANES][0]; p.tt_dim = c.tt_dim; p.tt_off = c.tt_off;
   p.k2 = (float)(2.0 * M_PI / (double)c.lambda_um);
-  p.nphotons = c.nphotons; p.noise = noise; p.cog_offset = c.cog_offset; p.pixsize = c.pixsize;
+  p.nphotons = ctx->nph_c; p.noise = noise; p.cog_offset = c.cog_offset; p.pixsize = c.pixsize;
+  // per-environment sensor values: every frame is scaled by each environment's photon count, a noisy frame (noise >= 0)
+  // draws each environment's own noise, a noise-free one none
+  p.nph_env = ctx->nph_env;
+  p.noise_env = (noise >= 0.f) ? ctx->noise_env : nullptr;
   p.frame = ctx->frame; p.wfs_index = (uint32_t)c.wfs_index; p.k0 = ctx->k0; p.k1 = ctx->k1;
   p.frame0 = ctx->staggered ? ctx->frame0 : nullptr;
   p.slopes = ctx->slopes_frame; p.lds = ctx->lds;
@@ -1558,8 +1583,18 @@ extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* st
     rc = umma ? wfs_umma_prepare(ctx) : wfs_fast_prepare(ctx);
     if (rc) return rc;
   }
+  // does any environment draw noise in this frame?  (host copies: no device read)
+  bool noisy = p.noise >= 0.f;
+  if (p.noise_env) {
+    noisy = false;
+    for (int e = 0; e < c.n_env && !noisy; ++e) noisy = ctx->noise_henv[e] >= 0.f;
+  }
   if (c.nfft == 64 && umma && ctx->umma_state == 1) {
-    cudaError_t le = wfs_umma_launch(p, ctx->umma, ctx->num_sms, !fast, path == AOM_WFS_UMMA_WS && p.noise < 0.f && p.bincube == nullptr, st);
+    // the specialised-warp kernel serves every frame without noise and kept image (it reads neither noise nor photon
+    // count); the others go to the fused kernel, in its per-environment form when per-environment values are in force
+    const bool ws = path == AOM_WFS_UMMA_WS && !noisy && p.bincube == nullptr;
+    if (ws) { p.noise = -1.f; p.noise_env = nullptr; p.nph_env = nullptr; }
+    cudaError_t le = wfs_umma_launch(p, ctx->umma, ctx->num_sms, !fast, ws, st);
     if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "wfs_umma_launch: %s", cudaGetErrorString(le));
   }
   else if (c.nfft == 64 && path != AOM_WFS_SIMT && p.frame0)
@@ -1568,6 +1603,9 @@ extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* st
   else if (c.nfft == 64 && path != AOM_WFS_SIMT && p.wind)
     return fail(ctx, AOM_ERR_UNSUPPORTED, "per-environment wind is not implemented in the round-1 sensor kernels "
                 "(wfs_frame_tma_kernel, wfs_frame_mma_kernel): use the umma, umma_ws or simt path");
+  else if (c.nfft == 64 && path != AOM_WFS_SIMT && (p.noise_env || p.nph_env))
+    return fail(ctx, AOM_ERR_UNSUPPORTED, "per-environment sensor noise and photon counts are not implemented in the round-1 "
+                "sensor kernels (wfs_frame_tma_kernel, wfs_frame_mma_kernel): use the umma, umma_ws or simt path");
   else if (c.nfft == 64 && staged && ctx->fast_state == 1) {
     rc = wfs_fast_launch(ctx, p, !fast, st);
     if (rc) return rc;
@@ -1582,6 +1620,12 @@ extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* st
       default: if (full) WFM_LAUNCH(1, -1); else WFM_LAUNCH(0, -1); break;
     }
 #undef WFM_LAUNCH
+  }
+  else if (p.noise_env || p.nph_env) {      // per-environment sensor values
+    if (c.nfft == 64 && p.wind) wfs_frame_kernel<4, true, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
+    else if (c.nfft == 64) wfs_frame_kernel<4, false, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
+    else if (p.wind) wfs_frame_kernel<8, true, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<8>(), st>>>(p);
+    else wfs_frame_kernel<8, false, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<8>(), st>>>(p);
   }
   else if (c.nfft == 64 && p.wind) wfs_frame_kernel<4, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
   else if (c.nfft == 64) wfs_frame_kernel<4><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
@@ -1910,6 +1954,59 @@ extern "C" int aom_set_gain(aom_ctx* ctx, float gain) {
   return AOM_OK;
 }
 
+// Per-environment value array: NULL frees it (back to the common value); otherwise checks every entry (finite, and > 0
+// when `positive`), keeps a host copy and uploads it.  The caller has synchronised the device.
+static int set_env_values(aom_ctx* ctx, const float* host, float** dev, float** hcopy, bool positive, const char* what) {
+  const size_t E = ctx->cfg.n_env;
+  if (!host) {
+    cudaFree(*dev); free(*hcopy);
+    *dev = *hcopy = nullptr;
+    return AOM_OK;
+  }
+  for (size_t e = 0; e < E; ++e) {
+    if (!isfinite(host[e])) return fail(ctx, AOM_ERR_INVALID, "%s of environment %zu is not finite", what, e);
+    if (positive && !(host[e] > 0.f)) return fail(ctx, AOM_ERR_INVALID, "%s of environment %zu must be > 0", what, e);
+  }
+  if (!*hcopy) {
+    *hcopy = (float*)malloc(E * sizeof(float));
+    if (!*hcopy) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+    CU(cudaMalloc((void**)dev, E * sizeof(float)));
+  }
+  memcpy(*hcopy, host, E * sizeof(float));
+  CU(cudaMemcpy(*dev, host, E * sizeof(float), cudaMemcpyHostToDevice));
+  return AOM_OK;
+}
+
+extern "C" int aom_set_gain_env(aom_ctx* ctx, const float* gain_host) {
+  if (!ctx) return AOM_ERR_INVALID;
+  CU(cudaDeviceSynchronize());                       // an integrator in flight may still read the old gains
+  return set_env_values(ctx, gain_host, &ctx->gain_env, &ctx->gain_henv, false, "gain");
+}
+
+extern "C" int aom_set_wfs_noise(aom_ctx* ctx, float noise, float nphotons) {
+  if (!ctx) return AOM_ERR_INVALID;
+  if (!isfinite(noise) || !isfinite(nphotons)) return fail(ctx, AOM_ERR_INVALID, "sensor noise and photon count must be finite");
+  if (!(nphotons > 0.f)) return fail(ctx, AOM_ERR_INVALID, "photon count must be > 0");
+  ctx->noise_c = noise;
+  ctx->nph_c = nphotons;
+  return AOM_OK;
+}
+
+extern "C" int aom_set_wfs_noise_env(aom_ctx* ctx, const float* noise_host, const float* nphotons_host) {
+  if (!ctx) return AOM_ERR_INVALID;
+  const size_t E = ctx->cfg.n_env;
+  // check both before changing either: a refused call leaves the state as it was
+  for (size_t e = 0; noise_host && e < E; ++e)
+    if (!isfinite(noise_host[e])) return fail(ctx, AOM_ERR_INVALID, "sensor noise of environment %zu is not finite", e);
+  for (size_t e = 0; nphotons_host && e < E; ++e)
+    if (!isfinite(nphotons_host[e]) || !(nphotons_host[e] > 0.f))
+      return fail(ctx, AOM_ERR_INVALID, "photon count of environment %zu must be finite and > 0", e);
+  CU(cudaDeviceSynchronize());                       // a sensor frame in flight may still read the old values
+  int rc = set_env_values(ctx, noise_host, &ctx->noise_env, &ctx->noise_henv, false, "sensor noise");
+  if (rc) return rc;
+  return set_env_values(ctx, nphotons_host, &ctx->nph_env, &ctx->nph_henv, true, "photon count");
+}
+
 extern "C" int aom_set_loop(aom_ctx* ctx, int closed) {
   if (!ctx) return AOM_ERR_INVALID;
   ctx->closed = closed ? 1 : 0;
@@ -2103,7 +2200,8 @@ extern "C" int aom_step(aom_ctx* ctx, int mode, int eval_mode, void* stream) {
   }
   const bool denoise = ctx->opt[AOM_OPT_DENOISE] != 0;
   const bool keep = denoise || ctx->opt[AOM_OPT_KEEP_IMAGE] != 0;
-  rc = aom_comp_wfs_image(ctx, keep ? 7 : 3, ctx->cfg.noise, stream); if (rc) return rc;
+  // the common noise, or with per-environment noise in force any value >= 0: each environment's own
+  rc = aom_comp_wfs_image(ctx, keep ? 7 : 3, ctx->noise_env ? 0.f : ctx->noise_c, stream); if (rc) return rc;
   if (denoise) { rc = aom_denoise(ctx, nullptr, nullptr, 0, stream); if (rc) return rc; }
   rc = aom_do_centroids(ctx, stream); if (rc) return rc;
   rc = aom_do_control(ctx, stream); if (rc) return rc;

@@ -10,6 +10,7 @@ static cudaError_t oz_attrs() {
   cudaError_t e = cudaFuncSetAttribute(oz_gemm_kernel<0, OZ_LEVELS>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_SMEM_BYTES);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_kernel<1, OZ_LEVELS_PRODUCT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_SMEM_BYTES);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_kernel<2, OZ_LEVELS_PRODUCT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_SMEM_BYTES);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(oz_gemm_kernel<3, OZ_LEVELS_PRODUCT>, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_SMEM_BYTES);
   attr_set = e == cudaSuccess;
   return e;
 }
@@ -31,7 +32,8 @@ cudaError_t oz_product_launch(const OzSliceParams& sl, const OzGemmParams& m, in
   oz_slice_rows_kernel<<<sl.E, 256, 0, st>>>(sl);
   e = cudaGetLastError();
   if (e != cudaSuccess) return e;
-  if (integrator) oz_gemm_kernel<2, OZ_LEVELS_PRODUCT><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);
+  if (integrator && m.gain_env) oz_gemm_kernel<3, OZ_LEVELS_PRODUCT><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);
+  else if (integrator) oz_gemm_kernel<2, OZ_LEVELS_PRODUCT><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);
   else oz_gemm_kernel<1, OZ_LEVELS_PRODUCT><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);
   return cudaGetLastError();
 }

@@ -77,6 +77,7 @@ struct OzGemmParams {
   float* com; int ldcom;    // integrator epilogue: com += gain * out when closed
   float gain; int closed;
   int* err;
+  const float* gain_env;    // EPI 3: one gain per environment [E]
 };
 
 // digit planes of a per-environment float32 matrix X [E][ld] (K valid columns): the A operand of oz_gemm_kernel
@@ -331,6 +332,7 @@ __device__ __forceinline__ void oz_mma_i8(uint32_t d_tmem, uint64_t a_desc, uint
 //   warps 2-5  epilogue: TMEM lane quarter warp % 4 -> 32 environments, five int32 accumulators -> float64 -> float32
 // EPI 0: screen extrusion (+ zref, every column of the row written)   1: plain product (pad columns zero)
 // EPI 2: least-squares integrator: out = -product, com += gain * out when the loop is closed (rtcCompass.py:527-547)
+// EPI 3: the same with one gain per environment, com += gain_env[e] * out
 // LEV: digit-pair levels kept (pairs with s + t < LEV).  6 (21 MMAs per k block) for the screen recursion, which
 // integrates any truncation; OZ_LEVELS_PRODUCT = 5 (15 MMAs) for the one-shot controller products, where the dropped
 // pairs are below 2^-35 of |x|max |W|max per term.
@@ -409,6 +411,7 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) oz_gemm_kernel(OzGemmParams p) 
     const bool live = e < p.E;
     const int ev = live ? p.ev[e] : 0;
     const double zr = (EPI == 0 && live) ? (double)p.zref[e] : 0.0;
+    const float gn = (EPI == 3 && live) ? p.gain_env[e] : p.gain;     // integrator gain of this row's environment
 #pragma unroll 1
     for (int cb = 0; cb < OZ_BN / 8; ++cb) {
       uint32_t v[LEV][8];
@@ -434,7 +437,7 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) oz_gemm_kernel(OzGemmParams p) 
           if (EPI == 0) o[j] = (float)fma(acc, sc, zr);        // pad columns get zref: harmless, the scatter reads n < N
           else {
             const float r = (float)(acc * sc);
-            o[j] = (n < p.N) ? (EPI == 2 ? -r : r) : 0.f;       // pad columns stay zero
+            o[j] = (n < p.N) ? (EPI >= 2 ? -r : r) : 0.f;       // pad columns stay zero
           }
         }
         const int n0 = nt * OZ_BN + cb * 8;
@@ -442,11 +445,11 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) oz_gemm_kernel(OzGemmParams p) 
         if (n0 + 8 <= p.ldo) {
           *reinterpret_cast<float4*>(dst) = make_float4(o[0], o[1], o[2], o[3]);
           *reinterpret_cast<float4*>(dst + 4) = make_float4(o[4], o[5], o[6], o[7]);
-          if (EPI == 2 && p.closed) {
+          if (EPI >= 2 && p.closed) {
             float4* cp = reinterpret_cast<float4*>(p.com + (size_t)e * p.ldcom + n0);
             float4 c0 = cp[0], c1 = cp[1];
-            c0.x = fmaf(p.gain, o[0], c0.x); c0.y = fmaf(p.gain, o[1], c0.y); c0.z = fmaf(p.gain, o[2], c0.z); c0.w = fmaf(p.gain, o[3], c0.w);
-            c1.x = fmaf(p.gain, o[4], c1.x); c1.y = fmaf(p.gain, o[5], c1.y); c1.z = fmaf(p.gain, o[6], c1.z); c1.w = fmaf(p.gain, o[7], c1.w);
+            c0.x = fmaf(gn, o[0], c0.x); c0.y = fmaf(gn, o[1], c0.y); c0.z = fmaf(gn, o[2], c0.z); c0.w = fmaf(gn, o[3], c0.w);
+            c1.x = fmaf(gn, o[4], c1.x); c1.y = fmaf(gn, o[5], c1.y); c1.z = fmaf(gn, o[6], c1.z); c1.w = fmaf(gn, o[7], c1.w);
             cp[0] = c0; cp[1] = c1;
           }
         } else {
@@ -454,7 +457,7 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) oz_gemm_kernel(OzGemmParams p) 
           for (int j = 0; j < 8; ++j)
             if (n0 + j < p.ldo) {
               dst[j] = o[j];
-              if (EPI == 2 && p.closed) p.com[(size_t)e * p.ldcom + n0 + j] = fmaf(p.gain, o[j], p.com[(size_t)e * p.ldcom + n0 + j]);
+              if (EPI >= 2 && p.closed) p.com[(size_t)e * p.ldcom + n0 + j] = fmaf(gn, o[j], p.com[(size_t)e * p.ldcom + n0 + j]);
             }
         }
       }

@@ -7,7 +7,8 @@
 cudaError_t oz_extrude_launch(const OzGatherParams& g, const OzGemmParams& m, int MT, int NT, cudaStream_t st);
 
 // out = X . OP^T for a per-environment float32 matrix X and an operator given as digit planes (integrator != 0: the
-// least-squares integrator epilogue): row digits of X, then the digit-pair GEMM; both asynchronous on `st`
+// least-squares integrator epilogue, with one gain per environment when m.gain_env is set): row digits of X, then the
+// digit-pair GEMM; both asynchronous on `st`
 cudaError_t oz_product_launch(const OzSliceParams& sl, const OzGemmParams& m, int integrator, int MT, int NT, cudaStream_t st);
 
 // Host: cut the rows of the operator [rows][ld] (K valid columns) into digit planes in the tile layout of the kernel.

@@ -27,6 +27,8 @@ struct GemmParams {
   // gemm_tc_kernel only: the B operand already split into TF32 hi / lo planes in the UMMA tile order of 128-column tiles
   // ([n tile][k block][hi, lo][128 x 16]; gtc_pretile_host), brought in by one bulk copy per stage.  Null: B is split on the fly.
   const float* Bt; long long sBt;
+  // epilogue 2: the integrator of epilogue 1 with one gain per row (environment): com += gain_env[row] * err
+  const float* gain_env;
 };
 
 template <int EPI>
@@ -124,11 +126,12 @@ __global__ void __launch_bounds__(256, 2) gemm_tn_kernel(GemmParams p) {
         v[j] = (c < p.N) ? x : 0.f;   // pad columns stay zero
       }
       *reinterpret_cast<float4*>(C + (long long)row * p.ldc + col) = make_float4(v[0], v[1], v[2], v[3]);
-      if (EPI == 1 && p.closed) {
+      if ((EPI == 1 || EPI == 2) && p.closed) {
+        const float g = (EPI == 2) ? p.gain_env[row] : p.gain;
         float4* cp = reinterpret_cast<float4*>(p.com + (long long)row * p.ldcom + col);
         float4 c4 = *cp;
-        c4.x = fmaf(p.gain, v[0], c4.x); c4.y = fmaf(p.gain, v[1], c4.y);
-        c4.z = fmaf(p.gain, v[2], c4.z); c4.w = fmaf(p.gain, v[3], c4.w);
+        c4.x = fmaf(g, v[0], c4.x); c4.y = fmaf(g, v[1], c4.y);
+        c4.z = fmaf(g, v[2], c4.z); c4.w = fmaf(g, v[3], c4.w);
         *cp = c4;
       }
     }

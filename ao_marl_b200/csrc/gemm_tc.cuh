@@ -288,11 +288,12 @@ __global__ void __launch_bounds__(GTC_THREADS, 2) gemm_tc_kernel(GemmParams p, i
             o[j] = (cc < p.N) ? x : 0.f;         // pad columns stay zero
           }
           *reinterpret_cast<float4*>(C + (long long)row * p.ldc + col) = make_float4(o[0], o[1], o[2], o[3]);
-          if (EPI == 1 && p.closed) {
+          if ((EPI == 1 || EPI == 2) && p.closed) {
+            const float g = (EPI == 2) ? p.gain_env[row] : p.gain;
             float4* cp = reinterpret_cast<float4*>(p.com + (long long)row * p.ldcom + col);
             float4 c4 = *cp;
-            c4.x = fmaf(p.gain, o[0], c4.x); c4.y = fmaf(p.gain, o[1], c4.y);
-            c4.z = fmaf(p.gain, o[2], c4.z); c4.w = fmaf(p.gain, o[3], c4.w);
+            c4.x = fmaf(g, o[0], c4.x); c4.y = fmaf(g, o[1], c4.y);
+            c4.z = fmaf(g, o[2], c4.z); c4.w = fmaf(g, o[3], c4.w);
             *cp = c4;
           }
         }

@@ -27,7 +27,8 @@ __device__ __forceinline__ float wfs_layer_row(const float* scr, int N, int prow
 }
 
 // PE: per-environment winds (the layer offsets come from p.wind)
-template <int R, bool PE = false>
+// NE: per-environment sensor values (each environment's noise and photon count from p.noise_env / p.nph_env)
+template <int R, bool PE = false, bool NE = false>
 __global__ void __launch_bounds__(WFS_WARPS * 32, 2) wfs_frame_kernel(WfsParams p) {
   constexpr int NFFT = 16 * R;
   constexpr int H = 4 * R;            // half width of the kept spectrum
@@ -216,14 +217,15 @@ __global__ void __launch_bounds__(WFS_WARPS * 32, 2) wfs_frame_kernel(WfsParams 
     for (int j = 0; j < 8; ++j) { px[j] = s_img[lane + 32 * j]; tot += px[j]; }
 #pragma unroll
     for (int sft = 16; sft > 0; sft >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, sft);
-    const float scale = p.nphotons * p.flux[k] / tot;
+    const float scale = nphotons_of<NE>(p, e) * p.flux[k] / tot;
+    const float noise = noise_of<NE>(p, e);
     const uint32_t k0 = p.k0[e], k1 = p.k1[e], fr = noise_frame(p, e);
     float s0 = 0.f, sy = 0.f;
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const int pidx = lane + 32 * j;
       float v = px[j] * scale;
-      v = aom_pixel_noise(v, p.noise, (uint32_t)(k * 256 + pidx), fr, p.wfs_index, k0, k1);
+      v = aom_pixel_noise(v, noise, (uint32_t)(k * 256 + pidx), fr, p.wfs_index, k0, k1);
       px[j] = v;
       s0 += v;
       sy += v * (float)(pidx >> 4);

@@ -40,7 +40,21 @@ struct WfsParams {
   // per-environment winds: offsets of every layer and environment [n_layers][E], read by the kernels' per-environment
   // instantiations in place of layer[l].ix .. w11 (null while every layer moves all environments alike)
   const WindRec* wind;
+  // per-environment sensor values [E] (aom_set_wfs_noise_env), read by the kernels' NE instantiations in place of noise /
+  // nphotons (null: the common value; noise_env is null in a frame drawn noise-free)
+  const float* noise_env;
+  const float* nph_env;
 };
+
+// sensor noise / photon count of environment e: the common value, or its own when NE (per-environment sensor values)
+template <bool NE>
+__device__ __forceinline__ float noise_of(const WfsParams& p, int e) {
+  return (NE && p.noise_env) ? p.noise_env[e] : p.noise;
+}
+template <bool NE>
+__device__ __forceinline__ float nphotons_of(const WfsParams& p, int e) {
+  return (NE && p.nph_env) ? p.nph_env[e] : p.nphotons;
+}
 
 // raytrace offset of layer l for environment e: the layer's common one, or its record when PE (per-environment winds)
 template <bool PE>

@@ -281,7 +281,9 @@ __device__ __forceinline__ void wu_layer(const float* __restrict__ t, const Wt& 
 // rounded fp16 (slopes ~3e-5 relative).
 // PE: per-environment winds (layer offsets from p.wind: the ring origin per environment, the weights per item through
 // the aux slot)
-template <int NL, int FULL, bool PE = false>
+// NE: per-environment sensor values (noise and photon count of the item's environment; whether the epilogue takes the
+// plain path is decided per item -- warp-uniform, a warp's item belongs to one environment)
+template <int NL, int FULL, bool PE = false, bool NE = false>
 __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const __grid_constant__ WfsUmmaParams P) {
   const WfsParams& p = P.p;
   const WfsUmmaTables& f = P.f;
@@ -558,11 +560,11 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
       }
     }
   };
-  auto epilogue = [&](const float (&qa)[8], const float (&qb)[8], wu_f2 s0p, wu_f2 syp, int ie, int ik) {
+  auto epilogue = [&](const float (&qa)[8], const float (&qb)[8], wu_f2 s0p, wu_f2 syp, int ie, int ik, bool pl) {
     const int pr = lane >> 1;                                  // fx pair: kept indices 2 pr, 2 pr + 1
     const int px = (pr < 8) ? 8 + pr : pr - 8;
     float s0 = 0.f, sx = 0.f, sy = 0.f;
-    if (plain) {
+    if (pl) {
       float a, b;
       wu_upk(s0p, a, b); s0 = a + b;
       wu_upk(syp, a, b); sy = a + b;
@@ -583,7 +585,8 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
       for (int j = 0; j < 8; ++j) tot += mine[j];
 #pragma unroll
       for (int sft = 16; sft > 0; sft >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, sft);
-      const float scale = p.nphotons * p.flux[ik] / tot;
+      const float scale = nphotons_of<NE>(p, ie) * p.flux[ik] / tot;
+      const float noise = noise_of<NE>(p, ie);
       const uint32_t k0 = p.k0[ie], k1 = p.k1[ie], fr = noise_frame(p, ie);
       float* cube = p.bincube ? p.bincube + ((size_t)ie * p.nvalid + ik) * 256 : nullptr;
 #pragma unroll
@@ -591,7 +594,7 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
         const int py = py0 + j;
         const int pidx = py * 16 + px;
         float v = mine[j] * scale;
-        v = aom_pixel_noise(v, p.noise, (uint32_t)(ik * 256 + pidx), fr, p.wfs_index, k0, k1);
+        v = aom_pixel_noise(v, noise, (uint32_t)(ik * 256 + pidx), fr, p.wfs_index, k0, k1);
         if (cube) cube[pidx] = v;
         s0 += v;
         sx = fmaf(v, (float)px, sx);
@@ -826,6 +829,9 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
     }
 
     // ---- E(it-2) ----
+    // plain path of item it-2: the batch's, or with NE its environment's (a noise-free environment of a mixed launch
+    // takes exactly the path of a uniform noise-free launch)
+    const bool pl = NE ? (p.bincube == nullptr && noise_of<NE>(p, (int)(ek2 >> 16)) < 0.f) : plain;
     float qa[8], qb[8];
     wu_f2 s0p = 0ull, syp = 0ull;
     if (epi) {
@@ -834,13 +840,13 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
       wu_tmem_ld32(d2_addr, yv);
 #endif
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      if (plain) sq_plain(yv, 8.f, s0p, syp, true); else sq_half(yv, qa);
+      if (pl) sq_plain(yv, 8.f, s0p, syp, true); else sq_half(yv, qa);
       wu_tmem_ld32(d2_addr + 32u, yv);
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      if (plain) sq_plain(yv, 0.f, s0p, syp, false); else sq_half(yv, qb);
+      if (pl) sq_plain(yv, 0.f, s0p, syp, false); else sq_half(yv, qb);
     }
     if (conv) arrive_and_issue(1, (uint32_t)((it - 1) & 1));                    // A2(it-1) written and Y(it-2) drained by this warp
-    if (epi && it - 2 < n_mine) epilogue(qa, qb, s0p, syp, (int)(ek2 >> 16), (int)(ek2 & 0xffffu));
+    if (epi && it - 2 < n_mine) epilogue(qa, qb, s0p, syp, (int)(ek2 >> 16), (int)(ek2 & 0xffffu), pl);
 
     xy_cur = xy_next;
     ek2 = ek1; ek1 = ek0;

@@ -13,5 +13,6 @@ struct WfsUmmaHost {
 // Launches wfs_frame_umma_kernel for the frame described by p.  full != 0: fp32-grade products in both stages.
 // Returns cudaSuccess or the error of the attribute / launch call.
 // ws != 0: the warp-specialised kernel (wfs_umma_ws.cuh) on the same tables.  p.wind != null: the per-environment wind
-// instantiations of either kernel.
+// instantiations of either kernel.  p.noise_env / p.nph_env != null: the per-environment sensor instantiations of the fused
+// kernel (ws must be 0).
 cudaError_t wfs_umma_launch(const WfsParams& p, const WfsUmmaHost& h, int num_sms, int full, int ws, cudaStream_t st);

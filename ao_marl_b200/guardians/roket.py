@@ -54,6 +54,12 @@ class Roket(RlSupervisor):
             raise ValueError("ROKET needs the geometric controller of the parameter file (p_controllers[1].type == 'geo')")
         self.iter_number = 0
 
+    def _common_gain(self):
+        """The loop filter of the breakdown uses one gain g for the whole batch."""
+        if self.sim.gain_env is not None:
+            raise NotImplementedError("ROKET's loop filter has one gain for the whole batch: per-environment gains "
+                                      "(set_gain with an [E] array) are not supported; set a scalar gain")
+
     def reset_envs(self, envs, seeds):
         """Not available: the error-breakdown buffers ([N_total, E, .]) hold one run of the whole batch."""
         raise NotImplementedError("ROKET's breakdown buffers are whole-batch: use reset()")
@@ -63,6 +69,7 @@ class Roket(RlSupervisor):
                           n_zernike_start=None, n_zernike_end=None):
         import torch
         assert N_total >= N_preloop
+        self._common_gain()
         t, E = self.tables, self.n_env
         dev = "cuda"
         self.agent, self.include_tip_tilt = agent, include_tip_tilt
@@ -132,6 +139,7 @@ class Roket(RlSupervisor):
         """roket_generalized_rl.py:171-188: record the RL command of this frame, run the breakdown, then apply the (RL
         corrected) command and evaluate the target."""
         import torch
+        self._common_gain()
         i = self.iter_number
         if a is not None and i < self.n:
             act = torch.as_tensor(a, dtype=torch.float32, device="cuda")

@@ -108,6 +108,15 @@ def compute_nphotons(ittime, optthroughput, diam, nxsub, zerop, gsmag):
     return zerop * 10.0 ** (-0.4 * gsmag) * ittime * optthroughput * (diam / nxsub) ** 2.0
 
 
+def nphotons_for_mags(ittime, optthroughput, diam, nxsub, zerop, gsmag):
+    """float32 photon counts of compute_nphotons for a scalar or an array of guide-star magnitudes.  Each value is the
+    scalar formula in float64 rounded once to float32, as the builder's _nphotons reaches aom_config.nphotons."""
+    mags = np.asarray(gsmag, dtype=np.float64)
+    out = np.array([compute_nphotons(ittime, optthroughput, diam, nxsub, zerop, float(m)) for m in mags.reshape(-1)],
+                   dtype=np.float64)
+    return out.astype(np.float32).reshape(mags.shape)
+
+
 def init_sh_geom(p_wfs, r0, p_tel, p_geom, ittime):
     """Valid subapertures and the phasemap / binmap / halfxy tables (geom_init.py:622-811)."""
     nx, pd, npix = p_wfs.nxsub, p_wfs._pdiam, p_wfs.npix

@@ -52,9 +52,9 @@ OPTIONS = ["WFS_PATH", "GEMM_PATH", "TIME_WFS", "GEO", "DENOISE", "PUPIL_PATH", 
 O = {name: i for i, name in enumerate(OPTIONS)}
 
 EXPORTS = ["aom_config_size", "aom_create", "aom_destroy", "aom_last_error", "aom_set_table", "aom_get_buffer",
-           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_reset_envs", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
+           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_reset_envs", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_set_wfs_noise", "aom_set_wfs_noise_env", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
            "aom_comp_strehl", "aom_reset_strehl", "aom_do_control_geo", "aom_apply_control_geo", "aom_denoise", "aom_set_bincube", "aom_do_centroids", "aom_do_centroids_geom", "aom_do_control", "aom_set_command", "aom_apply_control",
-           "aom_set_gain", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
+           "aom_set_gain", "aom_set_gain_env", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
            "aom_state_begin", "aom_state_end", "aom_reward", "aom_actor_forward", "aom_step", "aom_gemm_tn",
            "aom_pixel_noise"]
 
@@ -94,6 +94,8 @@ def load_library():
     lib.aom_set_layer_amp.argtypes = [vp, i32, vp]
     lib.aom_set_layer_wind.argtypes = [vp, i32, vp, vp]
     lib.aom_comp_wfs_image.argtypes = [vp, i32, f32, vp]
+    lib.aom_set_wfs_noise.argtypes = [vp, f32, f32]
+    lib.aom_set_wfs_noise_env.argtypes = [vp, vp, vp]
     lib.aom_raytrace_wfs.argtypes = [vp, i32, vp]
     lib.aom_wfs_time_ms.argtypes = [vp, ctypes.POINTER(f32), ctypes.POINTER(i32)]
     lib.aom_wfs_kernel.argtypes = [vp]
@@ -110,6 +112,7 @@ def load_library():
     lib.aom_set_command.argtypes = [vp, vp, i32, vp]
     lib.aom_apply_control.argtypes = [vp, i32, vp]
     lib.aom_set_gain.argtypes = [vp, f32]
+    lib.aom_set_gain_env.argtypes = [vp, vp]
     lib.aom_set_loop.argtypes = [vp, i32]
     lib.aom_reset_dm.argtypes = [vp, vp]
     lib.aom_set_dm_volts.argtypes = [vp, vp, i32, vp]
@@ -232,6 +235,10 @@ class Simulator:
             raise (ValueError if rc == -1 else RuntimeError)("aom_create: " + msg)
         self._stream = stream
         self._views = {}
+        # sensor noise / photon count / integrator gain: common values and the per-environment float32 [E] arrays in
+        # force (None: the common value), as the context holds them
+        self.wfs_noise, self.wfs_nphotons = float(np.float32(cfg.noise)), float(np.float32(cfg.nphotons))
+        self.wfs_noise_env = self.wfs_nphotons_env = self.gain_env = None
         # focal-plane grid of the target image (p_geom._ipupil, geom_init: 2^ceil(log2(pupdiam) + 1)) for the PSF core
         try:
             self.psf_nfft = int(np.asarray(t.config.p_geom._ipupil).shape[0])
@@ -421,9 +428,38 @@ class Simulator:
         amp = np.ascontiguousarray(np.broadcast_to(np.asarray(amp, dtype=np.float32), (self.n_env,)))
         self._check(self.lib.aom_set_layer_amp(self._ctx, int(layer), amp.ctypes.data_as(ctypes.c_void_p)), "aom_set_layer_amp")
 
+    def _env_array(self, x, what):
+        """float32 [E] from a scalar (broadcast) or a length-E sequence; ValueError otherwise."""
+        a = np.asarray(x, dtype=np.float32)
+        if a.ndim == 0:
+            a = np.full(self.n_env, a, dtype=np.float32)
+        if a.shape != (self.n_env,):
+            raise ValueError("%s: expected a scalar or %d values, got shape %s" % (what, self.n_env, a.shape))
+        return np.ascontiguousarray(a)
+
+    def set_wfs_noise(self, noise, nphotons=None):
+        """Common sensor noise (<0 none, 0 photon, >0 photon + read noise in e-) and photons per subaperture and frame
+        (None: unchanged).  aom_step and comp_wfs_image(noise=None) use them; per-environment values stay in force."""
+        nph = self.wfs_nphotons if nphotons is None else nphotons
+        self._check(self.lib.aom_set_wfs_noise(self._ctx, float(noise), float(nph)), "aom_set_wfs_noise")
+        self.wfs_noise, self.wfs_nphotons = float(np.float32(noise)), float(np.float32(nph))
+
+    def set_wfs_noise_env(self, noise=None, nphotons=None):
+        """Sensor noise and photon count per environment (scalar or [E] each; None: that quantity's common value).  A
+        noisy frame then draws each environment's own noise, and every frame is scaled by its own photon count."""
+        P = lambda a: None if a is None else a.ctypes.data_as(ctypes.c_void_p)
+        n = None if noise is None else self._env_array(noise, "set_wfs_noise_env(noise)")
+        f = None if nphotons is None else self._env_array(nphotons, "set_wfs_noise_env(nphotons)")
+        self._check(self.lib.aom_set_wfs_noise_env(self._ctx, P(n), P(f)), "aom_set_wfs_noise_env")
+        self.wfs_noise_env, self.wfs_nphotons_env = n, f
+
     def comp_wfs_image(self, atmos=True, dms=True, keep_image=False, noise=None, advance_frame=True):
+        """noise None: the common noise, or with per-environment noise in force a noisy frame (each environment's own);
+        a value < 0: noise-free for every environment."""
         flags = (1 if atmos else 0) | (2 if dms else 0) | (4 if keep_image else 0) | (0 if advance_frame else 8)
-        noise = float(self.cfg.noise if noise is None else noise)
+        if noise is None:
+            noise = 0.0 if self.wfs_noise_env is not None else self.wfs_noise
+        noise = float(noise)
         self._check(self.lib.aom_comp_wfs_image(self._ctx, flags, noise, self.stream), "aom_comp_wfs_image")
 
     def do_centroids_geom(self, atmos=True, dms=True, geo=False):
@@ -560,7 +596,19 @@ class Simulator:
         self._check(self.lib.aom_apply_control(self._ctx, int(bool(comp_voltage)), self.stream), "aom_apply_control")
 
     def set_gain(self, g):
-        self._check(self.lib.aom_set_gain(self._ctx, float(g)), "aom_set_gain")
+        """Integrator gain: a scalar sets the common gain (per-environment gains stay in force, as aom_set_gain); an [E]
+        array sets one gain per environment (set_gain_env)."""
+        if np.ndim(g) == 0:
+            self._check(self.lib.aom_set_gain(self._ctx, float(g)), "aom_set_gain")
+        else:
+            self.set_gain_env(g)
+
+    def set_gain_env(self, g):
+        """One integrator gain per environment ([E]; a scalar broadcasts); None: back to the common gain."""
+        a = None if g is None else self._env_array(g, "set_gain_env")
+        self._check(self.lib.aom_set_gain_env(self._ctx, None if a is None else a.ctypes.data_as(ctypes.c_void_p)),
+                    "aom_set_gain_env")
+        self.gain_env = a
 
     def set_loop(self, closed):
         self._check(self.lib.aom_set_loop(self._ctx, int(bool(closed))), "aom_set_loop")

@@ -7,7 +7,7 @@ arrays of the reference's shapes (float32), otherwise device tensors [E, ...] (n
 """
 import numpy as np
 
-from ..init.geom import DEG2RAD
+from ..init.geom import DEG2RAD, nphotons_for_mags
 
 
 class _Base:
@@ -127,7 +127,6 @@ class WfsB200(_Base):
         self._index = wfs_index
         self._atm = False
         self._dms = False
-        self._noise = float(sim.cfg.noise)
         self.keep_image = False
 
     def _chk(self, i):
@@ -145,13 +144,35 @@ class WfsB200(_Base):
 
     def compute_wfs_image(self, wfs_index, *, noise=True):
         self._chk(wfs_index)
+        # noise=True: the common noise, or each environment's own (Simulator.comp_wfs_image(noise=None))
         self._sim.comp_wfs_image(atmos=self._atm, dms=self._dms, keep_image=self.keep_image,
-                                 noise=self._noise if noise else -1.0)
+                                 noise=None if noise else -1.0)
 
     def set_noise(self, wfs_index, noise, *, seed=1234):
+        """Sensor noise (<0 none, 0 photon, >0 photon + read noise in e-): a scalar sets the common value and drops
+        per-environment noise, an [E] array sets one value per environment.  Both reach aom_step and compute_wfs_image."""
         self._chk(wfs_index)
-        self._noise = float(noise)
-        self._config.p_wfss[wfs_index].noise = noise
+        sim = self._sim
+        if np.ndim(noise) == 0:
+            sim.set_wfs_noise(float(noise))
+            sim.set_wfs_noise_env(noise=None, nphotons=sim.wfs_nphotons_env)
+            self._config.p_wfss[wfs_index].noise = noise
+        else:
+            sim.set_wfs_noise_env(noise=noise, nphotons=sim.wfs_nphotons_env)
+
+    def set_gs_mag(self, wfs_index, mag):
+        """Guide-star magnitude, scalar or [E]: photons per subaperture and frame from compute_nphotons with this
+        sensor's integration time, throughput, telescope diameter, nxsub and zero point (geom_init.py:343-407).  A scalar
+        sets the common photon count and drops per-environment ones; an [E] array sets one per environment."""
+        self._chk(wfs_index)
+        c, sim = self._config, self._sim
+        w = c.p_wfss[wfs_index]
+        nph = nphotons_for_mags(c.p_loop.ittime, w.optthroughput, c.p_tel.diam, w.nxsub, w.zerop, mag)
+        if np.ndim(mag) == 0:
+            sim.set_wfs_noise(sim.wfs_noise, float(nph))
+            sim.set_wfs_noise_env(noise=sim.wfs_noise_env, nphotons=None)
+        else:
+            sim.set_wfs_noise_env(noise=sim.wfs_noise_env, nphotons=nph)
 
     def reset_noise(self, seed):
         """Noise streams are keyed by the environment seed and the frame counter: reseeding happens in
@@ -234,8 +255,15 @@ class _Controller:
         self.gain = float(sim.cfg.gain)
 
     def set_gain(self, g):
-        self.gain = float(g)
-        self._sim.set_gain(g)
+        """A scalar sets the gain of every environment (and drops per-environment gains); an [E] array one gain per
+        environment."""
+        if np.ndim(g) == 0:
+            self._sim.set_gain(float(g))
+            self._sim.set_gain_env(None)
+            self.gain = float(g)
+        else:
+            self._sim.set_gain_env(g)
+            self.gain = self._sim.gain_env.copy()
 
 
 class _RtcHandle:

@@ -280,9 +280,30 @@ int aom_set_layer_wind(aom_ctx* ctx, int layer, const float* deltax_host, const 
 /* WfsCompass.raytrace + compute_wfs_image fused (wfsCompass.py:334-343, sourceCompass.py:54-85).
  * flags: bit0 atmosphere, bit1 mirrors, bit2 keep image (writes AOM_B_BINCUBE), bit3 do not advance the frame counter
  * of the noise streams (a second look at the same frame, e.g. d_binimg_notnoisy of roket_generalized_rl.py:197). noise: sensor noise for
- * this frame (pass cfg.noise for the configured value).  Also leaves the centre-of-gravity slopes of the
+ * this frame (pass the common value of aom_set_wfs_noise, initially cfg.noise, for the configured one; with per-environment
+ * noise in force any value >= 0 selects each environment's own).  Also leaves the centre-of-gravity slopes of the
  * frame for aom_do_centroids. */
 int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* stream);
+
+/* WfsCompass.set_noise + the guide-star flux (geom_init.py:343-407): common sensor noise (<0 none, 0 photon, >0 photon
+ * + read noise in e-) and photons per full subaperture and frame.  They start as aom_config.noise / nphotons; aom_step
+ * draws its frames with them, and aom_comp_wfs_image scales its frames with this photon count.  AOM_ERR_INVALID for a
+ * non-finite value or a photon count <= 0. */
+int aom_set_wfs_noise(aom_ctx* ctx, float noise, float nphotons);
+
+/* The same per environment (one guide-star magnitude and detector per environment of the batch): host float [E] each.
+ * NULL returns that quantity to the common value; both NULL return to the uniform state.
+ * - While per-environment noise is in force, aom_step and aom_comp_wfs_image with noise >= 0 draw each environment's
+ *   frame with its own noise (the value passed then only means "noisy frame"); aom_comp_wfs_image with noise < 0 stays
+ *   noise-free for every environment.  Every frame, and a kept image, is scaled by each environment's photon count.
+ * - Every environment computes bit for bit what it computes in a batch configured with its values through aom_config.
+ * - A frame in which no environment draws noise and no image is kept still runs the specialised-warp kernel
+ *   (AOM_WFS_UMMA_WS); otherwise the per-environment form of the fused kernel (AOM_WFS_UMMA) serves it.
+ * - Persists through aom_reset / aom_reset_envs: set the new episode's values before the reset call.
+ * - AOM_ERR_INVALID for a non-finite entry or a photon count <= 0.  The round-1 sensor kernels (tensor_reg / tensor /
+ *   tensor_fast) return AOM_ERR_UNSUPPORTED for a frame that would read per-environment sensor values.
+ * Waits for the device; not for the step path. */
+int aom_set_wfs_noise_env(aom_ctx* ctx, const float* noise_host, const float* nphotons_host);
 
 /* Name of the kernel the next aom_comp_wfs_image will launch under the current AOM_OPT_WFS_PATH
  * ("wfs_frame_umma_kernel", "wfs_frame_tma_kernel", "wfs_frame_mma_kernel" or "wfs_frame_kernel"); when the staged kernel is not
@@ -345,7 +366,12 @@ int aom_do_centroids_geom(aom_ctx* ctx, int flags, float alpha, void* stream);
 int aom_do_control(aom_ctx* ctx, void* stream);
 int aom_set_command(aom_ctx* ctx, const float* dcom, int ld, void* stream);
 int aom_apply_control(aom_ctx* ctx, int comp_voltage, void* stream);
-int aom_set_gain(aom_ctx* ctx, float gain);
+int aom_set_gain(aom_ctx* ctx, float gain);     /* common gain; per-environment gains (aom_set_gain_env) stay in force */
+/* RtcCompass.set_gain per environment (the reference tunes the integrator gain per parameter file, params.py): gain of
+ * every environment's integrator, host float [E] (NULL: back to the common gain of aom_config.gain / aom_set_gain).
+ * com += g[e] err in all three controller paths.  Persists through aom_reset / aom_reset_envs.  AOM_ERR_INVALID for a
+ * non-finite entry.  Waits for the device; not for the step path. */
+int aom_set_gain_env(aom_ctx* ctx, const float* gain_host);
 int aom_set_loop(aom_ctx* ctx, int closed);       /* rtc.open_loop / close_loop (rtcCompass.py:116-142) */
 int aom_reset_dm(aom_ctx* ctx, void* stream);     /* DmCompass.reset_dm */
 int aom_set_dm_volts(aom_ctx* ctx, const float* dvolts, int ld, void* stream); /* DmCompass.set_command */
