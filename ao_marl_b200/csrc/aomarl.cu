@@ -8,6 +8,7 @@
 #include <string.h>
 
 #include "../../include/aomarl.h"
+#include "dispatch.h"
 #include "atmos_kernels.cuh"
 #include "gemm_kernels.cuh"
 #include "gemm_tc.cuh"
@@ -177,6 +178,22 @@ static cudaError_t dalloc(T** p, size_t count) {
   return e;
 }
 
+// Kernels launched with more dynamic shared memory than the default: f(kernel, bytes, its template arguments) for every
+// instantiation.  aom_create sets the attribute of each and the launch sites launch from the same lists.
+template <class F>
+static void gemm_tc_each(F&& f) {     // tcgen05 GEMM: epilogue, column tile
+  each<0, 1, 2>([&](auto EPI) {
+    each<GTC_BN, GTC_BN_WIDE>([&](auto BN) { f(gemm_tc_kernel<EPI, BN>, (size_t)GTC_SMEM_BYTES_T(BN), EPI, BN); });
+  });
+}
+
+template <class F>
+static void wfs_simt_each(F&& f) {    // SIMT sensor frame: Nfft / 16, per-environment winds, per-environment sensor values
+  each<4, 8>([&](auto R) {
+    each<false, true>([&](auto PE) { each<false, true>([&](auto NE) { f(wfs_frame_kernel<R, PE, NE>, wfs_smem_bytes<R>(), R, PE, NE); }); });
+  });
+}
+
 extern "C" size_t aom_config_size(void) { return sizeof(aom_config); }
 
 extern "C" const char* aom_last_error(const aom_ctx* ctx) { return ctx ? ctx->err : g_create_error; }
@@ -285,20 +302,13 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   CU(cudaStreamCreateWithFlags(&ctx->side_stream, cudaStreamNonBlocking));
   CU(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
   CU(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
-  CU(cudaFuncSetAttribute(gemm_tc_kernel<0, GTC_BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES));
-  CU(cudaFuncSetAttribute(gemm_tc_kernel<1, GTC_BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES));
-  CU(cudaFuncSetAttribute(gemm_tc_kernel<0, GTC_BN_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES_T(GTC_BN_WIDE)));
-  CU(cudaFuncSetAttribute(gemm_tc_kernel<1, GTC_BN_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES_T(GTC_BN_WIDE)));
-  CU(cudaFuncSetAttribute(gemm_tc_kernel<2, GTC_BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES));
-  CU(cudaFuncSetAttribute(gemm_tc_kernel<2, GTC_BN_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, GTC_SMEM_BYTES_T(GTC_BN_WIDE)));
-  CU(cudaFuncSetAttribute(wfs_frame_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
-  CU(cudaFuncSetAttribute(wfs_frame_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
-  CU(cudaFuncSetAttribute(wfs_frame_kernel<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
-  CU(cudaFuncSetAttribute(wfs_frame_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
-  CU(cudaFuncSetAttribute(wfs_frame_kernel<4, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
-  CU(cudaFuncSetAttribute(wfs_frame_kernel<8, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
-  CU(cudaFuncSetAttribute(wfs_frame_kernel<4, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<4>()));
-  CU(cudaFuncSetAttribute(wfs_frame_kernel<8, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wfs_smem_bytes<8>()));
+  cudaError_t ae = cudaSuccess;
+  auto smem_attr = [&](auto kernel, size_t smem, auto...) {
+    if (ae == cudaSuccess) ae = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  };
+  gemm_tc_each(smem_attr);
+  wfs_simt_each(smem_attr);
+  if (ae != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "cudaFuncSetAttribute(dynamic shared memory) failed: %s", cudaGetErrorString(ae));
   return AOM_OK;
 }
 
@@ -521,20 +531,12 @@ static int sweep_launch(aom_ctx* ctx, const WfsParams& w, float* Tp, double* mom
   P.nb = ctx->sweep_nb;
   P.n_strips = (c.n + PSW_STRIP - 1) / PSW_STRIP;
   P.err = ctx->d_err;
-  if (w.wind) {          // per-environment winds
-    switch (w.n_layers) {
-      case 1: return sweep_launch_t<1, MODE, true>(ctx, P, st);
-      case 2: return sweep_launch_t<2, MODE, true>(ctx, P, st);
-      case 3: return sweep_launch_t<3, MODE, true>(ctx, P, st);
-      default: return sweep_launch_t<4, MODE, true>(ctx, P, st);
-    }
-  }
-  switch (w.n_layers) {
-    case 0: case 1: return sweep_launch_t<1, MODE, false>(ctx, P, st);
-    case 2: return sweep_launch_t<2, MODE, false>(ctx, P, st);
-    case 3: return sweep_launch_t<3, MODE, false>(ctx, P, st);
-    default: return sweep_launch_t<4, MODE, false>(ctx, P, st);
-  }
+  int rc = AOM_OK;
+  // no layer runs as one, more than three as four
+  with<1, 2, 3, 4>(std::min(std::max(w.n_layers, 1), 4), [&](auto NL) {
+    with<false, true>(w.wind != nullptr, [&](auto PE) { rc = sweep_launch_t<NL, MODE, PE>(ctx, P, st); });
+  });
+  return rc;
 }
 
 // buffers of the geometric controller (only configurations that use it pay for them)
@@ -634,17 +636,11 @@ static int launch_gemm(aom_ctx* ctx, int epi, const float* A, int lda, long long
     // column tile: the wide one when it saves CTA waves (two CTAs per SM)
     const long long slots = 2LL * ctx->num_sms, rows = (M + GTC_BM - 1) / GTC_BM;
     auto waves = [&](int bn) { return (double)((rows * ((ldc + bn - 1) / bn) * batch + slots - 1) / slots) * bn; };
-    if (!Bt && waves(GTC_BN_WIDE) < waves(GTC_BN)) {
-      dim3 grid((ldc + GTC_BN_WIDE - 1) / GTC_BN_WIDE, (unsigned)rows, batch);
-      if (epi == 0) gemm_tc_kernel<0, GTC_BN_WIDE><<<grid, GTC_THREADS, GTC_SMEM_BYTES_T(GTC_BN_WIDE), st>>>(p, ctx->d_err);
-      else if (epi == 1) gemm_tc_kernel<1, GTC_BN_WIDE><<<grid, GTC_THREADS, GTC_SMEM_BYTES_T(GTC_BN_WIDE), st>>>(p, ctx->d_err);
-      else gemm_tc_kernel<2, GTC_BN_WIDE><<<grid, GTC_THREADS, GTC_SMEM_BYTES_T(GTC_BN_WIDE), st>>>(p, ctx->d_err);
-    } else {
-      dim3 grid((ldc + GTC_BN - 1) / GTC_BN, (unsigned)rows, batch);
-      if (epi == 0) gemm_tc_kernel<0, GTC_BN><<<grid, GTC_THREADS, GTC_SMEM_BYTES, st>>>(p, ctx->d_err);
-      else if (epi == 1) gemm_tc_kernel<1, GTC_BN><<<grid, GTC_THREADS, GTC_SMEM_BYTES, st>>>(p, ctx->d_err);
-      else gemm_tc_kernel<2, GTC_BN><<<grid, GTC_THREADS, GTC_SMEM_BYTES, st>>>(p, ctx->d_err);
-    }
+    const int bn = (!Bt && waves(GTC_BN_WIDE) < waves(GTC_BN)) ? GTC_BN_WIDE : GTC_BN;
+    const dim3 grid((ldc + bn - 1) / bn, (unsigned)rows, batch);
+    gemm_tc_each([&](auto kernel, size_t smem, int e, int b) {
+      if (e == epi && b == bn) kernel<<<grid, GTC_THREADS, smem, st>>>(p, ctx->d_err);
+    });
   } else if (exact && epi == 0 && batch == 1 && !bias && !relu && ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT) {
     // shaped exact kernel: column tile 8 CN with the least padding.  Only columns < N are consumed by the
     // extrusion scatter; pad columns inside the last tile are written as zeros, the rest keep their zeros.
@@ -662,13 +658,10 @@ static int launch_gemm(aom_ctx* ctx, int epi, const float* A, int lda, long long
       if (e != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "cudaMemsetAsync: %s", cudaGetErrorString(e));
     }
     dim3 grid((N + bn - 1) / bn, (M + GEMM_BM - 1) / GEMM_BM, ksplit);
-    if (best == 8) gemm_tn_exact_kernel<8><<<grid, 128, 0, st>>>(p);
-    else gemm_tn_exact_kernel<9><<<grid, 128, 0, st>>>(p);
+    with<8, 9>(best, [&](auto CN) { gemm_tn_exact_kernel<CN><<<grid, 128, 0, st>>>(p); });
   } else {
     dim3 grid((ldc + GEMM_BN - 1) / GEMM_BN, (M + GEMM_BM - 1) / GEMM_BM, batch);
-    if (epi == 0) gemm_tn_kernel<0><<<grid, 256, 0, st>>>(p);
-    else if (epi == 1) gemm_tn_kernel<1><<<grid, 256, 0, st>>>(p);
-    else gemm_tn_kernel<2><<<grid, 256, 0, st>>>(p);
+    with<0, 1, 2>(epi, [&](auto EPI) { gemm_tn_kernel<EPI><<<grid, 256, 0, st>>>(p); });
   }
   KCHECK();
   return AOM_OK;
@@ -751,15 +744,13 @@ static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st
     ctx->launches += 2;
     p.zref = nullptr;                                  // the reference pixel is already in the new column
   } else {
-    if (steps) extrude_gather_kernel<true><<<rows, 256, 0, st>>>(p);
-    else extrude_gather_kernel<false><<<rows, 256, 0, st>>>(p);
+    with<false, true>(steps != nullptr, [&](auto PE) { extrude_gather_kernel<PE><<<rows, 256, 0, st>>>(p); });
     KCHECK();
     int rc = launch_gemm(ctx, 0, ctx->Z, p.ldz, 0, (const float*)ctx->tab[AOM_T_AB][l], p.ldz, 0, ctx->newcol, p.ldn, 0,
                          rows, p.N, p.S + p.N, nullptr, 0, 0, 1, st, nullptr, 0, true);
     if (rc) return rc;
   }
-  if (steps) extrude_scatter_kernel<true><<<rows, EXTRUDE_SCATTER_THREADS, 0, st>>>(p);
-  else extrude_scatter_kernel<false><<<rows, EXTRUDE_SCATTER_THREADS, 0, st>>>(p);
+  with<false, true>(steps != nullptr, [&](auto PE) { extrude_scatter_kernel<PE><<<rows, EXTRUDE_SCATTER_THREADS, 0, st>>>(p); });
   KCHECK();
   return AOM_OK;
 }
@@ -1495,17 +1486,12 @@ static int wfs_fast_launch_t(aom_ctx* ctx, const WfsParams& p, cudaStream_t st) 
   return AOM_OK;
 }
 
-static int wfs_fast_launch(aom_ctx* ctx, const WfsParams& p, int full, cudaStream_t st) {
-#define WFT_GO(NL) return full ? wfs_fast_launch_t<1, NL>(ctx, p, st) : wfs_fast_launch_t<0, NL>(ctx, p, st)
-  switch (p.n_layers) {
-    case 0: WFT_GO(0);
-    case 1: WFT_GO(1);
-    case 2: WFT_GO(2);
-    case 3: WFT_GO(3);
-    case 4: WFT_GO(4);
-  }
-#undef WFT_GO
-  return fail(ctx, AOM_ERR_UNSUPPORTED, "wfs_fast_launch: %d layers", p.n_layers);
+static int wfs_fast_launch(aom_ctx* ctx, const WfsParams& p, bool full, cudaStream_t st) {
+  int rc = AOM_OK;
+  const bool served = with<0, 1, 2, 3, 4>(p.n_layers, [&](auto NL) {
+    with<false, true>(full, [&](auto FULL) { rc = wfs_fast_launch_t<FULL, NL>(ctx, p, st); });
+  });
+  return served ? rc : fail(ctx, AOM_ERR_UNSUPPORTED, "wfs_fast_launch: %d layers", p.n_layers);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1553,6 +1539,58 @@ static int fill_wfs_params(aom_ctx* ctx, WfsParams& p, int flags, float noise) {
   return AOM_OK;
 }
 
+// The sensor kernel that serves a frame: its family with its compile-time choices, and whether the frame is refused
+enum WfsFamily { WFS_WS, WFS_UMMA, WFS_TMA, WFS_MMA, WFS_SIMT };
+static const char* const wfs_kernel_names[] = {"wfs_frame_ws_kernel", "wfs_frame_umma_kernel", "wfs_frame_tma_kernel",
+                                               "wfs_frame_mma_kernel", "wfs_frame_kernel"};
+struct WfsRoute {
+  WfsFamily family;
+  bool full, pe, ne;     // fp32-grade products in both DFT stages; per-environment winds; per-environment sensor values
+  int nl, r;             // layers of the instantiation (mma: 0, 1 or 3, else -1: its generic form); simt: Nfft / 16
+  const char* refused;   // not null: the frame is refused with this message (family still names the path's kernel)
+};
+
+// Routes a frame of parameters p (fill_wfs_params), noisy when any environment draws noise in it, with its image kept or
+// not.  Prepares the tables of the staged paths on first use.
+static int wfs_route(aom_ctx* ctx, const WfsParams& p, bool noisy, bool keep, WfsRoute& r) {
+  const aom_config& c = ctx->cfg;
+  const int path = ctx->opt[AOM_OPT_WFS_PATH];
+  const bool umma = (path == AOM_WFS_UMMA || path == AOM_WFS_UMMA_FAST || path == AOM_WFS_UMMA_WS);
+  const bool staged = umma || path == AOM_WFS_MMA_STAGED || path == AOM_WFS_MMA_STAGED_FAST;
+  memset(&r, 0, sizeof(r));
+  r.full = !(path == AOM_WFS_UMMA_FAST || path == AOM_WFS_MMA_STAGED_FAST);
+  r.nl = p.n_layers;
+  r.pe = p.wind != nullptr;
+  r.ne = p.noise_env || p.nph_env;
+  if (c.nfft != 64 || path == AOM_WFS_SIMT) {
+    r.family = WFS_SIMT;
+    r.r = c.nfft / 16;
+    return AOM_OK;
+  }
+  if (staged) {
+    int rc = umma ? wfs_umma_prepare(ctx) : wfs_fast_prepare(ctx);
+    if (rc) return rc;
+  }
+  if (umma && ctx->umma_state == 1) {
+    // the specialised-warp kernel serves every frame without noise and kept image (it reads neither noise nor photon
+    // count); the others go to the fused kernel, in its per-environment form when per-environment values are in force
+    r.family = (path == AOM_WFS_UMMA_WS && !noisy && !keep) ? WFS_WS : WFS_UMMA;
+    if (r.family == WFS_WS) r.ne = false;
+    return AOM_OK;
+  }
+  r.family = (staged && ctx->fast_state == 1) ? WFS_TMA : WFS_MMA;
+  if (r.family == WFS_MMA && r.nl != 0 && r.nl != 1 && r.nl != 3) r.nl = -1;
+  // the round-1 kernels have no per-environment form
+  r.refused = p.frame0 ? "staggered environments (aom_reset_envs) are not implemented in the round-1 sensor kernels "
+                         "(wfs_frame_tma_kernel, wfs_frame_mma_kernel) until the next aom_reset: use the umma, umma_ws or simt path"
+            : p.wind ? "per-environment wind is not implemented in the round-1 sensor kernels (wfs_frame_tma_kernel, "
+                       "wfs_frame_mma_kernel): use the umma, umma_ws or simt path"
+            : r.ne ? "per-environment sensor noise and photon counts are not implemented in the round-1 sensor kernels "
+                     "(wfs_frame_tma_kernel, wfs_frame_mma_kernel): use the umma, umma_ws or simt path"
+            : nullptr;
+  return AOM_OK;
+}
+
 extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
@@ -1565,72 +1603,42 @@ extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* st
     if (!ctx->bincube) CU(dalloc(&ctx->bincube, (size_t)c.n_env * c.nvalid * 256));
     p.bincube = ctx->bincube;
   }
-  long long total = (long long)c.n_env * c.nvalid;
-  long long blocks = (total + WFS_WARPS - 1) / WFS_WARPS;
-  long long cap = (long long)ctx->num_sms * 2 * 8;      // 2 resident CTAs per SM, 8 waves of work each
-  int grid = (int)(blocks < cap ? blocks : cap);
-  const int path = ctx->opt[AOM_OPT_WFS_PATH];
-  const bool timed = ctx->opt[AOM_OPT_TIME_WFS] && ctx->wev_n < AOM_WFS_TIMERS;
-  if (timed) {
-    for (int j = 0; j < 2; ++j)
-      if (!ctx->wev[j][ctx->wev_n]) CU(cudaEventCreate(&ctx->wev[j][ctx->wev_n]));
-    CU(cudaEventRecord(ctx->wev[0][ctx->wev_n], st));
-  }
-  const bool umma = (path == AOM_WFS_UMMA || path == AOM_WFS_UMMA_FAST || path == AOM_WFS_UMMA_WS);
-  const bool staged = umma || path == AOM_WFS_MMA_STAGED || path == AOM_WFS_MMA_STAGED_FAST;
-  const bool fast = (path == AOM_WFS_UMMA_FAST || path == AOM_WFS_MMA_STAGED_FAST);
-  if (c.nfft == 64 && staged) {
-    rc = umma ? wfs_umma_prepare(ctx) : wfs_fast_prepare(ctx);
-    if (rc) return rc;
-  }
   // does any environment draw noise in this frame?  (host copies: no device read)
   bool noisy = p.noise >= 0.f;
   if (p.noise_env) {
     noisy = false;
     for (int e = 0; e < c.n_env && !noisy; ++e) noisy = ctx->noise_henv[e] >= 0.f;
   }
-  if (c.nfft == 64 && umma && ctx->umma_state == 1) {
-    // the specialised-warp kernel serves every frame without noise and kept image (it reads neither noise nor photon
-    // count); the others go to the fused kernel, in its per-environment form when per-environment values are in force
-    const bool ws = path == AOM_WFS_UMMA_WS && !noisy && p.bincube == nullptr;
-    if (ws) { p.noise = -1.f; p.noise_env = nullptr; p.nph_env = nullptr; }
-    cudaError_t le = wfs_umma_launch(p, ctx->umma, ctx->num_sms, !fast, ws, st);
+  WfsRoute r;
+  rc = wfs_route(ctx, p, noisy, p.bincube != nullptr, r);
+  if (rc) return rc;
+  if (r.refused) return fail(ctx, AOM_ERR_UNSUPPORTED, "%s", r.refused);
+  const bool timed = ctx->opt[AOM_OPT_TIME_WFS] && ctx->wev_n < AOM_WFS_TIMERS;
+  if (timed) {
+    for (int j = 0; j < 2; ++j)
+      if (!ctx->wev[j][ctx->wev_n]) CU(cudaEventCreate(&ctx->wev[j][ctx->wev_n]));
+    CU(cudaEventRecord(ctx->wev[0][ctx->wev_n], st));
+  }
+  long long total = (long long)c.n_env * c.nvalid;
+  long long blocks = (total + WFS_WARPS - 1) / WFS_WARPS;
+  long long cap = (long long)ctx->num_sms * 2 * 8;      // 2 resident CTAs per SM, 8 waves of work each
+  int grid = (int)(blocks < cap ? blocks : cap);
+  if (r.family == WFS_WS || r.family == WFS_UMMA) {
+    if (r.family == WFS_WS) { p.noise = -1.f; p.noise_env = nullptr; p.nph_env = nullptr; }
+    cudaError_t le = wfs_umma_launch(p, ctx->umma, ctx->num_sms, r.family == WFS_WS, r.full, r.ne, st);
     if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "wfs_umma_launch: %s", cudaGetErrorString(le));
-  }
-  else if (c.nfft == 64 && path != AOM_WFS_SIMT && p.frame0)
-    return fail(ctx, AOM_ERR_UNSUPPORTED, "staggered environments (aom_reset_envs) are not implemented in the round-1 sensor "
-                "kernels (wfs_frame_tma_kernel, wfs_frame_mma_kernel) until the next aom_reset: use the umma, umma_ws or simt path");
-  else if (c.nfft == 64 && path != AOM_WFS_SIMT && p.wind)
-    return fail(ctx, AOM_ERR_UNSUPPORTED, "per-environment wind is not implemented in the round-1 sensor kernels "
-                "(wfs_frame_tma_kernel, wfs_frame_mma_kernel): use the umma, umma_ws or simt path");
-  else if (c.nfft == 64 && path != AOM_WFS_SIMT && (p.noise_env || p.nph_env))
-    return fail(ctx, AOM_ERR_UNSUPPORTED, "per-environment sensor noise and photon counts are not implemented in the round-1 "
-                "sensor kernels (wfs_frame_tma_kernel, wfs_frame_mma_kernel): use the umma, umma_ws or simt path");
-  else if (c.nfft == 64 && staged && ctx->fast_state == 1) {
-    rc = wfs_fast_launch(ctx, p, !fast, st);
+  } else if (r.family == WFS_TMA) {
+    rc = wfs_fast_launch(ctx, p, r.full, st);
     if (rc) return rc;
+  } else if (r.family == WFS_MMA) {
+    with<0, 1, 3, -1>(r.nl, [&](auto NL) {
+      with<false, true>(r.full, [&](auto FULL) { wfs_frame_mma_kernel<FULL, NL><<<grid, WFM_WARPS * 32, 0, st>>>(p); });
+    });
+  } else {
+    wfs_simt_each([&](auto kernel, size_t smem, int R, bool PE, bool NE) {
+      if (R == r.r && PE == r.pe && NE == r.ne) kernel<<<grid, WFS_WARPS * 32, smem, st>>>(p);
+    });
   }
-  else if (c.nfft == 64 && path != AOM_WFS_SIMT) {
-    const int full = !fast;
-#define WFM_LAUNCH(F, NL) wfs_frame_mma_kernel<F, NL><<<grid, WFM_WARPS * 32, 0, st>>>(p)
-    switch (p.n_layers) {
-      case 0: if (full) WFM_LAUNCH(1, 0); else WFM_LAUNCH(0, 0); break;
-      case 1: if (full) WFM_LAUNCH(1, 1); else WFM_LAUNCH(0, 1); break;
-      case 3: if (full) WFM_LAUNCH(1, 3); else WFM_LAUNCH(0, 3); break;
-      default: if (full) WFM_LAUNCH(1, -1); else WFM_LAUNCH(0, -1); break;
-    }
-#undef WFM_LAUNCH
-  }
-  else if (p.noise_env || p.nph_env) {      // per-environment sensor values
-    if (c.nfft == 64 && p.wind) wfs_frame_kernel<4, true, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
-    else if (c.nfft == 64) wfs_frame_kernel<4, false, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
-    else if (p.wind) wfs_frame_kernel<8, true, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<8>(), st>>>(p);
-    else wfs_frame_kernel<8, false, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<8>(), st>>>(p);
-  }
-  else if (c.nfft == 64 && p.wind) wfs_frame_kernel<4, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
-  else if (c.nfft == 64) wfs_frame_kernel<4><<<grid, WFS_WARPS * 32, wfs_smem_bytes<4>(), st>>>(p);
-  else if (p.wind) wfs_frame_kernel<8, true><<<grid, WFS_WARPS * 32, wfs_smem_bytes<8>(), st>>>(p);
-  else wfs_frame_kernel<8><<<grid, WFS_WARPS * 32, wfs_smem_bytes<8>(), st>>>(p);
   KCHECK();
   if (timed) {
     CU(cudaEventRecord(ctx->wev[1][ctx->wev_n], st));
@@ -1658,17 +1666,14 @@ extern "C" int aom_wfs_time_ms(aom_ctx* ctx, float* mean_ms, int* count) {
 
 extern "C" const char* aom_wfs_kernel(aom_ctx* ctx) {
   if (!ctx) return "";
-  const int path = ctx->opt[AOM_OPT_WFS_PATH];
-  if (ctx->cfg.nfft != 64 || path == AOM_WFS_SIMT) return "wfs_frame_kernel";
-  if (path == AOM_WFS_MMA_REG) return "wfs_frame_mma_kernel";
-  if (path == AOM_WFS_UMMA || path == AOM_WFS_UMMA_FAST || path == AOM_WFS_UMMA_WS) {
-    if (wfs_umma_prepare(ctx) != AOM_OK) return "";
-    if (ctx->umma_state == 1) return path == AOM_WFS_UMMA_WS ? "wfs_frame_ws_kernel" : "wfs_frame_umma_kernel";
-  }
-  if (wfs_fast_prepare(ctx) != AOM_OK) return "";
-  if (ctx->fast_state == 1) return "wfs_frame_tma_kernel";
-  snprintf(ctx->err, sizeof(ctx->err), "staged sensor kernels not eligible: %s", ctx->fast_why);
-  return "wfs_frame_mma_kernel";
+  // the route of a noise-free frame without kept image; the per-environment state does not change its family, so the
+  // fields the route reads for it stay empty (and a refusal it would cause is not reported)
+  const WfsParams p{};
+  WfsRoute r;
+  if (wfs_route(ctx, p, false, false, r) != AOM_OK) return "";
+  if (r.family == WFS_MMA && ctx->opt[AOM_OPT_WFS_PATH] != AOM_WFS_MMA_REG)
+    snprintf(ctx->err, sizeof(ctx->err), "staged sensor kernels not eligible: %s", ctx->fast_why);
+  return wfs_kernel_names[r.family];
 }
 
 extern "C" int aom_raytrace_wfs(aom_ctx* ctx, int flags, void* stream) {
@@ -1685,8 +1690,7 @@ extern "C" int aom_raytrace_wfs(aom_ctx* ctx, int flags, void* stream) {
   }
   if (!ctx->phase) CU(dalloc(&ctx->phase, (size_t)c.n_env * c.n * c.n));
   dim3 blk(32, 8), grid((c.n + 31) / 32, (c.n + 7) / 8, c.n_env);
-  if (p.wind) wfs_phase_kernel<true><<<grid, blk, 0, st>>>(p, ctx->phase);
-  else wfs_phase_kernel<false><<<grid, blk, 0, st>>>(p, ctx->phase);
+  with<false, true>(p.wind != nullptr, [&](auto PE) { wfs_phase_kernel<PE><<<grid, blk, 0, st>>>(p, ctx->phase); });
   KCHECK();
   return AOM_OK;
 }
@@ -1737,8 +1741,9 @@ extern "C" int aom_comp_strehl(aom_ctx* ctx, int flags, float lambda_um, int acc
       if (rc) return rc;
     } else {
       dim3 blk(32, 8), grid((c.n + 31) / 32, (c.n + 7) / 8, c.n_env);
-      if (p.wind) target_moments_kernel<true><<<grid, blk, 0, st>>>(p, mom, k2t, peak ? PSW_MOM2 : 5, peak ? 1.f / (float)nfft : 0.f);
-      else target_moments_kernel<false><<<grid, blk, 0, st>>>(p, mom, k2t, peak ? PSW_MOM2 : 5, peak ? 1.f / (float)nfft : 0.f);
+      with<false, true>(p.wind != nullptr, [&](auto PE) {
+        target_moments_kernel<PE><<<grid, blk, 0, st>>>(p, mom, k2t, peak ? PSW_MOM2 : 5, peak ? 1.f / (float)nfft : 0.f);
+      });
       KCHECK();
     }
     if (flags & AOM_TAR_TRACE) return AOM_OK;        // sums pending until AOM_TAR_PUBLISH
@@ -1775,8 +1780,9 @@ extern "C" int aom_do_control_geo(aom_ctx* ctx, void* stream) {
   } else {
     const size_t smem = (size_t)GEO_ROW_WARPS * (c.n + (c.n >> 4) + 2) * sizeof(float);
     dim3 grid((c.n + GEO_ROW_WARPS - 1) / GEO_ROW_WARPS, c.n_env);
-    if (p.wind) geo_rows_kernel<true><<<grid, GEO_ROW_WARPS * 32, smem, st>>>(p, ctx->geo_T, ctx->geo_gp, ctx->geo_mom);
-    else geo_rows_kernel<false><<<grid, GEO_ROW_WARPS * 32, smem, st>>>(p, ctx->geo_T, ctx->geo_gp, ctx->geo_mom);
+    with<false, true>(p.wind != nullptr, [&](auto PE) {
+      geo_rows_kernel<PE><<<grid, GEO_ROW_WARPS * 32, smem, st>>>(p, ctx->geo_T, ctx->geo_gp, ctx->geo_mom);
+    });
     KCHECK();
   }
   geo_cols_kernel<<<c.n_env, 256, 0, st>>>(p, ctx->geo_T, ctx->geo_gp, nb, ctx->geo_mom,

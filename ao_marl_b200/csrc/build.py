@@ -11,7 +11,7 @@ LIB = os.path.join(HERE, "libaomarl.so")
 SOURCES = ["aomarl.cu", "wfs_umma.cu", "extrude_i8.cu", "denoise_tc.cu"]
 HEADERS = ["atmos_kernels.cuh", "gemm_kernels.cuh", "gemm_tc.cuh", "gemm_tc_host.h", "rtc_kernels.cuh", "wfs_kernels.cuh", "wfs_params.cuh", "wind_host.h",
            "wfs_mma.cuh", "wfs_tma.cuh", "wfs_umma.cuh", "wfs_umma_ws.cuh", "wfs_umma_host.h", "extrude_i8.cuh", "extrude_i8_host.h", "geo_kernels.cuh",
-           "pupil_sweep.cuh", "denoise_kernels.cuh", "denoise_tc.cuh", "denoise_tc_host.h", "fft16.cuh", "twiddles.cuh", "rng.cuh", "../../include/aomarl.h"]
+           "pupil_sweep.cuh", "denoise_kernels.cuh", "denoise_tc.cuh", "denoise_tc_host.h", "fft16.cuh", "twiddles.cuh", "rng.cuh", "dispatch.h", "../../include/aomarl.h"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
 
 

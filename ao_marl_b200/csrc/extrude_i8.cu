@@ -2,6 +2,7 @@
 #define OZ_DEFINE_KERNELS
 #include <math.h>
 #include <string.h>
+#include "dispatch.h"
 #include "extrude_i8_host.h"
 
 static cudaError_t oz_attrs() {
@@ -18,8 +19,7 @@ static cudaError_t oz_attrs() {
 cudaError_t oz_extrude_launch(const OzGatherParams& g, const OzGemmParams& m, int MT, int NT, cudaStream_t st) {
   cudaError_t e = oz_attrs();
   if (e != cudaSuccess) return e;
-  if (g.steps) oz_gather_slice_kernel<true><<<g.E, 256, (size_t)g.KB * OZ_BK * sizeof(double), st>>>(g);
-  else oz_gather_slice_kernel<false><<<g.E, 256, (size_t)g.KB * OZ_BK * sizeof(double), st>>>(g);
+  with<false, true>(g.steps != nullptr, [&](auto PE) { oz_gather_slice_kernel<PE><<<g.E, 256, (size_t)g.KB * OZ_BK * sizeof(double), st>>>(g); });
   e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   oz_gemm_kernel<0, OZ_LEVELS><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);
@@ -32,9 +32,9 @@ cudaError_t oz_product_launch(const OzSliceParams& sl, const OzGemmParams& m, in
   oz_slice_rows_kernel<<<sl.E, 256, 0, st>>>(sl);
   e = cudaGetLastError();
   if (e != cudaSuccess) return e;
-  if (integrator && m.gain_env) oz_gemm_kernel<3, OZ_LEVELS_PRODUCT><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);
-  else if (integrator) oz_gemm_kernel<2, OZ_LEVELS_PRODUCT><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);
-  else oz_gemm_kernel<1, OZ_LEVELS_PRODUCT><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);
+  with<1, 2, 3>(!integrator ? 1 : m.gain_env ? 3 : 2, [&](auto EPI) {
+    oz_gemm_kernel<EPI, OZ_LEVELS_PRODUCT><<<dim3(NT, MT), OZ_THREADS, OZ_SMEM_BYTES, st>>>(m);
+  });
   return cudaGetLastError();
 }
 

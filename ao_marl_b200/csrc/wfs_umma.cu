@@ -1,9 +1,10 @@
 // Translation unit of the tcgen05 Shack-Hartmann frame kernel: instantiations per layer count + launch geometry.
 #include <string.h>
+#include "dispatch.h"
 #include "wfs_umma_host.h"
 #include "wfs_umma_ws.cuh"
 
-template <int NL, int FULL, int WS, bool PE, bool NE = false>
+template <int NL, int FULL, int WS, bool PE, bool NE>
 static cudaError_t launch_t(const WfsParams& p, const WfsUmmaHost& h, int num_sms, cudaStream_t st) {
   const long long total = (long long)p.E * p.nvalid;
   // persistent CTAs over contiguous ranges of work items: two CTAs per SM, about 4 waves, at least 8 iterations each
@@ -19,7 +20,7 @@ static cudaError_t launch_t(const WfsParams& p, const WfsUmmaHost& h, int num_sm
   P.f.items_per_cta = ipc;
   for (int l = 0; l < NL; ++l) P.maps[l] = h.maps[l];
   const size_t smem = wu_smem_bytes<NL, PE>(P.f.GW);
-  if (WS) {
+  if constexpr (WS != 0) {
     cudaError_t e = cudaFuncSetAttribute(wfs_frame_ws_kernel<NL, FULL, PE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     wfs_frame_ws_kernel<NL, FULL, PE><<<(unsigned)grid, WS_THREADS, smem, st>>>(P);
@@ -31,47 +32,19 @@ static cudaError_t launch_t(const WfsParams& p, const WfsUmmaHost& h, int num_sm
   return cudaGetLastError();
 }
 
-cudaError_t wfs_umma_launch(const WfsParams& p, const WfsUmmaHost& h, int num_sms, int full, int ws, cudaStream_t st) {
-  if (p.noise_env || p.nph_env) {     // per-environment sensor values: the fused kernel only (the library routes so)
-    if (ws) return cudaErrorInvalidValue;
-#define WU_GO_NE(NL, PE) return full ? launch_t<NL, 1, 0, PE, true>(p, h, num_sms, st) : launch_t<NL, 0, 0, PE, true>(p, h, num_sms, st)
-    if (p.wind && p.n_layers > 0) {
-      switch (p.n_layers) {
-        case 1: WU_GO_NE(1, true);
-        case 2: WU_GO_NE(2, true);
-        case 3: WU_GO_NE(3, true);
-        case 4: WU_GO_NE(4, true);
-      }
-      return cudaErrorInvalidValue;
-    }
-    switch (p.n_layers) {
-      case 0: WU_GO_NE(0, false);
-      case 1: WU_GO_NE(1, false);
-      case 2: WU_GO_NE(2, false);
-      case 3: WU_GO_NE(3, false);
-      case 4: WU_GO_NE(4, false);
-    }
-#undef WU_GO_NE
-    return cudaErrorInvalidValue;
-  }
-#define WU_GO(NL, PE) return ws ? launch_t<NL, 1, 1, PE>(p, h, num_sms, st) : full ? launch_t<NL, 1, 0, PE>(p, h, num_sms, st) \
-                                                                                : launch_t<NL, 0, 0, PE>(p, h, num_sms, st)
-  if (p.wind && p.n_layers > 0) {     // per-environment winds
-    switch (p.n_layers) {
-      case 1: WU_GO(1, true);
-      case 2: WU_GO(2, true);
-      case 3: WU_GO(3, true);
-      case 4: WU_GO(4, true);
-    }
-    return cudaErrorInvalidValue;
-  }
-  switch (p.n_layers) {
-    case 0: WU_GO(0, false);
-    case 1: WU_GO(1, false);
-    case 2: WU_GO(2, false);
-    case 3: WU_GO(3, false);
-    case 4: WU_GO(4, false);
-  }
-#undef WU_GO
-  return cudaErrorInvalidValue;
+cudaError_t wfs_umma_launch(const WfsParams& p, const WfsUmmaHost& h, int num_sms, bool ws, bool full, bool ne, cudaStream_t st) {
+  cudaError_t e = cudaErrorInvalidValue;
+  with<0, 1, 2, 3, 4>(p.n_layers, [&](auto NL) {
+    with<false, true>(p.wind && p.n_layers > 0, [&](auto PE) {
+      with<false, true>(ws, [&](auto WS) {
+        with<false, true>(full, [&](auto FULL) {
+          with<false, true>(ne, [&](auto NE) {
+            // per-environment winds need a layer; the specialised-warp kernel exists with FULL and without NE only
+            if constexpr ((NL > 0 || !PE) && (!WS || (FULL && !NE))) e = launch_t<NL, FULL, WS, PE, NE>(p, h, num_sms, st);
+          });
+        });
+      });
+    });
+  });
+  return e;
 }

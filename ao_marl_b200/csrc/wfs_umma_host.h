@@ -10,9 +10,9 @@ struct WfsUmmaHost {
   CUtensorMap maps[WU_MAX_LAYERS];
 };
 
-// Launches wfs_frame_umma_kernel for the frame described by p.  full != 0: fp32-grade products in both stages.
+// Launches wfs_frame_umma_kernel for the frame described by p.  full: fp32-grade products in both stages.
 // Returns cudaSuccess or the error of the attribute / launch call.
-// ws != 0: the warp-specialised kernel (wfs_umma_ws.cuh) on the same tables.  p.wind != null: the per-environment wind
-// instantiations of either kernel.  p.noise_env / p.nph_env != null: the per-environment sensor instantiations of the fused
-// kernel (ws must be 0).
-cudaError_t wfs_umma_launch(const WfsParams& p, const WfsUmmaHost& h, int num_sms, int full, int ws, cudaStream_t st);
+// ws: the warp-specialised kernel (wfs_umma_ws.cuh) on the same tables (needs full and not ne).  p.wind != null: the
+// per-environment wind instantiations of either kernel.  ne: the per-environment sensor instantiations of the fused
+// kernel, which read p.noise_env / p.nph_env.
+cudaError_t wfs_umma_launch(const WfsParams& p, const WfsUmmaHost& h, int num_sms, bool ws, bool full, bool ne, cudaStream_t st);

@@ -305,9 +305,10 @@ int aom_set_wfs_noise(aom_ctx* ctx, float noise, float nphotons);
  * Waits for the device; not for the step path. */
 int aom_set_wfs_noise_env(aom_ctx* ctx, const float* noise_host, const float* nphotons_host);
 
-/* Name of the kernel the next aom_comp_wfs_image will launch under the current AOM_OPT_WFS_PATH
- * ("wfs_frame_umma_kernel", "wfs_frame_tma_kernel", "wfs_frame_mma_kernel" or "wfs_frame_kernel"); when the staged kernel is not
- * eligible for the geometry, aom_last_error() says why. */
+/* Name of the kernel a noise-free aom_comp_wfs_image without kept image launches under the current AOM_OPT_WFS_PATH
+ * ("wfs_frame_ws_kernel", "wfs_frame_umma_kernel", "wfs_frame_tma_kernel", "wfs_frame_mma_kernel" or "wfs_frame_kernel"), the
+ * path's kernel also where the per-environment state makes that frame refused; when the staged kernel is not eligible for the
+ * geometry, aom_last_error() says why. */
 const char* aom_wfs_kernel(aom_ctx* ctx);
 
 /* Mean device time (ms) of the sensor-kernel launches recorded since the last call (AOM_OPT_TIME_WFS; at most
