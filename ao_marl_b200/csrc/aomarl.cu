@@ -15,6 +15,7 @@
 #include "rtc_kernels.cuh"
 #include "wfs_kernels.cuh"
 #include "wfs_mma.cuh"
+#include "wfs_lattice_host.h"
 #include "wfs_tma.cuh"
 #include "wfs_umma_host.h"
 #include "extrude_i8_host.h"
@@ -124,17 +125,17 @@ struct aom_ctx {
   uint32_t* step_env;          // device [E] actor decision counters
   int* le_n;                   // device [2][E] long-exposure counts (main target, geometric target)
   int* first;                  // device [E] first step pending
-  // TMA-staged Shack-Hartmann kernel (wfs_tma.cuh): host copies of the tables it derives from, derived tables
+  // staged Shack-Hartmann kernels: host copies of the tables their own tables derive from; fast_why says why the last
+  // refused preparation refused
   void* htab[AOM_T_COUNT];
   size_t htab_bytes[AOM_T_COUNT];
-  int fast_state;            // 0 = not prepared, 1 = eligible, -1 = not eligible (fast_why says why)
   char fast_why[160];
+  // TMA-staged kernel (wfs_tma.cuh): derived tables
+  int fast_state;            // 0 = not prepared, 1 = eligible, -1 = not eligible
   WfsFast fast;
   void* fast_dev[6];
   CUtensorMap fast_maps[WFT_MAX_LAYERS];
-  size_t fast_smem;
-  int fast_geom[6];          // joffx, joffy, c0x, c0y, GW, dm (lattice alignment of the subapertures, wfs_fast_prepare)
-  // tcgen05 Shack-Hartmann kernel (wfs_umma.cuh): derived tables
+  // tcgen05 kernels (wfs_umma.cuh, wfs_umma_ws.cuh): derived tables
   int umma_state;            // 0 = not prepared, 1 = eligible, -1 = not eligible
   WfsUmmaHost umma;
   void* umma_dev[6];
@@ -1112,7 +1113,9 @@ extern "C" int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const in
 }
 
 // ---------------------------------------------------------------------------------------------
-// Host side of wfs_frame_tma_kernel (wfs_tma.cuh): eligibility, derived tables, TMA descriptors.
+// Host side of the staged sensor kernels, wfs_frame_tma_kernel (wfs_tma.cuh) and the tcgen05 pair (wfs_umma.cuh,
+// wfs_umma_ws.cuh): eligibility, derived tables, TMA descriptors.  Both read the mirror through the same lattice
+// analysis (wfs_lattice_host.h) and lay out its tables their own way.
 static uint32_t half2_bits(float a, float b) {
   __half2 h = __floats2half2_rn(a, b);
   uint32_t u;
@@ -1137,84 +1140,83 @@ typedef CUresult (*aom_encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuin
                                         const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                         CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-#define FAST_NO(...)                                             \
-  do {                                                           \
-    snprintf(ctx->fast_why, sizeof(ctx->fast_why), __VA_ARGS__); \
-    ctx->fast_state = -1;                                        \
-    return AOM_OK;                                               \
-  } while (0)
+// A staged kernel cannot serve this configuration: its state becomes -1 and fast_why says why.  Returns AOM_OK.
+static int staged_refuse(aom_ctx* ctx, int& state, const char* fmt, ...) {
+  va_list ap;
+  va_start(ap, fmt);
+  vsnprintf(ctx->fast_why, sizeof(ctx->fast_why), fmt, ap);
+  va_end(ap);
+  state = -1;
+  return AOM_OK;
+}
+
+// The lattice analysis of the uploaded host tables: null, or why the staged kernels cannot serve them
+static const char* staged_lattice(aom_ctx* ctx, WfsLattice& L) {
+  return wfl_analyse(ctx->cfg, (const float*)ctx->htab[AOM_T_MPUPIL], (const int*)ctx->htab[AOM_T_SUB_X0],
+                     (const int*)ctx->htab[AOM_T_SUB_Y0], (const float*)ctx->htab[AOM_T_STAMP1D],
+                     (const int*)ctx->htab[AOM_T_ACT_MAP], L);
+}
+
+// One 3-D map [E][N][N] per screen layer, box bw x bh x 1, zero fill outside.  False: refused (state, fast_why).
+static bool encode_screen_maps(aom_ctx* ctx, CUtensorMap* maps, cuuint32_t bw, cuuint32_t bh, int& state) {
+  const aom_config& c = ctx->cfg;
+  if (c.n_layers == 0) return true;
+  void* fn = nullptr;
+  cudaDriverEntryPointQueryResult qres;
+  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn ||
+      qres != cudaDriverEntryPointSuccess) {
+    staged_refuse(ctx, state, "cuTensorMapEncodeTiled not available");
+    return false;
+  }
+  for (int l = 0; l < c.n_layers; ++l) {
+    const cuuint64_t N = (cuuint64_t)c.screen_dim[l];
+    const cuuint64_t dims[3] = {N, N, (cuuint64_t)c.n_env};
+    const cuuint64_t strides[2] = {N * 4, N * N * 4};
+    const cuuint32_t box[3] = {bw, bh, 1};
+    const cuuint32_t estr[3] = {1, 1, 1};
+    CUresult r = ((aom_encode_tiled_fn)fn)(&maps[l], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ctx->screen[l], dims, strides, box,
+                                           estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+      staged_refuse(ctx, state, "cuTensorMapEncodeTiled failed (%d)", (int)r);
+      return false;
+    }
+  }
+  return true;
+}
+
+// Copies the six host tables src[i] of bytes[i] into new device buffers dev[i]
+static cudaError_t upload_tables(void* (&dev)[6], const void* const (&src)[6], const size_t (&bytes)[6]) {
+  cudaError_t ce = cudaSuccess;
+  for (int i = 0; i < 6 && ce == cudaSuccess; ++i) {
+    ce = cudaMalloc(&dev[i], bytes[i]);
+    if (ce == cudaSuccess) ce = cudaMemcpy(dev[i], src[i], bytes[i], cudaMemcpyHostToDevice);
+  }
+  return ce;
+}
 
 static int wfs_fast_prepare(aom_ctx* ctx) {
   const aom_config& c = ctx->cfg;
   if (ctx->fast_state != 0) return AOM_OK;
   for (void*& b : ctx->fast_dev) { cudaFree(b); b = nullptr; }
-  if (c.nfft != 64 || c.nrebin != 2) FAST_NO("Nfft != 64");
-  if (c.n_layers > WFT_MAX_LAYERS) FAST_NO("more than %d layers", WFT_MAX_LAYERS);
-  if (c.pzt_pitch != 16) FAST_NO("actuator pitch is not 16 pixels");
-  if (c.nvalid > 65535 / 256 * 256 || c.n > 65535) FAST_NO("geometry too large for the packed tables");
-  if ((c.tt_dim & 3) || c.tt_dim <= 0) FAST_NO("tip-tilt support not a multiple of 4");
+  WfsLattice L;
+  if (const char* why = staged_lattice(ctx, L)) return staged_refuse(ctx, ctx->fast_state, "%s", why);
   const float* pup = (const float*)ctx->htab[AOM_T_MPUPIL];
   const int* sx = (const int*)ctx->htab[AOM_T_SUB_X0];
   const int* sy = (const int*)ctx->htab[AOM_T_SUB_Y0];
   const float* stamp = (const float*)ctx->htab[AOM_T_STAMP1D];
-  const int* amap = (const int*)ctx->htab[AOM_T_ACT_MAP];
-  if (!pup || !sx || !sy) FAST_NO("sensor tables not uploaded");
-  const bool dm = stamp && amap;
-  for (int l = 0; l < c.n_layers; ++l)
-    if (c.screen_dim[l] & 3) FAST_NO("screen side not a multiple of 4");
-  for (size_t i = 0; i < (size_t)c.n * c.n; ++i)
-    if (pup[i] != 0.f && pup[i] != 1.f) FAST_NO("pupil transmission is not binary");
-  const int ss = c.stamp_size, nv = c.nvalid;
-  int cx = 0, cy = 0;
-  for (int k = 0; k < nv; ++k) {
-    if (sx[k] < 0 || sy[k] < 0 || sx[k] + 16 > c.n || sy[k] + 16 > c.n) FAST_NO("subaperture outside the pupil frame");
-    if ((sx[k] + c.tt_off) & 3) FAST_NO("tip-tilt rows not 16-byte aligned");
-    const int mx = (((sx[k] + c.pzt_off - c.pzt_i1_0) % 16) + 16) % 16, my = (((sy[k] + c.pzt_off - c.pzt_j1_0) % 16) + 16) % 16;
-    if (k == 0) { cx = mx; cy = my; }
-    if (mx != cx || my != cy) FAST_NO("subapertures not aligned with the actuator lattice");
-  }
-  // lattice cells j = 0 .. NG-1 from gx_lo = m - joff, m = (X0 - cx) / 16; stamp index a = c0 + x - 16 j
-  auto axis = [&](int cm, int& joff, int& c0, int& ng) {
-    const int num = cm - (ss - 1);                       // ceil(num / 16) = -joff
-    joff = -((num >= 0) ? (num + 15) / 16 : -((-num) / 16));
-    c0 = cm + 16 * joff;
-    ng = (c0 + 15) / 16 + 1;
-  };
-  int joffx = 0, joffy = 0, c0x = 0, c0y = 0, ngx = 0, ngy = 0;
-  if (dm) {
-    axis(cx, joffx, c0x, ngx);
-    axis(cy, joffy, c0y, ngy);
-    if (ngx > WFT_NG || ngy > WFT_NG) FAST_NO("stamp spans more than %d lattice cells", WFT_NG);
-  }
-  const int GW = c.pzt_grid_n + 2 * WFT_PAD;
-  if ((size_t)GW * GW * 2 > 16384) FAST_NO("actuator lattice too large");
-
-  // ---- derived tables ----
+  const int nv = c.nvalid, GW = L.GW;
   uint2* h_sub = (uint2*)malloc((size_t)nv * sizeof(uint2));
   unsigned char* h_pm = (unsigned char*)malloc((size_t)nv * 32);
   short* h_amap = (short*)malloc((size_t)GW * GW * sizeof(short));
   float h_fxy[2 * WFT_NG * 16];
   uint4* h_c1 = (uint4*)malloc(8 * 32 * sizeof(uint4));
   uint4* h_c2 = (uint4*)malloc(12 * 32 * sizeof(uint4));
-  bool ok = h_sub && h_pm && h_amap && h_c1 && h_c2;
+  const bool ok = h_sub && h_pm && h_amap && h_c1 && h_c2;
   if (ok) {
-    for (int i = 0; i < GW * GW; ++i) h_amap[i] = -1;
-    if (dm)
-      for (int gy = 0; gy < c.pzt_grid_n; ++gy)
-        for (int gx = 0; gx < c.pzt_grid_n; ++gx) {
-          const int a = amap[gy * c.pzt_grid_n + gx];
-          if (a > 32767) ok = false;
-          h_amap[(gy + WFT_PAD) * GW + gx + WFT_PAD] = (short)a;
-        }
-    for (int k = 0; k < nv && ok; ++k) {
-      int gb = 0;
-      if (dm) {
-        const int gxl = (sx[k] + c.pzt_off - c.pzt_i1_0 - cx) / 16 - joffx + WFT_PAD;   // exact multiples of 16
-        const int gyl = (sy[k] + c.pzt_off - c.pzt_j1_0 - cy) / 16 - joffy + WFT_PAD;
-        if (gxl < 0 || gyl < 0 || gxl + WFT_NG > GW || gyl + WFT_NG > GW) { ok = false; break; }
-        gb = gyl * GW + gxl;
-      }
-      h_sub[k] = make_uint2(((uint32_t)sy[k] << 16) | (uint32_t)sx[k], (uint32_t)gb);
+    wfl_amap(c, L, (const int*)ctx->htab[AOM_T_ACT_MAP], h_amap);
+    for (int k = 0; k < nv; ++k) {
+      h_sub[k] = make_uint2(((uint32_t)sy[k] << 16) | (uint32_t)sx[k], (uint32_t)wfl_window(c, L, sx[k], sy[k]));
       for (int lane = 0; lane < 32; ++lane) {
         const int g = lane >> 2, q = lane & 3;
         unsigned m = 0;
@@ -1226,10 +1228,7 @@ static int wfs_fast_prepare(aom_ctx* ctx) {
     }
     for (int ax = 0; ax < 2; ++ax)
       for (int j = 0; j < WFT_NG; ++j)
-        for (int x = 0; x < 16; ++x) {
-          const int a = (ax ? c0y : c0x) + x - 16 * j;
-          h_fxy[(ax * WFT_NG + j) * 16 + x] = (dm && a >= 0 && a < ss) ? stamp[a] : 0.f;
-        }
+        for (int x = 0; x < 16; ++x) h_fxy[(ax * WFT_NG + j) * 16 + x] = wfl_factor(c, L, stamp, ax, j, x);
     // stage-1 A fragments: row r of m-tile mt <-> kept frequency 16 mt + 2 (r & 7) + (r >> 3); k <-> x = sigma(k)
     auto sigma = [](int kk) { return kk < 8 ? 4 * (kk >> 1) + (kk & 1) : 4 * ((kk - 8) >> 1) + 2 + (kk & 1); };
     auto yk = [](int kk) { return kk < 8 ? 2 * kk : 2 * (kk - 8) + 1; };
@@ -1265,37 +1264,14 @@ static int wfs_fast_prepare(aom_ctx* ctx) {
         h_c2[(b * 3 + 2) * 32 + lane] = make_uint4(nh[0], nh[1], nl[0], nl[1]);
       }
   }
-  cudaError_t ce = cudaSuccess;
-  const void* srcs[6] = {h_sub, h_amap, h_pm, h_c1, h_c2, h_fxy};
+  const void* const srcs[6] = {h_sub, h_amap, h_pm, h_c1, h_c2, h_fxy};
   const size_t sizes[6] = {(size_t)nv * sizeof(uint2), (size_t)GW * GW * sizeof(short), (size_t)nv * 32,
                            8 * 32 * sizeof(uint4), 12 * 32 * sizeof(uint4), sizeof(h_fxy)};
-  for (int i = 0; i < 6 && ok && ce == cudaSuccess; ++i) {
-    ce = cudaMalloc(&ctx->fast_dev[i], sizes[i]);
-    if (ce == cudaSuccess) ce = cudaMemcpy(ctx->fast_dev[i], srcs[i], sizes[i], cudaMemcpyHostToDevice);
-  }
+  const cudaError_t ce = ok ? upload_tables(ctx->fast_dev, srcs, sizes) : cudaSuccess;
   free(h_sub); free(h_pm); free(h_amap); free(h_c1); free(h_c2);
   if (ce != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "wfs_fast_prepare: %s", cudaGetErrorString(ce));
-  if (!ok) FAST_NO("derived tables out of range");
-
-  // ---- TMA descriptors: one 3-D map [E][N][N] per layer, box 24 x 17 x 1, zero fill outside ----
-  if (c.n_layers > 0) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn ||
-        qres != cudaDriverEntryPointSuccess)
-      FAST_NO("cuTensorMapEncodeTiled not available");
-    for (int l = 0; l < c.n_layers; ++l) {
-      const cuuint64_t N = (cuuint64_t)c.screen_dim[l];
-      const cuuint64_t dims[3] = {N, N, (cuuint64_t)c.n_env};
-      const cuuint64_t strides[2] = {N * 4, N * N * 4};
-      const cuuint32_t box[3] = {WFT_TILE_W, WFT_TILE_H, 1};
-      const cuuint32_t estr[3] = {1, 1, 1};
-      CUresult r = ((aom_encode_tiled_fn)fn)(&ctx->fast_maps[l], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ctx->screen[l], dims,
-                                             strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                             CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) FAST_NO("cuTensorMapEncodeTiled failed (%d)", (int)r);
-    }
-  }
+  if (!ok) return staged_refuse(ctx, ctx->fast_state, "out of host memory");
+  if (!encode_screen_maps(ctx, ctx->fast_maps, WFT_TILE_W, WFT_TILE_H, ctx->fast_state)) return AOM_OK;
   WfsFast& f = ctx->fast;
   f.sub = (const uint2*)ctx->fast_dev[0];
   f.amap = (const short*)ctx->fast_dev[1];
@@ -1306,21 +1282,9 @@ static int wfs_fast_prepare(aom_ctx* ctx) {
   f.GW = GW;
   f.sub_in_smem = (nv <= 1280) ? 1 : 0;
   f.err = ctx->d_err;
-  ctx->fast_geom[0] = joffx; ctx->fast_geom[1] = joffy; ctx->fast_geom[2] = c0x; ctx->fast_geom[3] = c0y;
-  ctx->fast_geom[4] = GW; ctx->fast_geom[5] = dm ? 1 : 0;
   ctx->fast_state = 1;
-  ctx->fast_why[0] = 0;
   return AOM_OK;
 }
-
-// Host side of wfs_frame_umma_kernel (wfs_umma.cuh): same eligibility as the staged kernel plus an analytic
-// half-pixel phasor; derived tables in the (h, y) lane layout, operand tiles of the two DFT stages, 20 x 17 TMA boxes.
-#define UMMA_NO(...)                                             \
-  do {                                                           \
-    snprintf(ctx->fast_why, sizeof(ctx->fast_why), __VA_ARGS__); \
-    ctx->umma_state = -1;                                        \
-    return AOM_OK;                                               \
-  } while (0)
 
 static void umma_put_half(unsigned short* tile_hi, unsigned short* tile_lo, int n, int kk, double v) {
   // UMMA canonical K-major no-swizzle layout: 8-row x 16-byte core matrices, LBO 128 B, SBO 512 B (K = 32 halves)
@@ -1331,54 +1295,36 @@ static void umma_put_half(unsigned short* tile_hi, unsigned short* tile_lo, int 
   memcpy((unsigned char*)tile_lo + off, &lo, 2);
 }
 
+// The tcgen05 kernels also need a full group of subapertures and the analytic half-pixel phasor; their tables are in the
+// (h, y) lane layout, with the operand tiles of the two DFT stages and 20 x 17 TMA boxes.
 static int wfs_umma_prepare(aom_ctx* ctx) {
   const aom_config& c = ctx->cfg;
   if (ctx->umma_state != 0) return AOM_OK;
-  int rc = wfs_fast_prepare(ctx);
-  if (rc) return rc;
   for (void*& b : ctx->umma_dev) { cudaFree(b); b = nullptr; }
-  if (ctx->fast_state != 1) { ctx->umma_state = -1; return AOM_OK; }      // fast_why already says why
-  if (c.nvalid < WU_WARPS) UMMA_NO("fewer than %d subapertures", WU_WARPS);
-  if (c.n_layers > WU_MAX_LAYERS) UMMA_NO("more than %d layers", WU_MAX_LAYERS);
+  WfsLattice L;
+  if (const char* why = staged_lattice(ctx, L)) return staged_refuse(ctx, ctx->umma_state, "%s", why);
+  if (c.nvalid < WU_WARPS) return staged_refuse(ctx, ctx->umma_state, "fewer than %d subapertures", WU_WARPS);
   const float* hxy = (const float*)ctx->htab[AOM_T_HALFXY];
-  if (!hxy) UMMA_NO("half-pixel phasor table not uploaded");
+  if (!hxy) return staged_refuse(ctx, ctx->umma_state, "half-pixel phasor table not uploaded");
   for (int i = 0; i < 16; ++i)
     for (int j = 0; j < 16; ++j)
-      if (fabs((double)hxy[i * 16 + j] - M_PI * (double)(i + j) / 64.0) > 2e-6) UMMA_NO("half-pixel phasor is not pi (x + y) / Nfft");
+      if (fabs((double)hxy[i * 16 + j] - M_PI * (double)(i + j) / 64.0) > 2e-6)
+        return staged_refuse(ctx, ctx->umma_state, "half-pixel phasor is not pi (x + y) / Nfft");
   const float* pup = (const float*)ctx->htab[AOM_T_MPUPIL];
   const int* sx = (const int*)ctx->htab[AOM_T_SUB_X0];
   const int* sy = (const int*)ctx->htab[AOM_T_SUB_Y0];
   const float* stamp = (const float*)ctx->htab[AOM_T_STAMP1D];
-  const int* amap = (const int*)ctx->htab[AOM_T_ACT_MAP];
-  const int joffx = ctx->fast_geom[0], joffy = ctx->fast_geom[1], c0x = ctx->fast_geom[2], c0y = ctx->fast_geom[3];
-  const int GW = ctx->fast_geom[4];
-  const bool dm = ctx->fast_geom[5] != 0;
-  const int ss = c.stamp_size, nv = c.nvalid;
-  int cx = 0, cy = 0;
-  if (nv > 0) {
-    cx = (((sx[0] + c.pzt_off - c.pzt_i1_0) % 16) + 16) % 16;
-    cy = (((sy[0] + c.pzt_off - c.pzt_j1_0) % 16) + 16) % 16;
-  }
+  const int nv = c.nvalid, GW = L.GW;
   uint2* h_sub = (uint2*)malloc((size_t)nv * sizeof(uint2));
   uint32_t* h_pm = (uint32_t*)malloc((size_t)nv * 32 * sizeof(uint32_t));
   short* h_amap = (short*)malloc((size_t)GW * GW * sizeof(short));
   unsigned short* h_b1 = (unsigned short*)calloc(2 * WU_B_BYTES, 1);     // [hi, lo] tiles of WU_B_BYTES each
   unsigned short* h_b2 = (unsigned short*)calloc(2 * WU_B_BYTES, 1);
   float h_fxy[2 * WU_NG * 16];
-  bool ok = h_sub && h_pm && h_amap && h_b1 && h_b2;
+  const bool ok = h_sub && h_pm && h_amap && h_b1 && h_b2;
   if (ok) {
-    for (int i = 0; i < GW * GW; ++i) h_amap[i] = -1;
-    if (dm)
-      for (int gy = 0; gy < c.pzt_grid_n; ++gy)
-        for (int gx = 0; gx < c.pzt_grid_n; ++gx)
-          h_amap[(gy + WU_PAD) * GW + gx + WU_PAD] = (short)amap[gy * c.pzt_grid_n + gx];
+    wfl_amap(c, L, (const int*)ctx->htab[AOM_T_ACT_MAP], h_amap);
     for (int k = 0; k < nv; ++k) {
-      int gb = 0;
-      if (dm) {
-        const int gxl = (sx[k] + c.pzt_off - c.pzt_i1_0 - cx) / 16 - joffx + WU_PAD;
-        const int gyl = (sy[k] + c.pzt_off - c.pzt_j1_0 - cy) / 16 - joffy + WU_PAD;
-        gb = gyl * GW + gxl;
-      }
       bool full = true;
       for (int lane = 0; lane < 32; ++lane) {
         const int yy = lane & 15, hh = lane >> 4;
@@ -1388,14 +1334,14 @@ static int wfs_umma_prepare(aom_ctx* ctx) {
         h_pm[(size_t)k * 32 + lane] = m;
         full = full && m == 0xffu;
       }
-      h_sub[k] = make_uint2(((uint32_t)sy[k] << 16) | (uint32_t)sx[k], (uint32_t)gb | (full ? 0x80000000u : 0u));
+      h_sub[k] = make_uint2(((uint32_t)sy[k] << 16) | (uint32_t)sx[k],
+                            (uint32_t)wfl_window(c, L, sx[k], sy[k]) | (full ? 0x80000000u : 0u));
     }
     // x stamp factors [j][x], y stamp factors transposed [y][j]
     for (int j = 0; j < WU_NG; ++j)
       for (int x = 0; x < 16; ++x) {
-        const int ax = c0x + x - 16 * j, ay = c0y + x - 16 * j;
-        h_fxy[j * 16 + x] = (dm && ax >= 0 && ax < ss) ? stamp[ax] : 0.f;
-        h_fxy[WU_NG * 16 + x * WU_NG + j] = (dm && ay >= 0 && ay < ss) ? stamp[ay] : 0.f;
+        h_fxy[j * 16 + x] = wfl_factor(c, L, stamp, 0, j, x);
+        h_fxy[WU_NG * 16 + x * WU_NG + j] = wfl_factor(c, L, stamp, 1, j, x);
       }
     // stage 1: B1[n = 32 ro + fx][k = 16 ri + x]:  Tr = Wr Xr - Wi Xi ; Ti = Wi Xr + Wr Xi
     // stage 2: B2[n = 2 fy + po][k = 16 ro + y]:   Yr = Tr Wr - Ti Wi ; Yi = Tr Wi + Ti Wr
@@ -1415,35 +1361,14 @@ static int wfs_umma_prepare(aom_ctx* ctx) {
         }
       }
   }
-  cudaError_t ce = cudaSuccess;
-  const void* srcs[6] = {h_sub, h_amap, h_pm, h_b1, h_b2, h_fxy};
+  const void* const srcs[6] = {h_sub, h_amap, h_pm, h_b1, h_b2, h_fxy};
   const size_t sizes[6] = {(size_t)nv * sizeof(uint2), (size_t)GW * GW * sizeof(short), (size_t)nv * 32 * sizeof(uint32_t),
                            (size_t)2 * WU_B_BYTES, (size_t)2 * WU_B_BYTES, sizeof(h_fxy)};
-  for (int i = 0; i < 6 && ok && ce == cudaSuccess; ++i) {
-    ce = cudaMalloc(&ctx->umma_dev[i], sizes[i]);
-    if (ce == cudaSuccess) ce = cudaMemcpy(ctx->umma_dev[i], srcs[i], sizes[i], cudaMemcpyHostToDevice);
-  }
+  const cudaError_t ce = ok ? upload_tables(ctx->umma_dev, srcs, sizes) : cudaSuccess;
   free(h_sub); free(h_pm); free(h_amap); free(h_b1); free(h_b2);
   if (ce != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "wfs_umma_prepare: %s", cudaGetErrorString(ce));
-  if (!ok) UMMA_NO("out of host memory");
-  if (c.n_layers > 0) {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn ||
-        qres != cudaDriverEntryPointSuccess)
-      UMMA_NO("cuTensorMapEncodeTiled not available");
-    for (int l = 0; l < c.n_layers; ++l) {
-      const cuuint64_t N = (cuuint64_t)c.screen_dim[l];
-      const cuuint64_t dims[3] = {N, N, (cuuint64_t)c.n_env};
-      const cuuint64_t strides[2] = {N * 4, N * N * 4};
-      const cuuint32_t box[3] = {WU_TILE_W, WU_TILE_H, 1};
-      const cuuint32_t estr[3] = {1, 1, 1};
-      CUresult r = ((aom_encode_tiled_fn)fn)(&ctx->umma.maps[l], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ctx->screen[l], dims,
-                                             strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                             CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) UMMA_NO("cuTensorMapEncodeTiled failed (%d)", (int)r);
-    }
-  }
+  if (!ok) return staged_refuse(ctx, ctx->umma_state, "out of host memory");
+  if (!encode_screen_maps(ctx, ctx->umma.maps, WU_TILE_W, WU_TILE_H, ctx->umma_state)) return AOM_OK;
   WfsUmmaTables& f = ctx->umma.f;
   memset(&f, 0, sizeof(f));
   f.sub = (const uint2*)ctx->umma_dev[0];
@@ -1454,22 +1379,18 @@ static int wfs_umma_prepare(aom_ctx* ctx) {
   f.fxy = (const float*)ctx->umma_dev[5];
   f.GW = GW;
   f.err = ctx->d_err;
-  {
-    const char* sw = getenv("AOM_UMMA_SWAP");
-    f.a2_swap = (sw && sw[0] == '1') ? 1 : 0;
-  }
   ctx->umma_state = 1;
   return AOM_OK;
 }
 
-template <int FULL, int NL, int NW = WFT_WARPS, int MINB = 2, int NST = 2, int TOKEN = 0>
+template <int FULL, int NL>
 static int wfs_fast_launch_t(aom_ctx* ctx, const WfsParams& p, cudaStream_t st) {
   const long long total = (long long)p.E * p.nvalid;
-  // contiguous ranges of work items per CTA: about 8 waves of MINB CTAs per SM, at least 16 items per warp
-  long long grid = (long long)ctx->num_sms * MINB * 8;
+  // contiguous ranges of work items per CTA: about 8 waves of resident CTAs per SM, at least 16 items per warp
+  long long grid = (long long)ctx->num_sms * WFT_MIN_CTAS * 8;
   long long ipc = (total + grid - 1) / grid;
-  if (ipc < 16 * NW) ipc = 16 * NW;
-  ipc = (ipc + NW - 1) / NW * NW;
+  if (ipc < 16 * WFT_WARPS) ipc = 16 * WFT_WARPS;
+  ipc = (ipc + WFT_WARPS - 1) / WFT_WARPS * WFT_WARPS;
   grid = (total + ipc - 1) / ipc;
   WfsTmaParams P;
   memset(&P, 0, sizeof(P));
@@ -1477,12 +1398,12 @@ static int wfs_fast_launch_t(aom_ctx* ctx, const WfsParams& p, cudaStream_t st) 
   P.f = ctx->fast;
   P.f.items_per_cta = ipc;
   for (int l = 0; l < NL; ++l) P.maps[l] = ctx->fast_maps[l];
-  const size_t smem = wft_smem_bytes<NL, NW, NST>(P.f.GW, P.f.sub_in_smem ? p.nvalid : 0);
+  const size_t smem = wft_smem_bytes<NL>(P.f.GW, P.f.sub_in_smem ? p.nvalid : 0);
   {
-    cudaError_t e = cudaFuncSetAttribute(wfs_frame_tma_kernel<FULL, NL, NW, MINB, NST, TOKEN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(wfs_frame_tma_kernel<FULL, NL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "cudaFuncSetAttribute(wfs_frame_tma_kernel): %s", cudaGetErrorString(e));
   }
-  wfs_frame_tma_kernel<FULL, NL, NW, MINB, NST, TOKEN><<<(unsigned)grid, NW * 32, smem, st>>>(P);
+  wfs_frame_tma_kernel<FULL, NL><<<(unsigned)grid, WFT_WARPS * 32, smem, st>>>(P);
   return AOM_OK;
 }
 
@@ -1551,7 +1472,7 @@ struct WfsRoute {
 };
 
 // Routes a frame of parameters p (fill_wfs_params), noisy when any environment draws noise in it, with its image kept or
-// not.  Prepares the tables of the staged paths on first use.
+// not.  Prepares the tables of a staged kernel on first use, and the round-1 kernel's only when the route can reach it.
 static int wfs_route(aom_ctx* ctx, const WfsParams& p, bool noisy, bool keep, WfsRoute& r) {
   const aom_config& c = ctx->cfg;
   const int path = ctx->opt[AOM_OPT_WFS_PATH];
@@ -1567,8 +1488,8 @@ static int wfs_route(aom_ctx* ctx, const WfsParams& p, bool noisy, bool keep, Wf
     r.r = c.nfft / 16;
     return AOM_OK;
   }
-  if (staged) {
-    int rc = umma ? wfs_umma_prepare(ctx) : wfs_fast_prepare(ctx);
+  if (umma) {
+    int rc = wfs_umma_prepare(ctx);
     if (rc) return rc;
   }
   if (umma && ctx->umma_state == 1) {
@@ -1577,6 +1498,10 @@ static int wfs_route(aom_ctx* ctx, const WfsParams& p, bool noisy, bool keep, Wf
     r.family = (path == AOM_WFS_UMMA_WS && !noisy && !keep) ? WFS_WS : WFS_UMMA;
     if (r.family == WFS_WS) r.ne = false;
     return AOM_OK;
+  }
+  if (staged) {
+    int rc = wfs_fast_prepare(ctx);
+    if (rc) return rc;
   }
   r.family = (staged && ctx->fast_state == 1) ? WFS_TMA : WFS_MMA;
   if (r.family == WFS_MMA && r.nl != 0 && r.nl != 1 && r.nl != 3) r.nl = -1;

@@ -21,7 +21,7 @@
 //     subaperture is prefetched one iteration ahead;
 //   * the pupil mask is one byte per lane per subaperture.
 //
-// Eligibility is decided on the host (aomarl.cu: wfs_fast_prepare); other geometries keep wfs_frame_mma_kernel.
+// Eligibility is decided on the host (wfs_lattice_host.h); other geometries keep wfs_frame_mma_kernel.
 // Replaces sutra's raytrace + fillcamplipup + cuFFT + abs2 + fillbincube + noise + centroid kernels behind
 // WfsCompass.raytrace / compute_wfs_image / RtcCompass.do_centroids (shesha/supervisor/components/
 // wfsCompass.py:334-343, sourceCompass.py:54-85, rtcCompass.py:557-563).
@@ -30,20 +30,21 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include "wfs_mma.cuh"
+#include "wfs_lattice_host.h"
 
 #define WFT_WARPS 8
+#define WFT_MIN_CTAS 2
 #define WFT_TILE_W 24                      // box width (floats): 17 needed, padded so that rows are 96 B apart
 #define WFT_TILE_H 17
 #define WFT_TILE_BYTES (WFT_TILE_W * WFT_TILE_H * 4)          // 1632 = bytes one box delivers
 #define WFT_TILE_STRIDE 1664                                  // 13 x 128: TMA destinations stay 128-byte aligned
-#define WFT_NG 4                           // lattice cells per axis whose stamp meets one subaperture
-#define WFT_PAD 4                          // border of the padded actuator map
-#define WFT_MAX_LAYERS 4
+#define WFT_NG WFL_NG
+#define WFT_MAX_LAYERS WFL_MAX_LAYERS
 #define WFT_WAIT_SPINS (1u << 22)
 
 struct WfsFast {
   const uint2* sub;          // [nvalid] {y0 << 16 | x0, padded-lattice index of the neighbourhood origin}
-  const short* amap;         // [GW * GW] actuator index or -1 (padded by WFT_PAD cells on every side)
+  const short* amap;         // [GW * GW] actuator index or -1 (padded by WFL_PAD cells on every side)
   const unsigned char* pmask;// [nvalid][32] bit r*4+c = pupil(2g + r, 4q + c) of lane (g, q)
   const uint4* c1;           // [8][32]  stage-1 A fragments  [(mt*2 + part)*2 + hl][lane]
   const uint4* c2;           // [12][32] stage-2 B fragments  [b*3 + {hi, lo, -Wi}][lane]
@@ -51,7 +52,6 @@ struct WfsFast {
   int GW;                    // side of the padded actuator map
   int sub_in_smem;           // stage the subaperture table in shared memory
   int* err;                  // device error word (bounded waits)
-  int dbg;                   // unused (development switches of round 1, see DESIGN.md section 4)
   long long items_per_cta;
 };
 
@@ -122,34 +122,26 @@ __device__ __forceinline__ void wft_layer(const float* __restrict__ t, const Wfs
     }
 }
 
-// NW warps per CTA, NST tile stages per warp (the volt buffers are always double)
-template <int NL, int NW = WFT_WARPS, int NST = 2>
+// WFT_WARPS warps per CTA, two tile stages and two volt buffers per warp
+template <int NL>
 constexpr size_t wft_smem_bytes(int gw, int nvalid_smem) {
-  return (size_t)NW * NST * (NL > 0 ? NL : 1) * WFT_TILE_STRIDE + NW * 2 * 8 +
-         8 * 32 * 16 + 12 * 32 * 16 + 256 * 4 + 2 * WFT_NG * 16 * 4 + NW * 2 * 32 * 4 +
+  return (size_t)WFT_WARPS * 2 * (NL > 0 ? NL : 1) * WFT_TILE_STRIDE + WFT_WARPS * 2 * 8 +
+         8 * 32 * 16 + 12 * 32 * 16 + 256 * 4 + 2 * WFT_NG * 16 * 4 + WFT_WARPS * 2 * 32 * 4 +
          (((size_t)gw * gw * 2 + 15) & ~(size_t)15) + (size_t)nvalid_smem * 8;
 }
 
 // FULL = 1: three MMAs per product in both stages (fp32-grade); 0 drops the twiddle-lo pass of stage 2.
-// NW / MINB: warps per CTA and CTAs per SM the register allocation is bounded for.  NST: tile stages per warp;
-// with one stage the boxes of the next item are issued as soon as the current item has been sampled (the tiles
-// are consumed at the very start of an iteration, so they still have ~90 % of it to land) -- the smaller
-// footprint is what lets more warps share a scheduler: every warp runs latency bound, so throughput follows the
-// warp count (DESIGN.md section 4).
-// TOKEN: experiment -- the warps that share a scheduler (warp % 4) take turns on the tensor pipe (a warp runs its
-// two MMA stages only while it holds the scheduler's token), to test whether identical warps convoy on the pipe.
-// Measured 13.5 ms against 10.8 ms without (16 warps, one CTA per SM): serialising the MMA phases exposes their
-// latency-bound critical path; kept off.
-template <int FULL, int NL, int NW = WFT_WARPS, int MINB = 2, int NST = 2, int TOKEN = 0>
-__global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __grid_constant__ WfsTmaParams P) {
-  __shared__ unsigned int s_tok[4];
+// The register allocation is bounded for WFT_WARPS warps per CTA and WFT_MIN_CTAS CTAs per SM.
+template <int FULL, int NL>
+__global__ void __launch_bounds__(WFT_WARPS * 32, WFT_MIN_CTAS) wfs_frame_tma_kernel(const __grid_constant__ WfsTmaParams P) {
+  constexpr int NW = WFT_WARPS;
   const WfsParams& p = P.p;
   const WfsFast& f = P.f;
   extern __shared__ __align__(128) unsigned char wft_smem_raw[];
   unsigned char* sm = wft_smem_raw;
   constexpr int NLS = NL > 0 ? NL : 1;
   unsigned char* s_tiles = sm;                                             // [warp][stage][layer][WFT_TILE_STRIDE]
-  uint64_t* s_bar = (uint64_t*)(s_tiles + (size_t)NW * NST * NLS * WFT_TILE_STRIDE);   // [warp][stage]
+  uint64_t* s_bar = (uint64_t*)(s_tiles + (size_t)NW * 2 * NLS * WFT_TILE_STRIDE);   // [warp][stage]
   uint4* s_c1 = (uint4*)(s_bar + NW * 2);                                  // [8][32]
   uint4* s_c2 = s_c1 + 8 * 32;                                             // [12][32]
   float* s_half = (float*)(s_c2 + 12 * 32);                                // [256]
@@ -171,14 +163,13 @@ __global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __gr
   for (int i = threadIdx.x; i < f.GW * f.GW; i += blockDim.x) s_amap[i] = f.amap[i];
   if (f.sub_in_smem)
     for (int i = threadIdx.x; i < p.nvalid; i += blockDim.x) s_sub[i] = f.sub[i];
-  if (threadIdx.x < 4) s_tok[threadIdx.x] = 0u;
   if (threadIdx.x < NW * 2)
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(wft_smem_u32(s_bar + threadIdx.x)) : "memory");
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   __syncthreads();
 
   const uint2* sub = f.sub_in_smem ? s_sub : f.sub;
-  unsigned char* my_tiles = s_tiles + (size_t)warp * NST * NLS * WFT_TILE_STRIDE;
+  unsigned char* my_tiles = s_tiles + (size_t)warp * 2 * NLS * WFT_TILE_STRIDE;
   const uint32_t my_tiles_u32 = wft_smem_u32(my_tiles);
   const uint32_t my_bar_u32 = wft_smem_u32(s_bar + warp * 2);
   float* s_v = s_vall + warp * 2 * 32;
@@ -203,11 +194,11 @@ __global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __gr
   uint32_t n_xy = 0, n_pm = 0, n_d = 0;      // n_d: 2 bits per layer = tile origin column & 3
   float n_v = 0.f;
   bool n_seam = false;
-  auto prefetch = [&](int pe, int pk, int stage, bool tiles, bool aux) {
+  auto prefetch = [&](int pe, int pk, int stage) {
     uint2 sb = sub[pk];
     sb.x = __shfl_sync(0xffffffffu, sb.x, 0); sb.y = __shfl_sync(0xffffffffu, sb.y, 0);
     n_xy = sb.x;
-    if (NL > 0 && tiles) {
+    if (NL > 0) {
       if (pe != ring_e) {
 #pragma unroll
         for (int l = 0; l < NL; ++l) {
@@ -247,22 +238,19 @@ __global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __gr
           wft_tma_load_3d(my_tiles_u32 + (stage * NL + l) * WFT_TILE_STRIDE, &P.maps[l], tc[l], tr[l], pe, bar);
       }
     }
-    if (aux) {
-      n_v = 0.f;
-      if (p.use_dm && lane < 18) {
-        int idx = (lane < 16) ? (int)s_amap[(int)sb.y + amap_lane] : p.pzt_nact + lane - 16;
-        if (idx >= 0) n_v = __ldg(p.volts + (size_t)pe * p.ldv + idx);
-      }
-      n_pm = f.pmask[(size_t)pk * 32 + lane];
+    n_v = 0.f;
+    if (p.use_dm && lane < 18) {
+      int idx = (lane < 16) ? (int)s_amap[(int)sb.y + amap_lane] : p.pzt_nact + lane - 16;
+      if (idx >= 0) n_v = __ldg(p.volts + (size_t)pe * p.ldv + idx);
     }
+    n_pm = f.pmask[(size_t)pk * 32 + lane];
   };
 
-  prefetch(e, k, 0, true, true);
+  prefetch(e, k, 0);
   s_v[lane] = n_v;
   __syncwarp();
   for (int it = 0; w < end; ++it, w += NW) {
-    const int s = it & 1;
-    const int ts = (NST == 2) ? s : 0;          // tile stage of the current item
+    const int s = it & 1;                       // stage of the current item
     const uint32_t c_xy = n_xy, c_pm = n_pm, c_d = n_d;
     const bool c_seam = n_seam;
     const int ce = e, ck = k;
@@ -273,7 +261,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __gr
     if (has_next) {
       k += NW;
       if (k >= p.nvalid) { k -= p.nvalid; e += 1; }
-      prefetch(e, k, s ^ 1, NST == 2, true);
+      prefetch(e, k, s ^ 1);
     }
 
     // ---- static planes of the current subaperture (L2-resident tables), issued before the wait ----
@@ -295,8 +283,8 @@ __global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __gr
     // ---- atmosphere: bilinear sample of the staged tiles ----
     if (NL > 0) {
       if (!c_seam) {
-        wft_mbar_wait(my_bar_u32 + ts * 8, (phase_bits >> ts) & 1u, f.err);
-        phase_bits ^= (1u << ts);
+        wft_mbar_wait(my_bar_u32 + s * 8, (phase_bits >> s) & 1u, f.err);
+        phase_bits ^= (1u << s);
       } else {
         // tile straddles the torus seam: fill the stage with wrapped plain loads
 #pragma unroll 1
@@ -305,7 +293,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __gr
           const float* scr = p.layer[l].screen + (size_t)ce * N * N;
           int c0 = x0 + p.layer[l].ix + p.layer[l].ox[ce];  c0 -= (c0 >= N) ? N : 0;  c0 -= (c0 >= N) ? N : 0;
           int r0 = y0 + p.layer[l].iy + p.layer[l].oy[ce];  r0 -= (r0 >= N) ? N : 0;  r0 -= (r0 >= N) ? N : 0;
-          float* tile = reinterpret_cast<float*>(my_tiles + (ts * NL + l) * WFT_TILE_STRIDE);
+          float* tile = reinterpret_cast<float*>(my_tiles + (s * NL + l) * WFT_TILE_STRIDE);
           for (int i = lane; i < WFT_TILE_H * WFT_TILE_H; i += 32) {
             const int r = i / WFT_TILE_H, c = i - r * WFT_TILE_H;
             int rr = r0 + r;  rr -= (rr >= N) ? N : 0;
@@ -317,17 +305,13 @@ __global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __gr
       }
 #pragma unroll
       for (int l = 0; l < NL; ++l) {
-        const float* t = reinterpret_cast<const float*>(my_tiles + (ts * NL + l) * WFT_TILE_STRIDE) + lane_off;
+        const float* t = reinterpret_cast<const float*>(my_tiles + (s * NL + l) * WFT_TILE_STRIDE) + lane_off;
         switch ((c_d >> (2 * l)) & 3u) {
           case 0: wft_layer<0>(t, p.layer[l], ph); break;
           case 1: wft_layer<1>(t, p.layer[l], ph); break;
           case 2: wft_layer<2>(t, p.layer[l], ph); break;
           default: wft_layer<3>(t, p.layer[l], ph); break;
         }
-      }
-      if (NST == 1 && has_next) {
-        __syncwarp();                          // every lane has drained the stage before lane 0 re-arms it
-        prefetch(e, k, 0, true, false);
       }
     }
 
@@ -405,11 +389,6 @@ __global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __gr
         for (int j = 0; j < 2; ++j)
 #pragma unroll
           for (int c = 0; c < 4; ++c) T[a][mt][j][c] = 0.f;
-    if (TOKEN) {
-      if (lane == 0)
-        while (atomicCAS(&s_tok[warp & 3], 0u, 1u) != 0u) __nanosleep(40);
-      __syncwarp();
-    }
     {
       uint32_t nxi_h[2][2], nxi_l[2][2];
 #pragma unroll
@@ -497,11 +476,6 @@ __global__ void __launch_bounds__(NW * 32, MINB) wfs_frame_tma_kernel(const __gr
         c = fmaf(yi[u][3], yi[u][3], c);
         pix[u][b] = a + c;
       }
-    }
-
-    if (TOKEN) {
-      __syncwarp();
-      if (lane == 0) atomicExch(&s_tok[warp & 3], 0u);
     }
 
     // ---- flux normalisation, noise, centre of gravity ----

@@ -36,18 +36,15 @@
 #include <stdint.h>
 #include "rng.cuh"
 #include "wfs_params.cuh"
+#include "wfs_lattice_host.h"
 
 #define WU_WARPS 8
-#ifndef WU_EARLY_Y
-#define WU_EARLY_Y 0
-#endif
 #define WU_TILE_W 20                       // box width (floats): 17 needed + up to 3 of alignment slack; rows 80 B apart
 #define WU_TILE_H 17
 #define WU_TILE_BYTES (WU_TILE_W * WU_TILE_H * 4)            // 1360 = bytes one box delivers
 #define WU_TILE_STRIDE 1408                                  // 11 x 128
-#define WU_NG 4
-#define WU_PAD 4
-#define WU_MAX_LAYERS 4
+#define WU_NG WFL_NG
+#define WU_MAX_LAYERS WFL_MAX_LAYERS
 #define WU_A_BYTES 8192                    // 128 rows x 32 fp16
 #define WU_B_BYTES 4096                    // 64 rows x 32 fp16
 #define WU_TMEM_COLS 256                   // D1: 64 columns, D2: 2 x 64
@@ -55,13 +52,12 @@
 
 struct WfsUmmaTables {
   const uint2* sub;           // [nvalid] {y0 << 16 | x0, padded-lattice index of the neighbourhood origin | fully lit << 31}
-  const short* amap;          // [GW * GW] actuator index or -1 (padded by WU_PAD cells on every side)
+  const short* amap;          // [GW * GW] actuator index or -1 (padded by WFL_PAD cells on every side)
   const uint32_t* pmask;      // [nvalid][32] bit c = pupil(y, 8h + c) of lane (h, y)
   const uint4* b1;            // [2][WU_B_BYTES / 16] stage-1 B tiles (hi, lo), K-major canonical layout
   const uint4* b2;            // [2][WU_B_BYTES / 16] stage-2 B tiles
   const float* fxy;           // [WU_NG][16] x stamp factors, then [16][WU_NG] y stamp factors (transposed)
   int GW;
-  int a2_swap;                // development switch: swap the LBO / SBO fields of the MN-major descriptor
   int* err;
   long long items_per_cta;
 };
@@ -510,8 +506,7 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
           wu_commit(mma1_bar);
         } else {
           const uint32_t b_hi = q_b2 + KM, b_lo = b_hi + (WU_B_BYTES >> 4);
-          const uint32_t lbo = f.a2_swap ? 512u : 128u, sbo = f.a2_swap ? 128u : 512u;
-          const uint32_t am = (lbo >> 4) << 16, hia = (sbo >> 4) | (1u << 14);
+          const uint32_t am = (128u >> 4) << 16, hia = (512u >> 4) | (1u << 14);     // MN-major: LBO 128, SBO 512
 #pragma unroll
           for (int j = 0; j < 2; ++j) {
             const uint32_t a_hi = q_a2 + j * (2 * WU_A_BYTES >> 4) + am, a_lo = a_hi + (WU_A_BYTES >> 4);
@@ -807,10 +802,6 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
     uint32_t yv[32];
     if (epi) {
       wu_mbar_wait(mma2_bar, (uint32_t)((it - 2) & 1), f.err);
-#if WU_EARLY_Y
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      wu_tmem_ld32(d2_addr, yv);                        // first half of Y(it-2): lands during the conversion below
-#endif
     }
     if (conv) {
       // ---- C(it-1): T -> fp16 hi / lo -> A2 (MN-major: 8 consecutive fx per 16-byte group) ----
@@ -835,10 +826,8 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
     float qa[8], qb[8];
     wu_f2 s0p = 0ull, syp = 0ull;
     if (epi) {
-#if !WU_EARLY_Y
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       wu_tmem_ld32(d2_addr, yv);
-#endif
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
       if (pl) sq_plain(yv, 8.f, s0p, syp, true); else sq_half(yv, qa);
       wu_tmem_ld32(d2_addr + 32u, yv);

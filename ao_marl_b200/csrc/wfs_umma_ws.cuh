@@ -549,8 +549,7 @@ __global__ void __launch_bounds__(WS_THREADS, WS_MIN_BLOCKS) wfs_frame_ws_kernel
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             constexpr uint32_t KM = (128u >> 4) << 16, HI = (512u >> 4) | (1u << 14);
             const uint32_t b_hi = q_b2 + KM, b_lo = b_hi + (WU_B_BYTES >> 4);
-            const uint32_t lbo = f.a2_swap ? 512u : 128u, sbo = f.a2_swap ? 128u : 512u;
-            const uint32_t am = (lbo >> 4) << 16, hia = (sbo >> 4) | (1u << 14);
+            const uint32_t am = (128u >> 4) << 16, hia = (512u >> 4) | (1u << 14);     // MN-major: LBO 128, SBO 512
 #pragma unroll
             for (int t = 0; t < 2; ++t) {
               const uint32_t a_hi = q_a2 + t * (2 * WU_A_BYTES >> 4) + am, a_lo = a_hi + (WU_A_BYTES >> 4);

@@ -1,5 +1,6 @@
-// Host build of the device math headers (rng.cuh, fft16.cuh) so that the exact code the kernels
-// run can be checked against the numpy oracle on a machine without a GPU.
+// Host build of the device math headers (rng.cuh, fft16.cuh) and of the host-only headers the library prepares its kernels
+// with (gemm_tc_host.h, wfs_lattice_host.h), so that the exact code the library runs can be checked against the numpy
+// oracle on a machine without a GPU.
 // Built by tests/test_cpu_kernels.py:  g++ -O2 -ffp-contract=off -shared -fPIC
 #include <cmath>
 #include <cstdint>
@@ -7,6 +8,7 @@
 #include "../../ao_marl_b200/csrc/rng.cuh"
 #include "../../ao_marl_b200/csrc/fft16.cuh"
 #include "../../ao_marl_b200/csrc/gemm_tc_host.h"
+#include "../../ao_marl_b200/csrc/wfs_lattice_host.h"
 
 extern "C" {
 
@@ -82,5 +84,23 @@ void h_spot(int R, const float* inr, const float* ini, float* inten) {
 long long h_pretile_floats(int n_cols_ld, int K) { return (long long)gtc_pretile_floats(n_cols_ld, K); }
 void h_pretile(const float* W, int batch, long long sB, int ldb, int rows, int n_cols_ld, int K, float* out) {
   gtc_pretile_host(W, batch, sB, ldb, rows, n_cols_ld, K, out);
+}
+
+// Lattice analysis of the staged sensor kernels (wfs_lattice_host.h).  Returns null and fills geom = {cx, cy, joffx, joffy,
+// c0x, c0y, GW, dm}, the padded actuator map amap_pad [GW * GW], each subaperture's window origin win [nvalid] and the
+// stamp factors fac [2][WFL_NG][16]; or returns the refusal.
+const char* h_wfs_lattice(const aom_config* c, const float* pup, const int* sx, const int* sy, const float* stamp,
+                          const int* amap, int* geom, short* amap_pad, int* win, float* fac) {
+  WfsLattice L;
+  const char* why = wfl_analyse(*c, pup, sx, sy, stamp, amap, L);
+  if (why) return why;
+  const int g[8] = {L.cx, L.cy, L.joffx, L.joffy, L.c0x, L.c0y, L.GW, L.dm ? 1 : 0};
+  for (int i = 0; i < 8; ++i) geom[i] = g[i];
+  wfl_amap(*c, L, amap, amap_pad);
+  for (int k = 0; k < c->nvalid; ++k) win[k] = wfl_window(*c, L, sx[k], sy[k]);
+  for (int ax = 0; ax < 2; ++ax)
+    for (int j = 0; j < WFL_NG; ++j)
+      for (int x = 0; x < 16; ++x) fac[(ax * WFL_NG + j) * 16 + x] = wfl_factor(*c, L, stamp, ax, j, x);
+  return nullptr;
 }
 }

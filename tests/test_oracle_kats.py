@@ -228,3 +228,94 @@ def test_pretiled_actor_weights_layout(harness):
             assert np.array_equal(out[b, 0, kb, 0][off], hi)
             assert np.array_equal(out[b, 0, kb, 1][off], tile - hi)
             assert np.array_equal(out[b, 0, kb, 0][off] + out[b, 0, kb, 1][off], tile)
+
+
+def _lattice_inputs(t):
+    """aom_config fields and host tables of the staged sensor kernels, as Simulator uploads them."""
+    from ao_marl_b200.lib import AomConfig, actuator_lattice, separable_factor
+    w = t.p_wfs
+    cfg = AomConfig()
+    cfg.n, cfg.n_layers, cfg.nvalid, cfg.nfft, cfg.nrebin = t.n, t.nscreens, w._nvalid, w._Nfft, w._nrebin
+    for l in range(t.nscreens):
+        cfg.screen_dim[l] = int(t.dim_screens[l])
+    cfg.pzt_pitch, cfg.pzt_grid_n, cfg.pzt_i1_0, cfg.pzt_j1_0, amap = actuator_lattice(t.p_pzt)
+    cfg.stamp_size, cfg.pzt_off, cfg.tt_dim, cfg.tt_off = t.p_pzt._influsize, t.pzt_off, t.tt_dim, t.tt_off
+    tab = dict(pup=t.mpupil.astype(np.float32), sx=w._tile_origin[:, 1].astype(np.int32),
+               sy=w._tile_origin[:, 0].astype(np.int32), stamp=separable_factor(t.p_pzt._influ[:, :, 0]), amap=amap)
+    return cfg, tab
+
+
+def _lattice(harness, cfg, tab):
+    """wfl_analyse and the lattice builders (wfs_lattice_host.h): (refusal or None, geom, amap_pad, win, fac)."""
+    harness.h_wfs_lattice.restype = ctypes.c_char_p
+    GW = cfg.pzt_grid_n + 8
+    geom, amap_pad = np.zeros(8, np.int32), np.zeros(GW * GW, np.int16)
+    win, fac = np.zeros(cfg.nvalid, np.int32), np.zeros((2, 4, 16), np.float32)
+    t = {k: np.ascontiguousarray(v) for k, v in tab.items()}
+    why = harness.h_wfs_lattice(ctypes.byref(cfg), P(t["pup"]), P(t["sx"]), P(t["sy"]), P(t["stamp"]), P(t["amap"]),
+                                P(geom), P(amap_pad), P(win), P(fac))
+    return (why.decode() if why else None), geom, amap_pad, win, fac
+
+
+@pytest.mark.parametrize("par", ["production_sh_10x10_2m.py",
+                                 pytest.param("production_sh_40x40_8m_3layers.py", marks=pytest.mark.slow)])
+def test_wfs_lattice_reproduces_mirror(harness, par):
+    """The padded actuator map, window origins and stamp factors both staged sensor kernels derive their tables from give,
+    for every pixel of every subaperture, the actuators and weights of the mirror sum of the SIMT kernel (wfs_kernels.cuh:
+    stamp1d[Y - (j1_0 + 16 gy)] * stamp1d[X - (i1_0 + 16 gx)] over the lattice cells whose stamp covers the pixel)."""
+    from ao_marl_b200 import tables
+    from ao_marl_b200.config import load_config_from_file
+    cfg, tab = _lattice_inputs(tables.build_static(load_config_from_file(par)))
+    why, geom, amap_pad, win, fac = _lattice(harness, cfg, tab)
+    assert why is None and geom[7] == 1
+    GW, gn, ss, nact = geom[6], cfg.pzt_grid_n, cfg.stamp_size, int(tab["amap"].max()) + 1
+    stamp, amap = tab["stamp"].astype(np.float64), tab["amap"]
+
+    def factors(origin, base):      # [16 pixels][grid_n cells] stamp factor of the SIMT kernel
+        d = origin + cfg.pzt_off + np.arange(16)[:, None] - (base + 16 * np.arange(gn))[None, :]
+        return np.where((d >= 0) & (d < ss), stamp[np.clip(d, 0, ss - 1)], 0.0)
+
+    on = amap >= 0
+    for k in range(cfg.nvalid):
+        fx, fy = factors(tab["sx"][k], cfg.pzt_i1_0), factors(tab["sy"][k], cfg.pzt_j1_0)
+        ref = np.zeros((256, nact))
+        ref[:, amap[on]] = np.einsum("yg,xh->yxgh", fy, fx).reshape(256, gn * gn)[:, on]
+        got = np.zeros((256, nact))
+        for jy in range(4):
+            for jx in range(4):
+                a = amap_pad[win[k] + jy * GW + jx]
+                if a >= 0:
+                    assert not got[:, a].any()
+                    got[:, a] = np.outer(fac[1, jy].astype(np.float64), fac[0, jx].astype(np.float64)).ravel()
+        assert np.array_equal(got, ref), k
+        assert np.count_nonzero(ref.any(axis=0)) > 0
+
+
+def test_wfs_lattice_refusals(harness, static10):
+    """Geometries outside the staged sensor kernels are refused with the reasons aom_wfs_kernel reports."""
+    from ao_marl_b200.lib import AomConfig
+    cfg, tab = _lattice_inputs(static10)
+    assert _lattice(harness, cfg, tab)[0] is None
+
+    def refusal(cfg_changes={}, **tables):
+        c = AomConfig()
+        ctypes.memmove(ctypes.byref(c), ctypes.byref(cfg), ctypes.sizeof(cfg))
+        for k, v in cfg_changes.items():
+            setattr(c, k, v)
+        return _lattice(harness, c, dict(tab, **tables))[0]
+
+    pup = tab["pup"].copy()
+    y, x = np.argwhere(pup == 1)[np.count_nonzero(pup) // 2]
+    pup[y, x] = 0.5
+    assert refusal(pup=pup) == "pupil transmission is not binary"
+    sx, k = tab["sx"].copy(), cfg.nvalid // 2
+    assert sx[k] + 4 + 16 <= cfg.n and 0 < k
+    sx[k] += 4                                   # tip-tilt rows stay 16-byte aligned
+    assert refusal(sx=sx) == "subapertures not aligned with the actuator lattice"
+    assert refusal({"pzt_pitch": 8}) == "actuator pitch is not 16 pixels"
+    assert refusal({"n_layers": 5}) == "more than 4 layers"
+    assert refusal({"nfft": 128}) == "Nfft != 64"
+    amap = tab["amap"].copy()
+    amap[amap >= 0] += 40000                     # actuator indices beyond a short
+    assert refusal(amap=amap) == "derived tables out of range"
+    assert refusal({"pzt_grid_n": 2}) == "derived tables out of range"     # windows leave the padded map

@@ -63,3 +63,47 @@ def test_routing_matrix(static10):
                 _leave(sim, state)
     finally:
         sim.close()
+
+
+def _non_binary_pupil(t):
+    pup = t.mpupil.astype(np.float32)
+    y, x = np.argwhere(pup == 1)[np.count_nonzero(pup) // 2]
+    pup[y, x] = 0.5
+    return pup
+
+
+def _perturbed_phasor(t):
+    h = t.p_wfs._halfxy.astype(np.float32)
+    h.flat[17] += 1e-3
+    return h
+
+
+# geometry -> (table re-uploaded, its new contents, kernel of each path, reason aom_wfs_kernel leaves in aom_last_error)
+STAGED_MMA = dict(KERNELS, **{p: "wfs_frame_mma_kernel" for p in ("umma_ws", "umma", "umma_fast", "tensor", "tensor_fast")})
+GEOMETRIES = {"non-binary pupil": ("MPUPIL", _non_binary_pupil, STAGED_MMA, "pupil transmission is not binary"),
+              "perturbed half-pixel phasor": ("HALFXY", _perturbed_phasor,
+                                              dict(KERNELS, umma_ws="wfs_frame_tma_kernel", umma="wfs_frame_tma_kernel",
+                                                   umma_fast="wfs_frame_tma_kernel"), None)}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("geometry", list(GEOMETRIES))
+def test_routing_ineligible_geometry(static10, geometry):
+    """A geometry a staged kernel cannot serve goes to the next kernel down, which computes its frames."""
+    import torch
+    assert torch.cuda.is_available(), "GPU tests need a CUDA device"
+    from ao_marl_b200.lib import Simulator
+    table, contents, kernels, reason = GEOMETRIES[geometry]
+    sim = Simulator(static10, len(SEEDS), rl=None)
+    try:
+        sim.set_table(table, contents(static10))
+        sim.reset(SEEDS)
+        for path in PATHS:
+            sim.set_wfs_path(path)
+            assert sim.wfs_kernel() == kernels[path], path
+            if reason and path != "tensor_reg" and path != "simt":
+                assert sim.lib.aom_last_error(sim._ctx).decode() == "staged sensor kernels not eligible: " + reason, path
+            sim.comp_wfs_image(noise=-1.0)
+            sim.check_device()
+    finally:
+        sim.close()
