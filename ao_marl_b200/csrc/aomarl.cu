@@ -389,6 +389,7 @@ static size_t table_expected_bytes(const aom_ctx* ctx, int t, int index) {
 // digit planes of an operator [rows][ld] (K valid columns) for the integer contraction (extrude_i8.cuh)
 static int oz_upload_operator(aom_ctx* ctx, const float* host, int rows, int ld, int K, uint8_t** planes_d, int** ea_d,
                               int* kb_out, int* nt_out) {
+  if (!oz_operator_finite(host, rows, ld, K)) return fail(ctx, AOM_ERR_INVALID, "operator table holds a NaN or an infinity");
   const int KB = (K + OZ_BK - 1) / OZ_BK, NT = (rows + OZ_BN - 1) / OZ_BN;
   const size_t bytes = (size_t)NT * KB * OZ_SLICES_B * OZ_B_TILE;
   uint8_t* planes = (uint8_t*)calloc(bytes, 1);
@@ -414,6 +415,24 @@ extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* hos
   size_t want = table_expected_bytes(ctx, table, index);
   if (want != nbytes)
     return fail(ctx, AOM_ERR_INVALID, "Dimension mismatch: table %d[%d] expects %zu bytes, got %zu", table, index, want, nbytes);
+  // operators of the integer contraction first: a non-finite one is refused before anything changes
+  if (table == AOM_T_AB) {
+    // digit planes of [A | B] for the exact integer extrusion
+    const aom_config& c = ctx->cfg;
+    const int N = c.screen_dim[index], K = c.stencil_size[index] + N;
+    int rc = oz_upload_operator(ctx, (const float*)host, N, AOM_LD(K), K, &ctx->oz_ab[index], &ctx->oz_ea[index],
+                                &ctx->oz_kb[index], &ctx->oz_nt[index]);
+    if (rc) return rc;
+  }
+  if (table == AOM_T_CMAT || table == AOM_T_V2M || table == AOM_T_M2V) {
+    // digit planes of the controller operators for the exact integer products
+    const aom_config& c = ctx->cfg;
+    const int rows = table == AOM_T_V2M ? c.nmodes : c.nactu;
+    const int K = table == AOM_T_CMAT ? c.nslopes : table == AOM_T_V2M ? c.nactu : c.nmodes;
+    int rc = oz_upload_operator(ctx, (const float*)host, rows, AOM_LD(K), K, &ctx->ozop[table], &ctx->ozop_ea[table],
+                                &ctx->ozop_kb[table], &ctx->ozop_nt[table]);
+    if (rc) return rc;
+  }
   if (ctx->tab[table][index]) { cudaFree(ctx->tab[table][index]); ctx->tab[table][index] = nullptr; }
   CU(cudaMalloc(&ctx->tab[table][index], nbytes ? nbytes : 4));
   CU(cudaMemcpy(ctx->tab[table][index], host, nbytes, cudaMemcpyHostToDevice));
@@ -430,14 +449,6 @@ extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* hos
   }
   if (table == AOM_T_MPUPIL || table == AOM_T_TT_PLANES) ctx->sweep_state = 0;
   if (table == AOM_T_DENOISER_TC) memcpy(ctx->dn_prm, host, (size_t)DT_NPARAM * 4);   // float parameters travel as kernel arguments
-  if (table == AOM_T_AB) {
-    // digit planes of [A | B] for the exact integer extrusion
-    const aom_config& c = ctx->cfg;
-    const int N = c.screen_dim[index], K = c.stencil_size[index] + N;
-    int rc = oz_upload_operator(ctx, (const float*)host, N, AOM_LD(K), K, &ctx->oz_ab[index], &ctx->oz_ea[index],
-                                &ctx->oz_kb[index], &ctx->oz_nt[index]);
-    if (rc) return rc;
-  }
   if (table == AOM_T_ACTOR_W1 || table == AOM_T_ACTOR_W2 || table == AOM_T_ACTOR_WH) {
     // the same weights pre-split into TF32 hi / lo planes in the tile order of gemm_tc_kernel: the actor GEMMs then take
     // their B operand by one bulk copy per stage instead of global loads + split + st.shared in the loader warps
@@ -456,14 +467,6 @@ extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* hos
     free(h);
     if (e != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "pre-tiled actor weights: %s", cudaGetErrorString(e));
     ctx->actor_bt_per[i] = per;
-  }
-  if (table == AOM_T_CMAT || table == AOM_T_V2M || table == AOM_T_M2V) {
-    const aom_config& c = ctx->cfg;
-    const int rows = table == AOM_T_V2M ? c.nmodes : c.nactu;
-    const int K = table == AOM_T_CMAT ? c.nslopes : table == AOM_T_V2M ? c.nactu : c.nmodes;
-    int rc = oz_upload_operator(ctx, (const float*)host, rows, AOM_LD(K), K, &ctx->ozop[table], &ctx->ozop_ea[table],
-                                &ctx->ozop_kb[table], &ctx->ozop_nt[table]);
-    if (rc) return rc;
   }
   return AOM_OK;
 }

@@ -37,24 +37,3 @@ cudaError_t oz_product_launch(const OzSliceParams& sl, const OzGemmParams& m, in
   });
   return cudaGetLastError();
 }
-
-void oz_slice_operator(const float* AB, int rows, int ld, int K, int KB, int NT, uint8_t* planes, int* ea) {
-  for (int n = 0; n < NT * OZ_BN; ++n) {
-    ea[n] = 0;
-    if (n >= rows) continue;
-    const float* row = AB + (size_t)n * ld;
-    double amax = 0.0;
-    for (int k = 0; k < K; ++k) amax = fmax(amax, fabs((double)row[k]));
-    const int ex = oz_exponent(amax);
-    ea[n] = ex;
-    const double scale = ldexp(1.0, -ex);
-    const int nt = n / OZ_BN, r = n % OZ_BN;
-    for (int k = 0; k < K; ++k) {
-      int q[OZ_SLICES_B];
-      oz_digits<OZ_SLICES_B>((double)row[k], scale, q);
-      const int kb = k / OZ_BK, kk = k % OZ_BK;
-      for (int s = 0; s < OZ_SLICES_B; ++s)
-        planes[((size_t)(nt * KB + kb) * OZ_SLICES_B + s) * OZ_B_TILE + oz_tile_offset(r, kk)] = (uint8_t)(int8_t)q[s];
-    }
-  }
-}

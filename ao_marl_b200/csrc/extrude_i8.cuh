@@ -29,21 +29,9 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "rng.cuh"
+#include "extrude_i8_digits.h"
 
-#define OZ_SLICES 6                               // digits of the per-extrusion inputs (41 bits below the row maximum)
-#define OZ_SLICES_B 6                             // digits of the operator rows (41 bits): its truncation is a FIXED perturbation
-                                                  // of the recursion and adds up coherently -- with 4 digits the 648^2 screens
-                                                  // were 9.5e-5 off after a reset (measured, and reproduced in numpy)
-#define OZ_LEVELS 6                               // digit pairs kept: s + t <= 5
-#define OZ_LEVELS_PRODUCT 5                       // controller products (no recursion behind them): s + t <= 4, 15 MMAs per k
-                                                  // block (with s + t <= 3 the 40x40 closed loop moved from 1e-6 to 1e-5 .. 4e-5
-                                                  // of the oracle: measured, profiles/r02_parity_levels4.json)
-#define OZ_BM 128
-#define OZ_BN 80
-#define OZ_BK 32
 #define OZ_STAGES 3
-#define OZ_A_TILE (OZ_BM * OZ_BK)                 // 4096 bytes: one digit plane of 128 rows x 32 k
-#define OZ_B_TILE (OZ_BN * OZ_BK)                 // 2560 bytes
 #define OZ_STAGE_BYTES (OZ_SLICES * OZ_A_TILE + OZ_SLICES_B * OZ_B_TILE)      // 39936
 #define OZ_SMEM_BYTES (OZ_STAGES * OZ_STAGE_BYTES + 256)
 #define OZ_THREADS 192
@@ -85,44 +73,6 @@ struct OzSliceParams {
   const float* X; int ld, K, E, KB;
   uint8_t* Zs; int* ev;
 };
-
-// element (row r, k) of a [rows x 32] int8 tile: 8-row x 16-byte core matrices, 128 B between the two k halves,
-// 256 B between 8-row groups
-__host__ __device__ __forceinline__ uint32_t oz_tile_offset(int r, int kk) {
-  return (uint32_t)((r >> 3) * 256 + (kk >> 4) * 128 + (r & 7) * 16 + (kk & 15));
-}
-
-// NS signed 7-bit digits of x * scale, |x * scale| < 1 (every step is exact in float64 for inputs of <= 48 bits)
-template <int NS>
-__host__ __device__ __forceinline__ void oz_digits(double x, double scale, int (&q)[NS]) {
-  double t = x * scale * 64.0;
-#pragma unroll
-  for (int s = 0; s < NS; ++s) {
-    const double r = rint(t);
-    q[s] = (int)r;
-    t = (t - r) * 128.0;
-  }
-}
-
-// the same digits of a float32 value: every step is exact in float32 (the remainders only lose leading bits)
-template <int NS>
-__host__ __device__ __forceinline__ void oz_digits_f32(float x, float scale, int (&q)[NS]) {
-  float t = x * scale * 64.0f;
-#pragma unroll
-  for (int s = 0; s < NS; ++s) {
-    const float r = rintf(t);
-    q[s] = (int)r;
-    t = (t - r) * 128.0f;
-  }
-}
-
-// power of two e with |x| * 2^-e in [0.5, 1) for the row maximum x (0 for an all-zero row)
-__host__ __device__ __forceinline__ int oz_exponent(double amax) {
-  if (!(amax > 0.0)) return 0;
-  int e;
-  frexp(amax, &e);           // amax = m 2^e, m in [0.5, 1)
-  return e;
-}
 
 #ifdef OZ_DEFINE_KERNELS   // the kernels are defined in one translation unit only (extrude_i8.cu)
 __device__ __forceinline__ void oz_logical(int r, int c, int N, int axis, int sign, int& lr, int& lc) {
@@ -220,17 +170,23 @@ __global__ void __launch_bounds__(256) oz_slice_rows_kernel(OzSliceParams p) {
   const int e = blockIdx.x, Kp = p.KB * OZ_BK;
   const float* x = p.X + (size_t)e * p.ld;
   float amax = 0.f;
-  for (int k = threadIdx.x; k < p.K; k += blockDim.x) amax = fmaxf(amax, fabsf(x[k]));
+  int bad = 0;                                                    // fmaxf ignores NaN: non-finite elements are flagged
+  for (int k = threadIdx.x; k < p.K; k += blockDim.x) {
+    const float a = fabsf(x[k]);
+    amax = fmaxf(amax, a);
+    bad |= !(a <= 3.402823466e38f);
+  }
 #pragma unroll
   for (int s = 16; s > 0; s >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, s));
   if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = amax;
-  __syncthreads();
+  bad = __syncthreads_or(bad);
   amax = s_red[0];
 #pragma unroll
   for (int i = 1; i < 8; ++i) amax = fmaxf(amax, s_red[i]);
-  const int ex = oz_exponent((double)amax);
-  if (threadIdx.x == 0) p.ev[e] = ex;
-  const float scale = __int_as_float((127 - ex) << 23);          // 2^-ex
+  const int ex = bad ? 0 : oz_exponent((double)amax);
+  if (threadIdx.x == 0) p.ev[e] = bad ? OZ_EV_NONFINITE : ex;    // the GEMM epilogue writes NaN for the whole row
+  // 2^-ex as two float32 factors: a single one overflows for a subnormal row maximum (ex < -126) or one >= 2^127
+  const float pre = __int_as_float((127 - (ex >> 1)) << 23), scale = __int_as_float((127 - (ex - (ex >> 1))) << 23);
   const int mt = e >> 7, r = e & 127;
   for (int j = threadIdx.x; j < Kp / 16; j += blockDim.x) {
     uint32_t w[OZ_SLICES][4];
@@ -253,7 +209,7 @@ __global__ void __launch_bounds__(256) oz_slice_rows_kernel(OzSliceParams p) {
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
       int q[OZ_SLICES];
-      oz_digits_f32<OZ_SLICES>((16 * j + i < p.K) ? v[i] : 0.f, scale, q);
+      oz_digits_f32<OZ_SLICES>((16 * j + i < p.K) ? v[i] * pre : 0.f, scale, q);
 #pragma unroll
       for (int s = 0; s < OZ_SLICES; ++s) w[s][i >> 2] |= ((uint32_t)q[s] & 0xffu) << (8 * (i & 3));
     }
@@ -409,7 +365,9 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) oz_gemm_kernel(OzGemmParams p) 
     const int q = warp & 3;                                   // TMEM lane quarter this warp may read
     const int e = mt * OZ_BM + 32 * q + lane;
     const bool live = e < p.E;
-    const int ev = live ? p.ev[e] : 0;
+    const int ev_row = live ? p.ev[e] : 0;
+    const bool nonfinite = EPI != 0 && ev_row == OZ_EV_NONFINITE;    // products only: the row held a NaN or an infinity
+    const int ev = nonfinite ? 0 : ev_row;
     const double zr = (EPI == 0 && live) ? (double)p.zref[e] : 0.0;
     const float gn = (EPI == 3 && live) ? p.gain_env[e] : p.gain;     // integrator gain of this row's environment
 #pragma unroll 1
@@ -436,7 +394,7 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) oz_gemm_kernel(OzGemmParams p) 
           const double sc = __longlong_as_double((long long)(1023 + ex) << 52);
           if (EPI == 0) o[j] = (float)fma(acc, sc, zr);        // pad columns get zref: harmless, the scatter reads n < N
           else {
-            const float r = (float)(acc * sc);
+            const float r = nonfinite ? __int_as_float(0x7fffffff) : (float)(acc * sc);
             o[j] = (n < p.N) ? (EPI >= 2 ? -r : r) : 0.f;       // pad columns stay zero
           }
         }

@@ -11,6 +11,3 @@ cudaError_t oz_extrude_launch(const OzGatherParams& g, const OzGemmParams& m, in
 // digit-pair GEMM; both asynchronous on `st`
 cudaError_t oz_product_launch(const OzSliceParams& sl, const OzGemmParams& m, int integrator, int MT, int NT, cudaStream_t st);
 
-// Host: cut the rows of the operator [rows][ld] (K valid columns) into digit planes in the tile layout of the kernel.
-// planes: NT * KB * OZ_SLICES_B * OZ_B_TILE bytes (zero-initialised by the caller); ea: NT * OZ_BN ints.
-void oz_slice_operator(const float* AB, int rows, int ld, int K, int KB, int NT, uint8_t* planes, int* ea);

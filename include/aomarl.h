@@ -218,6 +218,9 @@ size_t aom_config_size(void);                       /* sizeof(aom_config) the li
 int aom_create(const aom_config* cfg, aom_ctx** out);
 void aom_destroy(aom_ctx* ctx);
 const char* aom_last_error(const aom_ctx* ctx);     /* ctx may be NULL for create-time errors */
+/* Upload a table (host copy of nbytes).  The operators of the integer contractions (AOM_T_CMAT, AOM_T_V2M, AOM_T_M2V,
+ * AOM_T_AB) must be finite: a NaN or an infinity in one of their valid columns returns AOM_ERR_INVALID and leaves the
+ * table in force unchanged. */
 int aom_set_table(aom_ctx* ctx, int table, int index, const void* host, size_t nbytes);
 int aom_get_buffer(aom_ctx* ctx, int buffer, int index, void** dptr, size_t* count);
 int aom_device_count_launches(const aom_ctx* ctx, uint64_t* n_launches);  /* kernels launched so far */
@@ -364,6 +367,9 @@ int aom_do_centroids(aom_ctx* ctx, void* stream);
  * phase gradient per subaperture of the sensor-direction phase selected by flags (bit0 atmosphere, bit1 mirrors,
  * AOM_TAR_GEO: the geometric controller's mirrors), alpha = 0.206265 / subaperture size [m]. */
 int aom_do_centroids_geom(aom_ctx* ctx, int flags, float alpha, void* stream);
+/* err = -cmat.s and, loop closed, com += g err.  Non-finite inputs stay visible: an environment whose slopes (or, through
+ * aom_rl_control, whose commands) hold a NaN or an infinity gets non-finite outputs in its own row and no other.  The
+ * default tcgen05 path writes NaN to every output of that row; the SIMT path may give +-Inf instead. */
 int aom_do_control(aom_ctx* ctx, void* stream);
 int aom_set_command(aom_ctx* ctx, const float* dcom, int ld, void* stream);
 int aom_apply_control(aom_ctx* ctx, int comp_voltage, void* stream);

@@ -1,5 +1,5 @@
 // Host build of the device math headers (rng.cuh, fft16.cuh) and of the host-only headers the library prepares its kernels
-// with (gemm_tc_host.h, wfs_lattice_host.h), so that the exact code the library runs can be checked against the numpy
+// with (gemm_tc_host.h, wfs_lattice_host.h, extrude_i8_digits.h), so that the exact code the library runs can be checked against the numpy
 // oracle on a machine without a GPU.
 // Built by tests/test_cpu_kernels.py:  g++ -O2 -ffp-contract=off -shared -fPIC
 #include <cmath>
@@ -9,6 +9,7 @@
 #include "../../ao_marl_b200/csrc/fft16.cuh"
 #include "../../ao_marl_b200/csrc/gemm_tc_host.h"
 #include "../../ao_marl_b200/csrc/wfs_lattice_host.h"
+#include "../../ao_marl_b200/csrc/extrude_i8_digits.h"
 
 extern "C" {
 
@@ -102,5 +103,35 @@ const char* h_wfs_lattice(const aom_config* c, const float* pup, const int* sx, 
     for (int j = 0; j < WFL_NG; ++j)
       for (int x = 0; x < 16; ++x) fac[(ax * WFL_NG + j) * 16 + x] = wfl_factor(*c, L, stamp, ax, j, x);
   return nullptr;
+}
+
+// Digit code of the integer contraction (extrude_i8_digits.h).  Tile geometry: {OZ_SLICES, OZ_SLICES_B, OZ_LEVELS,
+// OZ_LEVELS_PRODUCT, OZ_BM, OZ_BN, OZ_BK, OZ_A_TILE, OZ_B_TILE, OZ_EV_NONFINITE}.
+void h_oz_constants(int* c) {
+  const int v[10] = {OZ_SLICES, OZ_SLICES_B, OZ_LEVELS, OZ_LEVELS_PRODUCT, OZ_BM, OZ_BN, OZ_BK, OZ_A_TILE, OZ_B_TILE, OZ_EV_NONFINITE};
+  for (int i = 0; i < 10; ++i) c[i] = v[i];
+}
+int h_oz_tile_offset(int r, int kk) { return (int)oz_tile_offset(r, kk); }
+void h_oz_exponent(int n, const double* amax, int* e) {
+  for (int i = 0; i < n; ++i) e[i] = oz_exponent(amax[i]);
+}
+// q [OZ_SLICES][n]: digits of x[i] * scale[i] in float32 (oz_digits_f32) and in float64 (oz_digits)
+void h_oz_digits_f32(int n, const float* x, const float* scale, int* q) {
+  for (int i = 0; i < n; ++i) {
+    int d[OZ_SLICES];
+    oz_digits_f32<OZ_SLICES>(x[i], scale[i], d);
+    for (int s = 0; s < OZ_SLICES; ++s) q[(size_t)s * n + i] = d[s];
+  }
+}
+void h_oz_digits(int n, const double* x, const double* scale, int* q) {
+  for (int i = 0; i < n; ++i) {
+    int d[OZ_SLICES_B];
+    oz_digits<OZ_SLICES_B>(x[i], scale[i], d);
+    for (int s = 0; s < OZ_SLICES_B; ++s) q[(size_t)s * n + i] = d[s];
+  }
+}
+int h_oz_operator_finite(const float* AB, int rows, int ld, int K) { return oz_operator_finite(AB, rows, ld, K); }
+void h_oz_slice_operator(const float* AB, int rows, int ld, int K, int KB, int NT, uint8_t* planes, int* ea) {
+  oz_slice_operator(AB, rows, ld, K, KB, NT, planes, ea);
 }
 }
