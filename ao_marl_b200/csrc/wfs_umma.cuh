@@ -273,6 +273,430 @@ __device__ __forceinline__ void wu_layer(const float* __restrict__ t, const Wt& 
   a.y7 = fmaf(wy1, v[1][D + 8 - B_X], fmaf(wy0, v[0][D + 8 - B_X], a.y7));
 }
 
+// ================= pieces shared by wfs_frame_umma_kernel and wfs_frame_ws_kernel (wfs_umma_ws.cuh) =================
+
+// Shared memory of one CTA (wu_smem_bytes).  The 128-byte barrier block is laid out by each kernel.
+struct WuSmem {
+  unsigned char* a1;        // [hi, lo][WU_A_BYTES]
+  unsigned char* a2;        // [tile][hi, lo][WU_A_BYTES]
+  unsigned char* b1;        // [hi, lo][WU_B_BYTES]
+  unsigned char* b2;
+  unsigned char* tiles;     // [warp][layer][WU_TILE_STRIDE]
+  uint64_t* bar;            // barrier block
+  float* fx;                // [NG][16]
+  float* fyT;               // [16][NG]
+  unsigned char* aux;       // [warp][parity][AUXB]
+  short* amap;
+};
+
+template <int NL, bool PE>
+__device__ __forceinline__ WuSmem wu_smem_layout() {
+  extern __shared__ __align__(1024) unsigned char wu_smem_raw[];
+  constexpr int NLS = NL > 0 ? NL : 1;
+  constexpr int AUXB = PE ? WU_AUX_BYTES_PE : WU_AUX_BYTES;
+  WuSmem S;
+  S.a1 = wu_smem_raw;
+  S.a2 = S.a1 + 2 * WU_A_BYTES;
+  S.b1 = S.a2 + 4 * WU_A_BYTES;
+  S.b2 = S.b1 + 2 * WU_B_BYTES;
+  S.tiles = S.b2 + 2 * WU_B_BYTES;
+  S.bar = (uint64_t*)(S.tiles + (size_t)WU_WARPS * NLS * WU_TILE_STRIDE);
+  S.fx = (float*)((unsigned char*)S.bar + 128);
+  S.fyT = S.fx + WU_NG * 16;
+  S.aux = (unsigned char*)(S.fyT + 16 * WU_NG);
+  S.amap = (short*)(S.aux + WU_WARPS * 2 * AUXB);
+  return S;
+}
+
+// lane through a volatile read: the compiler otherwise re-derives it from S2R SR_TID.X at ~25 places of the loop body
+// and each of those reads stalls its warp (5 % of the stall samples in profiles/r02_wfs_umma_v5)
+__device__ __forceinline__ int wu_lane() {
+  int lane;
+  asm volatile("mov.u32 %0, %%laneid;" : "=r"(lane));
+  return lane;
+}
+
+// CTA set-up: copies the constant tables, zeroes the operand tiles, initialises barriers 0 .. n_bar - 1 (count: the
+// arrival count of barrier tid) and allocates the tensor memory; returns its base address, which passes through
+// tmem_slot, a word of the barrier block.  tid / nthr are threadIdx.x / blockDim.x read in the kernel, where the compiler
+// bounds them by its launch bounds (read here, the copy loops compile to a longer trip-count computation).
+__device__ __forceinline__ uint32_t wu_cta_setup(const WuSmem& S, const WfsUmmaTables& f, uint32_t tid, uint32_t nthr, int warp,
+                                                 uint32_t n_bar, uint32_t count, uint32_t* tmem_slot) {
+  for (int i = tid; i < 2 * WU_B_BYTES / 16; i += nthr) {
+    reinterpret_cast<uint4*>(S.b1)[i] = f.b1[i];
+    reinterpret_cast<uint4*>(S.b2)[i] = f.b2[i];
+  }
+  for (int i = tid; i < 2 * WU_NG * 16; i += nthr) S.fx[i] = f.fxy[i];
+  for (int i = tid; i < f.GW * f.GW; i += nthr) S.amap[i] = f.amap[i];
+  // operand tiles start from zeros: rows of work items that do not exist are multiplied too
+  for (int i = tid; i < 6 * WU_A_BYTES / 16; i += nthr) reinterpret_cast<uint4*>(S.a1)[i] = make_uint4(0u, 0u, 0u, 0u);
+  if (tid < n_bar) asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(wu_smem_u32(S.bar + tid)), "r"(count) : "memory");
+  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");          // B tiles / zeroed A tiles are read by the tensor core
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(wu_smem_u32(tmem_slot)), "r"((uint32_t)WU_TMEM_COLS)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  return __shfl_sync(0xffffffffu, *tmem_slot, 0);
+}
+
+__device__ __forceinline__ void wu_cta_release(int warp, uint32_t tmem_base) {
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  if (warp == 0) {
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)WU_TMEM_COLS) : "memory");
+  }
+}
+
+// ---- the F phase of a field warp: its items are the CTA-local indices warp + 8 i; the tiles and per-lane inputs of
+//      the next item are in flight while the current one is sampled.  The kernels keep the per-warp state in locals
+//      and pass it by reference: the order of the loads, copies and fences below is what keeps the register budget
+//      (the specialised kernel fits in 80 registers) ----
+
+// tiles of one work item (record sb): TMA boxes, or element-wise wrapped cp.async copies on the torus seam.  ring_e /
+// rx / ry: the ring origins of the environment whose origins were computed last; n_d / n_seam: the tile column offsets
+// and the seam flag of this item.
+template <int NL, bool PE>
+__device__ __forceinline__ void wu_issue_tiles(const WfsUmmaParams& P, uint32_t my_tiles_u32, uint32_t my_bar_u32, int lane, int pe,
+                                               uint2 sb, int& ring_e, int (&rx)[NL > 0 ? NL : 1], int (&ry)[NL > 0 ? NL : 1],
+                                               uint32_t& n_d, bool& n_seam) {
+  constexpr int NLS = NL > 0 ? NL : 1;
+  const WfsParams& p = P.p;
+  if (NL == 0) return;
+  if (pe != ring_e) {
+#pragma unroll
+    for (int l = 0; l < NL; ++l) {
+      const int N = p.layer[l].N;
+      int a = (PE ? __ldg(&p.wind[(size_t)l * p.E + pe].ix) : p.layer[l].ix) + p.layer[l].ox[pe];  a -= (a >= N) ? N : 0;
+      int b = (PE ? __ldg(&p.wind[(size_t)l * p.E + pe].iy) : p.layer[l].iy) + p.layer[l].oy[pe];  b -= (b >= N) ? N : 0;
+      rx[l] = a; ry[l] = b;
+    }
+    ring_e = pe;
+  }
+  const int x0 = (int)(sb.x & 0xffffu), y0 = (int)(sb.x >> 16);
+  int tc[NLS], tr[NLS];
+  bool seam = false;
+  uint32_t dbits = 0;
+#pragma unroll
+  for (int l = 0; l < NL; ++l) {
+    const int N = p.layer[l].N;
+    int c = x0 + rx[l];  c -= (c >= N) ? N : 0;
+    int r = y0 + ry[l];  r -= (r >= N) ? N : 0;
+    tc[l] = c & ~3; tr[l] = r;
+    dbits |= (uint32_t)(c & 3) << (2 * l);
+    seam |= (c + WU_TILE_H > N) | (r + WU_TILE_H > N);
+  }
+  n_seam = seam;
+  n_d = dbits;
+  if (!seam) {
+    // the stage was read with plain loads: order them before the async-proxy writes of the new boxes
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    __syncwarp();
+    if (wu_elect()) {       // elect.sync: a warp-uniform issue path (no per-thread waterfall around the TMA instructions)
+      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(my_bar_u32), "r"(NL * WU_TILE_BYTES) : "memory");
+#pragma unroll
+      for (int l = 0; l < NL; ++l)
+        wu_tma_load_3d(my_tiles_u32 + l * WU_TILE_STRIDE, &P.maps[l], tc[l], tr[l], pe, my_bar_u32);
+    }
+  } else {
+    // (rare path: keep its per-lane index arithmetic here instead of in registers that live across the whole loop)
+    int ln = lane;
+    asm volatile("" : "+r"(ln));
+#pragma unroll
+    for (int l = 0; l < NL; ++l) {
+      const int N = p.layer[l].N;
+      const float* scr = p.layer[l].screen + (size_t)pe * N * N;
+      const int c0 = tc[l] + (int)((dbits >> (2 * l)) & 3u), r0 = tr[l];
+      const uint32_t dst0 = my_tiles_u32 + l * WU_TILE_STRIDE + ((dbits >> (2 * l)) & 3u) * 4u;
+#pragma unroll 1
+      for (int i0 = 0; i0 < WU_TILE_H * WU_TILE_H; i0 += 32) {
+        const int i = i0 + ln;
+        if (i < WU_TILE_H * WU_TILE_H) {
+          const int r = i / WU_TILE_H, c = i - r * WU_TILE_H;
+          int rr = r0 + r;  rr -= (rr >= N) ? N : 0;
+          int cc = c0 + c;  cc -= (cc >= N) ? N : 0;
+          wu_cp_async4(dst0 + (uint32_t)(r * WU_TILE_W + c) * 4u, scr + (size_t)rr * N + cc);
+        }
+      }
+    }
+    asm volatile("cp.async.commit_group;" ::: "memory");
+  }
+}
+
+// per-lane inputs of one work item into the parity slot of my_aux (pm[32] | volts[32] | record, then with PE the layer
+// offsets): pupil word, neighbourhood volts (cp.async: no register waits for them), and the record of the item after it
+template <int NL, bool PE>
+__device__ __forceinline__ void wu_issue_aux(const WfsParams& p, const WfsUmmaTables& f, unsigned char* my_aux, uint32_t my_aux_u32,
+                                             const short* amap, int amap_lane, int lane, int pe, int pk, uint2 sb, int slot,
+                                             int k_after, bool has_after) {
+  constexpr int AUXB = PE ? WU_AUX_BYTES_PE : WU_AUX_BYTES;
+  const uint32_t dst = my_aux_u32 + (uint32_t)slot * AUXB;
+  wu_cp_async4(dst + 4u * lane, f.pmask + (size_t)pk * 32 + lane);
+  if (p.use_dm && lane < 18) {
+    const int idx = (lane < 16) ? (int)amap[(int)(sb.y & 0x7fffffffu) + amap_lane] : p.pzt_nact + lane - 16;
+    if (idx >= 0) wu_cp_async4(dst + 128u + 4u * lane, p.volts + (size_t)pe * p.ldv + idx);
+    else *reinterpret_cast<float*>(my_aux + slot * AUXB + 128 + 4 * lane) = 0.f;
+  }
+  if (has_after && lane == 0) wu_cp_async8(my_aux_u32 + (uint32_t)(slot ^ 1) * AUXB + 256u, f.sub + k_after);
+  if (PE && lane < 8 * NL)      // the layer offsets of this item's environment, one word per lane
+    wu_cp_async4(dst + (uint32_t)WU_AUX_BYTES + 4u * lane,
+                 reinterpret_cast<const uint32_t*>(p.wind + (size_t)(lane >> 3) * p.E + pe) + (lane & 7));
+  asm volatile("cp.async.commit_group;" ::: "memory");
+}
+
+// The tip-tilt planes are tables (the reference's Zernike 2 / 3 are evaluated in float32 with offset centres,
+// dm_init.py:661-694 -> dm_util.py:300-380: up to 1.5 % away from a plane).  The 2 x 8 values of a lane are requested
+// at the top of the item and used after the atmosphere has been sampled (the layers are sampled one at a time so
+// that these 16 registers survive without a spill: a spill right behind the loads would wait for them).
+// tt_lane: this lane's first pixel in the tip-tilt support; xy: (y0 << 16 | x0) of the item.
+__device__ __forceinline__ void wu_load_tt(const WfsParams& p, const float* tt_plane1, int tt_lane, uint32_t xy, float4 (&tta)[2], float4 (&ttb)[2]) {
+  const int to = (int)(xy >> 16) * p.tt_dim + (int)(xy & 0xffffu) + tt_lane;
+  tta[0] = __ldg(reinterpret_cast<const float4*>(p.tt_planes + to));
+  tta[1] = __ldg(reinterpret_cast<const float4*>(p.tt_planes + to + 4));
+  ttb[0] = __ldg(reinterpret_cast<const float4*>(tt_plane1 + to));
+  ttb[1] = __ldg(reinterpret_cast<const float4*>(tt_plane1 + to + 4));
+}
+
+// mirror surface of the lane's 8 pixels as pairs P: the separable stamp of the 4 x 4 neighbourhood volts v0..v3 (fyv:
+// the y factors of the lane's row, fx: the x factors) and the tip-tilt volts vt0 / vt1 on the planes' values.  The
+// tip-tilt loads were requested before the stamp arithmetic, and the tiles of the atmosphere land meanwhile.
+__device__ __forceinline__ void wu_mirror(float4 v0, float4 v1r, float4 v2r, float4 v3, float vt0, float vt1, float4 fyv, const float* fx,
+                                          int h, const float4 (&tta)[2], const float4 (&ttb)[2], wu_f2 (&P)[4]) {
+  float u[WU_NG];
+  {
+    wu_f2 ua = wu_mul2(wu_bc(fyv.x), wu_pk(v0.x, v0.y)), ub = wu_mul2(wu_bc(fyv.x), wu_pk(v0.z, v0.w));
+    ua = wu_fma2(wu_bc(fyv.y), wu_pk(v1r.x, v1r.y), ua); ub = wu_fma2(wu_bc(fyv.y), wu_pk(v1r.z, v1r.w), ub);
+    ua = wu_fma2(wu_bc(fyv.z), wu_pk(v2r.x, v2r.y), ua); ub = wu_fma2(wu_bc(fyv.z), wu_pk(v2r.z, v2r.w), ub);
+    ua = wu_fma2(wu_bc(fyv.w), wu_pk(v3.x, v3.y), ua);   ub = wu_fma2(wu_bc(fyv.w), wu_pk(v3.z, v3.w), ub);
+    wu_upk(ua, u[0], u[1]); wu_upk(ub, u[2], u[3]);
+  }
+#pragma unroll
+  for (int jx = 0; jx < WU_NG; ++jx) {
+    const float4 fa = *reinterpret_cast<const float4*>(fx + jx * 16 + 8 * h);
+    const float4 fb = *reinterpret_cast<const float4*>(fx + jx * 16 + 8 * h + 4);
+    const wu_f2 U = wu_bc(u[jx]);
+    if (jx == 0) {
+      P[0] = wu_mul2(U, wu_pk(fa.x, fa.y)); P[1] = wu_mul2(U, wu_pk(fa.z, fa.w));
+      P[2] = wu_mul2(U, wu_pk(fb.x, fb.y)); P[3] = wu_mul2(U, wu_pk(fb.z, fb.w));
+    } else {
+      P[0] = wu_fma2(U, wu_pk(fa.x, fa.y), P[0]); P[1] = wu_fma2(U, wu_pk(fa.z, fa.w), P[1]);
+      P[2] = wu_fma2(U, wu_pk(fb.x, fb.y), P[2]); P[3] = wu_fma2(U, wu_pk(fb.z, fb.w), P[3]);
+    }
+  }
+  const wu_f2 T0 = wu_bc(vt0), T1 = wu_bc(vt1);
+  P[0] = wu_fma2(T0, wu_pk(tta[0].x, tta[0].y), P[0]); P[1] = wu_fma2(T0, wu_pk(tta[0].z, tta[0].w), P[1]);
+  P[2] = wu_fma2(T0, wu_pk(tta[1].x, tta[1].y), P[2]); P[3] = wu_fma2(T0, wu_pk(tta[1].z, tta[1].w), P[3]);
+  P[0] = wu_fma2(T1, wu_pk(ttb[0].x, ttb[0].y), P[0]); P[1] = wu_fma2(T1, wu_pk(ttb[0].z, ttb[0].w), P[1]);
+  P[2] = wu_fma2(T1, wu_pk(ttb[1].x, ttb[1].y), P[2]); P[3] = wu_fma2(T1, wu_pk(ttb[1].z, ttb[1].w), P[3]);
+}
+
+// the atmosphere on top of acc: every layer's staged tile (my_tiles + lane_off floats), with the common offsets or, with
+// PE, the item's own weights (WindRec [NL] at wind_slot); c_d: the tile column offsets of the item, 2 bits per layer
+template <int NL, bool PE>
+__device__ __forceinline__ void wu_layers(const unsigned char* my_tiles, int lane_off, const unsigned char* wind_slot, const WfsParams& p,
+                                          uint32_t c_d, WuPhase& acc) {
+#pragma unroll
+  for (int l = 0; l < NL; ++l) {
+    const float* t = reinterpret_cast<const float*>(my_tiles + l * WU_TILE_STRIDE) + lane_off;
+    if (PE) {
+      const WindRec* wr = reinterpret_cast<const WindRec*>(wind_slot);
+      switch ((c_d >> (2 * l)) & 3u) {
+        case 0: wu_layer<0>(t, wr[l], acc); break;
+        case 1: wu_layer<1>(t, wr[l], acc); break;
+        case 2: wu_layer<2>(t, wr[l], acc); break;
+        default: wu_layer<3>(t, wr[l], acc); break;
+      }
+    } else {
+      switch ((c_d >> (2 * l)) & 3u) {
+        case 0: wu_layer<0>(t, p.layer[l], acc); break;
+        case 1: wu_layer<1>(t, p.layer[l], acc); break;
+        case 2: wu_layer<2>(t, p.layer[l], acc); break;
+        default: wu_layer<3>(t, p.layer[l], acc); break;
+      }
+    }
+    asm volatile("" ::: "memory");                // one layer's window in registers at a time
+  }
+}
+
+// fold the right-hand taps into the pixel pairs
+__device__ __forceinline__ void wu_fold(const WuPhase& acc, wu_f2 (&P)[4]) {
+  float x0, x1, ya, yb;
+  wu_upk(acc.X[0], x0, x1); wu_upk(acc.Y[0], ya, yb);
+  P[0] = wu_pk(x0 + acc.y0, x1 + ya);
+  wu_upk(acc.X[1], x0, x1); x0 += yb; wu_upk(acc.Y[1], ya, yb);
+  P[1] = wu_pk(x0, x1 + ya);
+  wu_upk(acc.X[2], x0, x1); x0 += yb; wu_upk(acc.Y[2], ya, yb);
+  P[2] = wu_pk(x0, x1 + ya);
+  wu_upk(acc.X[3], x0, x1);
+  P[3] = wu_pk(x0 + yb, x1 + acc.y7);
+}
+
+// complex field exp(2 pi i t), t = phi / lambda - (x + y) / 128 turns (kt = k2 / 2 pi, hc01: -(x + y) / 128 of the
+// lane's first pixel pair), zero outside the pupil word pm; fp16 hi / lo
+__device__ __forceinline__ void wu_field(const wu_f2 (&P)[4], uint32_t pm, float kt, wu_f2 hc01, uint32_t (&re_h)[4], uint32_t (&re_l)[4],
+                                         uint32_t (&im_h)[4], uint32_t (&im_l)[4]) {
+  wu_f2 RE[4], IM[4];
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    const wu_f2 t = wu_fma2(P[c], wu_bc(kt), wu_add2(hc01, wu_bc(-(float)(2 * c) * 0.0078125f)));
+    float t0, t1;
+    wu_upk(t, t0, t1);
+    const wu_f2 ang = wu_mul2(wu_sub2(t, wu_pk(rintf(t0), rintf(t1))), wu_bc(6.283185307179586f));
+    float a0, a1;
+    wu_upk(ang, a0, a1);
+    RE[c] = wu_pk(__cosf(a0), __cosf(a1));
+    IM[c] = wu_pk(__sinf(a0), __sinf(a1));
+  }
+  if (pm != 0xffu) {
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      float r0, r1, i0, i1;
+      wu_upk(RE[c], r0, r1); wu_upk(IM[c], i0, i1);
+      const bool on0 = (pm >> (2 * c)) & 1u, on1 = (pm >> (2 * c + 1)) & 1u;
+      RE[c] = wu_pk(on0 ? r0 : 0.f, on1 ? r1 : 0.f);
+      IM[c] = wu_pk(on0 ? i0 : 0.f, on1 ? i1 : 0.f);
+    }
+  }
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    wu_split2(RE[c], re_h[c], re_l[c]);
+    wu_split2(IM[c], im_h[c], im_l[c]);
+  }
+}
+// A1 rows of the lane (a1_addr): chunks (re, h) (im, h) of the hi tile, the lo tile 8 KB further
+__device__ __forceinline__ void wu_store_a1(uint32_t a1_addr, const uint32_t (&re_h)[4], const uint32_t (&re_l)[4], const uint32_t (&im_h)[4],
+                                            const uint32_t (&im_l)[4]) {
+  wu_sts128(a1_addr, re_h[0], re_h[1], re_h[2], re_h[3]);
+  wu_sts128(a1_addr + 256u, im_h[0], im_h[1], im_h[2], im_h[3]);
+  wu_sts128(a1_addr + WU_A_BYTES, re_l[0], re_l[1], re_l[2], re_l[3]);
+  wu_sts128(a1_addr + WU_A_BYTES + 256u, im_l[0], im_l[1], im_l[2], im_l[3]);
+}
+
+// ---- tensor-core issue ----
+// The warps of a phase arrive on a count-N mbarrier, and the elected lane of the last of them issues the MMAs.  One
+// arrival per warp (release semantics, no memory barrier instruction, no atomic): the state it returns is the one before
+// the arrival, and its pending count tells the last warp (== 1), which acquires the phase it has just completed
+// (profiles/dev/mbar_count_probe.cu; a shared-memory counter with atom.acq_rel cost a MEMBAR.ALL.CTA and the compiler's
+// warp-aggregation sequence per arrival).  The count is broadcast through a shuffle and the issuing lane chosen by
+// elect.sync, so that the issue path is warp-uniform for the compiler (descriptors in uniform registers, UTCHMMA back to
+// back; under `lane == 0` every MMA sat in a per-thread waterfall loop of ~13 instructions).
+
+// the arrival of this warp's writes (generic proxy, and with tmem its tensor-memory reads); true in the last warp
+__device__ __forceinline__ bool wu_arrive(uint32_t bar, int lane, bool tmem) {
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  if (tmem) asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncwarp();
+  uint32_t pend = 0;
+  if (lane == 0) {
+    uint64_t st;
+    asm volatile("mbarrier.arrive.shared::cta.b64 %0, [%1];" : "=l"(st) : "r"(bar) : "memory");
+    asm volatile("mbarrier.pending_count.b64 %0, %1;" : "=r"(pend) : "l"(st));
+  }
+  pend = __shfl_sync(0xffffffffu, pend, 0);
+  return pend == 1u;
+}
+// in the last warp: true in the lane that issues, after it has acquired the completed phase
+__device__ __forceinline__ bool wu_elect_acquire(uint32_t bar, uint32_t parity, int* err) {
+  if (!wu_elect()) return false;
+  if (!wu_mbar_try(bar, parity)) atomicExch(err, 4);       // acquire; complete by construction
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  return true;
+}
+
+constexpr uint32_t wu_idesc1 = (1u << 4) | ((uint32_t)(64 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);  // f16 x f16 -> f32, K-major A and B
+constexpr uint32_t wu_idesc2 = wu_idesc1 | (1u << 15);                                                  // A operand MN-major
+constexpr uint32_t wu_km = (128u >> 4) << 16, wu_hi = (512u >> 4) | (1u << 14);     // LBO 128, SBO 512 (both majors)
+
+// MMA 1 into TMEM column d: D1 = A1 . B1^T in three fp16 products (q_*: shared addresses >> 4)
+__device__ __forceinline__ void wu_issue_mma1(uint32_t d, uint32_t q_a1, uint32_t q_b1) {
+  const uint32_t a_hi = q_a1 + wu_km, a_lo = a_hi + (WU_A_BYTES >> 4);
+  const uint32_t b_hi = q_b1 + wu_km, b_lo = b_hi + (WU_B_BYTES >> 4);
+#pragma unroll
+  for (int ks = 0; ks < 2; ++ks) wu_mma_f16_lo(d, a_hi + ks * 16, b_hi + ks * 16, wu_hi, wu_idesc1, ks ? 1u : 0u);
+#pragma unroll
+  for (int ks = 0; ks < 2; ++ks) wu_mma_f16_lo(d, a_lo + ks * 16, b_hi + ks * 16, wu_hi, wu_idesc1, 1u);
+#pragma unroll
+  for (int ks = 0; ks < 2; ++ks) wu_mma_f16_lo(d, a_hi + ks * 16, b_lo + ks * 16, wu_hi, wu_idesc1, 1u);
+}
+
+// MMA 2 of both A2 tiles into TMEM columns d, d + 64
+template <int FULL>
+__device__ __forceinline__ void wu_issue_mma2(uint32_t d, uint32_t q_a2, uint32_t q_b2) {
+  const uint32_t b_hi = q_b2 + wu_km, b_lo = b_hi + (WU_B_BYTES >> 4);
+#pragma unroll
+  for (int j = 0; j < 2; ++j) {
+    const uint32_t a_hi = q_a2 + j * (2 * WU_A_BYTES >> 4) + wu_km, a_lo = a_hi + (WU_A_BYTES >> 4);
+    const uint32_t dj = d + 64u * j;
+#pragma unroll
+    for (int ks = 0; ks < 2; ++ks) wu_mma2(dj, a_hi + ks * 16, wu_hi, b_hi + ks * 16, wu_hi, wu_idesc2, ks ? 1u : 0u);
+    if (FULL) {
+#pragma unroll
+      for (int ks = 0; ks < 2; ++ks) wu_mma2(dj, a_lo + ks * 16, wu_hi, b_hi + ks * 16, wu_hi, wu_idesc2, 1u);
+    }
+#pragma unroll
+    for (int ks = 0; ks < 2; ++ks) wu_mma2(dj, a_hi + ks * 16, wu_hi, b_lo + ks * 16, wu_hi, wu_idesc2, 1u);
+  }
+}
+
+// 32 stage-1 accumulator columns -> fp16 hi / lo -> A2 (MN-major: 8 consecutive fx per 16-byte group)
+template <int FULL>
+__device__ __forceinline__ void wu_store_a2(uint32_t addr, uint32_t off, const uint32_t (&tv)[32]) {
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+    uint32_t hw[4], lw[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float a = __uint_as_float(tv[8 * c + 2 * j]), b = __uint_as_float(tv[8 * c + 2 * j + 1]);
+      if (FULL) wu_split2(wu_pk(a, b), hw[j], lw[j]);
+      else { hw[j] = wu_pack(a, b); lw[j] = 0u; }
+    }
+    wu_sts128(addr + off + c * 512, hw[0], hw[1], hw[2], hw[3]);
+    if (FULL) wu_sts128(addr + WU_A_BYTES + off + c * 512, lw[0], lw[1], lw[2], lw[3]);
+  }
+}
+
+// ---- epilogue of one subaperture: lane = kept fx index ----
+// Plain path (no noise, no image kept): the centre of gravity is scale invariant and linear in |Y|^2, so the sums over
+// the lane's 32 values of a half run on packed pairs straight from the accumulator: s0p = sum, syp = sum of py x value.
+__device__ __forceinline__ void wu_sq_plain(const uint32_t (&v)[32], float py0, wu_f2& s0p, wu_f2& syp, bool first) {
+#pragma unroll
+  for (int m = 0; m < 8; ++m) {
+    const wu_f2 a = wu_pk(__uint_as_float(v[4 * m]), __uint_as_float(v[4 * m + 1]));
+    const wu_f2 b = wu_pk(__uint_as_float(v[4 * m + 2]), __uint_as_float(v[4 * m + 3]));
+    const wu_f2 t = wu_fma2(b, b, wu_mul2(a, a));
+    if (first && m == 0) {
+      s0p = t;
+      syp = wu_mul2(t, wu_bc(py0));
+    } else {
+      s0p = wu_add2(s0p, t);
+      syp = wu_fma2(t, wu_bc(py0 + (float)m), syp);
+    }
+  }
+}
+// centre of gravity from the lanes' partial sums and the slopes of item (ie, ik)
+__device__ __forceinline__ void wu_cog_store(const WfsParams& p, int lane, float s0, float sx, float sy, int ie, int ik) {
+#pragma unroll
+  for (int sft = 16; sft > 0; sft >>= 1) {
+    s0 += __shfl_xor_sync(0xffffffffu, s0, sft);
+    sx += __shfl_xor_sync(0xffffffffu, sx, sft);
+    sy += __shfl_xor_sync(0xffffffffu, sy, sft);
+  }
+  if (lane == 0) {
+    const float inv = __frcp_rn(s0);
+    const float gx = (s0 > 0.f) ? sx * inv : p.cog_offset;
+    const float gy = (s0 > 0.f) ? sy * inv : p.cog_offset;
+    float* sl = p.slopes + (size_t)ie * p.lds;
+    sl[ik] = (gx - p.cog_offset) * p.pixsize;
+    sl[p.nvalid + ik] = (gy - p.cog_offset) * p.pixsize;
+  }
+}
+
 // FULL = 1: three fp16 products in both stages (fp32-grade slopes).  0: the stage-1 result goes to stage 2 as a single
 // rounded fp16 (slopes ~3e-5 relative).
 // PE: per-environment winds (layer offsets from p.wind: the ring origin per environment, the weights per item through
@@ -283,88 +707,42 @@ template <int NL, int FULL, bool PE = false, bool NE = false>
 __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const __grid_constant__ WfsUmmaParams P) {
   const WfsParams& p = P.p;
   const WfsUmmaTables& f = P.f;
-  extern __shared__ __align__(1024) unsigned char wu_smem_raw[];
   constexpr int NLS = NL > 0 ? NL : 1;
   constexpr int AUXB = PE ? WU_AUX_BYTES_PE : WU_AUX_BYTES;
-  unsigned char* s_a1 = wu_smem_raw;                                   // [hi, lo][WU_A_BYTES]
-  unsigned char* s_a2 = s_a1 + 2 * WU_A_BYTES;                         // [tile][hi, lo][WU_A_BYTES]
-  unsigned char* s_b1 = s_a2 + 4 * WU_A_BYTES;                         // [hi, lo][WU_B_BYTES]
-  unsigned char* s_b2 = s_b1 + 2 * WU_B_BYTES;
-  unsigned char* s_tiles = s_b2 + 2 * WU_B_BYTES;                      // [warp][layer][WU_TILE_STRIDE]
-  uint64_t* s_bar = (uint64_t*)(s_tiles + (size_t)WU_WARPS * NLS * WU_TILE_STRIDE);   // [0..7] tiles, [8] MMA1 done, [9] MMA2 done
-  uint32_t* s_cnt = (uint32_t*)(s_bar + 12);                           // [2] TMEM slot   (s_bar[10], [11]: stage-1 / stage-2 arrivals of the 8 warps)
-  float* s_fx = (float*)((unsigned char*)s_bar + 128);                 // [NG][16]
-  float* s_fyT = s_fx + WU_NG * 16;                                    // [16][NG]
-  unsigned char* s_aux = (unsigned char*)(s_fyT + 16 * WU_NG);         // [warp][parity][AUXB]
-  short* s_amap = (short*)(s_aux + WU_WARPS * 2 * AUXB);
-
-  // lane through a volatile read: the compiler otherwise re-derives it from S2R SR_TID.X at ~25 places of the loop body
-  // and each of those reads stalls its warp (5 % of the stall samples in profiles/r02_wfs_umma_v5)
-  int lane;
-  asm volatile("mov.u32 %0, %%laneid;" : "=r"(lane));
+  // barrier block: [0..7] tiles, [8] MMA1 done, [9] MMA2 done, [10], [11] stage-1 / stage-2 arrivals of the 8 warps;
+  // the TMEM slot at byte 104
+  const WuSmem S = wu_smem_layout<NL, PE>();
+  const int lane = wu_lane();
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
   const int y = lane & 15, h = lane >> 4;
 
-  for (int i = threadIdx.x; i < 2 * WU_B_BYTES / 16; i += blockDim.x) {
-    reinterpret_cast<uint4*>(s_b1)[i] = f.b1[i];
-    reinterpret_cast<uint4*>(s_b2)[i] = f.b2[i];
-  }
-  for (int i = threadIdx.x; i < 2 * WU_NG * 16; i += blockDim.x) s_fx[i] = f.fxy[i];
-  for (int i = threadIdx.x; i < f.GW * f.GW; i += blockDim.x) s_amap[i] = f.amap[i];
-  // operand tiles start from zeros: rows of work items that do not exist are multiplied too
-  for (int i = threadIdx.x; i < 6 * WU_A_BYTES / 16; i += blockDim.x) reinterpret_cast<uint4*>(s_a1)[i] = make_uint4(0u, 0u, 0u, 0u);
-  if (threadIdx.x < 12)
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(wu_smem_u32(s_bar + threadIdx.x)), "r"(threadIdx.x < 10 ? 1u : (uint32_t)WU_WARPS) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");          // B tiles / zeroed A tiles are read by the tensor core
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(wu_smem_u32(s_cnt + 2)), "r"((uint32_t)WU_TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_base = __shfl_sync(0xffffffffu, s_cnt[2], 0);
+  const uint32_t tmem_base = wu_cta_setup(S, f, threadIdx.x, blockDim.x, warp, 12, threadIdx.x < 10 ? 1u : (uint32_t)WU_WARPS,
+                                          (uint32_t*)(S.bar + 13));
 
-  unsigned char* my_tiles = s_tiles + (size_t)warp * NLS * WU_TILE_STRIDE;
+  unsigned char* my_tiles = S.tiles + (size_t)warp * NLS * WU_TILE_STRIDE;
   const uint32_t my_tiles_u32 = wu_smem_u32(my_tiles);
-  const uint32_t my_bar_u32 = wu_smem_u32(s_bar + warp);
-  const uint32_t mma1_bar = wu_smem_u32(s_bar + 8), mma2_bar = wu_smem_u32(s_bar + 9);
-  unsigned char* my_aux = s_aux + (size_t)warp * 2 * AUXB;     // per parity: pm[32] | volts[32] | record
+  const uint32_t my_bar_u32 = wu_smem_u32(S.bar + warp);
+  const uint32_t mma1_bar = wu_smem_u32(S.bar + 8), mma2_bar = wu_smem_u32(S.bar + 9);
+  unsigned char* my_aux = S.aux + (size_t)warp * 2 * AUXB;     // per parity: pm[32] | volts[32] | record
   const uint32_t my_aux_u32 = wu_smem_u32(my_aux);
   const int lane_off = y * WU_TILE_W + 8 * h;                          // floats, inside a tile
   const int amap_lane = (lane >> 2) * f.GW + (lane & 3);
   const int tt_lane = (y + p.tt_off) * p.tt_dim + 8 * h + p.tt_off;    // this lane's first pixel in the tip-tilt support
   const float* const tt_plane1 = p.tt_planes + (size_t)p.tt_dim * p.tt_dim;
-  // The tip-tilt planes are tables (the reference's Zernike 2 / 3 are evaluated in float32 with offset centres,
-  // dm_init.py:661-694 -> dm_util.py:300-380: up to 1.5 % away from a plane).  The 2 x 8 values of a lane are requested
-  // at the top of the item and used after the atmosphere has been sampled (the layers are sampled one at a time so
-  // that these 16 registers survive without a spill: a spill right behind the loads would wait for them).
   float4 tta[2], ttb[2];
-  auto load_tta = [&](uint32_t xy) {       // first plane: requested at the top of the item
-    const int to = (int)(xy >> 16) * p.tt_dim + (int)(xy & 0xffffu) + tt_lane;
-    tta[0] = __ldg(reinterpret_cast<const float4*>(p.tt_planes + to));
-    tta[1] = __ldg(reinterpret_cast<const float4*>(p.tt_planes + to + 4));
-  };
-  auto load_ttb = [&](uint32_t xy) {       // second plane: requested once the tile windows have left the registers
-    const int to = (int)(xy >> 16) * p.tt_dim + (int)(xy & 0xffffu) + tt_lane;
-    ttb[0] = __ldg(reinterpret_cast<const float4*>(tt_plane1 + to));
-    ttb[1] = __ldg(reinterpret_cast<const float4*>(tt_plane1 + to + 4));
-  };
-  const float4 fyv = *reinterpret_cast<const float4*>(s_fyT + y * WU_NG);      // y stamp factors of this lane's row (constant)
+  const float4 fyv = *reinterpret_cast<const float4*>(S.fyT + y * WU_NG);      // y stamp factors of this lane's row (constant)
   // phase in turns: t = phi / lambda - (x + y) / 128   (halfxy = pi (x + y) / 64, geom_init.py:690-701)
   const float kt = p.k2 * 0.15915494309189535f;
   const float hc0 = -(float)(y + 8 * h) * 0.0078125f;
   const wu_f2 hc01 = wu_pk(hc0, hc0 - 0.0078125f);
 
   // A1 rows of this lane: r = 16 warp + y ; chunks (re, h) (im, h) of the hi tile, the lo tile 8 KB further
-  const uint32_t a1_addr = wu_smem_u32(s_a1) + (uint32_t)((2 * warp + (y >> 3)) * 512 + (y & 7) * 16 + h * 128);
+  const uint32_t a1_addr = wu_smem_u32(S.a1) + (uint32_t)((2 * warp + (y >> 3)) * 512 + (y & 7) * 16 + h * 128);
   // conversion role: TMEM lane quarter qq = warp & 3 (rows 32 qq .. = subapertures 2 qq, 2 qq + 1), part ro = warp >> 2
   const int qq = warp & 3, ro = warp >> 2;
   const uint32_t d1_addr = tmem_base + ((uint32_t)(32 * qq) << 16) + (uint32_t)(32 * ro);
   // A2: tile qq >> 1, rows m = 32 s' + fx with s' = 2 (qq & 1) + h, K index 16 ro + y
-  const uint32_t a2_addr = wu_smem_u32(s_a2) + (uint32_t)((qq >> 1) * 2 * WU_A_BYTES + (4 * (2 * (qq & 1) + h)) * 512 +
+  const uint32_t a2_addr = wu_smem_u32(S.a2) + (uint32_t)((qq >> 1) * 2 * WU_A_BYTES + (4 * (2 * (qq & 1) + h)) * 512 +
                                                          (2 * ro + (y >> 3)) * 128 + (y & 7) * 16);
   // epilogue role: own subaperture = rows 32 (warp & 3) .. of tile warp >> 2
   const uint32_t d2_addr = tmem_base + ((uint32_t)(32 * qq) << 16) + (uint32_t)(64 + 64 * ro);
@@ -384,144 +762,25 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
   uint32_t n_d = 0;                                              // tile column offsets of the item whose tiles were issued last
   bool n_seam = false;
 
-  // ---- tiles of one work item (record sb): TMA boxes, or element-wise wrapped cp.async copies on the torus seam ----
   auto issue_tiles = [&](int pe, uint2 sb) {
-    if (NL == 0) return;
-    if (pe != ring_e) {
-#pragma unroll
-      for (int l = 0; l < NL; ++l) {
-        const int N = p.layer[l].N;
-        int a = (PE ? __ldg(&p.wind[(size_t)l * p.E + pe].ix) : p.layer[l].ix) + p.layer[l].ox[pe];  a -= (a >= N) ? N : 0;
-        int b = (PE ? __ldg(&p.wind[(size_t)l * p.E + pe].iy) : p.layer[l].iy) + p.layer[l].oy[pe];  b -= (b >= N) ? N : 0;
-        rx[l] = a; ry[l] = b;
-      }
-      ring_e = pe;
-    }
-    const int x0 = (int)(sb.x & 0xffffu), y0 = (int)(sb.x >> 16);
-    int tc[NLS], tr[NLS];
-    bool seam = false;
-    uint32_t dbits = 0;
-#pragma unroll
-    for (int l = 0; l < NL; ++l) {
-      const int N = p.layer[l].N;
-      int c = x0 + rx[l];  c -= (c >= N) ? N : 0;
-      int r = y0 + ry[l];  r -= (r >= N) ? N : 0;
-      tc[l] = c & ~3; tr[l] = r;
-      dbits |= (uint32_t)(c & 3) << (2 * l);
-      seam |= (c + WU_TILE_H > N) | (r + WU_TILE_H > N);
-    }
-    n_seam = seam;
-    n_d = dbits;
-    if (!seam) {
-      // the stage was read with plain loads: order them before the async-proxy writes of the new boxes
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      __syncwarp();
-      if (wu_elect()) {       // elect.sync: a warp-uniform issue path (no per-thread waterfall around the TMA instructions)
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(my_bar_u32), "r"(NL * WU_TILE_BYTES) : "memory");
-#pragma unroll
-        for (int l = 0; l < NL; ++l)
-          wu_tma_load_3d(my_tiles_u32 + l * WU_TILE_STRIDE, &P.maps[l], tc[l], tr[l], pe, my_bar_u32);
-      }
-    } else {
-      // (rare path: keep its per-lane index arithmetic here instead of in registers that live across the whole loop)
-      int ln = lane;
-      asm volatile("" : "+r"(ln));
-#pragma unroll
-      for (int l = 0; l < NL; ++l) {
-        const int N = p.layer[l].N;
-        const float* scr = p.layer[l].screen + (size_t)pe * N * N;
-        const int c0 = tc[l] + (int)((dbits >> (2 * l)) & 3u), r0 = tr[l];
-        const uint32_t dst0 = my_tiles_u32 + l * WU_TILE_STRIDE + ((dbits >> (2 * l)) & 3u) * 4u;
-#pragma unroll 1
-        for (int i0 = 0; i0 < WU_TILE_H * WU_TILE_H; i0 += 32) {
-          const int i = i0 + ln;
-          if (i < WU_TILE_H * WU_TILE_H) {
-            const int r = i / WU_TILE_H, c = i - r * WU_TILE_H;
-            int rr = r0 + r;  rr -= (rr >= N) ? N : 0;
-            int cc = c0 + c;  cc -= (cc >= N) ? N : 0;
-            wu_cp_async4(dst0 + (uint32_t)(r * WU_TILE_W + c) * 4u, scr + (size_t)rr * N + cc);
-          }
-        }
-      }
-      asm volatile("cp.async.commit_group;" ::: "memory");
-    }
+    wu_issue_tiles<NL, PE>(P, my_tiles_u32, my_bar_u32, lane, pe, sb, ring_e, rx, ry, n_d, n_seam);
   };
-
-  // ---- per-lane inputs of one work item into the parity slot: pupil word, neighbourhood volts (cp.async: no register
-  //      waits for them), and the record of the item after it ----
   auto issue_aux = [&](int pe, int pk, uint2 sb, int slot, int k_after, bool has_after) {
-    const uint32_t dst = my_aux_u32 + (uint32_t)slot * AUXB;
-    wu_cp_async4(dst + 4u * lane, f.pmask + (size_t)pk * 32 + lane);
-    if (p.use_dm && lane < 18) {
-      const int idx = (lane < 16) ? (int)s_amap[(int)(sb.y & 0x7fffffffu) + amap_lane] : p.pzt_nact + lane - 16;
-      if (idx >= 0) wu_cp_async4(dst + 128u + 4u * lane, p.volts + (size_t)pe * p.ldv + idx);
-      else *reinterpret_cast<float*>(my_aux + slot * AUXB + 128 + 4 * lane) = 0.f;
-    }
-    if (has_after && lane == 0) wu_cp_async8(my_aux_u32 + (uint32_t)(slot ^ 1) * AUXB + 256u, f.sub + k_after);
-    if (PE && lane < 8 * NL)      // the layer offsets of this item's environment, one word per lane
-      wu_cp_async4(dst + (uint32_t)WU_AUX_BYTES + 4u * lane,
-                   reinterpret_cast<const uint32_t*>(p.wind + (size_t)(lane >> 3) * p.E + pe) + (lane & 7));
-    asm volatile("cp.async.commit_group;" ::: "memory");
+    wu_issue_aux<NL, PE>(p, f, my_aux, my_aux_u32, S.amap, amap_lane, lane, pe, pk, sb, slot, k_after, has_after);
   };
 
-  // ---- lane 0 of the last warp to arrive issues the tensor-core work of the group ----
-  const uint32_t idesc1 = (1u << 4) | ((uint32_t)(64 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);   // f16 x f16 -> f32, K-major A and B
-  const uint32_t idesc2 = idesc1 | (1u << 15);                                                      // A operand MN-major
-  // The arrival count is broadcast through a shuffle and the issuing lane chosen by elect.sync, so that the issue path is
-  // warp-uniform for the compiler (descriptors in uniform registers, UTCHMMA back to back; under `lane == 0` every MMA
-  // sat in a per-thread waterfall loop of ~13 instructions).
-  const uint32_t q_a1 = __shfl_sync(0xffffffffu, wu_smem_u32(s_a1) >> 4, 0), q_b1 = __shfl_sync(0xffffffffu, wu_smem_u32(s_b1) >> 4, 0);
-  const uint32_t q_a2 = __shfl_sync(0xffffffffu, wu_smem_u32(s_a2) >> 4, 0), q_b2 = __shfl_sync(0xffffffffu, wu_smem_u32(s_b2) >> 4, 0);
-  const uint32_t arr_bar = wu_smem_u32(s_bar + 10);
+  const uint32_t q_a1 = __shfl_sync(0xffffffffu, wu_smem_u32(S.a1) >> 4, 0), q_b1 = __shfl_sync(0xffffffffu, wu_smem_u32(S.b1) >> 4, 0);
+  const uint32_t q_a2 = __shfl_sync(0xffffffffu, wu_smem_u32(S.a2) >> 4, 0), q_b2 = __shfl_sync(0xffffffffu, wu_smem_u32(S.b2) >> 4, 0);
+  const uint32_t arr_bar = wu_smem_u32(S.bar + 10);
+  // which = 0: MMA 1 (A1 written, T drained), 1: MMA 2 (A2 written, Y drained)
   auto arrive_and_issue = [&](int which, uint32_t arr_parity) {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncwarp();
-    // One arrival per warp on a count-8 mbarrier (release semantics, no memory barrier instruction, no atomic): the state
-    // it returns is the one before the arrival, and its pending count tells the last of the eight warps (== 1), which
-    // acquires the phase it has just completed and issues (profiles/dev/mbar_count_probe.cu; a shared-memory counter
-    // with atom.acq_rel cost a MEMBAR.ALL.CTA and the compiler's warp-aggregation sequence per arrival).
-    uint32_t pend = 0;
-    if (lane == 0) {
-      uint64_t st;
-      asm volatile("mbarrier.arrive.shared::cta.b64 %0, [%1];" : "=l"(st) : "r"(arr_bar + 8u * which) : "memory");
-      asm volatile("mbarrier.pending_count.b64 %0, %1;" : "=r"(pend) : "l"(st));
-    }
-    pend = __shfl_sync(0xffffffffu, pend, 0);
-    if (pend == 1u) {
-      if (wu_elect()) {
-        if (!wu_mbar_try(arr_bar + 8u * which, arr_parity)) atomicExch(f.err, 4);       // acquire; complete by construction
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        constexpr uint32_t KM = (128u >> 4) << 16, HI = (512u >> 4) | (1u << 14);     // K-major: LBO 128, SBO 512
-        if (which == 0) {
-          const uint32_t a_hi = q_a1 + KM, a_lo = a_hi + (WU_A_BYTES >> 4);
-          const uint32_t b_hi = q_b1 + KM, b_lo = b_hi + (WU_B_BYTES >> 4);
-#pragma unroll
-          for (int ks = 0; ks < 2; ++ks) wu_mma_f16_lo(tmem_base, a_hi + ks * 16, b_hi + ks * 16, HI, idesc1, ks ? 1u : 0u);
-#pragma unroll
-          for (int ks = 0; ks < 2; ++ks) wu_mma_f16_lo(tmem_base, a_lo + ks * 16, b_hi + ks * 16, HI, idesc1, 1u);
-#pragma unroll
-          for (int ks = 0; ks < 2; ++ks) wu_mma_f16_lo(tmem_base, a_hi + ks * 16, b_lo + ks * 16, HI, idesc1, 1u);
-          wu_commit(mma1_bar);
-        } else {
-          const uint32_t b_hi = q_b2 + KM, b_lo = b_hi + (WU_B_BYTES >> 4);
-          const uint32_t am = (128u >> 4) << 16, hia = (512u >> 4) | (1u << 14);     // MN-major: LBO 128, SBO 512
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            const uint32_t a_hi = q_a2 + j * (2 * WU_A_BYTES >> 4) + am, a_lo = a_hi + (WU_A_BYTES >> 4);
-            const uint32_t d = tmem_base + 64u + 64u * j;
-#pragma unroll
-            for (int ks = 0; ks < 2; ++ks) wu_mma2(d, a_hi + ks * 16, hia, b_hi + ks * 16, HI, idesc2, ks ? 1u : 0u);
-            if (FULL) {
-#pragma unroll
-              for (int ks = 0; ks < 2; ++ks) wu_mma2(d, a_lo + ks * 16, hia, b_hi + ks * 16, HI, idesc2, 1u);
-            }
-#pragma unroll
-            for (int ks = 0; ks < 2; ++ks) wu_mma2(d, a_hi + ks * 16, hia, b_lo + ks * 16, HI, idesc2, 1u);
-          }
-          wu_commit(mma2_bar);
-        }
+    if (wu_arrive(arr_bar + 8u * which, lane, true) && wu_elect_acquire(arr_bar + 8u * which, arr_parity, f.err)) {
+      if (which == 0) {
+        wu_issue_mma1(tmem_base, q_a1, q_b1);
+        wu_commit(mma1_bar);
+      } else {
+        wu_issue_mma2<FULL>(tmem_base + 64u, q_a2, q_b2);
+        wu_commit(mma2_bar);
       }
     }
     __syncwarp();
@@ -538,23 +797,6 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
     }
   };
   // ---- epilogue of one subaperture: lane = kept fx index; qa / qb = the fy pairs of py 8..15 / 0..7 ----
-  // plain path (no noise, no image kept): the centre of gravity is scale invariant and linear in |Y|^2, so the sums
-  // over the lane's 32 values run on packed pairs straight from the accumulator: s0p = sum, syp = sum of py x value
-  auto sq_plain = [&](const uint32_t (&v)[32], float py0, wu_f2& s0p, wu_f2& syp, bool first) {
-#pragma unroll
-    for (int m = 0; m < 8; ++m) {
-      const wu_f2 a = wu_pk(__uint_as_float(v[4 * m]), __uint_as_float(v[4 * m + 1]));
-      const wu_f2 b = wu_pk(__uint_as_float(v[4 * m + 2]), __uint_as_float(v[4 * m + 3]));
-      const wu_f2 t = wu_fma2(b, b, wu_mul2(a, a));
-      if (first && m == 0) {
-        s0p = t;
-        syp = wu_mul2(t, wu_bc(py0));
-      } else {
-        s0p = wu_add2(s0p, t);
-        syp = wu_fma2(t, wu_bc(py0 + (float)m), syp);
-      }
-    }
-  };
   auto epilogue = [&](const float (&qa)[8], const float (&qb)[8], wu_f2 s0p, wu_f2 syp, int ie, int ik, bool pl) {
     const int pr = lane >> 1;                                  // fx pair: kept indices 2 pr, 2 pr + 1
     const int px = (pr < 8) ? 8 + pr : pr - 8;
@@ -596,20 +838,7 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
         sy = fmaf(v, (float)py, sy);
       }
     }
-#pragma unroll
-    for (int sft = 16; sft > 0; sft >>= 1) {
-      s0 += __shfl_xor_sync(0xffffffffu, s0, sft);
-      sx += __shfl_xor_sync(0xffffffffu, sx, sft);
-      sy += __shfl_xor_sync(0xffffffffu, sy, sft);
-    }
-    if (lane == 0) {
-      const float inv = __frcp_rn(s0);
-      const float gx = (s0 > 0.f) ? sx * inv : p.cog_offset;
-      const float gy = (s0 > 0.f) ? sy * inv : p.cog_offset;
-      float* sl = p.slopes + (size_t)ie * p.lds;
-      sl[ik] = (gx - p.cog_offset) * p.pixsize;
-      sl[p.nvalid + ik] = (gy - p.cog_offset) * p.pixsize;
-    }
+    wu_cog_store(p, lane, s0, sx, sy, ie, ik);
   };
 
   // ---- prologue: item 0 entirely, the record of item 1 ----
@@ -644,8 +873,7 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
       float4 v0 = make_float4(0.f, 0.f, 0.f, 0.f), v1r = v0, v2r = v0, v3 = v0;
       float vt0 = 0.f, vt1 = 0.f;
       if (p.use_dm) {
-        load_tta(xy_cur);
-        load_ttb(xy_cur);
+        wu_load_tt(p, tt_plane1, tt_lane, xy_cur, tta, ttb);
         v0 = *reinterpret_cast<const float4*>(V); v1r = *reinterpret_cast<const float4*>(V + 4);
         v2r = *reinterpret_cast<const float4*>(V + 8); v3 = *reinterpret_cast<const float4*>(V + 12);
         vt0 = V[16]; vt1 = V[17];
@@ -667,34 +895,9 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
       //      requested at once and consumed after the stamp arithmetic, and the tiles of the atmosphere get the whole
       //      section to land ----
       if (p.use_dm) {
-        float u[WU_NG];
-        {
-          wu_f2 ua = wu_mul2(wu_bc(fyv.x), wu_pk(v0.x, v0.y)), ub = wu_mul2(wu_bc(fyv.x), wu_pk(v0.z, v0.w));
-          ua = wu_fma2(wu_bc(fyv.y), wu_pk(v1r.x, v1r.y), ua); ub = wu_fma2(wu_bc(fyv.y), wu_pk(v1r.z, v1r.w), ub);
-          ua = wu_fma2(wu_bc(fyv.z), wu_pk(v2r.x, v2r.y), ua); ub = wu_fma2(wu_bc(fyv.z), wu_pk(v2r.z, v2r.w), ub);
-          ua = wu_fma2(wu_bc(fyv.w), wu_pk(v3.x, v3.y), ua);   ub = wu_fma2(wu_bc(fyv.w), wu_pk(v3.z, v3.w), ub);
-          wu_upk(ua, u[0], u[1]); wu_upk(ub, u[2], u[3]);
-        }
-#pragma unroll
-        for (int jx = 0; jx < WU_NG; ++jx) {
-          const float4 fa = *reinterpret_cast<const float4*>(s_fx + jx * 16 + 8 * h);
-          const float4 fb = *reinterpret_cast<const float4*>(s_fx + jx * 16 + 8 * h + 4);
-          const wu_f2 U = wu_bc(u[jx]);
-          if (jx == 0) {
-            P[0] = wu_mul2(U, wu_pk(fa.x, fa.y)); P[1] = wu_mul2(U, wu_pk(fa.z, fa.w));
-            P[2] = wu_mul2(U, wu_pk(fb.x, fb.y)); P[3] = wu_mul2(U, wu_pk(fb.z, fb.w));
-          } else {
-            P[0] = wu_fma2(U, wu_pk(fa.x, fa.y), P[0]); P[1] = wu_fma2(U, wu_pk(fa.z, fa.w), P[1]);
-            P[2] = wu_fma2(U, wu_pk(fb.x, fb.y), P[2]); P[3] = wu_fma2(U, wu_pk(fb.z, fb.w), P[3]);
-          }
-        }
-        const wu_f2 T0 = wu_bc(vt0), T1 = wu_bc(vt1);
-        P[0] = wu_fma2(T0, wu_pk(tta[0].x, tta[0].y), P[0]); P[1] = wu_fma2(T0, wu_pk(tta[0].z, tta[0].w), P[1]);
-        P[2] = wu_fma2(T0, wu_pk(tta[1].x, tta[1].y), P[2]); P[3] = wu_fma2(T0, wu_pk(tta[1].z, tta[1].w), P[3]);
-        P[0] = wu_fma2(T1, wu_pk(ttb[0].x, ttb[0].y), P[0]); P[1] = wu_fma2(T1, wu_pk(ttb[0].z, ttb[0].w), P[1]);
-        P[2] = wu_fma2(T1, wu_pk(ttb[1].x, ttb[1].y), P[2]); P[3] = wu_fma2(T1, wu_pk(ttb[1].z, ttb[1].w), P[3]);
+        wu_mirror(v0, v1r, v2r, v3, vt0, vt1, fyv, S.fx, h, tta, ttb, P);
       } else {
-#pragma unroll
+      #pragma unroll
         for (int j = 0; j < 4; ++j) P[j] = 0ull;
       }
 
@@ -710,39 +913,10 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
           wu_mbar_wait(my_bar_u32, tile_phase, f.err);
           tile_phase ^= 1u;
         }
-#pragma unroll
-        for (int l = 0; l < NL; ++l) {
-          const float* t = reinterpret_cast<const float*>(my_tiles + l * WU_TILE_STRIDE) + lane_off;
-          if (PE) {
-            const WindRec* wr = reinterpret_cast<const WindRec*>(my_aux + s * AUXB + WU_AUX_BYTES);
-            switch ((c_d >> (2 * l)) & 3u) {
-              case 0: wu_layer<0>(t, wr[l], acc); break;
-              case 1: wu_layer<1>(t, wr[l], acc); break;
-              case 2: wu_layer<2>(t, wr[l], acc); break;
-              default: wu_layer<3>(t, wr[l], acc); break;
-            }
-          } else {
-            switch ((c_d >> (2 * l)) & 3u) {
-              case 0: wu_layer<0>(t, p.layer[l], acc); break;
-              case 1: wu_layer<1>(t, p.layer[l], acc); break;
-              case 2: wu_layer<2>(t, p.layer[l], acc); break;
-              default: wu_layer<3>(t, p.layer[l], acc); break;
-            }
-          }
-          asm volatile("" ::: "memory");                // one layer's window in registers at a time
-        }
+        wu_layers<NL, PE>(my_tiles, lane_off, my_aux + s * AUXB + WU_AUX_BYTES, p, c_d, acc);
         __syncwarp();                                   // the stage is drained: re-arm it with the next item
         if (nx_valid) issue_tiles(e, sb1);
-        // fold the right-hand taps into the pixel pairs
-        float x0, x1, ya, yb;
-        wu_upk(acc.X[0], x0, x1); wu_upk(acc.Y[0], ya, yb);
-        P[0] = wu_pk(x0 + acc.y0, x1 + ya);
-        wu_upk(acc.X[1], x0, x1); x0 += yb; wu_upk(acc.Y[1], ya, yb);
-        P[1] = wu_pk(x0, x1 + ya);
-        wu_upk(acc.X[2], x0, x1); x0 += yb; wu_upk(acc.Y[2], ya, yb);
-        P[2] = wu_pk(x0, x1 + ya);
-        wu_upk(acc.X[3], x0, x1);
-        P[3] = wu_pk(x0 + yb, x1 + acc.y7);
+        wu_fold(acc, P);
       }
 
     }
@@ -758,41 +932,11 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
     }
 
     if (c_valid) {
-      // ---- complex field exp(2 pi i t), t = phi / lambda - (x + y) / 128 turns; fp16 hi / lo ----
-      wu_f2 RE[4], IM[4];
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        const wu_f2 t = wu_fma2(P[c], wu_bc(kt), wu_add2(hc01, wu_bc(-(float)(2 * c) * 0.0078125f)));
-        float t0, t1;
-        wu_upk(t, t0, t1);
-        const wu_f2 ang = wu_mul2(wu_sub2(t, wu_pk(rintf(t0), rintf(t1))), wu_bc(6.283185307179586f));
-        float a0, a1;
-        wu_upk(ang, a0, a1);
-        RE[c] = wu_pk(__cosf(a0), __cosf(a1));
-        IM[c] = wu_pk(__sinf(a0), __sinf(a1));
-      }
-      if (c_pm != 0xffu) {
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          float r0, r1, i0, i1;
-          wu_upk(RE[c], r0, r1); wu_upk(IM[c], i0, i1);
-          const bool on0 = (c_pm >> (2 * c)) & 1u, on1 = (c_pm >> (2 * c + 1)) & 1u;
-          RE[c] = wu_pk(on0 ? r0 : 0.f, on1 ? r1 : 0.f);
-          IM[c] = wu_pk(on0 ? i0 : 0.f, on1 ? i1 : 0.f);
-        }
-      }
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        wu_split2(RE[c], re_h[c], re_l[c]);
-        wu_split2(IM[c], im_h[c], im_l[c]);
-      }
+      wu_field(P, c_pm, kt, hc01, re_h, re_l, im_h, im_l);
     }
 
     if (c_valid) {
-      wu_sts128(a1_addr, re_h[0], re_h[1], re_h[2], re_h[3]);
-      wu_sts128(a1_addr + 256u, im_h[0], im_h[1], im_h[2], im_h[3]);
-      wu_sts128(a1_addr + WU_A_BYTES, re_l[0], re_l[1], re_l[2], re_l[3]);
-      wu_sts128(a1_addr + WU_A_BYTES + 256u, im_l[0], im_l[1], im_l[2], im_l[3]);
+      wu_store_a1(a1_addr, re_h, re_l, im_h, im_l);
     }
     if (conv) asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
     if (it < n_iter) arrive_and_issue(0, (uint32_t)(it & 1));             // A1(it) written and T(it-1) drained by this warp
@@ -803,21 +947,7 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
     if (epi) {
       wu_mbar_wait(mma2_bar, (uint32_t)((it - 2) & 1), f.err);
     }
-    if (conv) {
-      // ---- C(it-1): T -> fp16 hi / lo -> A2 (MN-major: 8 consecutive fx per 16-byte group) ----
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        uint32_t hw[4], lw[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float a = __uint_as_float(tv[8 * c + 2 * j]), b = __uint_as_float(tv[8 * c + 2 * j + 1]);
-          if (FULL) wu_split2(wu_pk(a, b), hw[j], lw[j]);
-          else { hw[j] = wu_pack(a, b); lw[j] = 0u; }
-        }
-        wu_sts128(a2_addr + c * 512, hw[0], hw[1], hw[2], hw[3]);
-        if (FULL) wu_sts128(a2_addr + WU_A_BYTES + c * 512, lw[0], lw[1], lw[2], lw[3]);
-      }
-    }
+    if (conv) wu_store_a2<FULL>(a2_addr, 0u, tv);   // C(it-1): T -> fp16 hi / lo -> A2
 
     // ---- E(it-2) ----
     // plain path of item it-2: the batch's, or with NE its environment's (a noise-free environment of a mixed launch
@@ -829,10 +959,10 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       wu_tmem_ld32(d2_addr, yv);
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      if (pl) sq_plain(yv, 8.f, s0p, syp, true); else sq_half(yv, qa);
+      if (pl) wu_sq_plain(yv, 8.f, s0p, syp, true); else sq_half(yv, qa);
       wu_tmem_ld32(d2_addr + 32u, yv);
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      if (pl) sq_plain(yv, 0.f, s0p, syp, false); else sq_half(yv, qb);
+      if (pl) wu_sq_plain(yv, 0.f, s0p, syp, false); else sq_half(yv, qb);
     }
     if (conv) arrive_and_issue(1, (uint32_t)((it - 1) & 1));                    // A2(it-1) written and Y(it-2) drained by this warp
     if (epi && it - 2 < n_mine) epilogue(qa, qb, s0p, syp, (int)(ek2 >> 16), (int)(ek2 & 0xffffu), pl);
@@ -842,10 +972,5 @@ __global__ void __launch_bounds__(WU_WARPS * 32, 2) wfs_frame_umma_kernel(const 
     ek0 = ((uint32_t)e << 16) | (uint32_t)k;          // the item prefetched in this iteration is sampled in the next
   }
 
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)WU_TMEM_COLS) : "memory");
-  }
+  wu_cta_release(warp, tmem_base);
 }
