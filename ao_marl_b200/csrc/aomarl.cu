@@ -13,6 +13,7 @@
 #include "gemm_kernels.cuh"
 #include "gemm_tc.cuh"
 #include "rtc_kernels.cuh"
+#include "snapshot_kernels.cuh"
 #include "wfs_kernels.cuh"
 #include "wfs_mma.cuh"
 #include "wfs_lattice_host.h"
@@ -125,6 +126,12 @@ struct aom_ctx {
   uint32_t* step_env;          // device [E] actor decision counters
   int* le_n;                   // device [2][E] long-exposure counts (main target, geometric target)
   int* first;                  // device [E] first step pending
+  // snapshots (aom_save_envs / aom_load_envs): device list of environments and loaded wind accumulators [L][2][n], and
+  // the host staging block they are copied from (kept until the stream has passed the copy)
+  int* snap_envs;
+  double* snap_acc;
+  void* snap_h;
+  size_t snap_h_bytes;
   // staged Shack-Hartmann kernels: host copies of the tables their own tables derive from; fast_why says why the last
   // refused preparation refused
   void* htab[AOM_T_COUNT];
@@ -331,7 +338,7 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
                   ctx->action_mean, ctx->strehl, ctx->tar_mom, ctx->tar_acc, ctx->aX, ctx->aH1, ctx->aH2, ctx->aHO, ctx->d_err,
                   ctx->geo_com, ctx->geo_volts, ctx->geo_b, ctx->geo_T, ctx->strehl_geo, ctx->geo_acc, ctx->geo_mom,
                   ctx->sweep_mask, ctx->sweep_ttp, ctx->rs_envs, ctx->rs_seeds, ctx->frame0, ctx->step_env,
-                  ctx->le_n, ctx->first};
+                  ctx->le_n, ctx->first, ctx->snap_envs, ctx->snap_acc};
   for (void* b : bufs) cudaFree(b);
   for (int l = 0; l < AOM_MAX_LAYERS; ++l) { cudaFree(ctx->oz_ab[l]); cudaFree(ctx->oz_ea[l]); }
   for (int t = 0; t < AOM_T_COUNT; ++t) { cudaFree(ctx->ozop[t]); cudaFree(ctx->ozop_ea[t]); }
@@ -348,6 +355,7 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
   if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
   if (ctx->ev_geo) cudaEventDestroy(ctx->ev_geo);
   for (int t = 0; t < AOM_T_COUNT; ++t) free(ctx->htab[t]);
+  free(ctx->snap_h);
   free(ctx);
 }
 
@@ -769,9 +777,10 @@ static bool wind_any_env(const aom_ctx* ctx) {
 
 // One transition of the wind state of every layer and environment (WIND_STEP / WIND_INIT / WIND_RESET, atmos_kernels.cuh)
 // on the device, asynchronously on `st`, and the same on the host mirror: passes per layer and offset bounds.
-// WIND_RESET_ENVS: WIND_RESET of the K environments listed in envs_d (device) / envs_h (host) only.
+// WIND_RESET_ENVS: WIND_RESET of the K environments listed in envs_d (device) / envs_h (host) only.  WIND_LOAD_ENVS:
+// their accumulators <- acc_d (device) / acc_h (host), both [L][2][K].
 static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st, const int* envs_d = nullptr, const int* envs_h = nullptr,
-                       int K = 0) {
+                       int K = 0, const double* acc_d = nullptr, const double* acc_h = nullptr) {
   const aom_config& c = ctx->cfg;
   const int E = c.n_env, L = c.n_layers;
   if (L == 0) return AOM_OK;
@@ -784,8 +793,17 @@ static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st, const int* envs_
   }
   P.acc = ctx->wind_acc; P.steps = ctx->wind_steps; P.rec = ctx->wind_rec; P.E = E; P.n_layers = L; P.mode = mode;
   P.envs = envs_d; P.K = K;
-  const int n = mode == WIND_RESET_ENVS ? K : E;
-  wind_state_kernel<<<(L * n + 255) / 256, 256, 0, st>>>(P);
+  if (mode == WIND_LOAD_ENVS) {
+    WindLoadParams Q;
+    memset(&Q, 0, sizeof(Q));
+    for (int l = 0; l < L; ++l) { Q.xoff[l] = c.wfs_xoff[l]; Q.yoff[l] = c.wfs_yoff[l]; }
+    Q.acc = ctx->wind_acc; Q.steps = ctx->wind_steps; Q.rec = ctx->wind_rec; Q.envs = envs_d; Q.acc_in = acc_d;
+    Q.E = E; Q.K = K; Q.n_layers = L;
+    wind_load_kernel<<<(L * K + 255) / 256, 256, 0, st>>>(Q);
+  } else {
+    const int n = mode == WIND_RESET_ENVS ? K : E;
+    wind_state_kernel<<<(L * n + 255) / 256, 256, 0, st>>>(P);
+  }
   KCHECK();
   for (int l = 0; l < L; ++l) {
     const WindLayerParams& W = P.layer[l];
@@ -797,6 +815,11 @@ static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st, const int* envs_
       for (int k = 0; k < K; ++k) ax[envs_h[k]] = ay[envs_h[k]] = 0.0;
       py = W.n2;
     }
+    if (mode == WIND_LOAD_ENVS)
+      for (int k = 0; k < K; ++k) {
+        ax[envs_h[k]] = acc_h[(size_t)2 * l * K + k];
+        ay[envs_h[k]] = acc_h[(size_t)(2 * l + 1) * K + k];
+      }
     for (int e = 0; e < E; ++e) {
       const float dx = ctx->wind_hdx[l] ? ctx->wind_hdx[l][e] : W.cdx, dy = ctx->wind_hdy[l] ? ctx->wind_hdy[l][e] : W.cdy;
       if (mode == WIND_STEP) {
@@ -1031,28 +1054,27 @@ static int start_screens(aom_ctx* ctx, const int* envs, int K, cudaStream_t st) 
   return AOM_OK;
 }
 
-extern "C" int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const int64_t* seeds, void* stream) {
-  if (!ctx) return AOM_ERR_INVALID;
-  const aom_config& c = ctx->cfg;
-  const int E = c.n_env;
-  if (n < 0) return fail(ctx, AOM_ERR_INVALID, "aom_reset_envs: negative environment count %d", n);
-  if (n > 0 && (!envs || !seeds)) return fail(ctx, AOM_ERR_INVALID, "null argument");
-  if (n > E) return fail(ctx, AOM_ERR_INVALID, "aom_reset_envs: %d environments listed, the batch has %d", n, E);
-  {
-    char* seen = (char*)calloc((size_t)E, 1);
-    if (!seen) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
-    for (int k = 0; k < n; ++k) {
-      const int e = envs[k];
-      if (e < 0 || e >= E) { free(seen); return fail(ctx, AOM_ERR_INVALID, "aom_reset_envs: environment %d out of range [0, %d)", e, E); }
-      if (seen[e]) { free(seen); return fail(ctx, AOM_ERR_INVALID, "aom_reset_envs: environment %d listed twice", e); }
-      seen[e] = 1;
-    }
-    free(seen);
+// Checks a host list of n environments of the batch: n >= 0, every index in range and listed once.
+static int check_env_list(aom_ctx* ctx, int n, const int32_t* envs, const char* what) {
+  const int E = ctx->cfg.n_env;
+  if (n < 0) return fail(ctx, AOM_ERR_INVALID, "%s: negative environment count %d", what, n);
+  if (n > 0 && !envs) return fail(ctx, AOM_ERR_INVALID, "null argument");
+  if (n > E) return fail(ctx, AOM_ERR_INVALID, "%s: %d environments listed, the batch has %d", what, n, E);
+  char* seen = (char*)calloc((size_t)E, 1);
+  if (!seen) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+  for (int k = 0; k < n; ++k) {
+    const int e = envs[k];
+    if (e < 0 || e >= E) { free(seen); return fail(ctx, AOM_ERR_INVALID, "%s: environment %d out of range [0, %d)", what, e, E); }
+    if (seen[e]) { free(seen); return fail(ctx, AOM_ERR_INVALID, "%s: environment %d listed twice", what, e); }
+    seen[e] = 1;
   }
-  if (!ctx->seeded) return fail(ctx, AOM_ERR_STATE, "aom_reset must be called before aom_reset_envs");
-  if (n == 0) return AOM_OK;
-  cudaStream_t st = (cudaStream_t)stream;
-  CU(cudaStreamSynchronize(st));                     // the wind mirror and the staging buffers are updated from the host
+  free(seen);
+  return AOM_OK;
+}
+
+// The batch leaves lockstep (aom_reset_envs, aom_load_envs): per-environment counters, every one at the batch's counts.
+static int stagger_begin(aom_ctx* ctx, cudaStream_t st) {
+  const int E = ctx->cfg.n_env;
   if (!ctx->first) {
     CU(dalloc(&ctx->rs_envs, (size_t)E));
     CU(dalloc(&ctx->rs_seeds, 2 * (size_t)E));
@@ -1062,12 +1084,59 @@ extern "C" int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const in
     CU(dalloc(&ctx->first, (size_t)E));
   }
   if (!ctx->staggered) {
-    // the batch leaves lockstep: every environment's counters start at the batch's
     stagger_counters_kernel<<<(E + 255) / 256, 256, 0, st>>>(ctx->frame0, ctx->step_env, ctx->le_n, ctx->first, E, ctx->step,
                                                              ctx->tar_n, ctx->geo_tar_n);
     KCHECK();
     ctx->staggered = true;
   }
+  return AOM_OK;
+}
+
+// The one enumeration of the per-environment rows of the context: word (s * slot_stride + e * ld + i) of buf for s <
+// slots, i < ld belongs to environment e.  aom_reset_envs clears the rows marked `clear`; aom_save_envs / aom_load_envs
+// pack and unpack all of them.  The others are the Philox keys (aom_reset_envs sets them from the new seeds) and the
+// pending target sums (a fresh trace overwrites them).  Buffers not allocated are skipped.
+struct EnvRow {
+  void* buf;
+  long long ld, slot_stride;
+  int slots, ring, clear;
+};
+
+static int env_rows(const aom_ctx* ctx, EnvRow* out) {
+  const aom_config& c = ctx->cfg;
+  const long long E = c.n_env;
+  int n = 0;
+  auto add = [&](void* b, long long ld, int clear = 1, int slots = 1, long long slot_stride = 0, int ring = 0) {
+    if (b) out[n++] = EnvRow{b, ld, slot_stride, slots, ring, clear};
+  };
+  add(ctx->slopes, ctx->lds); add(ctx->slopes_frame, ctx->lds); add(ctx->err_v, ctx->lda); add(ctx->com, ctx->lda);
+  add(ctx->com1, ctx->lda); add(ctx->volts, ctx->lda); add(ctx->com_before, ctx->lda); add(ctx->modes_res, ctx->ldm);
+  add(ctx->state, ctx->ldst); add(ctx->action, ctx->ldact); add(ctx->tar_acc, TAR_ACC); add(ctx->strehl, 4);
+  add(ctx->hist, c.state_modes, 1, c.n_hist, E * c.state_modes, 1);      // every slot of the ring
+  add(ctx->geo_com, ctx->lda); add(ctx->geo_volts, ctx->lda); add(ctx->geo_acc, TAR_ACC); add(ctx->strehl_geo, 4);
+  for (int l = 0; l < c.n_layers; ++l) {
+    add(ctx->screen[l], (long long)c.screen_dim[l] * c.screen_dim[l]);
+    add(ctx->ox[l], 1); add(ctx->oy[l], 1); add(ctx->ext_count[l], 1);
+  }
+  add(ctx->k0, 1, 0); add(ctx->k1, 1, 0);
+  add(ctx->tar_mom, 2 * PSW_MOM2, 0, 2, E * 2 * PSW_MOM2);                // doubles [2][E][PSW_MOM2]: both targets
+  add(ctx->geo_mom, 2 * 4, 0);                                           // doubles [E][4]
+  return n;
+}
+
+extern "C" int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const int64_t* seeds, void* stream) {
+  if (!ctx) return AOM_ERR_INVALID;
+  const aom_config& c = ctx->cfg;
+  const int E = c.n_env;
+  int rc = check_env_list(ctx, n, envs, "aom_reset_envs");
+  if (rc) return rc;
+  if (n > 0 && !seeds) return fail(ctx, AOM_ERR_INVALID, "null argument");
+  if (!ctx->seeded) return fail(ctx, AOM_ERR_STATE, "aom_reset must be called before aom_reset_envs");
+  if (n == 0) return AOM_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  CU(cudaStreamSynchronize(st));                     // the wind mirror and the staging buffers are updated from the host
+  rc = stagger_begin(ctx, st);
+  if (rc) return rc;
   {
     uint32_t* h = (uint32_t*)malloc(2 * (size_t)n * sizeof(uint32_t));
     if (!h) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
@@ -1085,19 +1154,13 @@ extern "C" int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const in
   // every per-environment row aom_reset clears, the listed environments' screens and ring state, keys and counters
   ResetEnvsParams P;
   memset(&P, 0, sizeof(P));
-  auto add = [&](void* b, long long ld, int slots = 1, long long slot_stride = 0) {
-    if (!b || P.nbuf == RESET_MAX_BUFS) return;
-    P.buf[P.nbuf] = (uint32_t*)b; P.ld[P.nbuf] = ld; P.slots[P.nbuf] = slots; P.slot_stride[P.nbuf] = slot_stride;
+  EnvRow rows[SNAP_MAX_SEGS];
+  const int nrows = env_rows(ctx, rows);
+  for (int i = 0; i < nrows && P.nbuf < RESET_MAX_BUFS; ++i) {
+    const EnvRow& r = rows[i];
+    if (!r.clear) continue;
+    P.buf[P.nbuf] = (uint32_t*)r.buf; P.ld[P.nbuf] = r.ld; P.slots[P.nbuf] = r.slots; P.slot_stride[P.nbuf] = r.slot_stride;
     P.nbuf++;
-  };
-  add(ctx->slopes, ctx->lds); add(ctx->slopes_frame, ctx->lds); add(ctx->err_v, ctx->lda); add(ctx->com, ctx->lda);
-  add(ctx->com1, ctx->lda); add(ctx->volts, ctx->lda); add(ctx->com_before, ctx->lda); add(ctx->modes_res, ctx->ldm);
-  add(ctx->state, ctx->ldst); add(ctx->action, ctx->ldact); add(ctx->tar_acc, TAR_ACC); add(ctx->strehl, 4);
-  if (ctx->hist) add(ctx->hist, c.state_modes, c.n_hist, (long long)E * c.state_modes);   // every slot of the ring
-  add(ctx->geo_com, ctx->lda); add(ctx->geo_volts, ctx->lda); add(ctx->geo_acc, TAR_ACC); add(ctx->strehl_geo, 4);
-  for (int l = 0; l < c.n_layers; ++l) {
-    add(ctx->screen[l], (long long)c.screen_dim[l] * c.screen_dim[l]);
-    add(ctx->ox[l], 1); add(ctx->oy[l], 1); add(ctx->ext_count[l], 1);
   }
   P.envs = ctx->rs_envs; P.seeds = ctx->rs_seeds; P.K = n; P.E = E;
   P.k0 = ctx->k0; P.k1 = ctx->k1; P.frame0 = ctx->frame0; P.step_env = ctx->step_env; P.le_n = ctx->le_n;
@@ -1108,11 +1171,223 @@ extern "C" int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const in
   if (c.n_layers == 0) return AOM_OK;
   // The listed environments' accumulators restart from 0 while the others keep theirs: the per-environment wind state
   // (common winds included) until they agree again (wind_try_uniform)
-  int rc;
   if (!ctx->wind_pe) { rc = wind_begin_pe(ctx, st); if (rc) return rc; }
   rc = wind_update(ctx, WIND_RESET_ENVS, st, ctx->rs_envs, envs, n);
   if (rc) return rc;
   return start_screens(ctx, ctx->rs_envs, n, st);
+}
+
+// ---------------------------------------------------------------------------------------------
+// per-environment snapshots (snapshot_kernels.cuh)
+
+// FNV-1a of the configuration without the batch size and the values setters change: two contexts whose records are
+// interchangeable have the same fingerprint
+static uint64_t config_fingerprint(const aom_config& cfg) {
+  aom_config c = cfg;
+  c.n_env = 0;
+  c.gain = c.noise = c.nphotons = 0.f;
+  for (int l = 0; l < AOM_MAX_LAYERS; ++l) c.deltax[l] = c.deltay[l] = c.amp[l] = 0.f;
+  uint64_t h = 1469598103934665603ull;
+  const unsigned char* b = (const unsigned char*)&c;
+  for (size_t i = 0; i < sizeof(c); ++i) h = (h ^ b[i]) * 1099511628211ull;
+  return h;
+}
+
+// Segment table of a record (the rows of env_rows after the head) and its size
+static size_t snap_layout(const aom_ctx* ctx, SnapParams& P) {
+  EnvRow rows[SNAP_MAX_SEGS];
+  const int nrows = env_rows(ctx, rows);
+  long long off = SNAP_HEAD_BYTES;
+  int chunks = 0;
+  P.nseg = nrows;
+  for (int i = 0; i < nrows; ++i) {
+    const EnvRow& r = rows[i];
+    SnapSeg& G = P.seg[i];
+    G.buf = (uint32_t*)r.buf; G.ld = r.ld; G.slot_stride = r.slot_stride; G.slots = r.slots; G.ring = r.ring;
+    G.off = off; G.pitch = (r.ld * 4 + 15) / 16 * 16;
+    G.cps = (int)((r.ld + SNAP_CHUNK_WORDS - 1) / SNAP_CHUNK_WORDS);
+    G.chunk0 = chunks;
+    chunks += G.cps * r.slots;
+    off += G.pitch * r.slots;
+  }
+  P.nchunks = chunks;
+  return (size_t)off;
+}
+
+extern "C" int aom_env_state_bytes(aom_ctx* ctx, size_t* bytes) {
+  if (!ctx || !bytes) return fail(ctx, AOM_ERR_INVALID, "null argument");
+  SnapParams P;
+  *bytes = snap_layout(ctx, P);
+  return AOM_OK;
+}
+
+// The parameters of a pack / unpack of n records at rec whose device list of environments is ctx->snap_envs
+static void snap_params(aom_ctx* ctx, SnapParams& P, int n, void* rec) {
+  const aom_config& c = ctx->cfg;
+  memset(&P, 0, sizeof(P));
+  const size_t bytes = snap_layout(ctx, P);
+  P.envs = ctx->snap_envs; P.rec = (unsigned char*)rec; P.bytes = (long long)bytes;
+  P.E = c.n_env; P.hist_head = ctx->hist_head;
+  P.magic = AOM_ENV_MAGIC; P.rec_bytes = (uint32_t)bytes; P.fingerprint = config_fingerprint(c); P.n_layers = c.n_layers;
+  P.frame = ctx->frame; P.step = ctx->step; P.le_c[0] = ctx->tar_n; P.le_c[1] = ctx->geo_tar_n;
+  if (ctx->staggered) { P.frame0 = ctx->frame0; P.step_env = ctx->step_env; P.le_n = ctx->le_n; P.first = ctx->first; }
+  P.wind_acc = ctx->wind_pe ? ctx->wind_acc : nullptr;
+  for (int l = 0; l < c.n_layers; ++l) {
+    P.acc_c[l][0] = ctx->accx[l]; P.acc_c[l][1] = ctx->accy[l];
+    P.wind_d[l][0] = ctx->wind_dx[l]; P.wind_d[l][1] = ctx->wind_dy[l];
+    P.wind_c[l][0] = c.deltax[l]; P.wind_c[l][1] = c.deltay[l];
+    P.amp_env[l] = ctx->amp_env[l]; P.amp_c[l] = c.amp[l];
+  }
+  P.noise_env = ctx->noise_env; P.nph_env = ctx->nph_env; P.gain_env = ctx->gain_env;
+  P.noise_c = ctx->noise_c; P.nph_c = ctx->nph_c; P.gain_c = ctx->gain;
+}
+
+// Host staging block of at least `bytes`, and the device list of environments envs[0..n) copied from it on `st`
+static int snap_stage(aom_ctx* ctx, int n, const int32_t* envs, size_t bytes, cudaStream_t st) {
+  if (!ctx->snap_envs) CU(dalloc(&ctx->snap_envs, (size_t)ctx->cfg.n_env));
+  if (bytes < (size_t)n * sizeof(int32_t)) bytes = (size_t)n * sizeof(int32_t);
+  if (bytes > ctx->snap_h_bytes) {
+    free(ctx->snap_h);
+    ctx->snap_h = malloc(bytes);
+    ctx->snap_h_bytes = ctx->snap_h ? bytes : 0;
+    if (!ctx->snap_h) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+  }
+  memcpy(ctx->snap_h, envs, (size_t)n * sizeof(int32_t));
+  CU(cudaMemcpyAsync(ctx->snap_envs, ctx->snap_h, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  return AOM_OK;
+}
+
+extern "C" int aom_save_envs(aom_ctx* ctx, int n, const int32_t* envs, void* dst, void* stream) {
+  if (!ctx) return AOM_ERR_INVALID;
+  int rc = check_env_list(ctx, n, envs, "aom_save_envs");
+  if (rc) return rc;
+  if (n > 0 && !dst) return fail(ctx, AOM_ERR_INVALID, "null argument");
+  if (!ctx->seeded) return fail(ctx, AOM_ERR_STATE, "aom_reset must be called before aom_save_envs");
+  if (n == 0) return AOM_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  CU(cudaStreamSynchronize(st));                     // the staging block is free and the host mirrors are current
+  rc = snap_stage(ctx, n, envs, 0, st);
+  if (rc) return rc;
+  SnapParams P;
+  snap_params(ctx, P, n, dst);
+  env_pack_kernel<<<dim3((unsigned)P.nchunks + 1, (unsigned)n), SNAP_THREADS, 0, st>>>(P);
+  KCHECK();
+  CU(cudaStreamSynchronize(st));
+  return AOM_OK;
+}
+
+// Value of each environment of the batch (E host floats): the per-environment host copy `henv` or the common value,
+// with the loaded records' values vals[k] (stride `stride` bytes) at envs[k].  True when one of those differs.
+static bool merge_env_values(int E, const float* henv, float common, int n, const int32_t* envs, const float* vals,
+                             size_t stride, float* out) {
+  for (int e = 0; e < E; ++e) out[e] = henv ? henv[e] : common;
+  bool differ = false;
+  for (int k = 0; k < n; ++k) {
+    const float v = *(const float*)((const char*)vals + k * stride);
+    differ = differ || memcmp(&v, &out[envs[k]], sizeof(float)) != 0;
+    out[envs[k]] = v;
+  }
+  return differ;
+}
+
+// Conditions of the loaded records that differ from those in force: per-environment arrays through the setters
+static int load_conditions(aom_ctx* ctx, int n, const int32_t* envs, const aom_env_head* h) {
+  const aom_config& c = ctx->cfg;
+  const int E = c.n_env, L = c.n_layers;
+  const size_t hs = sizeof(aom_env_head);
+  float* a = (float*)malloc(3 * (size_t)E * sizeof(float));
+  if (!a) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+  float *b = a + E, *cur = a + 2 * E;
+  int rc = AOM_OK;
+  for (int l = 0; l < L && !rc; ++l) {
+    // amplitude: the device array (no host copy) or the common value
+    if (ctx->amp_env[l]) {
+      cudaError_t e = cudaMemcpy(cur, ctx->amp_env[l], (size_t)E * sizeof(float), cudaMemcpyDeviceToHost);
+      if (e != cudaSuccess) { free(a); return fail(ctx, AOM_ERR_CUDA, "amplitudes: %s", cudaGetErrorString(e)); }
+    }
+    if (merge_env_values(E, ctx->amp_env[l] ? cur : nullptr, c.amp[l], n, envs, &h[0].amp[l], hs, a))
+      rc = aom_set_layer_amp(ctx, l, a);
+    if (rc) break;
+    const bool dx = merge_env_values(E, ctx->wind_hdx[l], c.deltax[l], n, envs, &h[0].wind[l][0], hs, a);
+    const bool dy = merge_env_values(E, ctx->wind_hdy[l], c.deltay[l], n, envs, &h[0].wind[l][1], hs, b);
+    if (dx || dy) rc = aom_set_layer_wind(ctx, l, a, b);
+  }
+  if (!rc) {
+    const bool dn = merge_env_values(E, ctx->noise_henv, ctx->noise_c, n, envs, &h[0].noise, hs, a);
+    const bool dp = merge_env_values(E, ctx->nph_henv, ctx->nph_c, n, envs, &h[0].nphotons, hs, b);
+    if (dn || dp) rc = aom_set_wfs_noise_env(ctx, (dn || ctx->noise_henv) ? a : nullptr, (dp || ctx->nph_henv) ? b : nullptr);
+  }
+  if (!rc && merge_env_values(E, ctx->gain_henv, ctx->gain, n, envs, &h[0].gain, hs, a)) rc = aom_set_gain_env(ctx, a);
+  free(a);
+  return rc;
+}
+
+extern "C" int aom_load_envs(aom_ctx* ctx, int n, const int32_t* envs, const void* src, void* stream) {
+  if (!ctx) return AOM_ERR_INVALID;
+  const aom_config& c = ctx->cfg;
+  const int L = c.n_layers;
+  int rc = check_env_list(ctx, n, envs, "aom_load_envs");
+  if (rc) return rc;
+  if (n > 0 && !src) return fail(ctx, AOM_ERR_INVALID, "null argument");
+  if (!ctx->seeded) return fail(ctx, AOM_ERR_STATE, "aom_reset must be called before aom_load_envs");
+  if (n == 0) return AOM_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  CU(cudaStreamSynchronize(st));
+  // the heads first, checked before anything changes
+  size_t bytes;
+  aom_env_state_bytes(ctx, &bytes);
+  const size_t hs = sizeof(aom_env_head);
+  // staging block: the list of environments, then (16-byte aligned) the heads, then the loaded accumulators [L][2][n]
+  const size_t at = ((size_t)n * sizeof(int32_t) + 15) / 16 * 16;
+  rc = snap_stage(ctx, n, envs, at + (size_t)n * (hs + 2 * L * sizeof(double)), st);
+  if (rc) return rc;
+  aom_env_head* h = (aom_env_head*)((char*)ctx->snap_h + at);
+  CU(cudaMemcpy2DAsync(h, hs, src, bytes, hs, (size_t)n, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  const uint64_t fp = config_fingerprint(c);
+  for (int k = 0; k < n; ++k) {
+    if (h[k].magic != AOM_ENV_MAGIC) return fail(ctx, AOM_ERR_INVALID, "aom_load_envs: record %d is not an environment record", k);
+    if (h[k].bytes != bytes || h[k].fingerprint != fp || h[k].n_layers != L)
+      return fail(ctx, AOM_ERR_INVALID, "aom_load_envs: record %d (%u bytes) was saved by a context of another configuration or "
+                  "allocation (this one: %zu bytes)", k, h[k].bytes, bytes);
+  }
+  rc = load_conditions(ctx, n, envs, h);
+  if (rc) return rc;
+  rc = stagger_begin(ctx, st);
+  if (rc) return rc;
+  SnapParams P;
+  snap_params(ctx, P, n, (void*)src);
+  env_unpack_kernel<<<dim3((unsigned)P.nchunks + 1, (unsigned)n), SNAP_THREADS, 0, st>>>(P);
+  KCHECK();
+  ctx->first_any = true;                             // a loaded environment may have its first step pending
+  if (L > 0) {
+    // wind accumulators: the per-environment state unless the loaded ones are the batch's common ones
+    bool differ = ctx->wind_pe;
+    for (int k = 0; k < n && !differ; ++k)
+      for (int l = 0; l < L; ++l) differ = differ || h[k].acc[l][0] != ctx->accx[l] || h[k].acc[l][1] != ctx->accy[l];
+    if (differ) {
+      if (!ctx->wind_pe) { rc = wind_begin_pe(ctx, st); if (rc) return rc; }
+      double* acc = (double*)(h + n);
+      for (int l = 0; l < L; ++l)
+        for (int k = 0; k < n; ++k) {
+          acc[(size_t)2 * l * n + k] = h[k].acc[l][0];
+          acc[(size_t)(2 * l + 1) * n + k] = h[k].acc[l][1];
+        }
+      if (!ctx->snap_acc) CU(dalloc(&ctx->snap_acc, (size_t)2 * L * c.n_env));
+      CU(cudaMemcpyAsync(ctx->snap_acc, acc, (size_t)2 * L * n * sizeof(double), cudaMemcpyHostToDevice, st));
+      rc = wind_update(ctx, WIND_LOAD_ENVS, st, ctx->snap_envs, envs, n, ctx->snap_acc, acc);
+      if (rc) return rc;
+      CU(cudaStreamSynchronize(st));
+      for (int l = 0; l < L; ++l) {
+        const int* bx = ctx->wind_box[l];
+        if (bx[0] < 0 || bx[2] < 0 || bx[1] + c.n + 1 > c.screen_dim[l] || bx[3] + c.n + 1 > c.screen_dim[l])
+          return fail(ctx, AOM_ERR_UNSUPPORTED, "layer %d: pupil footprint leaves the screen", l);
+      }
+      wind_try_uniform(ctx);
+    }
+  }
+  CU(cudaStreamSynchronize(st));
+  return AOM_OK;
 }
 
 // ---------------------------------------------------------------------------------------------

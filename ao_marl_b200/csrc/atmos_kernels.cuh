@@ -228,3 +228,25 @@ __global__ void wind_state_kernel(const __grid_constant__ WindStateParams P) {
   P.steps[(size_t)(2 * l + 1) * P.E + e] = ny;
   P.rec[(size_t)l * P.E + e] = wind_record(L.xoff, L.yoff, x, y);
 }
+
+// WIND_LOAD_ENVS (aom_load_envs): accumulators of the listed environments envs[0..K) <- acc_in [L][2][K], no extrusion.
+// One thread per (layer, listed environment); the others keep their state.
+#define WIND_LOAD_ENVS 4
+struct WindLoadParams {
+  float xoff[AOM_MAX_LAYERS], yoff[AOM_MAX_LAYERS];
+  double* acc; int* steps; WindRec* rec;
+  const int* envs; const double* acc_in;
+  int E, K, n_layers;
+};
+
+__global__ void wind_load_kernel(const __grid_constant__ WindLoadParams P) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.n_layers * P.K) return;
+  const int l = i / P.K, k = i - l * P.K, e = P.envs[k];
+  const double x = P.acc_in[(size_t)2 * l * P.K + k], y = P.acc_in[(size_t)(2 * l + 1) * P.K + k];
+  P.acc[(size_t)2 * l * P.E + e] = x;
+  P.acc[(size_t)(2 * l + 1) * P.E + e] = y;
+  P.steps[(size_t)2 * l * P.E + e] = 0;
+  P.steps[(size_t)(2 * l + 1) * P.E + e] = 0;
+  P.rec[(size_t)l * P.E + e] = wind_record(P.xoff[l], P.yoff[l], x, y);
+}

@@ -1,0 +1,130 @@
+// Per-environment snapshots (aom_save_envs / aom_load_envs): one record per environment, a run of 16-byte-aligned
+// segments.  The head (aom_env_head of aomarl.h: magic, size, configuration fingerprint, counters relative to the
+// environment, wind state and resolved conditions) comes first, then one segment per row of the enumeration of the
+// per-environment state (env_rows in aomarl.cu), each slot of a row padded to 16 bytes.
+//
+// grid (chunks + 1, n): block (c < chunks, k) moves chunk c of the segments of record k with 128-bit loads and stores
+// where the context's row is 16-byte aligned (32-bit words otherwise); block (chunks, k) writes (pack) or applies
+// (unpack) the head.  The command history is stored in logical order, oldest slot first: slot s of the record is
+// physical slot (s + hist_head) % n_hist of the context.  Counters are stored relative to the environment's reset and
+// rebased onto the context's global counters on unpack.
+#pragma once
+#include <cuda_runtime.h>
+#include <stdint.h>
+#include "../../include/aomarl.h"
+
+#define SNAP_MAX_SEGS (RESET_MAX_BUFS + 4)    // rows aom_reset_envs clears + keys and pending target sums
+#define SNAP_CHUNK_WORDS 8192                 // 32 KB of a slot per block
+#define SNAP_THREADS 256
+#define SNAP_HEAD_BYTES ((sizeof(aom_env_head) + 15) / 16 * 16)
+
+struct SnapSeg {
+  uint32_t* buf;            // word (s * slot_stride + e * ld + i) of the context, s < slots, i < ld
+  long long ld, slot_stride;
+  long long off, pitch;     // byte offset of the segment in the record, bytes per slot there (ld words rounded to 16 B)
+  int slots, ring;          // ring: the command history (logical slot order in the record)
+  int chunk0, cps;          // first chunk of the segment, chunks per slot
+};
+
+struct SnapParams {
+  SnapSeg seg[SNAP_MAX_SEGS];
+  int nseg, nchunks;
+  const int* envs;          // [n] environments (device)
+  unsigned char* rec;       // [n][bytes] records
+  long long bytes;
+  int E, hist_head;
+  // head: constants of this context
+  uint32_t magic, rec_bytes;
+  uint64_t fingerprint;
+  int n_layers;
+  // counters: global ones, and the per-environment arrays while environments are staggered (else null)
+  uint32_t frame, step;
+  int le_c[2];
+  uint32_t *frame0, *step_env;
+  int *le_n, *first;
+  // pack: wind state and conditions, each a per-environment array when one is in force, else the common value
+  const double* wind_acc;   // [L][2][E] or null
+  double acc_c[AOM_MAX_LAYERS][2];
+  const float* wind_d[AOM_MAX_LAYERS][2];
+  float wind_c[AOM_MAX_LAYERS][2];
+  const float* amp_env[AOM_MAX_LAYERS];
+  float amp_c[AOM_MAX_LAYERS];
+  const float *noise_env, *nph_env, *gain_env;
+  float noise_c, nph_c, gain_c;
+};
+
+template <bool LOAD>
+__device__ __forceinline__ void snap_words(uint32_t* ctx_row, uint32_t* rec_row, long long n) {
+  // the record side is always 16-byte aligned; the context side is when its row starts on 16 bytes
+  long long i = 0;
+  if (((uintptr_t)ctx_row & 15) == 0) {
+    const long long n4 = n >> 2;
+    uint4* a = reinterpret_cast<uint4*>(ctx_row);
+    uint4* b = reinterpret_cast<uint4*>(rec_row);
+    for (long long j = threadIdx.x; j < n4; j += blockDim.x) {
+      if (LOAD) a[j] = b[j];
+      else b[j] = a[j];
+    }
+    i = n4 << 2;
+  }
+  for (long long j = i + threadIdx.x; j < n; j += blockDim.x) {
+    if (LOAD) ctx_row[j] = rec_row[j];
+    else rec_row[j] = ctx_row[j];
+  }
+}
+
+template <bool LOAD>
+__device__ __forceinline__ void snap_head(const SnapParams& P, int e, aom_env_head* h) {
+  if (threadIdx.x) return;
+  const int E = P.E;
+  if (LOAD) {
+    // counters rebased onto this context: the environment's noise frame stays frame - frame0[e]
+    P.frame0[e] = P.frame - h->frame;
+    P.step_env[e] = h->step;
+    P.le_n[e] = h->le_n[0];
+    P.le_n[E + e] = h->le_n[1];
+    P.first[e] = h->first;
+    return;
+  }
+  aom_env_head r{};
+  r.magic = P.magic; r.bytes = P.rec_bytes; r.fingerprint = P.fingerprint; r.n_layers = P.n_layers;
+  r.frame = P.frame0 ? P.frame - P.frame0[e] : P.frame;
+  r.step = P.step_env ? P.step_env[e] : P.step;
+  r.le_n[0] = P.le_n ? P.le_n[e] : P.le_c[0];
+  r.le_n[1] = P.le_n ? P.le_n[E + e] : P.le_c[1];
+  r.first = P.first ? P.first[e] : 0;
+  for (int l = 0; l < P.n_layers; ++l) {
+    for (int a = 0; a < 2; ++a) {
+      r.acc[l][a] = P.wind_acc ? P.wind_acc[(size_t)(2 * l + a) * E + e] : P.acc_c[l][a];
+      r.wind[l][a] = P.wind_d[l][a] ? P.wind_d[l][a][e] : P.wind_c[l][a];
+    }
+    r.amp[l] = P.amp_env[l] ? P.amp_env[l][e] : P.amp_c[l];
+  }
+  r.noise = P.noise_env ? P.noise_env[e] : P.noise_c;
+  r.nphotons = P.nph_env ? P.nph_env[e] : P.nph_c;
+  r.gain = P.gain_env ? P.gain_env[e] : P.gain_c;
+  *h = r;
+}
+
+template <bool LOAD>
+__device__ __forceinline__ void snap_move(const SnapParams& P) {
+  const int k = blockIdx.y, e = P.envs[k], c = blockIdx.x;
+  unsigned char* rec = P.rec + (size_t)k * P.bytes;
+  if (c == P.nchunks) {
+    snap_head<LOAD>(P, e, reinterpret_cast<aom_env_head*>(rec));
+    return;
+  }
+  int s = 0;
+  while (s + 1 < P.nseg && P.seg[s + 1].chunk0 <= c) ++s;
+  const SnapSeg& G = P.seg[s];
+  const int cc = c - G.chunk0, slot = cc / G.cps, part = cc - slot * G.cps;
+  const int phys = G.ring ? (slot + P.hist_head) % G.slots : slot;
+  const long long i0 = (long long)part * SNAP_CHUNK_WORDS;
+  const long long n = min((long long)SNAP_CHUNK_WORDS, G.ld - i0);
+  uint32_t* row = G.buf + (long long)phys * G.slot_stride + (long long)e * G.ld + i0;
+  uint32_t* dst = reinterpret_cast<uint32_t*>(rec + G.off + (long long)slot * G.pitch) + i0;
+  snap_words<LOAD>(row, dst, n);
+}
+
+__global__ void __launch_bounds__(SNAP_THREADS) env_pack_kernel(const __grid_constant__ SnapParams P) { snap_move<false>(P); }
+__global__ void __launch_bounds__(SNAP_THREADS) env_unpack_kernel(const __grid_constant__ SnapParams P) { snap_move<true>(P); }

@@ -75,6 +75,18 @@ class AoEnv:
         episode's conditions (set_r0 / set_wind with [E] arrays) before the call."""
         self.supervisor.reset_envs(envs, seeds)
 
+    def save_envs(self, envs):
+        """Snapshots of the environments `envs` (RlSupervisor.save_envs)."""
+        return self.supervisor.save_envs(envs)
+
+    def load_envs(self, envs, snap):
+        """Resume the environments `envs` from records of save_envs (RlSupervisor.load_envs)."""
+        self.supervisor.load_envs(envs, snap)
+
+    def copy_envs(self, src, dst):
+        """Environments `dst` continue as copies of environments `src` (RlSupervisor.copy_envs)."""
+        self.supervisor.copy_envs(src, dst)
+
     def state(self):
         return self.sim.rows("STATE", self.state_size)
 

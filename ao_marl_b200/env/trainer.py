@@ -127,6 +127,16 @@ class StepLearner:
         self.sim.reset_envs(envs, seeds)
         self._first[np.asarray(envs, dtype=np.int64)] = self._t + 1
 
+    def load_envs(self, envs, snap):
+        """Resume the environments `envs` from records of Simulator.save_envs.  Their credit-assignment window restarts as
+        after reset_envs: no transition spans the load."""
+        self.sim.load_envs(envs, snap)
+        self._first[np.asarray(envs, dtype=np.int64)] = self._t + 1
+
+    def copy_envs(self, src, dst):
+        """Environments `dst` continue as copies of environments `src`; their windows restart as in load_envs."""
+        self.load_envs(dst, self.sim.save_envs(src))
+
     def states_per_agent(self, state):
         return state[:, self._idx].permute(1, 0, 2) * self._idx_ok[:, None, :]
 

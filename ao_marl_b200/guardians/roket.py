@@ -64,6 +64,14 @@ class Roket(RlSupervisor):
         """Not available: the error-breakdown buffers ([N_total, E, .]) hold one run of the whole batch."""
         raise NotImplementedError("ROKET's breakdown buffers are whole-batch: use reset()")
 
+    def load_envs(self, envs, snap):
+        """Not available: the error-breakdown buffers ([N_total, E, .]) hold one run of the whole batch."""
+        raise NotImplementedError("ROKET's breakdown buffers are whole-batch: environments cannot be loaded")
+
+    def copy_envs(self, src, dst):
+        """Not available, as load_envs."""
+        raise NotImplementedError("ROKET's breakdown buffers are whole-batch: environments cannot be copied")
+
     # -- buffers ----------------------------------------------------------------------------------------------------------
     def init_config_roket(self, N_total=3000, N_preloop=1000, agent=None, nfiltered=None, gamma=1.0, include_tip_tilt=True,
                           n_zernike_start=None, n_zernike_end=None):

@@ -47,12 +47,17 @@ BUFFERS = ["SCREEN", "RING_OX", "RING_OY", "SLOPES", "ERR", "COM", "VOLTS", "BIN
            "RES_MODES", "STATE", "REWARD", "ACTION", "ACTION_MEAN", "STREHL", "GEO_COM", "GEO_VOLTS", "STREHL_GEO", "GEO_PROJ",
            "EXT_COUNT"]
 B = {name: i for i, name in enumerate(BUFFERS)}
+# head of an environment record (aom_env_head, aom_save_envs)
+ENV_HEAD = np.dtype([("magic", "<u4"), ("bytes", "<u4"), ("fingerprint", "<u8"), ("frame", "<u4"), ("step", "<u4"),
+                     ("le_n", "<i4", 2), ("first", "<i4"), ("n_layers", "<i4"), ("acc", "<f8", (MAX_LAYERS, 2)),
+                     ("wind", "<f4", (MAX_LAYERS, 2)), ("amp", "<f4", MAX_LAYERS), ("noise", "<f4"), ("nphotons", "<f4"),
+                     ("gain", "<f4"), ("reserved", "<u4")])
 _INT_BUFFERS = {"RING_OX", "RING_OY", "EXT_COUNT"}
 OPTIONS = ["WFS_PATH", "GEMM_PATH", "TIME_WFS", "GEO", "DENOISE", "PUPIL_PATH", "KEEP_IMAGE", "STREHL", "STREHL_LAMBDA_NM", "EXTRUDE_PATH", "STREHL_PEAK", "PSF_NFFT", "DENOISE_PATH"]
 O = {name: i for i, name in enumerate(OPTIONS)}
 
 EXPORTS = ["aom_config_size", "aom_create", "aom_destroy", "aom_last_error", "aom_set_table", "aom_get_buffer",
-           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_reset_envs", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_set_wfs_noise", "aom_set_wfs_noise_env", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
+           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_reset_envs", "aom_env_state_bytes", "aom_save_envs", "aom_load_envs", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_set_wfs_noise", "aom_set_wfs_noise_env", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
            "aom_comp_strehl", "aom_reset_strehl", "aom_do_control_geo", "aom_apply_control_geo", "aom_denoise", "aom_set_bincube", "aom_do_centroids", "aom_do_centroids_geom", "aom_do_control", "aom_set_command", "aom_apply_control",
            "aom_set_gain", "aom_set_gain_env", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
            "aom_state_begin", "aom_state_end", "aom_reward", "aom_actor_forward", "aom_step", "aom_gemm_tn",
@@ -89,6 +94,9 @@ def load_library():
     lib.aom_check_device.argtypes = [vp]
     lib.aom_reset.argtypes = [vp, vp, vp]
     lib.aom_reset_envs.argtypes = [vp, i32, vp, vp, vp]
+    lib.aom_env_state_bytes.argtypes = [vp, ctypes.POINTER(sz)]
+    lib.aom_save_envs.argtypes = [vp, i32, vp, vp, vp]
+    lib.aom_load_envs.argtypes = [vp, i32, vp, vp, vp]
     lib.aom_move_atmos.argtypes = [vp, vp]
     lib.aom_set_layer.argtypes = [vp, i32, f32, f32, f32]
     lib.aom_set_layer_amp.argtypes = [vp, i32, vp]
@@ -239,6 +247,7 @@ class Simulator:
         # force (None: the common value), as the context holds them
         self.wfs_noise, self.wfs_nphotons = float(np.float32(cfg.noise)), float(np.float32(cfg.nphotons))
         self.wfs_noise_env = self.wfs_nphotons_env = self.gain_env = None
+        self._gain = float(np.float32(cfg.gain))
         # focal-plane grid of the target image (p_geom._ipupil, geom_init: 2^ceil(log2(pupdiam) + 1)) for the PSF core
         try:
             self.psf_nfft = int(np.asarray(t.config.p_geom._ipupil).shape[0])
@@ -382,6 +391,76 @@ class Simulator:
     def reset(self, seeds):
         seeds = np.ascontiguousarray(np.broadcast_to(np.asarray(seeds, dtype=np.int64), (self.n_env,)))
         self._check(self.lib.aom_reset(self._ctx, seeds.ctypes.data_as(ctypes.c_void_p), self.stream), "aom_reset")
+
+    def _env_list(self, envs, what):
+        """int32 [n] of distinct environment indices of the batch; ValueError / TypeError otherwise."""
+        envs = np.asarray(envs)
+        if envs.ndim != 1:
+            raise ValueError("%s: environments must be a 1-D array" % what)
+        if envs.size and envs.dtype.kind not in "iu":
+            raise TypeError("%s: environments must be integers" % what)
+        if envs.size and (envs.min() < 0 or envs.max() >= self.n_env):
+            raise ValueError("%s: environment index out of range [0, %d)" % (what, self.n_env))
+        if np.unique(envs).size != envs.size:
+            raise ValueError("%s: duplicate environment index" % what)
+        return np.ascontiguousarray(envs, dtype=np.int32)
+
+    def env_state_bytes(self):
+        """Bytes of one environment's record (aom_env_state_bytes) under the context's current allocation."""
+        n = ctypes.c_size_t()
+        self._check(self.lib.aom_env_state_bytes(self._ctx, ctypes.byref(n)), "aom_env_state_bytes")
+        return int(n.value)
+
+    def save_envs(self, envs):
+        """Snapshots of the environments `envs` (distinct indices): torch.uint8 [n, env_state_bytes()] on the device, one
+        record per environment holding everything its future depends on (aom_save_envs).  torch.save keeps it."""
+        envs = self._env_list(envs, "save_envs")
+        out = self.torch.empty((envs.size, self.env_state_bytes()), dtype=self.torch.uint8, device="cuda")
+        if envs.size:
+            self._check(self.lib.aom_save_envs(self._ctx, int(envs.size), envs.ctypes.data_as(ctypes.c_void_p),
+                                               ctypes.c_void_p(out.data_ptr()), self.stream), "aom_save_envs")
+        return out
+
+    def load_envs(self, envs, snap):
+        """Load the records `snap` ([n, env_state_bytes()] uint8, CPU or CUDA; from save_envs of this context or of one with
+        the same configuration and tables) into the slots `envs` (aom_load_envs).  From then on each of those
+        environments computes bit for bit what the saved one would have computed; the others are unaffected.  Conditions
+        carried by a record (amplitude, wind, sensor noise, photon count, gain) that differ from those in force become
+        per-environment values."""
+        torch = self.torch
+        envs = self._env_list(envs, "load_envs")
+        if not isinstance(snap, torch.Tensor) or snap.dtype != torch.uint8:
+            raise TypeError("load_envs: records must be a torch.uint8 tensor (save_envs)")
+        nb = self.env_state_bytes()
+        if tuple(snap.shape) != (envs.size, nb):
+            raise ValueError("load_envs: expected records of shape (%d, %d), got %s" % (envs.size, nb, tuple(snap.shape)))
+        if not envs.size:
+            return
+        src = snap.to(device="cuda").contiguous()
+        head = np.frombuffer(src[:, :ENV_HEAD.itemsize].cpu().numpy().tobytes(), dtype=ENV_HEAD)
+        # the host copies of the per-environment sensor values and gains, as the context updates them
+        new = {}
+        for name, attr, common in (("noise", "wfs_noise_env", self.wfs_noise), ("nphotons", "wfs_nphotons_env",
+                                                                                  self.wfs_nphotons),
+                                   ("gain", "gain_env", self._gain)):
+            cur = getattr(self, attr)
+            a = np.full(self.n_env, common, np.float32) if cur is None else cur.copy()
+            differ = not np.array_equal(a[envs].view(np.uint32), head[name].astype(np.float32).view(np.uint32))
+            a[envs] = head[name]
+            new[attr] = a if (differ or cur is not None) else None
+        self._check(self.lib.aom_load_envs(self._ctx, int(envs.size), envs.ctypes.data_as(ctypes.c_void_p),
+                                           ctypes.c_void_p(src.data_ptr()), self.stream), "aom_load_envs")
+        if new["wfs_noise_env"] is not None or new["wfs_nphotons_env"] is not None:
+            self.wfs_noise_env, self.wfs_nphotons_env = new["wfs_noise_env"], new["wfs_nphotons_env"]
+        self.gain_env = new["gain_env"]
+
+    def copy_envs(self, src, dst):
+        """Environments `dst` continue as copies of environments `src` (save_envs then load_envs): same screens, loop
+        state, counters, random streams and conditions, so each pair then draws the same turbulence and noise."""
+        src, dst = np.asarray(src), np.asarray(dst)
+        if src.shape != dst.shape:
+            raise ValueError("copy_envs: src and dst must have the same length")
+        self.load_envs(dst, self.save_envs(src))
 
     def reset_envs(self, envs, seeds):
         """Restart the environments `envs` (distinct indices, int [n]) with `seeds` (int [n]) while the others run on
@@ -600,6 +679,7 @@ class Simulator:
         array sets one gain per environment (set_gain_env)."""
         if np.ndim(g) == 0:
             self._check(self.lib.aom_set_gain(self._ctx, float(g)), "aom_set_gain")
+            self._gain = float(np.float32(g))
         else:
             self.set_gain_env(g)
 

@@ -128,6 +128,19 @@ class RlSupervisor:
         must be set before the call, so that the start-up of their screens uses them."""
         self.sim.reset_envs(envs, seeds)
 
+    def save_envs(self, envs):
+        """Snapshots of the environments `envs` (Simulator.save_envs): uint8 [n, bytes] records on the device."""
+        return self.sim.save_envs(envs)
+
+    def load_envs(self, envs, snap):
+        """Load records of save_envs into the slots `envs` (Simulator.load_envs): those environments continue bit for bit
+        where the saved ones were, with their conditions; the others run on."""
+        self.sim.load_envs(envs, snap)
+
+    def copy_envs(self, src, dst):
+        """Environments `dst` continue as copies of environments `src` (Simulator.copy_envs)."""
+        self.sim.copy_envs(src, dst)
+
     def get_m_pupil(self):
         return self.config.p_geom._mpupil
 

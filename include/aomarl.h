@@ -251,6 +251,56 @@ int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream);
  *   staggered, until the next aom_reset.  Waits for `stream`; cost about that of aom_reset for n = E, less for fewer. */
 int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const int64_t* seeds, void* stream);
 
+/* Per-environment snapshots: save any subset of the batch to device records and load them back, into the same slots (a
+ * rewind), other slots (a copy) or another context with the same configuration (a resume; a record saved right after
+ * aom_reset_envs makes an autoreset a memory copy).
+ * - Contract: a record of environment e holds everything its future depends on.  After a load into slot d, in this
+ *   context or another one with the same aom_config fields of the fingerprint below and the same tables, environment d
+ *   computes bit for bit what e would have computed from the save on, given the same actions.  Every environment not
+ *   listed computes what it would have computed without the call.  Tables (operators, actor weights) are not part of a
+ *   record: bit-exactness needs the same tables in both contexts.
+ * - A record is aom_env_state_bytes long (a multiple of 16): the head below, then the environment's rows of the state
+ *   aom_reset_envs clears (screens in physical order with their ring origins and extrusion counts; slopes, err, com,
+ *   com1, volts, com_before, residual modes, state, action, Strehl figures and accumulators, the geometric controller's
+ *   rows when they are allocated), the command history in logical order (oldest first), the Philox keys and the pending
+ *   target sums of both targets (AOM_TAR_TRACE / AOM_TAR_PUBLISH), each row padded to 16 bytes.
+ * - aom_load_envs rebases the counters onto the context's own (noise frame, actor decisions, long-exposure counts and the
+ *   first-step-pending flag of aom_reset_envs) and the history onto its ring head: the batch becomes staggered as after
+ *   aom_reset_envs.  Loaded wind accumulators or winds that differ from the batch's common state put the batch into the
+ *   per-environment wind state (aom_set_layer_wind); loaded amplitudes, sensor noise, photon counts and gains that
+ *   differ from those in force create the per-environment arrays (aom_set_layer_amp, aom_set_wfs_noise_env,
+ *   aom_set_gain_env) with every other environment's value kept.  The uniform kernels return as they do otherwise, at
+ *   the latest at the next aom_reset.
+ * - Errors: AOM_ERR_INVALID for n < 0, a slot out of range or listed twice, a null buffer, or (load) a record whose
+ *   magic, size or fingerprint does not match this context -- nothing changes then.  AOM_ERR_STATE before the first
+ *   aom_reset.  AOM_ERR_UNSUPPORTED (load) when a loaded wind state puts a pupil footprint off a screen.  As after
+ *   aom_reset_envs, the round-1 sensor kernels (tensor_reg / tensor / tensor_fast) return AOM_ERR_UNSUPPORTED while
+ *   environments are staggered.
+ * - Both calls wait for `stream` and return once their work is done on it; they are not for the step path. */
+#define AOM_ENV_MAGIC 0x31564e45u   /* "ENV1" */
+typedef struct aom_env_head {
+  uint32_t magic;                   /* AOM_ENV_MAGIC */
+  uint32_t bytes;                   /* record size (aom_env_state_bytes of the saving context) */
+  uint64_t fingerprint;             /* FNV-1a of aom_config without n_env and the values setters change (deltax, deltay,
+                                       amp, gain, noise, nphotons) */
+  uint32_t frame;                   /* noise frames since the environment's reset */
+  uint32_t step;                    /* actor decisions since its reset */
+  int32_t le_n[2];                  /* long-exposure counts: main target, geometric target */
+  int32_t first;                    /* its first step after aom_reset_envs is pending */
+  int32_t n_layers;
+  double acc[AOM_MAX_LAYERS][2];    /* wind accumulators (x, y) */
+  float wind[AOM_MAX_LAYERS][2];    /* wind step (x, y), pixels / frame */
+  float amp[AOM_MAX_LAYERS];        /* innovation amplitude */
+  float noise, nphotons, gain;      /* sensor noise, photons per subaperture and frame, integrator gain */
+  uint32_t reserved;
+} aom_env_head;
+/* Size in bytes of one environment's record under the context's current allocation. */
+int aom_env_state_bytes(aom_ctx* ctx, size_t* bytes);
+/* Pack the records of environments envs[0..n) (host int32, distinct) into dst (device, n * bytes). */
+int aom_save_envs(aom_ctx* ctx, int n, const int32_t* envs, void* dst, void* stream);
+/* Unpack the n records of src (device, n * bytes) into slots envs[0..n) (host int32, distinct). */
+int aom_load_envs(aom_ctx* ctx, int n, const int32_t* envs, const void* src, void* stream);
+
 /* AtmosCompass.move_atmos (atmosCompass.py:158-161) */
 int aom_move_atmos(aom_ctx* ctx, void* stream);
 
