@@ -27,6 +27,15 @@
 
 static char g_create_error[512] = "";
 
+// One per-episode condition (aom_condition): the common value, and while per-environment values are in force their
+// device array [E] and its host copy (both null otherwise).  Host readers take at(e); kernels take dev or common.
+struct EnvCond {
+  float common;
+  float* dev;
+  float* host;
+  float at(int e) const { return host ? host[e] : common; }
+};
+
 struct aom_ctx {
   aom_config cfg;
   char err[512];
@@ -41,13 +50,10 @@ struct aom_ctx {
   int* ox[AOM_MAX_LAYERS];
   int* oy[AOM_MAX_LAYERS];
   uint32_t* ext_count[AOM_MAX_LAYERS];
-  float* amp_env[AOM_MAX_LAYERS];     // optional per-environment innovation amplitude (aom_set_layer_amp)
   double accx[AOM_MAX_LAYERS], accy[AOM_MAX_LAYERS];
   // per-environment winds (aom_set_layer_wind).  While wind_pe is set every layer keeps one accumulator per environment
   // on the device (wind_state_kernel) and in a host mirror that only sizes the extrusion passes; the extrusion and
   // sampling kernels run their per-environment instantiations.  Otherwise accx / accy above hold the state.
-  float *wind_dx[AOM_MAX_LAYERS], *wind_dy[AOM_MAX_LAYERS];     // device [E] steps of layers with their own winds, else null
-  float *wind_hdx[AOM_MAX_LAYERS], *wind_hdy[AOM_MAX_LAYERS];   // host copies
   bool wind_pe;
   double* wind_acc;            // device [L][2][E] accumulators (x, y)
   int* wind_steps;             // device [L][2][E] whole-pixel counts of the last frame (x, y)
@@ -94,15 +100,11 @@ struct aom_ctx {
   float* sweep_ttp;
   int sweep_nb;               // 128-pixel column blocks per pupil row
   int lds, lda, ldm;
-  float gain;
   int closed;
   uint32_t frame;
-  // sensor noise / photon count / integrator gain: common values (aom_set_wfs_noise, aom_set_gain) and optional
-  // per-environment ones (aom_set_wfs_noise_env, aom_set_gain_env): device [E] arrays while in force, else null, with
-  // host copies that route the frames without a device read
-  float noise_c, nph_c;
-  float *noise_env, *nph_env, *gain_env;
-  float *noise_henv, *nph_henv, *gain_henv;
+  // the conditions [aom_condition][layer] (layer 0 for those of the sensor and the controller); the only copy of them
+  // after aom_create, which clears their initial values in cfg
+  EnvCond cond[AOM_COND_COUNT][AOM_MAX_LAYERS];
   int opt[AOM_OPT_COUNT];
   long long* dn_dbg;
   float dn_prm[DT_NPARAM];    // float parameters of the tensor-core denoiser (head of AOM_T_DENOISER_TC)
@@ -228,9 +230,16 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   if (!ctx) return fail(nullptr, AOM_ERR_INVALID, "out of host memory");
   memset(ctx, 0, sizeof(aom_ctx));
   ctx->cfg = *cfg;
-  ctx->gain = cfg->gain;
-  ctx->noise_c = cfg->noise;
-  ctx->nph_c = cfg->nphotons;
+  for (int l = 0; l < AOM_MAX_LAYERS; ++l) {
+    ctx->cond[AOM_COND_AMP][l].common = cfg->amp[l];
+    ctx->cond[AOM_COND_WIND_X][l].common = cfg->deltax[l];
+    ctx->cond[AOM_COND_WIND_Y][l].common = cfg->deltay[l];
+    ctx->cfg.amp[l] = ctx->cfg.deltax[l] = ctx->cfg.deltay[l] = 0.f;
+  }
+  ctx->cond[AOM_COND_NOISE][0].common = cfg->noise;
+  ctx->cond[AOM_COND_NPHOTONS][0].common = cfg->nphotons;
+  ctx->cond[AOM_COND_GAIN][0].common = cfg->gain;
+  ctx->cfg.noise = ctx->cfg.nphotons = ctx->cfg.gain = 0.f;
   ctx->closed = 1;
   ctx->opt[AOM_OPT_WFS_PATH] = AOM_WFS_UMMA_WS;
   {
@@ -326,12 +335,9 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
     for (int l = 0; l < AOM_MAX_LAYERS; ++l) cudaFree(ctx->tab[t][l]);
   for (int l = 0; l < AOM_MAX_LAYERS; ++l) {
     cudaFree(ctx->screen[l]); cudaFree(ctx->ox[l]); cudaFree(ctx->oy[l]); cudaFree(ctx->ext_count[l]);
-    cudaFree(ctx->amp_env[l]);
-    cudaFree(ctx->wind_dx[l]); cudaFree(ctx->wind_dy[l]); free(ctx->wind_hdx[l]); free(ctx->wind_hdy[l]);
+    for (int k = 0; k < AOM_COND_COUNT; ++k) { cudaFree(ctx->cond[k][l].dev); free(ctx->cond[k][l].host); }
   }
   cudaFree(ctx->wind_acc); cudaFree(ctx->wind_steps); cudaFree(ctx->wind_rec); free(ctx->wind_hacc);
-  cudaFree(ctx->noise_env); cudaFree(ctx->nph_env); cudaFree(ctx->gain_env);
-  free(ctx->noise_henv); free(ctx->nph_henv); free(ctx->gain_henv);
   void* bufs[] = {ctx->k0, ctx->k1, ctx->Z, ctx->zref, ctx->newcol, ctx->slopes_frame, ctx->slopes, ctx->err_v,
                   ctx->com, ctx->com1, ctx->volts, ctx->com_before, ctx->bincube, ctx->phase, ctx->modes,
                   ctx->modes_before, ctx->modes_res, ctx->state, ctx->hist, ctx->reward, ctx->action,
@@ -639,9 +645,10 @@ static int launch_gemm(aom_ctx* ctx, int epi, const float* A, int lda, long long
   p.A = A; p.B = B; p.C = C; p.bias = bias;
   p.lda = lda; p.ldb = ldb; p.ldc = ldc; p.M = M; p.N = N; p.K = Kp;
   p.sA = sA; p.sB = sB; p.sC = sC; p.sBias = sBias; p.relu = relu;
-  p.com = com; p.ldcom = ldcom; p.gain = ctx->gain; p.closed = ctx->closed;
+  p.com = com; p.ldcom = ldcom; p.gain = ctx->cond[AOM_COND_GAIN][0].common; p.closed = ctx->closed;
   p.Bt = Bt; p.sBt = sBt;
-  if (epi == 1 && ctx->gain_env) { epi = 2; p.gain_env = ctx->gain_env; }   // integrator with one gain per environment
+  const float* gain_env = ctx->cond[AOM_COND_GAIN][0].dev;
+  if (epi == 1 && gain_env) { epi = 2; p.gain_env = gain_env; }   // integrator with one gain per environment
   // `exact`: float32 FFMA accumulation with round-to-nearest (the recursive screen extrusion needs it: the
   // tensor core truncates its float32 accumulator, a ~1e-5 systematic shrink that an autoregression integrates)
   if (!exact && ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT) {
@@ -698,8 +705,8 @@ static int launch_oz_product(aom_ctx* ctx, int op, const float* X, int ldx, int 
   OzGemmParams m;
   memset(&m, 0, sizeof(m));
   m.Zs = ctx->oz_xs; m.ABs = ctx->ozop[op]; m.ev = ctx->oz_xev; m.ea = ctx->ozop_ea[op]; m.out = out; m.ldo = ldo;
-  m.E = c.n_env; m.N = N; m.KB = KB; m.com = com; m.ldcom = ldcom; m.gain = ctx->gain; m.closed = ctx->closed; m.err = ctx->d_err;
-  m.gain_env = integrator ? ctx->gain_env : nullptr;
+  m.E = c.n_env; m.N = N; m.KB = KB; m.com = com; m.ldcom = ldcom; m.closed = ctx->closed; m.err = ctx->d_err;
+  m.gain = ctx->cond[AOM_COND_GAIN][0].common; m.gain_env = integrator ? ctx->cond[AOM_COND_GAIN][0].dev : nullptr;
   cudaError_t le = oz_product_launch(sl, m, integrator, MT, NT, st);
   if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "oz_product_launch: %s", cudaGetErrorString(le));
   ctx->launches += 2;
@@ -726,7 +733,7 @@ static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st
   p.screen = ctx->screen[l]; p.ox = ctx->ox[l]; p.oy = ctx->oy[l]; p.count = ctx->ext_count[l];
   p.k0 = ctx->k0; p.k1 = ctx->k1; p.stencil = (const int*)ctx->tab[AOM_T_STENCIL][l];
   p.N = c.screen_dim[l]; p.S = c.stencil_size[l]; p.E = c.n_env; p.layer = l; p.axis = axis; p.sign = sign;
-  p.amp = c.amp[l]; p.amp_env = ctx->amp_env[l];
+  p.amp = ctx->cond[AOM_COND_AMP][l].common; p.amp_env = ctx->cond[AOM_COND_AMP][l].dev;
   p.ldz = AOM_LD(p.S + p.N); p.Z = ctx->Z; p.zref = ctx->zref; p.ldn = AOM_LD(p.N); p.newcol = ctx->newcol;
   p.steps = steps; p.pass = pass; p.envs = envs;
   if (ctx->opt[AOM_OPT_EXTRUDE_PATH] == AOM_EXTRUDE_I8) {
@@ -746,7 +753,7 @@ static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st
     OzGatherParams g;
     g.screen = p.screen; g.ox = p.ox; g.oy = p.oy; g.count = p.count; g.k0 = p.k0; g.k1 = p.k1; g.stencil = p.stencil;
     g.zref = p.zref; g.ev = ev; g.Zs = zs; g.N = p.N; g.S = p.S; g.E = rows; g.KB = KB; g.layer = l;
-    g.axis = axis; g.sign = sign; g.amp = p.amp; g.amp_env = ctx->amp_env[l];
+    g.axis = axis; g.sign = sign; g.amp = p.amp; g.amp_env = p.amp_env;
     g.steps = steps; g.pass = pass; g.envs = envs;
     OzGemmParams m;
     m.Zs = zs; m.ABs = ctx->oz_ab[l]; m.ev = ev; m.ea = ctx->oz_ea[l]; m.zref = p.zref;
@@ -768,10 +775,79 @@ static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st
 }
 
 // ---------------------------------------------------------------------------------------------
+// the conditions (aom_condition)
+static const char* const cond_names[AOM_COND_COUNT] = {"amplitude", "wind x", "wind y", "sensor noise", "photon count", "gain"};
+
+// One change of condition (k, l): env false sets the common value *v; env true sets the per-environment values v[E]
+// (host), or with v null returns to the common value.
+struct CondSet {
+  int k, l;
+  bool env;
+  const float* v;
+};
+
+// The one setter of the conditions.  Checks every value of the n changes first (finite; photon counts > 0), then
+// allocates the arrays of those that become per-environment, all or none: a refused call changes nothing.  Waits for the
+// device when per-environment values change (a kernel in flight may still read the old ones).
+static int set_conditions(aom_ctx* ctx, int n, const CondSet* s) {
+  if (!ctx) return AOM_ERR_INVALID;
+  const int E = ctx->cfg.n_env;
+  bool env = false;
+  for (int i = 0; i < n; ++i) {
+    const CondSet& c = s[i];
+    if (c.l < 0 || c.l >= cond_layers(c.k, ctx->cfg.n_layers)) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
+    env = env || c.env;
+    for (int e = 0; e < (!c.v ? 0 : c.env ? E : 1); ++e) {
+      const float v = c.v[e];
+      if (isfinite(v) && (c.k != AOM_COND_NPHOTONS || v > 0.f)) continue;
+      char where[32] = "", who[32] = "";
+      if (c.k <= AOM_COND_WIND_Y) snprintf(where, sizeof(where), "layer %d: ", c.l);
+      if (c.env) snprintf(who, sizeof(who), " of environment %d", e);
+      return fail(ctx, AOM_ERR_INVALID, "%s%s%s %s", where, cond_names[c.k], who, isfinite(v) ? "must be > 0" : "is not finite");
+    }
+  }
+  if (env) CU(cudaDeviceSynchronize());
+  bool fresh[AOM_COND_COUNT * AOM_MAX_LAYERS] = {}, ok = true;
+  for (int i = 0; i < n && ok; ++i) {
+    EnvCond& C = ctx->cond[s[i].k][s[i].l];
+    if (!(fresh[i] = s[i].env && s[i].v && !C.host)) continue;
+    C.host = (float*)malloc((size_t)E * sizeof(float));
+    ok = C.host && cudaMalloc((void**)&C.dev, (size_t)E * sizeof(float)) == cudaSuccess;
+  }
+  for (int i = 0; i < n && !ok; ++i)
+    if (fresh[i]) { EnvCond& C = ctx->cond[s[i].k][s[i].l]; free(C.host); cudaFree(C.dev); C.host = C.dev = nullptr; }
+  if (!ok) return fail(ctx, AOM_ERR_CUDA, "out of memory for per-environment values");
+  for (int i = 0; i < n; ++i) {
+    EnvCond& C = ctx->cond[s[i].k][s[i].l];
+    if (!s[i].env) {
+      C.common = *s[i].v;
+    } else if (!s[i].v) {
+      cudaFree(C.dev); free(C.host);
+      C.dev = C.host = nullptr;
+    } else {
+      CU(cudaMemcpy(C.dev, s[i].v, (size_t)E * sizeof(float), cudaMemcpyHostToDevice));
+      memcpy(C.host, s[i].v, (size_t)E * sizeof(float));
+    }
+  }
+  return AOM_OK;
+}
+
+extern "C" int aom_get_condition(aom_ctx* ctx, int cond, int layer, float* common, float* values_host, int* per_env) {
+  if (!ctx) return AOM_ERR_INVALID;
+  if (cond < 0 || cond >= AOM_COND_COUNT) return fail(ctx, AOM_ERR_INVALID, "unknown condition %d", cond);
+  if (layer < 0 || layer >= cond_layers(cond, ctx->cfg.n_layers)) return fail(ctx, AOM_ERR_INVALID, "%s: layer %d out of range", cond_names[cond], layer);
+  const EnvCond& C = ctx->cond[cond][layer];
+  if (common) *common = C.common;
+  if (per_env) *per_env = C.host != nullptr;
+  for (int e = 0; values_host && e < ctx->cfg.n_env; ++e) values_host[e] = C.at(e);
+  return AOM_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
 // per-environment winds
 static bool wind_any_env(const aom_ctx* ctx) {
   for (int l = 0; l < ctx->cfg.n_layers; ++l)
-    if (ctx->wind_dx[l]) return true;
+    if (ctx->cond[AOM_COND_WIND_X][l].host || ctx->cond[AOM_COND_WIND_Y][l].host) return true;
   return false;
 }
 
@@ -788,7 +864,8 @@ static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st, const int* envs_
   memset(&P, 0, sizeof(P));
   for (int l = 0; l < L; ++l) {
     WindLayerParams& W = P.layer[l];
-    W.dx = ctx->wind_dx[l]; W.dy = ctx->wind_dy[l]; W.cdx = c.deltax[l]; W.cdy = c.deltay[l];
+    const EnvCond &wx = ctx->cond[AOM_COND_WIND_X][l], &wy = ctx->cond[AOM_COND_WIND_Y][l];
+    W.dx = wx.dev; W.dy = wy.dev; W.cdx = wx.common; W.cdy = wy.common;
     W.ax0 = ctx->accx[l]; W.ay0 = ctx->accy[l]; W.xoff = c.wfs_xoff[l]; W.yoff = c.wfs_yoff[l]; W.n2 = 2 * c.screen_dim[l];
   }
   P.acc = ctx->wind_acc; P.steps = ctx->wind_steps; P.rec = ctx->wind_rec; P.E = E; P.n_layers = L; P.mode = mode;
@@ -821,7 +898,7 @@ static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st, const int* envs_
         ay[envs_h[k]] = acc_h[(size_t)(2 * l + 1) * K + k];
       }
     for (int e = 0; e < E; ++e) {
-      const float dx = ctx->wind_hdx[l] ? ctx->wind_hdx[l][e] : W.cdx, dy = ctx->wind_hdy[l] ? ctx->wind_hdy[l][e] : W.cdy;
+      const float dx = ctx->cond[AOM_COND_WIND_X][l].at(e), dy = ctx->cond[AOM_COND_WIND_Y][l].at(e);
       if (mode == WIND_STEP) {
         const int nx = wind_advance(ax[e], dx), ny = wind_advance(ay[e], dy);
         px = std::max(px, abs(nx)); py = std::max(py, abs(ny));
@@ -876,35 +953,15 @@ static int wind_begin_pe(aom_ctx* ctx, cudaStream_t st) {
   return AOM_OK;
 }
 
-extern "C" int aom_set_layer_wind(aom_ctx* ctx, int layer, const float* deltax_host, const float* deltay_host) {
-  if (!ctx) return AOM_ERR_INVALID;
+// After a change of the per-environment winds of `layer`: the uniform state when it can, else every environment continues
+// from the common accumulators (the screens do not jump), and its pupil footprint must stay on the screen.
+static int wind_settle(aom_ctx* ctx, int layer) {
   const aom_config& c = ctx->cfg;
-  if (layer < 0 || layer >= c.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
-  if (!deltax_host != !deltay_host) return fail(ctx, AOM_ERR_INVALID, "per-environment winds need both components (or neither)");
-  const size_t E = c.n_env;
-  CU(cudaDeviceSynchronize());                       // an extrusion in flight may still read the old steps
-  if (!deltax_host) {
-    cudaFree(ctx->wind_dx[layer]); cudaFree(ctx->wind_dy[layer]); free(ctx->wind_hdx[layer]); free(ctx->wind_hdy[layer]);
-    ctx->wind_dx[layer] = ctx->wind_dy[layer] = ctx->wind_hdx[layer] = ctx->wind_hdy[layer] = nullptr;
+  if (!ctx->cond[AOM_COND_WIND_X][layer].host) {
     wind_try_uniform(ctx);
     return AOM_OK;
   }
-  for (size_t e = 0; e < E; ++e)
-    if (!isfinite(deltax_host[e]) || !isfinite(deltay_host[e]))
-      return fail(ctx, AOM_ERR_INVALID, "layer %d: wind of environment %zu is not finite", layer, e);
-  if (!ctx->wind_hdx[layer]) {
-    ctx->wind_hdx[layer] = (float*)malloc(E * sizeof(float));
-    ctx->wind_hdy[layer] = (float*)malloc(E * sizeof(float));
-    if (!ctx->wind_hdx[layer] || !ctx->wind_hdy[layer]) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
-    CU(cudaMalloc((void**)&ctx->wind_dx[layer], E * sizeof(float)));
-    CU(cudaMalloc((void**)&ctx->wind_dy[layer], E * sizeof(float)));
-  }
-  memcpy(ctx->wind_hdx[layer], deltax_host, E * sizeof(float));
-  memcpy(ctx->wind_hdy[layer], deltay_host, E * sizeof(float));
-  CU(cudaMemcpy(ctx->wind_dx[layer], deltax_host, E * sizeof(float), cudaMemcpyHostToDevice));
-  CU(cudaMemcpy(ctx->wind_dy[layer], deltay_host, E * sizeof(float), cudaMemcpyHostToDevice));
   if (!ctx->wind_pe) {
-    // every environment continues from the common accumulators: the screens do not jump
     int rc = wind_begin_pe(ctx, 0);
     if (rc) return rc;
     CU(cudaStreamSynchronize(0));                    // the legacy stream: the state is read next on any stream
@@ -913,6 +970,13 @@ extern "C" int aom_set_layer_wind(aom_ctx* ctx, int layer, const float* deltax_h
   if (b[0] < 0 || b[2] < 0 || b[1] + c.n + 1 > c.screen_dim[layer] || b[3] + c.n + 1 > c.screen_dim[layer])
     return fail(ctx, AOM_ERR_UNSUPPORTED, "layer %d: pupil footprint leaves the screen", layer);
   return AOM_OK;
+}
+
+extern "C" int aom_set_layer_wind(aom_ctx* ctx, int layer, const float* deltax_host, const float* deltay_host) {
+  if (!deltax_host != !deltay_host) return fail(ctx, AOM_ERR_INVALID, "per-environment winds need both components (or neither)");
+  const CondSet s[2] = {{AOM_COND_WIND_X, layer, true, deltax_host}, {AOM_COND_WIND_Y, layer, true, deltay_host}};
+  int rc = set_conditions(ctx, 2, s);
+  return rc ? rc : wind_settle(ctx, layer);
 }
 
 extern "C" int aom_move_atmos(aom_ctx* ctx, void* stream) {
@@ -936,8 +1000,8 @@ extern "C" int aom_move_atmos(aom_ctx* ctx, void* stream) {
     return AOM_OK;
   }
   for (int l = 0; l < c.n_layers; ++l) {
-    ctx->accx[l] += (double)c.deltax[l];
-    ctx->accy[l] += (double)c.deltay[l];
+    ctx->accx[l] += (double)ctx->cond[AOM_COND_WIND_X][l].common;
+    ctx->accy[l] += (double)ctx->cond[AOM_COND_WIND_Y][l].common;
     int nx = (int)ctx->accx[l], ny = (int)ctx->accy[l];
     ctx->accx[l] -= nx;
     ctx->accy[l] -= ny;
@@ -1035,7 +1099,7 @@ static int start_screens(aom_ctx* ctx, const int* envs, int K, cudaStream_t st) 
   int rc;
   for (int l = 0; l < c.n_layers; ++l) {
     size_t N = c.screen_dim[l];
-    int sign = c.deltax[l] < 0 ? -1 : 1;
+    int sign = ctx->cond[AOM_COND_WIND_X][l].common < 0 ? -1 : 1;
     const int* steps = ctx->wind_pe ? ctx->wind_steps + (2 * l + 1) * E : nullptr;
     // The reference starts a screen with 2N extrusions along x (columns: 648 pixels in 648 different DRAM rows per
     // environment, the expensive direction of the [y][x] layout -- 0.32 ms per extrusion at 4096 environments against
@@ -1180,13 +1244,11 @@ extern "C" int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const in
 // ---------------------------------------------------------------------------------------------
 // per-environment snapshots (snapshot_kernels.cuh)
 
-// FNV-1a of the configuration without the batch size and the values setters change: two contexts whose records are
-// interchangeable have the same fingerprint
+// FNV-1a of the configuration without the batch size (the conditions are cleared in ctx->cfg): two contexts whose
+// records are interchangeable have the same fingerprint
 static uint64_t config_fingerprint(const aom_config& cfg) {
   aom_config c = cfg;
   c.n_env = 0;
-  c.gain = c.noise = c.nphotons = 0.f;
-  for (int l = 0; l < AOM_MAX_LAYERS; ++l) c.deltax[l] = c.deltay[l] = c.amp[l] = 0.f;
   uint64_t h = 1469598103934665603ull;
   const unsigned char* b = (const unsigned char*)&c;
   for (size_t i = 0; i < sizeof(c); ++i) h = (h ^ b[i]) * 1099511628211ull;
@@ -1232,14 +1294,9 @@ static void snap_params(aom_ctx* ctx, SnapParams& P, int n, void* rec) {
   P.frame = ctx->frame; P.step = ctx->step; P.le_c[0] = ctx->tar_n; P.le_c[1] = ctx->geo_tar_n;
   if (ctx->staggered) { P.frame0 = ctx->frame0; P.step_env = ctx->step_env; P.le_n = ctx->le_n; P.first = ctx->first; }
   P.wind_acc = ctx->wind_pe ? ctx->wind_acc : nullptr;
-  for (int l = 0; l < c.n_layers; ++l) {
-    P.acc_c[l][0] = ctx->accx[l]; P.acc_c[l][1] = ctx->accy[l];
-    P.wind_d[l][0] = ctx->wind_dx[l]; P.wind_d[l][1] = ctx->wind_dy[l];
-    P.wind_c[l][0] = c.deltax[l]; P.wind_c[l][1] = c.deltay[l];
-    P.amp_env[l] = ctx->amp_env[l]; P.amp_c[l] = c.amp[l];
-  }
-  P.noise_env = ctx->noise_env; P.nph_env = ctx->nph_env; P.gain_env = ctx->gain_env;
-  P.noise_c = ctx->noise_c; P.nph_c = ctx->nph_c; P.gain_c = ctx->gain;
+  for (int l = 0; l < c.n_layers; ++l) { P.acc_c[l][0] = ctx->accx[l]; P.acc_c[l][1] = ctx->accy[l]; }
+  for (int k = 0; k < AOM_COND_COUNT; ++k)
+    for (int l = 0; l < AOM_MAX_LAYERS; ++l) { P.cond_env[k][l] = ctx->cond[k][l].dev; P.cond_c[k][l] = ctx->cond[k][l].common; }
 }
 
 // Host staging block of at least `bytes`, and the device list of environments envs[0..n) copied from it on `st`
@@ -1276,49 +1333,35 @@ extern "C" int aom_save_envs(aom_ctx* ctx, int n, const int32_t* envs, void* dst
   return AOM_OK;
 }
 
-// Value of each environment of the batch (E host floats): the per-environment host copy `henv` or the common value,
-// with the loaded records' values vals[k] (stride `stride` bytes) at envs[k].  True when one of those differs.
-static bool merge_env_values(int E, const float* henv, float common, int n, const int32_t* envs, const float* vals,
-                             size_t stride, float* out) {
-  for (int e = 0; e < E; ++e) out[e] = henv ? henv[e] : common;
-  bool differ = false;
-  for (int k = 0; k < n; ++k) {
-    const float v = *(const float*)((const char*)vals + k * stride);
-    differ = differ || memcmp(&v, &out[envs[k]], sizeof(float)) != 0;
-    out[envs[k]] = v;
-  }
-  return differ;
-}
-
-// Conditions of the loaded records that differ from those in force: per-environment arrays through the setters
-static int load_conditions(aom_ctx* ctx, int n, const int32_t* envs, const aom_env_head* h) {
-  const aom_config& c = ctx->cfg;
-  const int E = c.n_env, L = c.n_layers;
-  const size_t hs = sizeof(aom_env_head);
-  float* a = (float*)malloc(3 * (size_t)E * sizeof(float));
+// The conditions of the loaded records: each environment keeps its value in force except envs[k], which takes that of
+// record k.  A condition where one of them differs becomes per-environment (a wind both components of its layer), all
+// in one set_conditions call: refused values change nothing.
+static int load_conditions(aom_ctx* ctx, int n, const int32_t* envs, aom_env_head* h) {
+  const int E = ctx->cfg.n_env, L = ctx->cfg.n_layers;
+  float* a = (float*)malloc((size_t)AOM_COND_COUNT * AOM_MAX_LAYERS * E * sizeof(float));
   if (!a) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
-  float *b = a + E, *cur = a + 2 * E;
-  int rc = AOM_OK;
-  for (int l = 0; l < L && !rc; ++l) {
-    // amplitude: the device array (no host copy) or the common value
-    if (ctx->amp_env[l]) {
-      cudaError_t e = cudaMemcpy(cur, ctx->amp_env[l], (size_t)E * sizeof(float), cudaMemcpyDeviceToHost);
-      if (e != cudaSuccess) { free(a); return fail(ctx, AOM_ERR_CUDA, "amplitudes: %s", cudaGetErrorString(e)); }
+  bool differ[AOM_COND_COUNT][AOM_MAX_LAYERS] = {};
+  for (int k = 0; k < AOM_COND_COUNT; ++k)
+    for (int l = 0; l < cond_layers(k, L); ++l) {
+      float* v = a + (size_t)(k * AOM_MAX_LAYERS + l) * E;
+      for (int e = 0; e < E; ++e) v[e] = ctx->cond[k][l].at(e);
+      for (int i = 0; i < n; ++i) {
+        const float x = head_cond(h[i], k, l);
+        differ[k][l] = differ[k][l] || memcmp(&x, &v[envs[i]], sizeof(float)) != 0;
+        v[envs[i]] = x;
+      }
     }
-    if (merge_env_values(E, ctx->amp_env[l] ? cur : nullptr, c.amp[l], n, envs, &h[0].amp[l], hs, a))
-      rc = aom_set_layer_amp(ctx, l, a);
-    if (rc) break;
-    const bool dx = merge_env_values(E, ctx->wind_hdx[l], c.deltax[l], n, envs, &h[0].wind[l][0], hs, a);
-    const bool dy = merge_env_values(E, ctx->wind_hdy[l], c.deltay[l], n, envs, &h[0].wind[l][1], hs, b);
-    if (dx || dy) rc = aom_set_layer_wind(ctx, l, a, b);
-  }
-  if (!rc) {
-    const bool dn = merge_env_values(E, ctx->noise_henv, ctx->noise_c, n, envs, &h[0].noise, hs, a);
-    const bool dp = merge_env_values(E, ctx->nph_henv, ctx->nph_c, n, envs, &h[0].nphotons, hs, b);
-    if (dn || dp) rc = aom_set_wfs_noise_env(ctx, (dn || ctx->noise_henv) ? a : nullptr, (dp || ctx->nph_henv) ? b : nullptr);
-  }
-  if (!rc && merge_env_values(E, ctx->gain_henv, ctx->gain, n, envs, &h[0].gain, hs, a)) rc = aom_set_gain_env(ctx, a);
+  for (int l = 0; l < L; ++l)
+    differ[AOM_COND_WIND_X][l] = differ[AOM_COND_WIND_Y][l] = differ[AOM_COND_WIND_X][l] || differ[AOM_COND_WIND_Y][l];
+  CondSet s[AOM_COND_COUNT * AOM_MAX_LAYERS];
+  int ns = 0;
+  for (int k = 0; k < AOM_COND_COUNT; ++k)
+    for (int l = 0; l < cond_layers(k, L); ++l)
+      if (differ[k][l]) s[ns++] = CondSet{k, l, true, a + (size_t)(k * AOM_MAX_LAYERS + l) * E};
+  int rc = set_conditions(ctx, ns, s);
   free(a);
+  for (int l = 0; l < L && !rc; ++l)
+    if (differ[AOM_COND_WIND_X][l]) rc = wind_settle(ctx, l);
   return rc;
 }
 
@@ -1727,11 +1770,11 @@ static int fill_wfs_params(aom_ctx* ctx, WfsParams& p, int flags, float noise) {
   p.pzt_off = c.pzt_off; p.pzt_nact = c.pzt_nact;
   p.tt_planes = (const float*)ctx->tab[AOM_T_TT_PLANES][0]; p.tt_dim = c.tt_dim; p.tt_off = c.tt_off;
   p.k2 = (float)(2.0 * M_PI / (double)c.lambda_um);
-  p.nphotons = ctx->nph_c; p.noise = noise; p.cog_offset = c.cog_offset; p.pixsize = c.pixsize;
+  p.nphotons = ctx->cond[AOM_COND_NPHOTONS][0].common; p.noise = noise; p.cog_offset = c.cog_offset; p.pixsize = c.pixsize;
   // per-environment sensor values: every frame is scaled by each environment's photon count, a noisy frame (noise >= 0)
   // draws each environment's own noise, a noise-free one none
-  p.nph_env = ctx->nph_env;
-  p.noise_env = (noise >= 0.f) ? ctx->noise_env : nullptr;
+  p.nph_env = ctx->cond[AOM_COND_NPHOTONS][0].dev;
+  p.noise_env = (noise >= 0.f) ? ctx->cond[AOM_COND_NOISE][0].dev : nullptr;
   p.frame = ctx->frame; p.wfs_index = (uint32_t)c.wfs_index; p.k0 = ctx->k0; p.k1 = ctx->k1;
   p.frame0 = ctx->staggered ? ctx->frame0 : nullptr;
   p.slopes = ctx->slopes_frame; p.lds = ctx->lds;
@@ -1807,11 +1850,8 @@ extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* st
     p.bincube = ctx->bincube;
   }
   // does any environment draw noise in this frame?  (host copies: no device read)
-  bool noisy = p.noise >= 0.f;
-  if (p.noise_env) {
-    noisy = false;
-    for (int e = 0; e < c.n_env && !noisy; ++e) noisy = ctx->noise_henv[e] >= 0.f;
-  }
+  bool noisy = p.noise >= 0.f && !p.noise_env;
+  for (int e = 0; p.noise_env && e < c.n_env && !noisy; ++e) noisy = ctx->cond[AOM_COND_NOISE][0].host[e] >= 0.f;
   WfsRoute r;
   rc = wfs_route(ctx, p, noisy, p.bincube != nullptr, r);
   if (rc) return rc;
@@ -2158,62 +2198,23 @@ extern "C" int aom_check_device(aom_ctx* ctx) {
 }
 
 extern "C" int aom_set_gain(aom_ctx* ctx, float gain) {
-  if (!ctx) return AOM_ERR_INVALID;
-  ctx->gain = gain;
-  return AOM_OK;
-}
-
-// Per-environment value array: NULL frees it (back to the common value); otherwise checks every entry (finite, and > 0
-// when `positive`), keeps a host copy and uploads it.  The caller has synchronised the device.
-static int set_env_values(aom_ctx* ctx, const float* host, float** dev, float** hcopy, bool positive, const char* what) {
-  const size_t E = ctx->cfg.n_env;
-  if (!host) {
-    cudaFree(*dev); free(*hcopy);
-    *dev = *hcopy = nullptr;
-    return AOM_OK;
-  }
-  for (size_t e = 0; e < E; ++e) {
-    if (!isfinite(host[e])) return fail(ctx, AOM_ERR_INVALID, "%s of environment %zu is not finite", what, e);
-    if (positive && !(host[e] > 0.f)) return fail(ctx, AOM_ERR_INVALID, "%s of environment %zu must be > 0", what, e);
-  }
-  if (!*hcopy) {
-    *hcopy = (float*)malloc(E * sizeof(float));
-    if (!*hcopy) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
-    CU(cudaMalloc((void**)dev, E * sizeof(float)));
-  }
-  memcpy(*hcopy, host, E * sizeof(float));
-  CU(cudaMemcpy(*dev, host, E * sizeof(float), cudaMemcpyHostToDevice));
-  return AOM_OK;
+  const CondSet s = {AOM_COND_GAIN, 0, false, &gain};
+  return set_conditions(ctx, 1, &s);
 }
 
 extern "C" int aom_set_gain_env(aom_ctx* ctx, const float* gain_host) {
-  if (!ctx) return AOM_ERR_INVALID;
-  CU(cudaDeviceSynchronize());                       // an integrator in flight may still read the old gains
-  return set_env_values(ctx, gain_host, &ctx->gain_env, &ctx->gain_henv, false, "gain");
+  const CondSet s = {AOM_COND_GAIN, 0, true, gain_host};
+  return set_conditions(ctx, 1, &s);
 }
 
 extern "C" int aom_set_wfs_noise(aom_ctx* ctx, float noise, float nphotons) {
-  if (!ctx) return AOM_ERR_INVALID;
-  if (!isfinite(noise) || !isfinite(nphotons)) return fail(ctx, AOM_ERR_INVALID, "sensor noise and photon count must be finite");
-  if (!(nphotons > 0.f)) return fail(ctx, AOM_ERR_INVALID, "photon count must be > 0");
-  ctx->noise_c = noise;
-  ctx->nph_c = nphotons;
-  return AOM_OK;
+  const CondSet s[2] = {{AOM_COND_NOISE, 0, false, &noise}, {AOM_COND_NPHOTONS, 0, false, &nphotons}};
+  return set_conditions(ctx, 2, s);
 }
 
 extern "C" int aom_set_wfs_noise_env(aom_ctx* ctx, const float* noise_host, const float* nphotons_host) {
-  if (!ctx) return AOM_ERR_INVALID;
-  const size_t E = ctx->cfg.n_env;
-  // check both before changing either: a refused call leaves the state as it was
-  for (size_t e = 0; noise_host && e < E; ++e)
-    if (!isfinite(noise_host[e])) return fail(ctx, AOM_ERR_INVALID, "sensor noise of environment %zu is not finite", e);
-  for (size_t e = 0; nphotons_host && e < E; ++e)
-    if (!isfinite(nphotons_host[e]) || !(nphotons_host[e] > 0.f))
-      return fail(ctx, AOM_ERR_INVALID, "photon count of environment %zu must be finite and > 0", e);
-  CU(cudaDeviceSynchronize());                       // a sensor frame in flight may still read the old values
-  int rc = set_env_values(ctx, noise_host, &ctx->noise_env, &ctx->noise_henv, false, "sensor noise");
-  if (rc) return rc;
-  return set_env_values(ctx, nphotons_host, &ctx->nph_env, &ctx->nph_henv, true, "photon count");
+  const CondSet s[2] = {{AOM_COND_NOISE, 0, true, noise_host}, {AOM_COND_NPHOTONS, 0, true, nphotons_host}};
+  return set_conditions(ctx, 2, s);
 }
 
 extern "C" int aom_set_loop(aom_ctx* ctx, int closed) {
@@ -2223,22 +2224,14 @@ extern "C" int aom_set_loop(aom_ctx* ctx, int closed) {
 }
 
 extern "C" int aom_set_layer(aom_ctx* ctx, int layer, float deltax, float deltay, float amp) {
-  if (!ctx) return AOM_ERR_INVALID;
-  if (layer < 0 || layer >= ctx->cfg.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
-  ctx->cfg.deltax[layer] = deltax;
-  ctx->cfg.deltay[layer] = deltay;
-  ctx->cfg.amp[layer] = amp;
-  return AOM_OK;
+  const CondSet s[3] = {{AOM_COND_WIND_X, layer, false, &deltax}, {AOM_COND_WIND_Y, layer, false, &deltay},
+                        {AOM_COND_AMP, layer, false, &amp}};
+  return set_conditions(ctx, 3, s);
 }
 
 extern "C" int aom_set_layer_amp(aom_ctx* ctx, int layer, const float* amp_host) {
-  if (!ctx) return AOM_ERR_INVALID;
-  if (layer < 0 || layer >= ctx->cfg.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
-  if (!amp_host) { cudaFree(ctx->amp_env[layer]); ctx->amp_env[layer] = nullptr; return AOM_OK; }
-  CU(cudaDeviceSynchronize());                       // an extrusion in flight may still read the old amplitudes
-  if (!ctx->amp_env[layer]) CU(cudaMalloc((void**)&ctx->amp_env[layer], (size_t)ctx->cfg.n_env * sizeof(float)));
-  CU(cudaMemcpy(ctx->amp_env[layer], amp_host, (size_t)ctx->cfg.n_env * sizeof(float), cudaMemcpyHostToDevice));
-  return AOM_OK;
+  const CondSet s = {AOM_COND_AMP, layer, true, amp_host};
+  return set_conditions(ctx, 1, &s);
 }
 
 extern "C" int aom_reset_dm(aom_ctx* ctx, void* stream) {
@@ -2410,7 +2403,8 @@ extern "C" int aom_step(aom_ctx* ctx, int mode, int eval_mode, void* stream) {
   const bool denoise = ctx->opt[AOM_OPT_DENOISE] != 0;
   const bool keep = denoise || ctx->opt[AOM_OPT_KEEP_IMAGE] != 0;
   // the common noise, or with per-environment noise in force any value >= 0: each environment's own
-  rc = aom_comp_wfs_image(ctx, keep ? 7 : 3, ctx->noise_env ? 0.f : ctx->noise_c, stream); if (rc) return rc;
+  const EnvCond& noise = ctx->cond[AOM_COND_NOISE][0];
+  rc = aom_comp_wfs_image(ctx, keep ? 7 : 3, noise.dev ? 0.f : noise.common, stream); if (rc) return rc;
   if (denoise) { rc = aom_denoise(ctx, nullptr, nullptr, 0, stream); if (rc) return rc; }
   rc = aom_do_centroids(ctx, stream); if (rc) return rc;
   rc = aom_do_control(ctx, stream); if (rc) return rc;

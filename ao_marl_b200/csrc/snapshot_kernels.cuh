@@ -42,16 +42,26 @@ struct SnapParams {
   int le_c[2];
   uint32_t *frame0, *step_env;
   int *le_n, *first;
-  // pack: wind state and conditions, each a per-environment array when one is in force, else the common value
+  // pack: wind state and conditions [aom_condition][layer], each a per-environment array while in force, else null
   const double* wind_acc;   // [L][2][E] or null
   double acc_c[AOM_MAX_LAYERS][2];
-  const float* wind_d[AOM_MAX_LAYERS][2];
-  float wind_c[AOM_MAX_LAYERS][2];
-  const float* amp_env[AOM_MAX_LAYERS];
-  float amp_c[AOM_MAX_LAYERS];
-  const float *noise_env, *nph_env, *gain_env;
-  float noise_c, nph_c, gain_c;
+  const float* cond_env[AOM_COND_COUNT][AOM_MAX_LAYERS];
+  float cond_c[AOM_COND_COUNT][AOM_MAX_LAYERS];
 };
+
+// Layers of condition k in a context of L layers, and its field of layer l in a record head
+__host__ __device__ __forceinline__ int cond_layers(int k, int L) { return k <= AOM_COND_WIND_Y ? L : 1; }
+
+__host__ __device__ __forceinline__ float& head_cond(aom_env_head& h, int k, int l) {
+  switch (k) {
+    case AOM_COND_AMP: return h.amp[l];
+    case AOM_COND_WIND_X: return h.wind[l][0];
+    case AOM_COND_WIND_Y: return h.wind[l][1];
+    case AOM_COND_NOISE: return h.noise;
+    case AOM_COND_NPHOTONS: return h.nphotons;
+    default: return h.gain;
+  }
+}
 
 template <bool LOAD>
 __device__ __forceinline__ void snap_words(uint32_t* ctx_row, uint32_t* rec_row, long long n) {
@@ -93,16 +103,10 @@ __device__ __forceinline__ void snap_head(const SnapParams& P, int e, aom_env_he
   r.le_n[0] = P.le_n ? P.le_n[e] : P.le_c[0];
   r.le_n[1] = P.le_n ? P.le_n[E + e] : P.le_c[1];
   r.first = P.first ? P.first[e] : 0;
-  for (int l = 0; l < P.n_layers; ++l) {
-    for (int a = 0; a < 2; ++a) {
-      r.acc[l][a] = P.wind_acc ? P.wind_acc[(size_t)(2 * l + a) * E + e] : P.acc_c[l][a];
-      r.wind[l][a] = P.wind_d[l][a] ? P.wind_d[l][a][e] : P.wind_c[l][a];
-    }
-    r.amp[l] = P.amp_env[l] ? P.amp_env[l][e] : P.amp_c[l];
-  }
-  r.noise = P.noise_env ? P.noise_env[e] : P.noise_c;
-  r.nphotons = P.nph_env ? P.nph_env[e] : P.nph_c;
-  r.gain = P.gain_env ? P.gain_env[e] : P.gain_c;
+  for (int l = 0; l < P.n_layers; ++l)
+    for (int a = 0; a < 2; ++a) r.acc[l][a] = P.wind_acc ? P.wind_acc[(size_t)(2 * l + a) * E + e] : P.acc_c[l][a];
+  for (int k = 0; k < AOM_COND_COUNT; ++k)
+    for (int l = 0; l < cond_layers(k, P.n_layers); ++l) head_cond(r, k, l) = P.cond_env[k][l] ? P.cond_env[k][l][e] : P.cond_c[k][l];
   *h = r;
 }
 

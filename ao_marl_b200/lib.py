@@ -53,11 +53,13 @@ ENV_HEAD = np.dtype([("magic", "<u4"), ("bytes", "<u4"), ("fingerprint", "<u8"),
                      ("wind", "<f4", (MAX_LAYERS, 2)), ("amp", "<f4", MAX_LAYERS), ("noise", "<f4"), ("nphotons", "<f4"),
                      ("gain", "<f4"), ("reserved", "<u4")])
 _INT_BUFFERS = {"RING_OX", "RING_OY", "EXT_COUNT"}
+CONDITIONS = ["AMP", "WIND_X", "WIND_Y", "NOISE", "NPHOTONS", "GAIN"]
+COND = {name: i for i, name in enumerate(CONDITIONS)}
 OPTIONS = ["WFS_PATH", "GEMM_PATH", "TIME_WFS", "GEO", "DENOISE", "PUPIL_PATH", "KEEP_IMAGE", "STREHL", "STREHL_LAMBDA_NM", "EXTRUDE_PATH", "STREHL_PEAK", "PSF_NFFT", "DENOISE_PATH"]
 O = {name: i for i, name in enumerate(OPTIONS)}
 
 EXPORTS = ["aom_config_size", "aom_create", "aom_destroy", "aom_last_error", "aom_set_table", "aom_get_buffer",
-           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_reset_envs", "aom_env_state_bytes", "aom_save_envs", "aom_load_envs", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_set_wfs_noise", "aom_set_wfs_noise_env", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
+           "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_reset_envs", "aom_env_state_bytes", "aom_save_envs", "aom_load_envs", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_set_wfs_noise", "aom_set_wfs_noise_env", "aom_get_condition", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
            "aom_comp_strehl", "aom_reset_strehl", "aom_do_control_geo", "aom_apply_control_geo", "aom_denoise", "aom_set_bincube", "aom_do_centroids", "aom_do_centroids_geom", "aom_do_control", "aom_set_command", "aom_apply_control",
            "aom_set_gain", "aom_set_gain_env", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
            "aom_state_begin", "aom_state_end", "aom_reward", "aom_actor_forward", "aom_step", "aom_gemm_tn",
@@ -104,6 +106,7 @@ def load_library():
     lib.aom_comp_wfs_image.argtypes = [vp, i32, f32, vp]
     lib.aom_set_wfs_noise.argtypes = [vp, f32, f32]
     lib.aom_set_wfs_noise_env.argtypes = [vp, vp, vp]
+    lib.aom_get_condition.argtypes = [vp, i32, i32, ctypes.POINTER(f32), vp, ctypes.POINTER(i32)]
     lib.aom_raytrace_wfs.argtypes = [vp, i32, vp]
     lib.aom_wfs_time_ms.argtypes = [vp, ctypes.POINTER(f32), ctypes.POINTER(i32)]
     lib.aom_wfs_kernel.argtypes = [vp]
@@ -243,11 +246,6 @@ class Simulator:
             raise (ValueError if rc == -1 else RuntimeError)("aom_create: " + msg)
         self._stream = stream
         self._views = {}
-        # sensor noise / photon count / integrator gain: common values and the per-environment float32 [E] arrays in
-        # force (None: the common value), as the context holds them
-        self.wfs_noise, self.wfs_nphotons = float(np.float32(cfg.noise)), float(np.float32(cfg.nphotons))
-        self.wfs_noise_env = self.wfs_nphotons_env = self.gain_env = None
-        self._gain = float(np.float32(cfg.gain))
         # focal-plane grid of the target image (p_geom._ipupil, geom_init: 2^ceil(log2(pupdiam) + 1)) for the PSF core
         try:
             self.psf_nfft = int(np.asarray(t.config.p_geom._ipupil).shape[0])
@@ -295,6 +293,22 @@ class Simulator:
         """[E, n] view (pad columns dropped) of a per-environment vector buffer."""
         flat = self.buffer(name, index)
         return flat.view(self.n_env, -1)[:, :n]
+
+    def _condition(self, name, layer=0):
+        """(common value, float32 [E] per-environment values in force or None) of a condition (aom_get_condition)."""
+        common, per_env, values = ctypes.c_float(), ctypes.c_int(), np.empty(self.n_env, np.float32)
+        self._check(self.lib.aom_get_condition(self._ctx, COND[name], int(layer), ctypes.byref(common),
+                                               values.ctypes.data_as(ctypes.c_void_p), ctypes.byref(per_env)),
+                    "aom_get_condition")
+        return float(common.value), (values if per_env.value else None)
+
+    # sensor noise, photon count and integrator gain in force: common values, and per-environment float32 [E] or None
+    wfs_noise = property(lambda self: self._condition("NOISE")[0])
+    wfs_nphotons = property(lambda self: self._condition("NPHOTONS")[0])
+    gain = property(lambda self: self._condition("GAIN")[0])
+    wfs_noise_env = property(lambda self: self._condition("NOISE")[1])
+    wfs_nphotons_env = property(lambda self: self._condition("NPHOTONS")[1])
+    gain_env = property(lambda self: self._condition("GAIN")[1])
 
     def launches(self):
         n = ctypes.c_uint64()
@@ -437,22 +451,8 @@ class Simulator:
         if not envs.size:
             return
         src = snap.to(device="cuda").contiguous()
-        head = np.frombuffer(src[:, :ENV_HEAD.itemsize].cpu().numpy().tobytes(), dtype=ENV_HEAD)
-        # the host copies of the per-environment sensor values and gains, as the context updates them
-        new = {}
-        for name, attr, common in (("noise", "wfs_noise_env", self.wfs_noise), ("nphotons", "wfs_nphotons_env",
-                                                                                  self.wfs_nphotons),
-                                   ("gain", "gain_env", self._gain)):
-            cur = getattr(self, attr)
-            a = np.full(self.n_env, common, np.float32) if cur is None else cur.copy()
-            differ = not np.array_equal(a[envs].view(np.uint32), head[name].astype(np.float32).view(np.uint32))
-            a[envs] = head[name]
-            new[attr] = a if (differ or cur is not None) else None
         self._check(self.lib.aom_load_envs(self._ctx, int(envs.size), envs.ctypes.data_as(ctypes.c_void_p),
                                            ctypes.c_void_p(src.data_ptr()), self.stream), "aom_load_envs")
-        if new["wfs_noise_env"] is not None or new["wfs_nphotons_env"] is not None:
-            self.wfs_noise_env, self.wfs_nphotons_env = new["wfs_noise_env"], new["wfs_nphotons_env"]
-        self.gain_env = new["gain_env"]
 
     def copy_envs(self, src, dst):
         """Environments `dst` continue as copies of environments `src` (save_envs then load_envs): same screens, loop
@@ -521,7 +521,6 @@ class Simulator:
         (None: unchanged).  aom_step and comp_wfs_image(noise=None) use them; per-environment values stay in force."""
         nph = self.wfs_nphotons if nphotons is None else nphotons
         self._check(self.lib.aom_set_wfs_noise(self._ctx, float(noise), float(nph)), "aom_set_wfs_noise")
-        self.wfs_noise, self.wfs_nphotons = float(np.float32(noise)), float(np.float32(nph))
 
     def set_wfs_noise_env(self, noise=None, nphotons=None):
         """Sensor noise and photon count per environment (scalar or [E] each; None: that quantity's common value).  A
@@ -530,7 +529,6 @@ class Simulator:
         n = None if noise is None else self._env_array(noise, "set_wfs_noise_env(noise)")
         f = None if nphotons is None else self._env_array(nphotons, "set_wfs_noise_env(nphotons)")
         self._check(self.lib.aom_set_wfs_noise_env(self._ctx, P(n), P(f)), "aom_set_wfs_noise_env")
-        self.wfs_noise_env, self.wfs_nphotons_env = n, f
 
     def comp_wfs_image(self, atmos=True, dms=True, keep_image=False, noise=None, advance_frame=True):
         """noise None: the common noise, or with per-environment noise in force a noisy frame (each environment's own);
@@ -679,7 +677,6 @@ class Simulator:
         array sets one gain per environment (set_gain_env)."""
         if np.ndim(g) == 0:
             self._check(self.lib.aom_set_gain(self._ctx, float(g)), "aom_set_gain")
-            self._gain = float(np.float32(g))
         else:
             self.set_gain_env(g)
 
@@ -688,7 +685,6 @@ class Simulator:
         a = None if g is None else self._env_array(g, "set_gain_env")
         self._check(self.lib.aom_set_gain_env(self._ctx, None if a is None else a.ctypes.data_as(ctypes.c_void_p)),
                     "aom_set_gain_env")
-        self.gain_env = a
 
     def set_loop(self, closed):
         self._check(self.lib.aom_set_loop(self._ctx, int(bool(closed))), "aom_set_loop")

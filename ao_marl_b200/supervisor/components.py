@@ -252,7 +252,12 @@ class _Controller:
     def __init__(self, sim, ctype):
         self._sim = sim
         self.type = ctype
-        self.gain = float(sim.cfg.gain)
+
+    @property
+    def gain(self):
+        """The integrator gain in force: the common one, or the float32 [E] per-environment gains."""
+        g = self._sim.gain_env
+        return self._sim.gain if g is None else g
 
     def set_gain(self, g):
         """A scalar sets the gain of every environment (and drops per-environment gains); an [E] array one gain per
@@ -260,10 +265,8 @@ class _Controller:
         if np.ndim(g) == 0:
             self._sim.set_gain(float(g))
             self._sim.set_gain_env(None)
-            self.gain = float(g)
         else:
             self._sim.set_gain_env(g)
-            self.gain = self._sim.gain_env.copy()
 
 
 class _RtcHandle:

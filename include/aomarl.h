@@ -305,13 +305,14 @@ int aom_load_envs(aom_ctx* ctx, int n, const int32_t* envs, const void* src, voi
 int aom_move_atmos(aom_ctx* ctx, void* stream);
 
 /* AtmosCompass.set_wind / set_r0 (atmosCompass.py:79-135): new wind step (pixels / frame) and innovation
- * amplitude of one layer; a sign change of the wind needs no stencil upload (mirroring is index arithmetic). */
+ * amplitude of one layer; a sign change of the wind needs no stencil upload (mirroring is index arithmetic).
+ * AOM_ERR_INVALID for a non-finite value. */
 int aom_set_layer(aom_ctx* ctx, int layer, float deltax, float deltay, float amp);
 
 /* AtmosCompass.set_r0 per environment (the reference changes r0 of its single simulator at run time,
  * train_rpc.py:429-449; a batch can hold one condition per environment): innovation amplitude of `layer` for every
  * environment, host float [E] (NULL: back to the layer's common amplitude).  The wind is set per environment by
- * aom_set_layer_wind. */
+ * aom_set_layer_wind.  AOM_ERR_INVALID for a non-finite entry. */
 int aom_set_layer_amp(aom_ctx* ctx, int layer, const float* amp_host);
 
 /* AtmosCompass.set_wind per environment (atmosCompass.py:79-135; the reference changes the wind of its single simulator
@@ -324,6 +325,7 @@ int aom_set_layer_amp(aom_ctx* ctx, int layer, const float* amp_host);
  * - Back on the common wind, the library returns to its uniform kernels as soon as every layer's accumulators agree
  *   over the batch, at the latest after the next aom_reset (whose start-up extrudes each environment in the direction
  *   of its own x wind).
+ * - AOM_ERR_INVALID for a non-finite entry or only one of the two arrays (nothing changes then).
  * - AOM_ERR_UNSUPPORTED when the pupil footprint of an environment leaves the screen.  The round-1 sensor kernels (wfs
  *   paths tensor_reg / tensor / tensor_fast) have no per-environment form: their frames return AOM_ERR_UNSUPPORTED
  *   ("per-environment wind is not implemented in the round-1 sensor kernels ...") while such winds are in force.
@@ -357,6 +359,24 @@ int aom_set_wfs_noise(aom_ctx* ctx, float noise, float nphotons);
  *   tensor_fast) return AOM_ERR_UNSUPPORTED for a frame that would read per-environment sensor values.
  * Waits for the device; not for the step path. */
 int aom_set_wfs_noise_env(aom_ctx* ctx, const float* noise_host, const float* nphotons_host);
+
+/* Per-episode conditions: each is one common value or one value per environment of the batch.  The setters above and
+ * aom_set_gain / aom_set_gain_env change them (every value must be finite, photon counts > 0); aom_load_envs merges
+ * those of loaded records.  The values of aom_config are only their initial common values. */
+typedef enum aom_condition {
+  AOM_COND_AMP = 0,    /* innovation amplitude of a layer (aom_set_layer, aom_set_layer_amp) */
+  AOM_COND_WIND_X,     /* wind step of a layer, pixels / frame (aom_set_layer, aom_set_layer_wind) */
+  AOM_COND_WIND_Y,
+  AOM_COND_NOISE,      /* sensor noise (aom_set_wfs_noise, aom_set_wfs_noise_env); layer 0 */
+  AOM_COND_NPHOTONS,   /* photons per subaperture and frame; layer 0 */
+  AOM_COND_GAIN,       /* integrator gain (aom_set_gain, aom_set_gain_env); layer 0 */
+  AOM_COND_COUNT
+} aom_condition;
+/* Read back one condition (layer: that of AOM_COND_AMP / WIND_X / WIND_Y, 0 for the others).  Any output may be NULL.
+ * common: the common value; per_env: 1 while per-environment values are in force, else 0; values_host (host float [E]):
+ * each environment's value in force.  Answers from host copies, never touches the device.  AOM_ERR_INVALID for an
+ * unknown condition or a layer out of range. */
+int aom_get_condition(aom_ctx* ctx, int cond, int layer, float* common, float* values_host, int* per_env);
 
 /* Name of the kernel a noise-free aom_comp_wfs_image without kept image launches under the current AOM_OPT_WFS_PATH
  * ("wfs_frame_ws_kernel", "wfs_frame_umma_kernel", "wfs_frame_tma_kernel", "wfs_frame_mma_kernel" or "wfs_frame_kernel"), the
@@ -423,7 +443,7 @@ int aom_do_centroids_geom(aom_ctx* ctx, int flags, float alpha, void* stream);
 int aom_do_control(aom_ctx* ctx, void* stream);
 int aom_set_command(aom_ctx* ctx, const float* dcom, int ld, void* stream);
 int aom_apply_control(aom_ctx* ctx, int comp_voltage, void* stream);
-int aom_set_gain(aom_ctx* ctx, float gain);     /* common gain; per-environment gains (aom_set_gain_env) stay in force */
+int aom_set_gain(aom_ctx* ctx, float gain);     /* common gain (finite); per-environment gains (aom_set_gain_env) stay in force */
 /* RtcCompass.set_gain per environment (the reference tunes the integrator gain per parameter file, params.py): gain of
  * every environment's integrator, host float [E] (NULL: back to the common gain of aom_config.gain / aom_set_gain).
  * com += g[e] err in all three controller paths.  Persists through aom_reset / aom_reset_envs.  AOM_ERR_INVALID for a

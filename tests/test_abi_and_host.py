@@ -32,6 +32,8 @@ def test_table_and_buffer_enums_match_header():
     assert [b for b in bufs if b != "COUNT"] == binding.BUFFERS
     opts = re.findall(r"^\s*AOM_OPT_([A-Z0-9_]+)", header, flags=re.M)
     assert [o for o in opts if o != "COUNT"] == binding.OPTIONS
+    conds = re.findall(r"^\s*AOM_COND_([A-Z0-9_]+)", header, flags=re.M)
+    assert [c for c in conds if c != "COUNT"] == binding.CONDITIONS
 
 
 def test_no_cpu_path():
