@@ -14,11 +14,8 @@
 #include "gemm_tc.cuh"
 #include "rtc_kernels.cuh"
 #include "snapshot_kernels.cuh"
-#include "wfs_kernels.cuh"
-#include "wfs_mma.cuh"
-#include "wfs_lattice_host.h"
-#include "wfs_tma.cuh"
-#include "wfs_umma_host.h"
+#include "pupil_kernels.cuh"
+#include "wfs_frame_host.h"
 #include "extrude_i8_host.h"
 #include "geo_kernels.cuh"
 #include "pupil_sweep.cuh"
@@ -134,20 +131,8 @@ struct aom_ctx {
   double* snap_acc;
   void* snap_h;
   size_t snap_h_bytes;
-  // staged Shack-Hartmann kernels: host copies of the tables their own tables derive from; fast_why says why the last
-  // refused preparation refused
-  void* htab[AOM_T_COUNT];
-  size_t htab_bytes[AOM_T_COUNT];
-  char fast_why[160];
-  // TMA-staged kernel (wfs_tma.cuh): derived tables
-  int fast_state;            // 0 = not prepared, 1 = eligible, -1 = not eligible
-  WfsFast fast;
-  void* fast_dev[6];
-  CUtensorMap fast_maps[WFT_MAX_LAYERS];
-  // tcgen05 kernels (wfs_umma.cuh, wfs_umma_ws.cuh): derived tables
-  int umma_state;            // 0 = not prepared, 1 = eligible, -1 = not eligible
-  WfsUmmaHost umma;
-  void* umma_dev[6];
+  // the sensor frame's kernel routing and the derived tables of its staged kernels (wfs_frame.cu)
+  WfsFrame* wfs;
   // aom_step runs the turbulence update next to the actor / controller GEMMs on a second stream
   cudaStream_t side_stream;
   cudaEvent_t ev_fork, ev_join;
@@ -197,13 +182,6 @@ static void gemm_tc_each(F&& f) {     // tcgen05 GEMM: epilogue, column tile
   });
 }
 
-template <class F>
-static void wfs_simt_each(F&& f) {    // SIMT sensor frame: Nfft / 16, per-environment winds, per-environment sensor values
-  each<4, 8>([&](auto R) {
-    each<false, true>([&](auto PE) { each<false, true>([&](auto NE) { f(wfs_frame_kernel<R, PE, NE>, wfs_smem_bytes<R>(), R, PE, NE); }); });
-  });
-}
-
 extern "C" size_t aom_config_size(void) { return sizeof(aom_config); }
 
 extern "C" const char* aom_last_error(const aom_ctx* ctx) { return ctx ? ctx->err : g_create_error; }
@@ -225,10 +203,8 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
     return fail(nullptr, AOM_ERR_UNSUPPORTED, "actuator pitch too small for the %d-cell neighbourhood", WFS_NG_MAX);
   if (cfg->delay != 0 && cfg->delay != 1) return fail(nullptr, AOM_ERR_UNSUPPORTED, "controller delay must be 0 or 1 frame");
 
-  // the context embeds CUtensorMap objects (64-byte aligned)
-  ctx = (aom_ctx*)aligned_alloc(64, (sizeof(aom_ctx) + 63) / 64 * 64);
+  ctx = (aom_ctx*)calloc(1, sizeof(aom_ctx));
   if (!ctx) return fail(nullptr, AOM_ERR_INVALID, "out of host memory");
-  memset(ctx, 0, sizeof(aom_ctx));
   ctx->cfg = *cfg;
   for (int l = 0; l < AOM_MAX_LAYERS; ++l) {
     ctx->cond[AOM_COND_AMP][l].common = cfg->amp[l];
@@ -316,6 +292,8 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
     CU(dalloc(&ctx->aHO, A * E * ctx->ld_aho));
   }
   CU(dalloc(&ctx->d_err, 1));
+  ctx->wfs = wfs_frame_create(ctx->cfg, ctx->screen, ctx->d_err, ctx->num_sms);
+  if (!ctx->wfs) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
   CU(cudaStreamCreateWithFlags(&ctx->side_stream, cudaStreamNonBlocking));
   CU(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
   CU(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
@@ -324,7 +302,6 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
     if (ae == cudaSuccess) ae = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   };
   gemm_tc_each(smem_attr);
-  wfs_simt_each(smem_attr);
   if (ae != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "cudaFuncSetAttribute(dynamic shared memory) failed: %s", cudaGetErrorString(ae));
   return AOM_OK;
 }
@@ -350,9 +327,7 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
   for (int t = 0; t < AOM_T_COUNT; ++t) { cudaFree(ctx->ozop[t]); cudaFree(ctx->ozop_ea[t]); }
   cudaFree(ctx->oz_zs); cudaFree(ctx->oz_ev); cudaFree(ctx->oz_xs); cudaFree(ctx->oz_xev);
   for (int i = 0; i < 3; ++i) cudaFree(ctx->actor_bt[i]);
-
-  for (void* b : ctx->fast_dev) cudaFree(b);
-  for (void* b : ctx->umma_dev) cudaFree(b);
+  wfs_frame_destroy(ctx->wfs);
   for (int i = 0; i < AOM_WFS_TIMERS; ++i)
     for (int j = 0; j < 2; ++j)
       if (ctx->wev[j][i]) cudaEventDestroy(ctx->wev[j][i]);
@@ -360,7 +335,6 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
   if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
   if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
   if (ctx->ev_geo) cudaEventDestroy(ctx->ev_geo);
-  for (int t = 0; t < AOM_T_COUNT; ++t) free(ctx->htab[t]);
   free(ctx->snap_h);
   free(ctx);
 }
@@ -451,16 +425,7 @@ extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* hos
   CU(cudaMalloc(&ctx->tab[table][index], nbytes ? nbytes : 4));
   CU(cudaMemcpy(ctx->tab[table][index], host, nbytes, cudaMemcpyHostToDevice));
   ctx->tab_bytes[table][index] = nbytes;
-  if (table == AOM_T_MPUPIL || table == AOM_T_SUB_X0 || table == AOM_T_SUB_Y0 || table == AOM_T_STAMP1D ||
-      table == AOM_T_ACT_MAP || table == AOM_T_HALFXY || table == AOM_T_TT_PLANES) {
-    free(ctx->htab[table]);
-    ctx->htab[table] = malloc(nbytes ? nbytes : 4);
-    if (!ctx->htab[table]) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
-    memcpy(ctx->htab[table], host, nbytes);
-    ctx->htab_bytes[table] = nbytes;
-    ctx->fast_state = 0;     // derived tables of the staged sensor kernels are rebuilt on the next frame
-    ctx->umma_state = 0;
-  }
+  if (!wfs_frame_set_table(ctx->wfs, table, host, nbytes)) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
   if (table == AOM_T_MPUPIL || table == AOM_T_TT_PLANES) ctx->sweep_state = 0;
   if (table == AOM_T_DENOISER_TC) memcpy(ctx->dn_prm, host, (size_t)DT_NPARAM * 4);   // float parameters travel as kernel arguments
   if (table == AOM_T_ACTOR_W1 || table == AOM_T_ACTOR_W2 || table == AOM_T_ACTOR_WH) {
@@ -1434,309 +1399,6 @@ extern "C" int aom_load_envs(aom_ctx* ctx, int n, const int32_t* envs, const voi
 }
 
 // ---------------------------------------------------------------------------------------------
-// Host side of the staged sensor kernels, wfs_frame_tma_kernel (wfs_tma.cuh) and the tcgen05 pair (wfs_umma.cuh,
-// wfs_umma_ws.cuh): eligibility, derived tables, TMA descriptors.  Both read the mirror through the same lattice
-// analysis (wfs_lattice_host.h) and lay out its tables their own way.
-static uint32_t half2_bits(float a, float b) {
-  __half2 h = __floats2half2_rn(a, b);
-  uint32_t u;
-  memcpy(&u, &h, 4);
-  return u;
-}
-
-static void split_pair(double a, double b, int lo_part, uint32_t& out) {
-  const float ah = __half2float(__float2half_rn((float)a)), bh = __half2float(__float2half_rn((float)b));
-  out = lo_part ? half2_bits((float)(a - (double)ah), (float)(b - (double)bh)) : half2_bits(ah, bh);
-}
-
-// W[n][i] = exp(-2 pi i n F(i) / 64), F = the 32 kept frequencies (0..15, 48..63); part 0 = real, 1 = imaginary
-static double wft_w(int n, int i, int part) {
-  const int F = (i < 16) ? i : i + 32;
-  const int ang = (n * F) & 63;
-  const double th = -2.0 * M_PI * (double)ang / 64.0;
-  return part ? sin(th) : cos(th);
-}
-
-typedef CUresult (*aom_encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                        const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                        CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-// A staged kernel cannot serve this configuration: its state becomes -1 and fast_why says why.  Returns AOM_OK.
-static int staged_refuse(aom_ctx* ctx, int& state, const char* fmt, ...) {
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(ctx->fast_why, sizeof(ctx->fast_why), fmt, ap);
-  va_end(ap);
-  state = -1;
-  return AOM_OK;
-}
-
-// The lattice analysis of the uploaded host tables: null, or why the staged kernels cannot serve them
-static const char* staged_lattice(aom_ctx* ctx, WfsLattice& L) {
-  return wfl_analyse(ctx->cfg, (const float*)ctx->htab[AOM_T_MPUPIL], (const int*)ctx->htab[AOM_T_SUB_X0],
-                     (const int*)ctx->htab[AOM_T_SUB_Y0], (const float*)ctx->htab[AOM_T_STAMP1D],
-                     (const int*)ctx->htab[AOM_T_ACT_MAP], L);
-}
-
-// One 3-D map [E][N][N] per screen layer, box bw x bh x 1, zero fill outside.  False: refused (state, fast_why).
-static bool encode_screen_maps(aom_ctx* ctx, CUtensorMap* maps, cuuint32_t bw, cuuint32_t bh, int& state) {
-  const aom_config& c = ctx->cfg;
-  if (c.n_layers == 0) return true;
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn ||
-      qres != cudaDriverEntryPointSuccess) {
-    staged_refuse(ctx, state, "cuTensorMapEncodeTiled not available");
-    return false;
-  }
-  for (int l = 0; l < c.n_layers; ++l) {
-    const cuuint64_t N = (cuuint64_t)c.screen_dim[l];
-    const cuuint64_t dims[3] = {N, N, (cuuint64_t)c.n_env};
-    const cuuint64_t strides[2] = {N * 4, N * N * 4};
-    const cuuint32_t box[3] = {bw, bh, 1};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = ((aom_encode_tiled_fn)fn)(&maps[l], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, ctx->screen[l], dims, strides, box,
-                                           estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      staged_refuse(ctx, state, "cuTensorMapEncodeTiled failed (%d)", (int)r);
-      return false;
-    }
-  }
-  return true;
-}
-
-// Copies the six host tables src[i] of bytes[i] into new device buffers dev[i]
-static cudaError_t upload_tables(void* (&dev)[6], const void* const (&src)[6], const size_t (&bytes)[6]) {
-  cudaError_t ce = cudaSuccess;
-  for (int i = 0; i < 6 && ce == cudaSuccess; ++i) {
-    ce = cudaMalloc(&dev[i], bytes[i]);
-    if (ce == cudaSuccess) ce = cudaMemcpy(dev[i], src[i], bytes[i], cudaMemcpyHostToDevice);
-  }
-  return ce;
-}
-
-static int wfs_fast_prepare(aom_ctx* ctx) {
-  const aom_config& c = ctx->cfg;
-  if (ctx->fast_state != 0) return AOM_OK;
-  for (void*& b : ctx->fast_dev) { cudaFree(b); b = nullptr; }
-  WfsLattice L;
-  if (const char* why = staged_lattice(ctx, L)) return staged_refuse(ctx, ctx->fast_state, "%s", why);
-  const float* pup = (const float*)ctx->htab[AOM_T_MPUPIL];
-  const int* sx = (const int*)ctx->htab[AOM_T_SUB_X0];
-  const int* sy = (const int*)ctx->htab[AOM_T_SUB_Y0];
-  const float* stamp = (const float*)ctx->htab[AOM_T_STAMP1D];
-  const int nv = c.nvalid, GW = L.GW;
-  uint2* h_sub = (uint2*)malloc((size_t)nv * sizeof(uint2));
-  unsigned char* h_pm = (unsigned char*)malloc((size_t)nv * 32);
-  short* h_amap = (short*)malloc((size_t)GW * GW * sizeof(short));
-  float h_fxy[2 * WFT_NG * 16];
-  uint4* h_c1 = (uint4*)malloc(8 * 32 * sizeof(uint4));
-  uint4* h_c2 = (uint4*)malloc(12 * 32 * sizeof(uint4));
-  const bool ok = h_sub && h_pm && h_amap && h_c1 && h_c2;
-  if (ok) {
-    wfl_amap(c, L, (const int*)ctx->htab[AOM_T_ACT_MAP], h_amap);
-    for (int k = 0; k < nv; ++k) {
-      h_sub[k] = make_uint2(((uint32_t)sy[k] << 16) | (uint32_t)sx[k], (uint32_t)wfl_window(c, L, sx[k], sy[k]));
-      for (int lane = 0; lane < 32; ++lane) {
-        const int g = lane >> 2, q = lane & 3;
-        unsigned m = 0;
-        for (int r = 0; r < 2; ++r)
-          for (int cc = 0; cc < 4; ++cc)
-            if (pup[(size_t)(sy[k] + 2 * g + r) * c.n + sx[k] + 4 * q + cc] != 0.f) m |= 1u << (r * 4 + cc);
-        h_pm[(size_t)k * 32 + lane] = (unsigned char)m;
-      }
-    }
-    for (int ax = 0; ax < 2; ++ax)
-      for (int j = 0; j < WFT_NG; ++j)
-        for (int x = 0; x < 16; ++x) h_fxy[(ax * WFT_NG + j) * 16 + x] = wfl_factor(c, L, stamp, ax, j, x);
-    // stage-1 A fragments: row r of m-tile mt <-> kept frequency 16 mt + 2 (r & 7) + (r >> 3); k <-> x = sigma(k)
-    auto sigma = [](int kk) { return kk < 8 ? 4 * (kk >> 1) + (kk & 1) : 4 * ((kk - 8) >> 1) + 2 + (kk & 1); };
-    auto yk = [](int kk) { return kk < 8 ? 2 * kk : 2 * (kk - 8) + 1; };
-    for (int mt = 0; mt < 2; ++mt)
-      for (int part = 0; part < 2; ++part)
-        for (int hl = 0; hl < 2; ++hl)
-          for (int lane = 0; lane < 32; ++lane) {
-            const int g = lane >> 2, q = lane & 3;
-            const int rows[2] = {g, g + 8};
-            const int ks[4] = {2 * q, 2 * q + 1, 2 * q + 8, 2 * q + 9};
-            uint32_t w[4];
-            for (int reg = 0; reg < 4; ++reg) {      // a0 (g; 2q..) a1 (g+8; 2q..) a2 (g; 2q+8..) a3 (g+8; 2q+8..)
-              const int r = rows[reg & 1], fi = 16 * mt + 2 * (r & 7) + (r >> 3);
-              const int k0 = ks[(reg >> 1) * 2], k1 = ks[(reg >> 1) * 2 + 1];
-              split_pair(wft_w(sigma(k0), fi, part), wft_w(sigma(k1), fi, part), hl, w[reg]);
-            }
-            h_c1[((mt * 2 + part) * 2 + hl) * 32 + lane] = make_uint4(w[0], w[1], w[2], w[3]);
-          }
-    // stage-2 B fragments: k <-> y = yk(k), n = g <-> kept frequency 8 b + g
-    for (int b = 0; b < 4; ++b)
-      for (int lane = 0; lane < 32; ++lane) {
-        const int g = lane >> 2, q = lane & 3;
-        const int ks[4] = {2 * q, 2 * q + 1, 2 * q + 8, 2 * q + 9};
-        uint32_t hi[4], lo[4], nh[2], nl[2];
-        for (int reg = 0; reg < 4; ++reg) {        // {Wr b0, Wr b1, Wi b0, Wi b1}
-          const int part = reg >> 1, k0 = ks[(reg & 1) * 2], k1 = ks[(reg & 1) * 2 + 1];
-          split_pair(wft_w(yk(k0), 8 * b + g, part), wft_w(yk(k1), 8 * b + g, part), 0, hi[reg]);
-          split_pair(wft_w(yk(k0), 8 * b + g, part), wft_w(yk(k1), 8 * b + g, part), 1, lo[reg]);
-        }
-        for (int h = 0; h < 2; ++h) { nh[h] = hi[2 + h] ^ 0x80008000u; nl[h] = lo[2 + h] ^ 0x80008000u; }
-        h_c2[(b * 3 + 0) * 32 + lane] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-        h_c2[(b * 3 + 1) * 32 + lane] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-        h_c2[(b * 3 + 2) * 32 + lane] = make_uint4(nh[0], nh[1], nl[0], nl[1]);
-      }
-  }
-  const void* const srcs[6] = {h_sub, h_amap, h_pm, h_c1, h_c2, h_fxy};
-  const size_t sizes[6] = {(size_t)nv * sizeof(uint2), (size_t)GW * GW * sizeof(short), (size_t)nv * 32,
-                           8 * 32 * sizeof(uint4), 12 * 32 * sizeof(uint4), sizeof(h_fxy)};
-  const cudaError_t ce = ok ? upload_tables(ctx->fast_dev, srcs, sizes) : cudaSuccess;
-  free(h_sub); free(h_pm); free(h_amap); free(h_c1); free(h_c2);
-  if (ce != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "wfs_fast_prepare: %s", cudaGetErrorString(ce));
-  if (!ok) return staged_refuse(ctx, ctx->fast_state, "out of host memory");
-  if (!encode_screen_maps(ctx, ctx->fast_maps, WFT_TILE_W, WFT_TILE_H, ctx->fast_state)) return AOM_OK;
-  WfsFast& f = ctx->fast;
-  f.sub = (const uint2*)ctx->fast_dev[0];
-  f.amap = (const short*)ctx->fast_dev[1];
-  f.pmask = (const unsigned char*)ctx->fast_dev[2];
-  f.c1 = (const uint4*)ctx->fast_dev[3];
-  f.c2 = (const uint4*)ctx->fast_dev[4];
-  f.fxy = (const float*)ctx->fast_dev[5];
-  f.GW = GW;
-  f.sub_in_smem = (nv <= 1280) ? 1 : 0;
-  f.err = ctx->d_err;
-  ctx->fast_state = 1;
-  return AOM_OK;
-}
-
-static void umma_put_half(unsigned short* tile_hi, unsigned short* tile_lo, int n, int kk, double v) {
-  // UMMA canonical K-major no-swizzle layout: 8-row x 16-byte core matrices, LBO 128 B, SBO 512 B (K = 32 halves)
-  const __half hi = __float2half_rn((float)v);
-  const __half lo = __float2half_rn((float)(v - (double)__half2float(hi)));
-  const size_t off = (size_t)(n >> 3) * 512 + (size_t)(kk >> 3) * 128 + (size_t)(n & 7) * 16 + (size_t)(kk & 7) * 2;
-  memcpy((unsigned char*)tile_hi + off, &hi, 2);
-  memcpy((unsigned char*)tile_lo + off, &lo, 2);
-}
-
-// The tcgen05 kernels also need a full group of subapertures and the analytic half-pixel phasor; their tables are in the
-// (h, y) lane layout, with the operand tiles of the two DFT stages and 20 x 17 TMA boxes.
-static int wfs_umma_prepare(aom_ctx* ctx) {
-  const aom_config& c = ctx->cfg;
-  if (ctx->umma_state != 0) return AOM_OK;
-  for (void*& b : ctx->umma_dev) { cudaFree(b); b = nullptr; }
-  WfsLattice L;
-  if (const char* why = staged_lattice(ctx, L)) return staged_refuse(ctx, ctx->umma_state, "%s", why);
-  if (c.nvalid < WU_WARPS) return staged_refuse(ctx, ctx->umma_state, "fewer than %d subapertures", WU_WARPS);
-  const float* hxy = (const float*)ctx->htab[AOM_T_HALFXY];
-  if (!hxy) return staged_refuse(ctx, ctx->umma_state, "half-pixel phasor table not uploaded");
-  for (int i = 0; i < 16; ++i)
-    for (int j = 0; j < 16; ++j)
-      if (fabs((double)hxy[i * 16 + j] - M_PI * (double)(i + j) / 64.0) > 2e-6)
-        return staged_refuse(ctx, ctx->umma_state, "half-pixel phasor is not pi (x + y) / Nfft");
-  const float* pup = (const float*)ctx->htab[AOM_T_MPUPIL];
-  const int* sx = (const int*)ctx->htab[AOM_T_SUB_X0];
-  const int* sy = (const int*)ctx->htab[AOM_T_SUB_Y0];
-  const float* stamp = (const float*)ctx->htab[AOM_T_STAMP1D];
-  const int nv = c.nvalid, GW = L.GW;
-  uint2* h_sub = (uint2*)malloc((size_t)nv * sizeof(uint2));
-  uint32_t* h_pm = (uint32_t*)malloc((size_t)nv * 32 * sizeof(uint32_t));
-  short* h_amap = (short*)malloc((size_t)GW * GW * sizeof(short));
-  unsigned short* h_b1 = (unsigned short*)calloc(2 * WU_B_BYTES, 1);     // [hi, lo] tiles of WU_B_BYTES each
-  unsigned short* h_b2 = (unsigned short*)calloc(2 * WU_B_BYTES, 1);
-  float h_fxy[2 * WU_NG * 16];
-  const bool ok = h_sub && h_pm && h_amap && h_b1 && h_b2;
-  if (ok) {
-    wfl_amap(c, L, (const int*)ctx->htab[AOM_T_ACT_MAP], h_amap);
-    for (int k = 0; k < nv; ++k) {
-      bool full = true;
-      for (int lane = 0; lane < 32; ++lane) {
-        const int yy = lane & 15, hh = lane >> 4;
-        unsigned m = 0;
-        for (int cc = 0; cc < 8; ++cc)
-          if (pup[(size_t)(sy[k] + yy) * c.n + sx[k] + 8 * hh + cc] != 0.f) m |= 1u << cc;
-        h_pm[(size_t)k * 32 + lane] = m;
-        full = full && m == 0xffu;
-      }
-      h_sub[k] = make_uint2(((uint32_t)sy[k] << 16) | (uint32_t)sx[k],
-                            (uint32_t)wfl_window(c, L, sx[k], sy[k]) | (full ? 0x80000000u : 0u));
-    }
-    // x stamp factors [j][x], y stamp factors transposed [y][j]
-    for (int j = 0; j < WU_NG; ++j)
-      for (int x = 0; x < 16; ++x) {
-        h_fxy[j * 16 + x] = wfl_factor(c, L, stamp, 0, j, x);
-        h_fxy[WU_NG * 16 + x * WU_NG + j] = wfl_factor(c, L, stamp, 1, j, x);
-      }
-    // stage 1: B1[n = 32 ro + fx][k = 16 ri + x]:  Tr = Wr Xr - Wi Xi ; Ti = Wi Xr + Wr Xi
-    // stage 2: B2[n = 2 fy + po][k = 16 ro + y]:   Yr = Tr Wr - Ti Wi ; Yi = Tr Wi + Ti Wr
-    unsigned short* b1_lo = (unsigned short*)((unsigned char*)h_b1 + WU_B_BYTES);
-    unsigned short* b2_lo = (unsigned short*)((unsigned char*)h_b2 + WU_B_BYTES);
-    for (int n = 0; n < 64; ++n)
-      for (int kk = 0; kk < 32; ++kk) {
-        {
-          const int ro = n >> 5, fx = n & 31, ri = kk >> 4, x = kk & 15;
-          const double wr = wft_w(x, fx, 0), wi = wft_w(x, fx, 1);
-          umma_put_half(h_b1, b1_lo, n, kk, ro == 0 ? (ri == 0 ? wr : -wi) : (ri == 0 ? wi : wr));
-        }
-        {
-          const int fy = n >> 1, po = n & 1, ro = kk >> 4, yy = kk & 15;
-          const double wr = wft_w(yy, fy, 0), wi = wft_w(yy, fy, 1);
-          umma_put_half(h_b2, b2_lo, n, kk, po == 0 ? (ro == 0 ? wr : -wi) : (ro == 0 ? wi : wr));
-        }
-      }
-  }
-  const void* const srcs[6] = {h_sub, h_amap, h_pm, h_b1, h_b2, h_fxy};
-  const size_t sizes[6] = {(size_t)nv * sizeof(uint2), (size_t)GW * GW * sizeof(short), (size_t)nv * 32 * sizeof(uint32_t),
-                           (size_t)2 * WU_B_BYTES, (size_t)2 * WU_B_BYTES, sizeof(h_fxy)};
-  const cudaError_t ce = ok ? upload_tables(ctx->umma_dev, srcs, sizes) : cudaSuccess;
-  free(h_sub); free(h_pm); free(h_amap); free(h_b1); free(h_b2);
-  if (ce != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "wfs_umma_prepare: %s", cudaGetErrorString(ce));
-  if (!ok) return staged_refuse(ctx, ctx->umma_state, "out of host memory");
-  if (!encode_screen_maps(ctx, ctx->umma.maps, WU_TILE_W, WU_TILE_H, ctx->umma_state)) return AOM_OK;
-  WfsUmmaTables& f = ctx->umma.f;
-  memset(&f, 0, sizeof(f));
-  f.sub = (const uint2*)ctx->umma_dev[0];
-  f.amap = (const short*)ctx->umma_dev[1];
-  f.pmask = (const uint32_t*)ctx->umma_dev[2];
-  f.b1 = (const uint4*)ctx->umma_dev[3];
-  f.b2 = (const uint4*)ctx->umma_dev[4];
-  f.fxy = (const float*)ctx->umma_dev[5];
-  f.GW = GW;
-  f.err = ctx->d_err;
-  ctx->umma_state = 1;
-  return AOM_OK;
-}
-
-template <int FULL, int NL>
-static int wfs_fast_launch_t(aom_ctx* ctx, const WfsParams& p, cudaStream_t st) {
-  const long long total = (long long)p.E * p.nvalid;
-  // contiguous ranges of work items per CTA: about 8 waves of resident CTAs per SM, at least 16 items per warp
-  long long grid = (long long)ctx->num_sms * WFT_MIN_CTAS * 8;
-  long long ipc = (total + grid - 1) / grid;
-  if (ipc < 16 * WFT_WARPS) ipc = 16 * WFT_WARPS;
-  ipc = (ipc + WFT_WARPS - 1) / WFT_WARPS * WFT_WARPS;
-  grid = (total + ipc - 1) / ipc;
-  WfsTmaParams P;
-  memset(&P, 0, sizeof(P));
-  P.p = p;
-  P.f = ctx->fast;
-  P.f.items_per_cta = ipc;
-  for (int l = 0; l < NL; ++l) P.maps[l] = ctx->fast_maps[l];
-  const size_t smem = wft_smem_bytes<NL>(P.f.GW, P.f.sub_in_smem ? p.nvalid : 0);
-  {
-    cudaError_t e = cudaFuncSetAttribute(wfs_frame_tma_kernel<FULL, NL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "cudaFuncSetAttribute(wfs_frame_tma_kernel): %s", cudaGetErrorString(e));
-  }
-  wfs_frame_tma_kernel<FULL, NL><<<(unsigned)grid, WFT_WARPS * 32, smem, st>>>(P);
-  return AOM_OK;
-}
-
-static int wfs_fast_launch(aom_ctx* ctx, const WfsParams& p, bool full, cudaStream_t st) {
-  int rc = AOM_OK;
-  const bool served = with<0, 1, 2, 3, 4>(p.n_layers, [&](auto NL) {
-    with<false, true>(full, [&](auto FULL) { rc = wfs_fast_launch_t<FULL, NL>(ctx, p, st); });
-  });
-  return served ? rc : fail(ctx, AOM_ERR_UNSUPPORTED, "wfs_fast_launch: %d layers", p.n_layers);
-}
-
-// ---------------------------------------------------------------------------------------------
 static int fill_wfs_params(aom_ctx* ctx, WfsParams& p, int flags, float noise) {
   const aom_config& c = ctx->cfg;
   memset(&p, 0, sizeof(p));
@@ -1781,62 +1443,6 @@ static int fill_wfs_params(aom_ctx* ctx, WfsParams& p, int flags, float noise) {
   return AOM_OK;
 }
 
-// The sensor kernel that serves a frame: its family with its compile-time choices, and whether the frame is refused
-enum WfsFamily { WFS_WS, WFS_UMMA, WFS_TMA, WFS_MMA, WFS_SIMT };
-static const char* const wfs_kernel_names[] = {"wfs_frame_ws_kernel", "wfs_frame_umma_kernel", "wfs_frame_tma_kernel",
-                                               "wfs_frame_mma_kernel", "wfs_frame_kernel"};
-struct WfsRoute {
-  WfsFamily family;
-  bool full, pe, ne;     // fp32-grade products in both DFT stages; per-environment winds; per-environment sensor values
-  int nl, r;             // layers of the instantiation (mma: 0, 1 or 3, else -1: its generic form); simt: Nfft / 16
-  const char* refused;   // not null: the frame is refused with this message (family still names the path's kernel)
-};
-
-// Routes a frame of parameters p (fill_wfs_params), noisy when any environment draws noise in it, with its image kept or
-// not.  Prepares the tables of a staged kernel on first use, and the round-1 kernel's only when the route can reach it.
-static int wfs_route(aom_ctx* ctx, const WfsParams& p, bool noisy, bool keep, WfsRoute& r) {
-  const aom_config& c = ctx->cfg;
-  const int path = ctx->opt[AOM_OPT_WFS_PATH];
-  const bool umma = (path == AOM_WFS_UMMA || path == AOM_WFS_UMMA_FAST || path == AOM_WFS_UMMA_WS);
-  const bool staged = umma || path == AOM_WFS_MMA_STAGED || path == AOM_WFS_MMA_STAGED_FAST;
-  memset(&r, 0, sizeof(r));
-  r.full = !(path == AOM_WFS_UMMA_FAST || path == AOM_WFS_MMA_STAGED_FAST);
-  r.nl = p.n_layers;
-  r.pe = p.wind != nullptr;
-  r.ne = p.noise_env || p.nph_env;
-  if (c.nfft != 64 || path == AOM_WFS_SIMT) {
-    r.family = WFS_SIMT;
-    r.r = c.nfft / 16;
-    return AOM_OK;
-  }
-  if (umma) {
-    int rc = wfs_umma_prepare(ctx);
-    if (rc) return rc;
-  }
-  if (umma && ctx->umma_state == 1) {
-    // the specialised-warp kernel serves every frame without noise and kept image (it reads neither noise nor photon
-    // count); the others go to the fused kernel, in its per-environment form when per-environment values are in force
-    r.family = (path == AOM_WFS_UMMA_WS && !noisy && !keep) ? WFS_WS : WFS_UMMA;
-    if (r.family == WFS_WS) r.ne = false;
-    return AOM_OK;
-  }
-  if (staged) {
-    int rc = wfs_fast_prepare(ctx);
-    if (rc) return rc;
-  }
-  r.family = (staged && ctx->fast_state == 1) ? WFS_TMA : WFS_MMA;
-  if (r.family == WFS_MMA && r.nl != 0 && r.nl != 1 && r.nl != 3) r.nl = -1;
-  // the round-1 kernels have no per-environment form
-  r.refused = p.frame0 ? "staggered environments (aom_reset_envs) are not implemented in the round-1 sensor kernels "
-                         "(wfs_frame_tma_kernel, wfs_frame_mma_kernel) until the next aom_reset: use the umma, umma_ws or simt path"
-            : p.wind ? "per-environment wind is not implemented in the round-1 sensor kernels (wfs_frame_tma_kernel, "
-                       "wfs_frame_mma_kernel): use the umma, umma_ws or simt path"
-            : r.ne ? "per-environment sensor noise and photon counts are not implemented in the round-1 sensor kernels "
-                     "(wfs_frame_tma_kernel, wfs_frame_mma_kernel): use the umma, umma_ws or simt path"
-            : nullptr;
-  return AOM_OK;
-}
-
 extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
   cudaStream_t st = (cudaStream_t)stream;
@@ -1852,36 +1458,12 @@ extern "C" int aom_comp_wfs_image(aom_ctx* ctx, int flags, float noise, void* st
   // does any environment draw noise in this frame?  (host copies: no device read)
   bool noisy = p.noise >= 0.f && !p.noise_env;
   for (int e = 0; p.noise_env && e < c.n_env && !noisy; ++e) noisy = ctx->cond[AOM_COND_NOISE][0].host[e] >= 0.f;
-  WfsRoute r;
-  rc = wfs_route(ctx, p, noisy, p.bincube != nullptr, r);
-  if (rc) return rc;
-  if (r.refused) return fail(ctx, AOM_ERR_UNSUPPORTED, "%s", r.refused);
   const bool timed = ctx->opt[AOM_OPT_TIME_WFS] && ctx->wev_n < AOM_WFS_TIMERS;
-  if (timed) {
+  if (timed)
     for (int j = 0; j < 2; ++j)
       if (!ctx->wev[j][ctx->wev_n]) CU(cudaEventCreate(&ctx->wev[j][ctx->wev_n]));
-    CU(cudaEventRecord(ctx->wev[0][ctx->wev_n], st));
-  }
-  long long total = (long long)c.n_env * c.nvalid;
-  long long blocks = (total + WFS_WARPS - 1) / WFS_WARPS;
-  long long cap = (long long)ctx->num_sms * 2 * 8;      // 2 resident CTAs per SM, 8 waves of work each
-  int grid = (int)(blocks < cap ? blocks : cap);
-  if (r.family == WFS_WS || r.family == WFS_UMMA) {
-    if (r.family == WFS_WS) { p.noise = -1.f; p.noise_env = nullptr; p.nph_env = nullptr; }
-    cudaError_t le = wfs_umma_launch(p, ctx->umma, ctx->num_sms, r.family == WFS_WS, r.full, r.ne, st);
-    if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "wfs_umma_launch: %s", cudaGetErrorString(le));
-  } else if (r.family == WFS_TMA) {
-    rc = wfs_fast_launch(ctx, p, r.full, st);
-    if (rc) return rc;
-  } else if (r.family == WFS_MMA) {
-    with<0, 1, 3, -1>(r.nl, [&](auto NL) {
-      with<false, true>(r.full, [&](auto FULL) { wfs_frame_mma_kernel<FULL, NL><<<grid, WFM_WARPS * 32, 0, st>>>(p); });
-    });
-  } else {
-    wfs_simt_each([&](auto kernel, size_t smem, int R, bool PE, bool NE) {
-      if (R == r.r && PE == r.pe && NE == r.ne) kernel<<<grid, WFS_WARPS * 32, smem, st>>>(p);
-    });
-  }
+  rc = wfs_frame_launch(ctx->wfs, p, ctx->opt[AOM_OPT_WFS_PATH], noisy, timed ? ctx->wev[0][ctx->wev_n] : nullptr, st, ctx->err);
+  if (rc) return rc;
   KCHECK();
   if (timed) {
     CU(cudaEventRecord(ctx->wev[1][ctx->wev_n], st));
@@ -1909,14 +1491,7 @@ extern "C" int aom_wfs_time_ms(aom_ctx* ctx, float* mean_ms, int* count) {
 
 extern "C" const char* aom_wfs_kernel(aom_ctx* ctx) {
   if (!ctx) return "";
-  // the route of a noise-free frame without kept image; the per-environment state does not change its family, so the
-  // fields the route reads for it stay empty (and a refusal it would cause is not reported)
-  const WfsParams p{};
-  WfsRoute r;
-  if (wfs_route(ctx, p, false, false, r) != AOM_OK) return "";
-  if (r.family == WFS_MMA && ctx->opt[AOM_OPT_WFS_PATH] != AOM_WFS_MMA_REG)
-    snprintf(ctx->err, sizeof(ctx->err), "staged sensor kernels not eligible: %s", ctx->fast_why);
-  return wfs_kernel_names[r.family];
+  return wfs_frame_kernel_name(ctx->wfs, ctx->opt[AOM_OPT_WFS_PATH], ctx->err);
 }
 
 extern "C" int aom_raytrace_wfs(aom_ctx* ctx, int flags, void* stream) {

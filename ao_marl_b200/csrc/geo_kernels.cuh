@@ -15,7 +15,7 @@
 // On the production lattices (pitch 16) the row pass is MODE 0 of pupil_sweep.cuh (staged screen rows, vector loads);
 // geo_rows_kernel below is the generic form for any pitch.
 #pragma once
-#include "wfs_kernels.cuh"
+#include "pupil_kernels.cuh"
 
 #define GEO_ROW_WARPS 4
 
@@ -35,21 +35,7 @@ __global__ void __launch_bounds__(GEO_ROW_WARPS * 32) geo_rows_kernel(WfsParams 
   for (int x = lane; x < p.n; x += 32) {
     float v = 0.f;
     if (mrow[x] != 0.f) {
-      for (int l = 0; l < p.n_layers; ++l) {
-        const WfsLayer& L = p.layer[l];
-        const int N = L.N;
-        const float* scr = L.screen + (size_t)e * N * N;
-        const int ox = L.ox[e], oy = L.oy[e];
-        const WindRec w = wind_of<PE>(p, l, e);
-        // footprint inside the screen (checked on the host) and 0 <= ox, oy < N: one conditional subtract wraps
-        int pc0 = x + w.ix + ox; pc0 -= (pc0 >= N) ? N : 0;
-        int pc1 = pc0 + 1;       pc1 -= (pc1 >= N) ? N : 0;
-        int pr0 = y + w.iy + oy; pr0 -= (pr0 >= N) ? N : 0;
-        int pr1 = pr0 + 1;       pr1 -= (pr1 >= N) ? N : 0;
-        float top = wfs_layer_row(scr, N, pr0, pc0, pc1, w.fx);
-        float bot = wfs_layer_row(scr, N, pr1, pc0, pc1, w.fx);
-        v += top + w.fy * (bot - top);
-      }
+      v = pupil_screens<PE>(p, e, x, y);
       s1 += v;
       sx = fmaf(v, __ldg(ttx + x), sx);
       sy = fmaf(v, __ldg(tty + x), sy);

@@ -31,8 +31,8 @@
 // writes its 11 partial sums (g = 8 cb - 3 .. 8 cb + 7) to Tp[e][y][cb][12] and geo_cols_kernel adds the two
 // blocks that can contribute to a lattice column -- no atomics, deterministic.
 #pragma once
-#include "wfs_kernels.cuh"
-#include "wfs_tma.cuh"
+#include "device_common.cuh"
+#include "pupil_kernels.cuh"
 
 #define PSW_WARPS 8
 #define PSW_SLOTS 3

@@ -20,6 +20,7 @@
 #pragma once
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
+#include "device_common.cuh"
 #include "wfs_kernels.cuh"
 
 #define WFM_WARPS 8
@@ -59,17 +60,6 @@ __device__ __forceinline__ float wfm_w(int n, int i, int part) {
   float s, c;
   sincospif(-(float)ang * (1.0f / 32.0f), &s, &c);
   return part ? s : c;
-}
-
-// sin / cos of a float32 argument of any magnitude met here (|x| < ~1e4): three-term Cody-Waite
-// reduction by 2 pi, then the SFU approximations on [-pi, pi] (absolute error < 5e-7)
-__device__ __forceinline__ void wfm_sincos(float x, float& s, float& c) {
-  const float n = rintf(x * 0.15915494309189535f);
-  float r = fmaf(n, -6.28125f, x);                    // 2 pi = 6.28125 + 1.9350051879882812e-3 + 3.0199159819995e-7
-  r = fmaf(n, -1.9350051879882812e-3f, r);
-  r = fmaf(n, -3.0199159819995e-7f, r);
-  s = __sinf(r);
-  c = __cosf(r);
 }
 
 // three consecutive floats p[0..2]; `even` = p is 8-byte aligned (warp-uniform), else p + 1 is

@@ -1,9 +1,12 @@
 // Parameter blocks shared by every Shack-Hartmann frame kernel (wfs_kernels.cuh, wfs_mma.cuh, wfs_tma.cuh,
-// wfs_umma.cuh): one turbulence layer as the raytrace sees it, and the per-frame sensor / mirror description.
+// wfs_umma.cuh) and the per-pixel pupil kernels (pupil_kernels.cuh): one turbulence layer as the raytrace sees it, and
+// the per-frame sensor / mirror description.
 #pragma once
 #include <stdint.h>
 #include "../../include/aomarl.h"
 #include "wind_host.h"
+
+#define WFS_NG_MAX 6   // actuator lattice cells per side that can reach a 16-pixel subaperture (checked in aom_create)
 
 struct WfsLayer {
   const float* screen;   // [E][N][N]
@@ -64,6 +67,13 @@ __device__ __forceinline__ WindRec wind_of(const WfsParams& p, int l, int e) {
   WindRec r;
   r.ix = L.ix; r.iy = L.iy; r.fx = L.fx; r.fy = L.fy; r.w00 = L.w00; r.w01 = L.w01; r.w10 = L.w10; r.w11 = L.w11;
   return r;
+}
+
+// one bilinear row tap of a screen: row prow between columns pc0 and pc1 at fraction fx
+__device__ __forceinline__ float wfs_layer_row(const float* scr, int N, int prow, int pc0, int pc1, float fx) {
+  const float* r = scr + (size_t)prow * N;
+  float a = __ldg(r + pc0), b = __ldg(r + pc1);
+  return a + fx * (b - a);
 }
 
 // noise frame of environment e: its frames count from its own reset once environments are staggered

@@ -29,6 +29,7 @@
 #include <cuda.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
+#include "device_common.cuh"
 #include "wfs_mma.cuh"
 #include "wfs_lattice_host.h"
 
@@ -40,7 +41,6 @@
 #define WFT_TILE_STRIDE 1664                                  // 13 x 128: TMA destinations stay 128-byte aligned
 #define WFT_NG WFL_NG
 #define WFT_MAX_LAYERS WFL_MAX_LAYERS
-#define WFT_WAIT_SPINS (1u << 22)
 
 struct WfsFast {
   const uint2* sub;          // [nvalid] {y0 << 16 | x0, padded-lattice index of the neighbourhood origin}
@@ -60,27 +60,6 @@ struct WfsTmaParams {
   WfsFast f;
   CUtensorMap maps[WFT_MAX_LAYERS];
 };
-
-__device__ __forceinline__ uint32_t wft_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ bool wft_mbar_wait(uint32_t bar, uint32_t parity, int* err) {
-  for (uint32_t it = 0; it < WFT_WAIT_SPINS; ++it) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    if (ok) return true;
-  }
-  // an expired wait would let the warp read a stage that was never filled: raise the error word and stop the kernel
-  atomicExch(err, 2);
-  __threadfence_system();
-  __trap();
-  return false;
-}
 
 __device__ __forceinline__ void wft_tma_load_3d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, uint32_t bar) {
   asm volatile(
