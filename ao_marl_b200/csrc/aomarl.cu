@@ -9,9 +9,10 @@
 
 #include "../../include/aomarl.h"
 #include "dispatch.h"
-#include "atmos_kernels.cuh"
-#include "gemm_kernels.cuh"
-#include "gemm_tc.cuh"
+#include "dalloc.h"
+#include "atmos_host.h"
+#include "gemm_host.h"
+#include "gemm_tc_host.h"
 #include "rtc_kernels.cuh"
 #include "snapshot_kernels.cuh"
 #include "pupil_kernels.cuh"
@@ -24,15 +25,6 @@
 
 static char g_create_error[512] = "";
 
-// One per-episode condition (aom_condition): the common value, and while per-environment values are in force their
-// device array [E] and its host copy (both null otherwise).  Host readers take at(e); kernels take dev or common.
-struct EnvCond {
-  float common;
-  float* dev;
-  float* host;
-  float at(int e) const { return host ? host[e] : common; }
-};
-
 struct aom_ctx {
   aom_config cfg;
   char err[512];
@@ -42,40 +34,13 @@ struct aom_ctx {
   // tables
   void* tab[AOM_T_COUNT][AOM_MAX_LAYERS];
   size_t tab_bytes[AOM_T_COUNT][AOM_MAX_LAYERS];
-  // atmosphere
-  float* screen[AOM_MAX_LAYERS];
-  int* ox[AOM_MAX_LAYERS];
-  int* oy[AOM_MAX_LAYERS];
-  uint32_t* ext_count[AOM_MAX_LAYERS];
-  double accx[AOM_MAX_LAYERS], accy[AOM_MAX_LAYERS];
-  // per-environment winds (aom_set_layer_wind).  While wind_pe is set every layer keeps one accumulator per environment
-  // on the device (wind_state_kernel) and in a host mirror that only sizes the extrusion passes; the extrusion and
-  // sampling kernels run their per-environment instantiations.  Otherwise accx / accy above hold the state.
-  bool wind_pe;
-  double* wind_acc;            // device [L][2][E] accumulators (x, y)
-  int* wind_steps;             // device [L][2][E] whole-pixel counts of the last frame (x, y)
-  WindRec* wind_rec;           // device [L][E] offsets for the samplers
-  double* wind_hacc;           // host mirror of wind_acc
-  int wind_passes[AOM_MAX_LAYERS][2];   // extrusion passes of the last frame: max over the batch of |count| (x, y)
-  int wind_box[AOM_MAX_LAYERS][4];      // min / max over the batch of ix, then of iy (pupil footprint check)
-  uint32_t *k0, *k1;
-  float *Z, *zref, *newcol;
-  int ldz_max, ldn_max;
-  // exact integer extrusion (extrude_i8.cuh): operator digit planes per layer, environment digit planes, row scales
-  uint8_t* oz_ab[AOM_MAX_LAYERS];
-  int* oz_ea[AOM_MAX_LAYERS];
-  int oz_kb[AOM_MAX_LAYERS], oz_nt[AOM_MAX_LAYERS];
-  uint8_t* oz_zs;
-  int* oz_ev;
-  size_t oz_zs_bytes;
-  // the same integer contraction for the controller's operator products (cmat, v2m, m2v): operator digit planes per
-  // table, scratch digit planes of the per-environment vectors (main stream; the extrusion has its own on the side stream)
-  uint8_t* ozop[AOM_T_COUNT];
-  int* ozop_ea[AOM_T_COUNT];
-  int ozop_kb[AOM_T_COUNT], ozop_nt[AOM_T_COUNT];
-  uint8_t* oz_xs;
-  int* oz_xev;
-  size_t oz_xs_bytes;
+  // the turbulence layers: screens, wind state, extrusion (atmos.cu)
+  Atmos* atmos;
+  uint32_t *k0, *k1;          // device [E] Philox keys (environment seeds)
+  // the integer contraction (extrude_i8.cuh) of the controller's operator products (cmat, v2m, m2v): operator digit
+  // planes per table, and the scratch of the main stream (the extrusion has its own on the side stream)
+  OzOperator ozop[AOM_T_COUNT];
+  OzScratch oz;
   // actor weights as pre-split TF32 hi / lo planes in the tile order of gemm_tc_kernel (W1, W2, WH), floats per agent
   float* actor_bt[3];
   size_t actor_bt_per[3];
@@ -125,10 +90,9 @@ struct aom_ctx {
   uint32_t* step_env;          // device [E] actor decision counters
   int* le_n;                   // device [2][E] long-exposure counts (main target, geometric target)
   int* first;                  // device [E] first step pending
-  // snapshots (aom_save_envs / aom_load_envs): device list of environments and loaded wind accumulators [L][2][n], and
-  // the host staging block they are copied from (kept until the stream has passed the copy)
+  // snapshots (aom_save_envs / aom_load_envs): device list of environments, and the host staging block it is copied
+  // from (kept until the stream has passed the copy)
   int* snap_envs;
-  double* snap_acc;
   void* snap_h;
   size_t snap_h_bytes;
   // the sensor frame's kernel routing and the derived tables of its staged kernels (wfs_frame.cu)
@@ -163,24 +127,6 @@ static int fail(aom_ctx* c, int code, const char* fmt, ...) {
     if (_e != cudaSuccess)                                                                        \
       return fail(ctx, AOM_ERR_CUDA, "kernel launch failed: %s (%s:%d)", cudaGetErrorString(_e), __FILE__, __LINE__); \
   } while (0)
-
-template <typename T>
-static cudaError_t dalloc(T** p, size_t count) {
-  cudaError_t e = cudaMalloc((void**)p, count * sizeof(T));
-  if (e == cudaSuccess) e = cudaMemset(*p, 0, count * sizeof(T));
-  // the fill runs on the legacy stream, the buffer may be used next on a non-blocking one: finish it here
-  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
-  return e;
-}
-
-// Kernels launched with more dynamic shared memory than the default: f(kernel, bytes, its template arguments) for every
-// instantiation.  aom_create sets the attribute of each and the launch sites launch from the same lists.
-template <class F>
-static void gemm_tc_each(F&& f) {     // tcgen05 GEMM: epilogue, column tile
-  each<0, 1, 2>([&](auto EPI) {
-    each<GTC_BN, GTC_BN_WIDE>([&](auto BN) { f(gemm_tc_kernel<EPI, BN>, (size_t)GTC_SMEM_BYTES_T(BN), EPI, BN); });
-  });
-}
 
 extern "C" size_t aom_config_size(void) { return sizeof(aom_config); }
 
@@ -237,23 +183,12 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   ctx->lds = AOM_LD(cfg->nslopes);
   ctx->lda = AOM_LD(cfg->nactu);
   ctx->ldm = AOM_LD(cfg->nmodes > 0 ? cfg->nmodes : 1);
-  for (int l = 0; l < cfg->n_layers; ++l) {
-    size_t N = cfg->screen_dim[l];
-    CU(dalloc(&ctx->screen[l], E * N * N));
-    CU(dalloc(&ctx->ox[l], E));
-    CU(dalloc(&ctx->oy[l], E));
-    CU(dalloc(&ctx->ext_count[l], E));
-    int ldz = AOM_LD(cfg->stencil_size[l] + (int)N);
-    if (ldz > ctx->ldz_max) ctx->ldz_max = ldz;
-    if (AOM_LD((int)N) > ctx->ldn_max) ctx->ldn_max = AOM_LD((int)N);
-  }
   CU(dalloc(&ctx->k0, E));
   CU(dalloc(&ctx->k1, E));
-  if (cfg->n_layers > 0) {
-    CU(dalloc(&ctx->Z, E * ctx->ldz_max));
-    CU(dalloc(&ctx->zref, E));
-    CU(dalloc(&ctx->newcol, E * ctx->ldn_max));
-  }
+  CU(dalloc(&ctx->d_err, 1));
+  const AtmosLinks links = {ctx->cond, ctx->tab, ctx->opt, ctx->k0, ctx->k1, ctx->d_err, &ctx->launches, ctx->num_sms};
+  int rc = atmos_create(ctx->cfg, links, &ctx->atmos, ctx->err);
+  if (rc) return rc;
   CU(dalloc(&ctx->slopes_frame, E * ctx->lds));
   CU(dalloc(&ctx->slopes, E * ctx->lds));
   CU(dalloc(&ctx->err_v, E * ctx->lda));
@@ -291,17 +226,14 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
     CU(dalloc(&ctx->aH2, A * E * ctx->ld_ah));
     CU(dalloc(&ctx->aHO, A * E * ctx->ld_aho));
   }
-  CU(dalloc(&ctx->d_err, 1));
-  ctx->wfs = wfs_frame_create(ctx->cfg, ctx->screen, ctx->d_err, ctx->num_sms);
+  float* screens[AOM_MAX_LAYERS] = {};
+  for (int l = 0; l < cfg->n_layers; ++l) screens[l] = atmos_layer(ctx->atmos, l).screen;
+  ctx->wfs = wfs_frame_create(ctx->cfg, screens, ctx->d_err, ctx->num_sms);
   if (!ctx->wfs) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
   CU(cudaStreamCreateWithFlags(&ctx->side_stream, cudaStreamNonBlocking));
   CU(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
   CU(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
-  cudaError_t ae = cudaSuccess;
-  auto smem_attr = [&](auto kernel, size_t smem, auto...) {
-    if (ae == cudaSuccess) ae = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  };
-  gemm_tc_each(smem_attr);
+  cudaError_t ae = gemm_init();
   if (ae != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "cudaFuncSetAttribute(dynamic shared memory) failed: %s", cudaGetErrorString(ae));
   return AOM_OK;
 }
@@ -310,22 +242,19 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
   if (!ctx) return;
   for (int t = 0; t < AOM_T_COUNT; ++t)
     for (int l = 0; l < AOM_MAX_LAYERS; ++l) cudaFree(ctx->tab[t][l]);
-  for (int l = 0; l < AOM_MAX_LAYERS; ++l) {
-    cudaFree(ctx->screen[l]); cudaFree(ctx->ox[l]); cudaFree(ctx->oy[l]); cudaFree(ctx->ext_count[l]);
+  for (int l = 0; l < AOM_MAX_LAYERS; ++l)
     for (int k = 0; k < AOM_COND_COUNT; ++k) { cudaFree(ctx->cond[k][l].dev); free(ctx->cond[k][l].host); }
-  }
-  cudaFree(ctx->wind_acc); cudaFree(ctx->wind_steps); cudaFree(ctx->wind_rec); free(ctx->wind_hacc);
-  void* bufs[] = {ctx->k0, ctx->k1, ctx->Z, ctx->zref, ctx->newcol, ctx->slopes_frame, ctx->slopes, ctx->err_v,
+  atmos_destroy(ctx->atmos);
+  void* bufs[] = {ctx->k0, ctx->k1, ctx->slopes_frame, ctx->slopes, ctx->err_v,
                   ctx->com, ctx->com1, ctx->volts, ctx->com_before, ctx->bincube, ctx->phase, ctx->modes,
                   ctx->modes_before, ctx->modes_res, ctx->state, ctx->hist, ctx->reward, ctx->action,
                   ctx->action_mean, ctx->strehl, ctx->tar_mom, ctx->tar_acc, ctx->aX, ctx->aH1, ctx->aH2, ctx->aHO, ctx->d_err,
                   ctx->geo_com, ctx->geo_volts, ctx->geo_b, ctx->geo_T, ctx->strehl_geo, ctx->geo_acc, ctx->geo_mom,
                   ctx->sweep_mask, ctx->sweep_ttp, ctx->rs_envs, ctx->rs_seeds, ctx->frame0, ctx->step_env,
-                  ctx->le_n, ctx->first, ctx->snap_envs, ctx->snap_acc};
+                  ctx->le_n, ctx->first, ctx->snap_envs};
   for (void* b : bufs) cudaFree(b);
-  for (int l = 0; l < AOM_MAX_LAYERS; ++l) { cudaFree(ctx->oz_ab[l]); cudaFree(ctx->oz_ea[l]); }
-  for (int t = 0; t < AOM_T_COUNT; ++t) { cudaFree(ctx->ozop[t]); cudaFree(ctx->ozop_ea[t]); }
-  cudaFree(ctx->oz_zs); cudaFree(ctx->oz_ev); cudaFree(ctx->oz_xs); cudaFree(ctx->oz_xev);
+  for (int t = 0; t < AOM_T_COUNT; ++t) oz_operator_free(ctx->ozop[t]);
+  oz_scratch_free(ctx->oz);
   for (int i = 0; i < 3; ++i) cudaFree(ctx->actor_bt[i]);
   wfs_frame_destroy(ctx->wfs);
   for (int i = 0; i < AOM_WFS_TIMERS; ++i)
@@ -374,28 +303,6 @@ static size_t table_expected_bytes(const aom_ctx* ctx, int t, int index) {
   return 0;
 }
 
-// digit planes of an operator [rows][ld] (K valid columns) for the integer contraction (extrude_i8.cuh)
-static int oz_upload_operator(aom_ctx* ctx, const float* host, int rows, int ld, int K, uint8_t** planes_d, int** ea_d,
-                              int* kb_out, int* nt_out) {
-  if (!oz_operator_finite(host, rows, ld, K)) return fail(ctx, AOM_ERR_INVALID, "operator table holds a NaN or an infinity");
-  const int KB = (K + OZ_BK - 1) / OZ_BK, NT = (rows + OZ_BN - 1) / OZ_BN;
-  const size_t bytes = (size_t)NT * KB * OZ_SLICES_B * OZ_B_TILE;
-  uint8_t* planes = (uint8_t*)calloc(bytes, 1);
-  int* ea = (int*)calloc((size_t)NT * OZ_BN, sizeof(int));
-  if (!planes || !ea) { free(planes); free(ea); return fail(ctx, AOM_ERR_INVALID, "out of host memory"); }
-  oz_slice_operator(host, rows, ld, K, KB, NT, planes, ea);
-  cudaFree(*planes_d); cudaFree(*ea_d);
-  *planes_d = nullptr; *ea_d = nullptr;
-  cudaError_t e = cudaMalloc((void**)planes_d, bytes);
-  if (e == cudaSuccess) e = cudaMalloc((void**)ea_d, (size_t)NT * OZ_BN * sizeof(int));
-  if (e == cudaSuccess) e = cudaMemcpy(*planes_d, planes, bytes, cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(*ea_d, ea, (size_t)NT * OZ_BN * sizeof(int), cudaMemcpyHostToDevice);
-  free(planes); free(ea);
-  if (e != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "operator digit planes: %s", cudaGetErrorString(e));
-  *kb_out = KB; *nt_out = NT;
-  return AOM_OK;
-}
-
 extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* host, size_t nbytes) {
   if (!ctx || !host) return fail(ctx, AOM_ERR_INVALID, "null argument");
   if (table < 0 || table >= AOM_T_COUNT || index < 0 || index >= AOM_MAX_LAYERS)
@@ -404,21 +311,14 @@ extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* hos
   if (want != nbytes)
     return fail(ctx, AOM_ERR_INVALID, "Dimension mismatch: table %d[%d] expects %zu bytes, got %zu", table, index, want, nbytes);
   // operators of the integer contraction first: a non-finite one is refused before anything changes
-  if (table == AOM_T_AB) {
-    // digit planes of [A | B] for the exact integer extrusion
-    const aom_config& c = ctx->cfg;
-    const int N = c.screen_dim[index], K = c.stencil_size[index] + N;
-    int rc = oz_upload_operator(ctx, (const float*)host, N, AOM_LD(K), K, &ctx->oz_ab[index], &ctx->oz_ea[index],
-                                &ctx->oz_kb[index], &ctx->oz_nt[index]);
-    if (rc) return rc;
-  }
+  int rc = atmos_set_table(ctx->atmos, table, index, host, ctx->err);
+  if (rc) return rc;
   if (table == AOM_T_CMAT || table == AOM_T_V2M || table == AOM_T_M2V) {
     // digit planes of the controller operators for the exact integer products
     const aom_config& c = ctx->cfg;
     const int rows = table == AOM_T_V2M ? c.nmodes : c.nactu;
     const int K = table == AOM_T_CMAT ? c.nslopes : table == AOM_T_V2M ? c.nactu : c.nmodes;
-    int rc = oz_upload_operator(ctx, (const float*)host, rows, AOM_LD(K), K, &ctx->ozop[table], &ctx->ozop_ea[table],
-                                &ctx->ozop_kb[table], &ctx->ozop_nt[table]);
+    rc = oz_operator_upload(ctx->ozop[table], (const float*)host, rows, AOM_LD(K), K, ctx->err);
     if (rc) return rc;
   }
   if (ctx->tab[table][index]) { cudaFree(ctx->tab[table][index]); ctx->tab[table][index] = nullptr; }
@@ -555,16 +455,16 @@ extern "C" int aom_get_buffer(aom_ctx* ctx, int buffer, int index, void** dptr, 
   switch (buffer) {
     case AOM_B_SCREEN:
       if (index < 0 || index >= c.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
-      p = ctx->screen[index]; n = E * c.screen_dim[index] * c.screen_dim[index]; break;
+      p = atmos_layer(ctx->atmos, index).screen; n = E * c.screen_dim[index] * c.screen_dim[index]; break;
     case AOM_B_RING_OX:
       if (index < 0 || index >= c.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
-      p = ctx->ox[index]; n = E; break;
+      p = atmos_layer(ctx->atmos, index).ox; n = E; break;
     case AOM_B_RING_OY:
       if (index < 0 || index >= c.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
-      p = ctx->oy[index]; n = E; break;
+      p = atmos_layer(ctx->atmos, index).oy; n = E; break;
     case AOM_B_EXT_COUNT:
       if (index < 0 || index >= c.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
-      p = ctx->ext_count[index]; n = E; break;
+      p = atmos_layer(ctx->atmos, index).count; n = E; break;
     case AOM_B_SLOPES: p = ctx->slopes; n = E * ctx->lds; break;
     case AOM_B_ERR: p = ctx->err_v; n = E * ctx->lda; break;
     case AOM_B_COM: p = ctx->com; n = E * ctx->lda; break;
@@ -604,49 +504,15 @@ static int launch_gemm(aom_ctx* ctx, int epi, const float* A, int lda, long long
                        bool exact = false, const float* Bt = nullptr, long long sBt = 0) {
   GemmParams p;
   memset(&p, 0, sizeof(p));
-  int Kp = AOM_LD(K);
-  if (lda < Kp || ldb < Kp || (lda & 3) || (ldb & 3) || (ldc & 3) || ldc < N)
-    return fail(ctx, AOM_ERR_INVALID, "gemm: leading dimensions must cover K rounded to 16 (lda %d ldb %d ldc %d K %d N %d)", lda, ldb, ldc, K, N);
   p.A = A; p.B = B; p.C = C; p.bias = bias;
-  p.lda = lda; p.ldb = ldb; p.ldc = ldc; p.M = M; p.N = N; p.K = Kp;
+  p.lda = lda; p.ldb = ldb; p.ldc = ldc; p.M = M; p.N = N; p.K = K;
   p.sA = sA; p.sB = sB; p.sC = sC; p.sBias = sBias; p.relu = relu;
   p.com = com; p.ldcom = ldcom; p.gain = ctx->cond[AOM_COND_GAIN][0].common; p.closed = ctx->closed;
   p.Bt = Bt; p.sBt = sBt;
   const float* gain_env = ctx->cond[AOM_COND_GAIN][0].dev;
   if (epi == 1 && gain_env) { epi = 2; p.gain_env = gain_env; }   // integrator with one gain per environment
-  // `exact`: float32 FFMA accumulation with round-to-nearest (the recursive screen extrusion needs it: the
-  // tensor core truncates its float32 accumulator, a ~1e-5 systematic shrink that an autoregression integrates)
-  if (!exact && ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT) {
-    // column tile: the wide one when it saves CTA waves (two CTAs per SM)
-    const long long slots = 2LL * ctx->num_sms, rows = (M + GTC_BM - 1) / GTC_BM;
-    auto waves = [&](int bn) { return (double)((rows * ((ldc + bn - 1) / bn) * batch + slots - 1) / slots) * bn; };
-    const int bn = (!Bt && waves(GTC_BN_WIDE) < waves(GTC_BN)) ? GTC_BN_WIDE : GTC_BN;
-    const dim3 grid((ldc + bn - 1) / bn, (unsigned)rows, batch);
-    gemm_tc_each([&](auto kernel, size_t smem, int e, int b) {
-      if (e == epi && b == bn) kernel<<<grid, GTC_THREADS, smem, st>>>(p, ctx->d_err);
-    });
-  } else if (exact && epi == 0 && batch == 1 && !bias && !relu && ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT) {
-    // shaped exact kernel: column tile 8 CN with the least padding.  Only columns < N are consumed by the
-    // extrusion scatter; pad columns inside the last tile are written as zeros, the rest keep their zeros.
-    int best = 9, waste = 1 << 30;
-    for (int cn = 9; cn >= 8; --cn) {
-      const int bn = 8 * cn, w = (N + bn - 1) / bn * bn - N;
-      if (w < waste) { waste = w; best = cn; }
-    }
-    const int bn = 8 * best;
-    // two K halves per tile when the tiles alone leave the SMs at two CTAs (8 warps) each
-    const int tiles = ((N + bn - 1) / bn) * ((M + GEMM_BM - 1) / GEMM_BM);
-    const int ksplit = (tiles <= 2 * ctx->num_sms && K >= 512) ? 2 : 1;
-    if (ksplit > 1) {
-      cudaError_t e = cudaMemsetAsync(C, 0, (size_t)M * ldc * sizeof(float), st);
-      if (e != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "cudaMemsetAsync: %s", cudaGetErrorString(e));
-    }
-    dim3 grid((N + bn - 1) / bn, (M + GEMM_BM - 1) / GEMM_BM, ksplit);
-    with<8, 9>(best, [&](auto CN) { gemm_tn_exact_kernel<CN><<<grid, 128, 0, st>>>(p); });
-  } else {
-    dim3 grid((ldc + GEMM_BN - 1) / GEMM_BN, (M + GEMM_BM - 1) / GEMM_BM, batch);
-    with<0, 1, 2>(epi, [&](auto EPI) { gemm_tn_kernel<EPI><<<grid, 256, 0, st>>>(p); });
-  }
+  int rc = gemm_launch(p, epi, batch, exact, ctx->opt[AOM_OPT_GEMM_PATH], ctx->num_sms, ctx->d_err, st, ctx->err);
+  if (rc) return rc;
   KCHECK();
   return AOM_OK;
 }
@@ -656,23 +522,17 @@ static int launch_gemm(aom_ctx* ctx, int epi, const float* A, int lda, long long
 static int launch_oz_product(aom_ctx* ctx, int op, const float* X, int ldx, int K, float* out, int ldo, int N, int integrator,
                              float* com, int ldcom, cudaStream_t st) {
   const aom_config& c = ctx->cfg;
-  const int KB = ctx->ozop_kb[op], NT = ctx->ozop_nt[op], MT = (c.n_env + OZ_BM - 1) / OZ_BM;
-  const size_t need = (size_t)MT * KB * OZ_SLICES * OZ_A_TILE;
-  if (need > ctx->oz_xs_bytes) {
-    cudaFree(ctx->oz_xs); ctx->oz_xs = nullptr; ctx->oz_xs_bytes = 0;
-    CU(cudaMalloc((void**)&ctx->oz_xs, need));
-    CU(cudaMemsetAsync(ctx->oz_xs, 0, need, st));
-    ctx->oz_xs_bytes = need;
-  }
-  if (!ctx->oz_xev) CU(dalloc(&ctx->oz_xev, (size_t)c.n_env));
+  const OzOperator& P = ctx->ozop[op];
+  const int MT = (c.n_env + OZ_BM - 1) / OZ_BM;
+  CU(oz_scratch_reserve(ctx->oz, MT, P.kb, c.n_env, st));
   OzSliceParams sl;
-  sl.X = X; sl.ld = ldx; sl.K = K; sl.E = c.n_env; sl.KB = KB; sl.Zs = ctx->oz_xs; sl.ev = ctx->oz_xev;
+  sl.X = X; sl.ld = ldx; sl.K = K; sl.E = c.n_env; sl.KB = P.kb; sl.Zs = ctx->oz.zs; sl.ev = ctx->oz.ev;
   OzGemmParams m;
   memset(&m, 0, sizeof(m));
-  m.Zs = ctx->oz_xs; m.ABs = ctx->ozop[op]; m.ev = ctx->oz_xev; m.ea = ctx->ozop_ea[op]; m.out = out; m.ldo = ldo;
-  m.E = c.n_env; m.N = N; m.KB = KB; m.com = com; m.ldcom = ldcom; m.closed = ctx->closed; m.err = ctx->d_err;
+  m.Zs = ctx->oz.zs; m.ABs = P.planes; m.ev = ctx->oz.ev; m.ea = P.ea; m.out = out; m.ldo = ldo;
+  m.E = c.n_env; m.N = N; m.KB = P.kb; m.com = com; m.ldcom = ldcom; m.closed = ctx->closed; m.err = ctx->d_err;
   m.gain = ctx->cond[AOM_COND_GAIN][0].common; m.gain_env = integrator ? ctx->cond[AOM_COND_GAIN][0].dev : nullptr;
-  cudaError_t le = oz_product_launch(sl, m, integrator, MT, NT, st);
+  cudaError_t le = oz_product_launch(sl, m, integrator, MT, P.nt, st);
   if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "oz_product_launch: %s", cudaGetErrorString(le));
   ctx->launches += 2;
   return AOM_OK;
@@ -682,61 +542,6 @@ extern "C" int aom_gemm_tn(aom_ctx* ctx, const float* A, int lda, const float* B
                            int M, int N, int K, const float* bias, int relu, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
   return launch_gemm(ctx, 0, A, lda, 0, B, ldb, 0, C, ldc, 0, M, N, K, bias, 0, relu, 1, (cudaStream_t)stream);
-}
-
-// ---------------------------------------------------------------------------------------------
-// steps != null: per-environment winds -- pass `pass` of the signed counts steps [E] of this axis (`sign` unused).
-// envs != null: only the K environments envs[0..K) (device), compacted into the first K rows of the scratch and the
-// contraction (the start-up of aom_reset_envs).
-static int extrude_once(aom_ctx* ctx, int l, int axis, int sign, cudaStream_t st, const int* steps = nullptr, int pass = 0,
-                        const int* envs = nullptr, int K = 0) {
-  const aom_config& c = ctx->cfg;
-  const int rows = envs ? K : c.n_env;
-  NEED(AOM_T_AB, l);
-  NEED(AOM_T_STENCIL, l);
-  ExtrudeParams p;
-  p.screen = ctx->screen[l]; p.ox = ctx->ox[l]; p.oy = ctx->oy[l]; p.count = ctx->ext_count[l];
-  p.k0 = ctx->k0; p.k1 = ctx->k1; p.stencil = (const int*)ctx->tab[AOM_T_STENCIL][l];
-  p.N = c.screen_dim[l]; p.S = c.stencil_size[l]; p.E = c.n_env; p.layer = l; p.axis = axis; p.sign = sign;
-  p.amp = ctx->cond[AOM_COND_AMP][l].common; p.amp_env = ctx->cond[AOM_COND_AMP][l].dev;
-  p.ldz = AOM_LD(p.S + p.N); p.Z = ctx->Z; p.zref = ctx->zref; p.ldn = AOM_LD(p.N); p.newcol = ctx->newcol;
-  p.steps = steps; p.pass = pass; p.envs = envs;
-  if (ctx->opt[AOM_OPT_EXTRUDE_PATH] == AOM_EXTRUDE_I8) {
-    // exact integer contraction on tcgen05 (extrude_i8.cuh): digits of the inputs, 13 int8 digit-pair products with
-    // int32 accumulators, one rounding to float32 after adding the reference pixel
-    const int KB = ctx->oz_kb[l], NT = ctx->oz_nt[l], MT = (rows + OZ_BM - 1) / OZ_BM;
-    const size_t need = (size_t)MT * KB * OZ_SLICES * OZ_A_TILE;
-    if (need > ctx->oz_zs_bytes) {
-      cudaFree(ctx->oz_zs); ctx->oz_zs = nullptr; ctx->oz_zs_bytes = 0;
-      CU(cudaMalloc((void**)&ctx->oz_zs, need));
-      CU(cudaMemsetAsync(ctx->oz_zs, 0, need, st));      // on the consuming stream: a default-stream memset does not order with it
-      ctx->oz_zs_bytes = need;
-    }
-    if (!ctx->oz_ev) CU(dalloc(&ctx->oz_ev, (size_t)c.n_env));
-    uint8_t* zs = ctx->oz_zs;
-    int* ev = ctx->oz_ev;
-    OzGatherParams g;
-    g.screen = p.screen; g.ox = p.ox; g.oy = p.oy; g.count = p.count; g.k0 = p.k0; g.k1 = p.k1; g.stencil = p.stencil;
-    g.zref = p.zref; g.ev = ev; g.Zs = zs; g.N = p.N; g.S = p.S; g.E = rows; g.KB = KB; g.layer = l;
-    g.axis = axis; g.sign = sign; g.amp = p.amp; g.amp_env = p.amp_env;
-    g.steps = steps; g.pass = pass; g.envs = envs;
-    OzGemmParams m;
-    m.Zs = zs; m.ABs = ctx->oz_ab[l]; m.ev = ev; m.ea = ctx->oz_ea[l]; m.zref = p.zref;
-    m.out = p.newcol; m.ldo = p.ldn; m.E = rows; m.N = p.N; m.KB = KB; m.err = ctx->d_err;
-    cudaError_t le = oz_extrude_launch(g, m, MT, NT, st);
-    if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "oz_extrude_launch: %s", cudaGetErrorString(le));
-    ctx->launches += 2;
-    p.zref = nullptr;                                  // the reference pixel is already in the new column
-  } else {
-    with<false, true>(steps != nullptr, [&](auto PE) { extrude_gather_kernel<PE><<<rows, 256, 0, st>>>(p); });
-    KCHECK();
-    int rc = launch_gemm(ctx, 0, ctx->Z, p.ldz, 0, (const float*)ctx->tab[AOM_T_AB][l], p.ldz, 0, ctx->newcol, p.ldn, 0,
-                         rows, p.N, p.S + p.N, nullptr, 0, 0, 1, st, nullptr, 0, true);
-    if (rc) return rc;
-  }
-  with<false, true>(steps != nullptr, [&](auto PE) { extrude_scatter_kernel<PE><<<rows, EXTRUDE_SCATTER_THREADS, 0, st>>>(p); });
-  KCHECK();
-  return AOM_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -809,171 +614,17 @@ extern "C" int aom_get_condition(aom_ctx* ctx, int cond, int layer, float* commo
 }
 
 // ---------------------------------------------------------------------------------------------
-// per-environment winds
-static bool wind_any_env(const aom_ctx* ctx) {
-  for (int l = 0; l < ctx->cfg.n_layers; ++l)
-    if (ctx->cond[AOM_COND_WIND_X][l].host || ctx->cond[AOM_COND_WIND_Y][l].host) return true;
-  return false;
-}
-
-// One transition of the wind state of every layer and environment (WIND_STEP / WIND_INIT / WIND_RESET, atmos_kernels.cuh)
-// on the device, asynchronously on `st`, and the same on the host mirror: passes per layer and offset bounds.
-// WIND_RESET_ENVS: WIND_RESET of the K environments listed in envs_d (device) / envs_h (host) only.  WIND_LOAD_ENVS:
-// their accumulators <- acc_d (device) / acc_h (host), both [L][2][K].
-static int wind_update(aom_ctx* ctx, int mode, cudaStream_t st, const int* envs_d = nullptr, const int* envs_h = nullptr,
-                       int K = 0, const double* acc_d = nullptr, const double* acc_h = nullptr) {
-  const aom_config& c = ctx->cfg;
-  const int E = c.n_env, L = c.n_layers;
-  if (L == 0) return AOM_OK;
-  WindStateParams P;
-  memset(&P, 0, sizeof(P));
-  for (int l = 0; l < L; ++l) {
-    WindLayerParams& W = P.layer[l];
-    const EnvCond &wx = ctx->cond[AOM_COND_WIND_X][l], &wy = ctx->cond[AOM_COND_WIND_Y][l];
-    W.dx = wx.dev; W.dy = wy.dev; W.cdx = wx.common; W.cdy = wy.common;
-    W.ax0 = ctx->accx[l]; W.ay0 = ctx->accy[l]; W.xoff = c.wfs_xoff[l]; W.yoff = c.wfs_yoff[l]; W.n2 = 2 * c.screen_dim[l];
-  }
-  P.acc = ctx->wind_acc; P.steps = ctx->wind_steps; P.rec = ctx->wind_rec; P.E = E; P.n_layers = L; P.mode = mode;
-  P.envs = envs_d; P.K = K;
-  if (mode == WIND_LOAD_ENVS) {
-    WindLoadParams Q;
-    memset(&Q, 0, sizeof(Q));
-    for (int l = 0; l < L; ++l) { Q.xoff[l] = c.wfs_xoff[l]; Q.yoff[l] = c.wfs_yoff[l]; }
-    Q.acc = ctx->wind_acc; Q.steps = ctx->wind_steps; Q.rec = ctx->wind_rec; Q.envs = envs_d; Q.acc_in = acc_d;
-    Q.E = E; Q.K = K; Q.n_layers = L;
-    wind_load_kernel<<<(L * K + 255) / 256, 256, 0, st>>>(Q);
-  } else {
-    const int n = mode == WIND_RESET_ENVS ? K : E;
-    wind_state_kernel<<<(L * n + 255) / 256, 256, 0, st>>>(P);
-  }
-  KCHECK();
-  for (int l = 0; l < L; ++l) {
-    const WindLayerParams& W = P.layer[l];
-    double* ax = ctx->wind_hacc + (size_t)2 * l * E;
-    double* ay = ax + E;
-    int px = 0, py = 0;
-    int* box = ctx->wind_box[l];
-    if (mode == WIND_RESET_ENVS) {
-      for (int k = 0; k < K; ++k) ax[envs_h[k]] = ay[envs_h[k]] = 0.0;
-      py = W.n2;
-    }
-    if (mode == WIND_LOAD_ENVS)
-      for (int k = 0; k < K; ++k) {
-        ax[envs_h[k]] = acc_h[(size_t)2 * l * K + k];
-        ay[envs_h[k]] = acc_h[(size_t)(2 * l + 1) * K + k];
-      }
-    for (int e = 0; e < E; ++e) {
-      const float dx = ctx->cond[AOM_COND_WIND_X][l].at(e), dy = ctx->cond[AOM_COND_WIND_Y][l].at(e);
-      if (mode == WIND_STEP) {
-        const int nx = wind_advance(ax[e], dx), ny = wind_advance(ay[e], dy);
-        px = std::max(px, abs(nx)); py = std::max(py, abs(ny));
-      } else if (mode == WIND_INIT) {
-        ax[e] = W.ax0; ay[e] = W.ay0;
-      } else if (mode == WIND_RESET) {
-        ax[e] = ay[e] = 0.0;
-        py = W.n2;
-      }
-      const WindRec r = wind_record(W.xoff, W.yoff, ax[e], ay[e]);
-      if (e == 0 || r.ix < box[0]) box[0] = r.ix;
-      if (e == 0 || r.ix > box[1]) box[1] = r.ix;
-      if (e == 0 || r.iy < box[2]) box[2] = r.iy;
-      if (e == 0 || r.iy > box[3]) box[3] = r.iy;
-    }
-    ctx->wind_passes[l][0] = px; ctx->wind_passes[l][1] = py;
-  }
-  return AOM_OK;
-}
-
-// Back to the common accumulators once no layer has winds of its own and every layer's accumulators agree over the batch
-// (at the latest after the next aom_reset, which zeroes them): the uniform kernels then run again.
-static void wind_try_uniform(aom_ctx* ctx) {
-  if (!ctx->wind_pe || wind_any_env(ctx)) return;
-  const int E = ctx->cfg.n_env;
-  for (int l = 0; l < ctx->cfg.n_layers; ++l) {
-    const double* a = ctx->wind_hacc + (size_t)2 * l * E;
-    for (int e = 1; e < E; ++e)
-      if (a[e] != a[0] || a[E + e] != a[E]) return;
-  }
-  for (int l = 0; l < ctx->cfg.n_layers; ++l) {
-    ctx->accx[l] = ctx->wind_hacc[(size_t)2 * l * E];
-    ctx->accy[l] = ctx->wind_hacc[(size_t)(2 * l + 1) * E];
-  }
-  ctx->wind_pe = false;
-}
-
-// Per-environment wind state from the common one (WIND_INIT on `st`): every environment continues from the layer's
-// common accumulators.
-static int wind_begin_pe(aom_ctx* ctx, cudaStream_t st) {
-  const size_t LE = (size_t)ctx->cfg.n_layers * ctx->cfg.n_env;
-  if (!ctx->wind_acc) {
-    CU(dalloc(&ctx->wind_acc, 2 * LE));
-    CU(dalloc(&ctx->wind_steps, 2 * LE));
-    CU(cudaMalloc((void**)&ctx->wind_rec, LE * sizeof(WindRec)));
-    ctx->wind_hacc = (double*)calloc(2 * LE, sizeof(double));
-    if (!ctx->wind_hacc) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
-  }
-  int rc = wind_update(ctx, WIND_INIT, st);
-  if (rc) return rc;
-  ctx->wind_pe = true;
-  return AOM_OK;
-}
-
-// After a change of the per-environment winds of `layer`: the uniform state when it can, else every environment continues
-// from the common accumulators (the screens do not jump), and its pupil footprint must stay on the screen.
-static int wind_settle(aom_ctx* ctx, int layer) {
-  const aom_config& c = ctx->cfg;
-  if (!ctx->cond[AOM_COND_WIND_X][layer].host) {
-    wind_try_uniform(ctx);
-    return AOM_OK;
-  }
-  if (!ctx->wind_pe) {
-    int rc = wind_begin_pe(ctx, 0);
-    if (rc) return rc;
-    CU(cudaStreamSynchronize(0));                    // the legacy stream: the state is read next on any stream
-  }
-  const int* b = ctx->wind_box[layer];
-  if (b[0] < 0 || b[2] < 0 || b[1] + c.n + 1 > c.screen_dim[layer] || b[3] + c.n + 1 > c.screen_dim[layer])
-    return fail(ctx, AOM_ERR_UNSUPPORTED, "layer %d: pupil footprint leaves the screen", layer);
-  return AOM_OK;
-}
-
 extern "C" int aom_set_layer_wind(aom_ctx* ctx, int layer, const float* deltax_host, const float* deltay_host) {
   if (!deltax_host != !deltay_host) return fail(ctx, AOM_ERR_INVALID, "per-environment winds need both components (or neither)");
   const CondSet s[2] = {{AOM_COND_WIND_X, layer, true, deltax_host}, {AOM_COND_WIND_Y, layer, true, deltay_host}};
   int rc = set_conditions(ctx, 2, s);
-  return rc ? rc : wind_settle(ctx, layer);
+  return rc ? rc : atmos_settle(ctx->atmos, layer, ctx->err);
 }
 
 extern "C" int aom_move_atmos(aom_ctx* ctx, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
   if (!ctx->seeded) return fail(ctx, AOM_ERR_STATE, "aom_reset must be called before aom_move_atmos");
-  cudaStream_t st = (cudaStream_t)stream;
-  const aom_config& c = ctx->cfg;
-  if (ctx->wind_pe) {
-    // per-environment winds: counts and offsets on the device, passes sized by the host mirror (x then y, as below);
-    // an environment takes part in the first |count| passes of each axis
-    int rc = wind_update(ctx, WIND_STEP, st);
-    if (rc) return rc;
-    const size_t E = c.n_env;
-    for (int l = 0; l < c.n_layers; ++l)
-      for (int a = 0; a < 2; ++a)
-        for (int i = 0; i < ctx->wind_passes[l][a]; ++i) {
-          rc = extrude_once(ctx, l, a, 1, st, ctx->wind_steps + (2 * l + a) * E, i);
-          if (rc) return rc;
-        }
-    wind_try_uniform(ctx);
-    return AOM_OK;
-  }
-  for (int l = 0; l < c.n_layers; ++l) {
-    ctx->accx[l] += (double)ctx->cond[AOM_COND_WIND_X][l].common;
-    ctx->accy[l] += (double)ctx->cond[AOM_COND_WIND_Y][l].common;
-    int nx = (int)ctx->accx[l], ny = (int)ctx->accy[l];
-    ctx->accx[l] -= nx;
-    ctx->accy[l] -= ny;
-    for (int i = 0; i < abs(nx); ++i) { int rc = extrude_once(ctx, l, 0, nx > 0 ? 1 : -1, st); if (rc) return rc; }
-    for (int i = 0; i < abs(ny); ++i) { int rc = extrude_once(ctx, l, 1, ny > 0 ? 1 : -1, st); if (rc) return rc; }
-  }
-  return AOM_OK;
+  return atmos_move(ctx->atmos, (cudaStream_t)stream, ctx->err);
 }
 
 static int clear_loop_state(aom_ctx* ctx, cudaStream_t st) {
@@ -1005,8 +656,6 @@ static int clear_loop_state(aom_ctx* ctx, cudaStream_t st) {
   return AOM_OK;
 }
 
-static int start_screens(aom_ctx* ctx, const int* envs, int K, cudaStream_t st);
-
 extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
   if (!ctx || !seeds) return fail(ctx, AOM_ERR_INVALID, "null argument");
   cudaStream_t st = (cudaStream_t)stream;
@@ -1036,51 +685,7 @@ extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
     CU(cudaMemsetAsync(ctx->le_n, 0, 2 * E * sizeof(int), st));
     CU(cudaMemsetAsync(ctx->first, 0, E * sizeof(int), st));
   }
-  for (int l = 0; l < c.n_layers; ++l) ctx->accx[l] = ctx->accy[l] = 0.0;
-  if (ctx->wind_pe && !wind_any_env(ctx)) ctx->wind_pe = false;      // every accumulator restarts from 0: common again
-  if (ctx->wind_pe) {
-    // per-environment winds: accumulators 0, start-up counts 2N along y signed like each environment's x wind
-    rc = wind_update(ctx, WIND_RESET, st);
-    if (rc) return rc;
-  }
-  for (int l = 0; l < c.n_layers; ++l) {
-    size_t N = c.screen_dim[l];
-    CU(cudaMemsetAsync(ctx->screen[l], 0, E * N * N * 4, st));
-    CU(cudaMemsetAsync(ctx->ox[l], 0, E * 4, st));
-    CU(cudaMemsetAsync(ctx->oy[l], 0, E * 4, st));
-    CU(cudaMemsetAsync(ctx->ext_count[l], 0, E * 4, st));
-  }
-  return start_screens(ctx, nullptr, 0, st);
-}
-
-// Start-up of the screens of every environment (envs null) or of the K environments envs[0..K) (device list, compacted
-// extrusions): zero screens, ring origins and counters are expected, and the wind state of WIND_RESET (WIND_RESET_ENVS).
-// (The layers' start-up chains are independent, but running them on separate streams with private scratch gained
-// nothing for the whole batch -- 1.35 s either way at 4096 environments: every extrusion kernel fills the GPU by itself.)
-static int start_screens(aom_ctx* ctx, const int* envs, int K, cudaStream_t st) {
-  const aom_config& c = ctx->cfg;
-  const size_t E = c.n_env;
-  const unsigned rows = envs ? (unsigned)K : (unsigned)E;
-  int rc;
-  for (int l = 0; l < c.n_layers; ++l) {
-    size_t N = c.screen_dim[l];
-    int sign = ctx->cond[AOM_COND_WIND_X][l].common < 0 ? -1 : 1;
-    const int* steps = ctx->wind_pe ? ctx->wind_steps + (2 * l + 1) * E : nullptr;
-    // The reference starts a screen with 2N extrusions along x (columns: 648 pixels in 648 different DRAM rows per
-    // environment, the expensive direction of the [y][x] layout -- 0.32 ms per extrusion at 4096 environments against
-    // 0.19 ms along y).  From a zero screen with zero ring offsets the recursion along y produces exactly the transpose
-    // (same stencil, same operator, same innovation counters; every index expression of the gather / scatter swaps its
-    // roles, atmos_kernels.cuh / extrude_i8.cuh), and 2N extrusions bring the ring origin back to zero: so the start-up
-    // runs along y and the screens are transposed in place once at the end -- bit-identical pixels, 1.29 -> 0.8 s.
-    for (size_t i = 0; i < 2 * N; ++i) { rc = extrude_once(ctx, l, 1, sign, st, steps, (int)i, envs, K); if (rc) return rc; }
-    {
-      const int T = (int)((N + 31) / 32);
-      transpose_screens_kernel<<<dim3((unsigned)(T * (T + 1) / 2), rows), dim3(32, 8), 0, st>>>(ctx->screen[l], (int)N, envs);
-      KCHECK();
-      // ring origin: 2N steps along y leave oy = 0 as 2N steps along x leave ox = 0 (2N mod N); nothing to swap
-    }
-  }
-  return AOM_OK;
+  return atmos_reset(ctx->atmos, st, ctx->err);
 }
 
 // Checks a host list of n environments of the batch: n >= 0, every index in range and listed once.
@@ -1144,8 +749,9 @@ static int env_rows(const aom_ctx* ctx, EnvRow* out) {
   add(ctx->hist, c.state_modes, 1, c.n_hist, E * c.state_modes, 1);      // every slot of the ring
   add(ctx->geo_com, ctx->lda); add(ctx->geo_volts, ctx->lda); add(ctx->geo_acc, TAR_ACC); add(ctx->strehl_geo, 4);
   for (int l = 0; l < c.n_layers; ++l) {
-    add(ctx->screen[l], (long long)c.screen_dim[l] * c.screen_dim[l]);
-    add(ctx->ox[l], 1); add(ctx->oy[l], 1); add(ctx->ext_count[l], 1);
+    const AtmosLayer a = atmos_layer(ctx->atmos, l);
+    add(a.screen, (long long)c.screen_dim[l] * c.screen_dim[l]);
+    add(a.ox, 1); add(a.oy, 1); add(a.count, 1);
   }
   add(ctx->k0, 1, 0); add(ctx->k1, 1, 0);
   add(ctx->tar_mom, 2 * PSW_MOM2, 0, 2, E * 2 * PSW_MOM2);                // doubles [2][E][PSW_MOM2]: both targets
@@ -1197,13 +803,7 @@ extern "C" int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const in
   reset_envs_kernel<<<dim3((unsigned)n, (unsigned)P.nbuf + 1), 256, 0, st>>>(P);
   KCHECK();
   ctx->first_any = true;
-  if (c.n_layers == 0) return AOM_OK;
-  // The listed environments' accumulators restart from 0 while the others keep theirs: the per-environment wind state
-  // (common winds included) until they agree again (wind_try_uniform)
-  if (!ctx->wind_pe) { rc = wind_begin_pe(ctx, st); if (rc) return rc; }
-  rc = wind_update(ctx, WIND_RESET_ENVS, st, ctx->rs_envs, envs, n);
-  if (rc) return rc;
-  return start_screens(ctx, ctx->rs_envs, n, st);
+  return atmos_reset_envs(ctx->atmos, ctx->rs_envs, envs, n, st, ctx->err);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1258,8 +858,7 @@ static void snap_params(aom_ctx* ctx, SnapParams& P, int n, void* rec) {
   P.magic = AOM_ENV_MAGIC; P.rec_bytes = (uint32_t)bytes; P.fingerprint = config_fingerprint(c); P.n_layers = c.n_layers;
   P.frame = ctx->frame; P.step = ctx->step; P.le_c[0] = ctx->tar_n; P.le_c[1] = ctx->geo_tar_n;
   if (ctx->staggered) { P.frame0 = ctx->frame0; P.step_env = ctx->step_env; P.le_n = ctx->le_n; P.first = ctx->first; }
-  P.wind_acc = ctx->wind_pe ? ctx->wind_acc : nullptr;
-  for (int l = 0; l < c.n_layers; ++l) { P.acc_c[l][0] = ctx->accx[l]; P.acc_c[l][1] = ctx->accy[l]; }
+  P.wind_acc = atmos_snap_view(ctx->atmos, P.acc_c);
   for (int k = 0; k < AOM_COND_COUNT; ++k)
     for (int l = 0; l < AOM_MAX_LAYERS; ++l) { P.cond_env[k][l] = ctx->cond[k][l].dev; P.cond_c[k][l] = ctx->cond[k][l].common; }
 }
@@ -1326,7 +925,7 @@ static int load_conditions(aom_ctx* ctx, int n, const int32_t* envs, aom_env_hea
   int rc = set_conditions(ctx, ns, s);
   free(a);
   for (int l = 0; l < L && !rc; ++l)
-    if (differ[AOM_COND_WIND_X][l]) rc = wind_settle(ctx, l);
+    if (differ[AOM_COND_WIND_X][l]) rc = atmos_settle(ctx->atmos, l, ctx->err);
   return rc;
 }
 
@@ -1368,32 +967,8 @@ extern "C" int aom_load_envs(aom_ctx* ctx, int n, const int32_t* envs, const voi
   env_unpack_kernel<<<dim3((unsigned)P.nchunks + 1, (unsigned)n), SNAP_THREADS, 0, st>>>(P);
   KCHECK();
   ctx->first_any = true;                             // a loaded environment may have its first step pending
-  if (L > 0) {
-    // wind accumulators: the per-environment state unless the loaded ones are the batch's common ones
-    bool differ = ctx->wind_pe;
-    for (int k = 0; k < n && !differ; ++k)
-      for (int l = 0; l < L; ++l) differ = differ || h[k].acc[l][0] != ctx->accx[l] || h[k].acc[l][1] != ctx->accy[l];
-    if (differ) {
-      if (!ctx->wind_pe) { rc = wind_begin_pe(ctx, st); if (rc) return rc; }
-      double* acc = (double*)(h + n);
-      for (int l = 0; l < L; ++l)
-        for (int k = 0; k < n; ++k) {
-          acc[(size_t)2 * l * n + k] = h[k].acc[l][0];
-          acc[(size_t)(2 * l + 1) * n + k] = h[k].acc[l][1];
-        }
-      if (!ctx->snap_acc) CU(dalloc(&ctx->snap_acc, (size_t)2 * L * c.n_env));
-      CU(cudaMemcpyAsync(ctx->snap_acc, acc, (size_t)2 * L * n * sizeof(double), cudaMemcpyHostToDevice, st));
-      rc = wind_update(ctx, WIND_LOAD_ENVS, st, ctx->snap_envs, envs, n, ctx->snap_acc, acc);
-      if (rc) return rc;
-      CU(cudaStreamSynchronize(st));
-      for (int l = 0; l < L; ++l) {
-        const int* bx = ctx->wind_box[l];
-        if (bx[0] < 0 || bx[2] < 0 || bx[1] + c.n + 1 > c.screen_dim[l] || bx[3] + c.n + 1 > c.screen_dim[l])
-          return fail(ctx, AOM_ERR_UNSUPPORTED, "layer %d: pupil footprint leaves the screen", l);
-      }
-      wind_try_uniform(ctx);
-    }
-  }
+  rc = atmos_load(ctx->atmos, n, ctx->snap_envs, envs, h, (double*)(h + n), st, ctx->err);
+  if (rc) return rc;
   CU(cudaStreamSynchronize(st));
   return AOM_OK;
 }
@@ -1404,17 +979,8 @@ static int fill_wfs_params(aom_ctx* ctx, WfsParams& p, int flags, float noise) {
   memset(&p, 0, sizeof(p));
   NEED(AOM_T_MPUPIL, 0); NEED(AOM_T_HALFXY, 0); NEED(AOM_T_SUB_X0, 0); NEED(AOM_T_SUB_Y0, 0); NEED(AOM_T_FLUX, 0);
   p.n_layers = (flags & 1) ? c.n_layers : 0;
-  for (int l = 0; l < p.n_layers; ++l) {
-    WfsLayer& L = p.layer[l];
-    L.screen = ctx->screen[l]; L.ox = ctx->ox[l]; L.oy = ctx->oy[l]; L.N = c.screen_dim[l];
-    const WindRec r = wind_record(c.wfs_xoff[l], c.wfs_yoff[l], ctx->accx[l], ctx->accy[l]);
-    L.ix = r.ix; L.iy = r.iy; L.fx = r.fx; L.fy = r.fy; L.w00 = r.w00; L.w01 = r.w01; L.w10 = r.w10; L.w11 = r.w11;
-    int box[4] = {L.ix, L.ix, L.iy, L.iy};          // with per-environment winds: the extremes over the batch
-    if (ctx->wind_pe) memcpy(box, ctx->wind_box[l], sizeof(box));
-    if (box[0] < 0 || box[2] < 0 || box[1] + c.n + 1 > L.N || box[3] + c.n + 1 > L.N)
-      return fail(ctx, AOM_ERR_UNSUPPORTED, "layer %d: pupil footprint leaves the screen", l);
-  }
-  p.wind = (ctx->wind_pe && p.n_layers > 0) ? ctx->wind_rec : nullptr;
+  int rc = atmos_fill_layers(ctx->atmos, p, ctx->err);
+  if (rc) return rc;
   p.use_dm = (flags & 2) ? 1 : 0;
   if (p.use_dm) {
     NEED(AOM_T_STAMP1D, 0); NEED(AOM_T_ACT_MAP, 0); NEED(AOM_T_TT_PLANES, 0);
@@ -1711,7 +1277,7 @@ extern "C" int aom_do_control(aom_ctx* ctx, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
   const aom_config& c = ctx->cfg;
   NEED(AOM_T_CMAT, 0);
-  if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_CMAT])
+  if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_CMAT].planes)
     return launch_oz_product(ctx, AOM_T_CMAT, ctx->slopes, ctx->lds, c.nslopes, ctx->err_v, ctx->lda, c.nactu, 1, ctx->com,
                              ctx->lda, (cudaStream_t)stream);
   return launch_gemm(ctx, 1, ctx->slopes, ctx->lds, 0, (const float*)ctx->tab[AOM_T_CMAT][0], ctx->lds, 0, ctx->err_v,
@@ -1819,7 +1385,7 @@ extern "C" int aom_reset_dm(aom_ctx* ctx, void* stream) {
 static int project_v2m(aom_ctx* ctx, const float* v, float* out, cudaStream_t st) {
   const aom_config& c = ctx->cfg;
   NEED(AOM_T_V2M, 0);
-  if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_V2M])
+  if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_V2M].planes)
     return launch_oz_product(ctx, AOM_T_V2M, v, ctx->lda, c.nactu, out, ctx->ldm, c.nmodes, 0, nullptr, 0, st);
   return launch_gemm(ctx, 0, v, ctx->lda, 0, (const float*)ctx->tab[AOM_T_V2M][0], ctx->lda, 0, out, ctx->ldm, 0, c.n_env,
                      c.nmodes, c.nactu, nullptr, 0, 0, 1, st);
@@ -1839,7 +1405,7 @@ extern "C" int aom_rl_control(aom_ctx* ctx, const float* daction, void* stream) 
                                              (const float*)ctx->tab[AOM_T_FREEDOM][0], c.action_dim, c.n_env,
                                              c.env_act_scale, c.env_act_bias, ctx->first_any ? ctx->first : nullptr);
   KCHECK();
-  if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_M2V])
+  if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_M2V].planes)
     return launch_oz_product(ctx, AOM_T_M2V, ctx->modes, ctx->ldm, c.nmodes, ctx->com, ctx->lda, c.nactu, 0, nullptr, 0, st);
   return launch_gemm(ctx, 0, ctx->modes, ctx->ldm, 0, (const float*)ctx->tab[AOM_T_M2V][0], ctx->ldm, 0, ctx->com, ctx->lda, 0,
                      c.n_env, c.nactu, c.nmodes, nullptr, 0, 0, 1, st);

@@ -174,26 +174,10 @@ __global__ void __launch_bounds__(256) transpose_screens_kernel(float* __restric
   }
 }
 
-// grid-stride fill helpers
-__global__ void fill_i32_kernel(int* p, int v, size_t n) {
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = v;
-}
-
 // Wind state of every layer and environment when the environments have their own winds: accumulators acc [L][2][E]
 // (x, y), whole-pixel counts of the frame steps [L][2][E] (x, y) and the samplers' offsets rec [L][E].  One thread per
 // (layer, environment), the arithmetic of wind_host.h (the host keeps a mirror of the accumulators with the same
-// functions to know how many extrusion passes to launch).
-#define WIND_STEP 0      // one frame of wind: acc += delta, counts = whole pixels
-#define WIND_INIT 1      // accumulators <- the layer's common ones (ax0, ay0), no extrusion
-#define WIND_RESET 2     // accumulators <- 0; counts of the start-up: 2N along y, signed like the environment's x wind
-#define WIND_RESET_ENVS 3  // WIND_RESET of the listed environments envs[0..K) only (aom_reset_envs); the others keep their state
-struct WindLayerParams {
-  const float* dx; const float* dy;      // [E] steps in pixels per frame, or null: the common cdx / cdy
-  float cdx, cdy;
-  double ax0, ay0;                       // WIND_INIT
-  float xoff, yoff;                      // sensor offsets of the layer (aom_config.wfs_xoff / wfs_yoff)
-  int n2;                                // WIND_RESET: 2 N
-};
+// functions, wind_mirror, to know how many extrusion passes to launch).  The modes are those of wind_host.h.
 struct WindStateParams {
   WindLayerParams layer[AOM_MAX_LAYERS];
   double* acc; int* steps; WindRec* rec;
@@ -231,7 +215,6 @@ __global__ void wind_state_kernel(const __grid_constant__ WindStateParams P) {
 
 // WIND_LOAD_ENVS (aom_load_envs): accumulators of the listed environments envs[0..K) <- acc_in [L][2][K], no extrusion.
 // One thread per (layer, listed environment); the others keep their state.
-#define WIND_LOAD_ENVS 4
 struct WindLoadParams {
   float xoff[AOM_MAX_LAYERS], yoff[AOM_MAX_LAYERS];
   double* acc; int* steps; WindRec* rec;

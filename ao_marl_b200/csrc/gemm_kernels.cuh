@@ -10,26 +10,12 @@
 // commands / rewards stay within rel 1e-4 of the oracle; the tcgen05 (3xTF32) version replaces it.
 #pragma once
 #include <cuda_runtime.h>
+#include "gemm_host.h"
 
 #define GEMM_BM 128
 #define GEMM_BN 128
 #define GEMM_BK 16
 #define GEMM_PAD 4
-
-struct GemmParams {
-  const float* A; const float* B; float* C; const float* bias;
-  int lda, ldb, ldc;
-  int M, N, K;          // K rounded up to a multiple of 16 by the caller (operands are zero padded)
-  long long sA, sB, sC, sBias;   // batch strides (elements)
-  int relu;
-  // epilogue 1 (integrator): err = -acc ; C = err ; com += gain * err
-  float* com; int ldcom; float gain; int closed;
-  // gemm_tc_kernel only: the B operand already split into TF32 hi / lo planes in the UMMA tile order of 128-column tiles
-  // ([n tile][k block][hi, lo][128 x 16]; gtc_pretile_host), brought in by one bulk copy per stage.  Null: B is split on the fly.
-  const float* Bt; long long sBt;
-  // epilogue 2: the integrator of epilogue 1 with one gain per row (environment): com += gain_env[row] * err
-  const float* gain_env;
-};
 
 template <int EPI>
 __global__ void __launch_bounds__(256, 2) gemm_tn_kernel(GemmParams p) {

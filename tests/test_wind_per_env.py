@@ -30,13 +30,25 @@ extern "C" void wind_run(int E, int T, const float* dx, const float* dy, float x
     }
   }
 }
+// the host mirror of the batch through the same T frames: passes [T][2] and offset bounds [T][4] per frame
+extern "C" void wind_run_mirror(int E, int T, const float* dx, const float* dy, float xoff, float yoff, int* passes, int* box) {
+  double* acc = new double[2 * E]();
+  WindLayerParams W = {};
+  W.xoff = xoff; W.yoff = yoff;
+  for (int t = 0; t < T; ++t) {
+    W.dx = dx + (size_t)t * E; W.dy = dy + (size_t)t * E;
+    wind_mirror(WIND_STEP, W, E, acc, acc + E, nullptr, 0, nullptr, nullptr, passes + 2 * t, box + 4 * t);
+  }
+  delete[] acc;
+}
 """
 
 
 def test_wind_accumulator_matches_oracle(tmp_path):
     """The accumulator / offset header shared by the host mirror and wind_state_kernel, built by a host compiler: whole
     pixels and accumulators equal OracleAtmos.move exactly, offsets and weights equal fill_wfs_params' formula (the
-    oracle's raytrace_layer)."""
+    oracle's raytrace_layer).  The host mirror of the batch sizes each frame's extrusion passes as the largest |whole
+    pixels| over the batch and bounds the pupil footprint by the least and greatest offsets."""
     import ctypes
     from oracle import aoframe
     src = tmp_path / "wind_shim.cpp"
@@ -57,6 +69,13 @@ def test_wind_accumulator_matches_oracle(tmp_path):
     P = lambda a: a.ctypes.data_as(ctypes.c_void_p)
     L.wind_run.argtypes = [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 2 + [ctypes.c_float] * 2 + [ctypes.c_void_p] * 4
     L.wind_run(E, T, P(dx), P(dy), float(xoff), float(yoff), P(n), P(acc), P(ij), P(w))
+    passes = np.zeros((T, 2), np.int32)
+    box = np.zeros((T, 4), np.int32)
+    L.wind_run_mirror.argtypes = [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 2 + [ctypes.c_float] * 2 + [ctypes.c_void_p] * 2
+    L.wind_run_mirror(E, T, P(dx), P(dy), float(xoff), float(yoff), P(passes), P(box))
+    assert np.array_equal(passes, np.abs(n).max(axis=1))
+    assert np.array_equal(box, np.stack([ij[:, :, 0].min(1), ij[:, :, 0].max(1), ij[:, :, 1].min(1), ij[:, :, 1].max(1)], 1))
+    assert passes.max() >= 3 and (box[:, 0] < box[:, 1]).any() and (box[:, 2] < box[:, 3]).any()   # not a degenerate batch
     F32 = np.float32
     for e in range(E):
         tab = {"nscreens": 1, "dim_screens": [8], "deltax": np.zeros(1, F32), "deltay": np.zeros(1, F32)}
