@@ -1469,6 +1469,33 @@ extern "C" int aom_actor_forward(aom_ctx* ctx, int eval_mode, void* stream) {
   NEED(AOM_T_AGENT_IDX, 0); NEED(AOM_T_AGENT_ACT, 0); NEED(AOM_T_ACTOR_W1, 0); NEED(AOM_T_ACTOR_B1, 0);
   NEED(AOM_T_ACTOR_W2, 0); NEED(AOM_T_ACTOR_B2, 0); NEED(AOM_T_ACTOR_WH, 0); NEED(AOM_T_ACTOR_BH, 0);
   const int E = c.n_env, A = c.n_agents;
+  if (ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT && actor_fused_fits(c.actor_in, c.actor_hidden, 2 * c.actor_out)) {
+    ActorParams p;
+    memset(&p, 0, sizeof(p));
+    p.state = ctx->state; p.ldst = ctx->ldst; p.E = E;
+    p.idx = (const int*)ctx->tab[AOM_T_AGENT_IDX][0]; p.actor_in = c.actor_in;
+    p.hidden = c.actor_hidden; p.heads = 2 * c.actor_out; p.ldh = ctx->ld_aho;
+    p.nkb_in = ctx->ld_ain / 16; p.nkb_h = ctx->ld_ah / 16;
+    p.nt_hidden = (ctx->ld_ah + 127) / 128; p.nt_heads = (ctx->ld_aho + 127) / 128;
+    for (int i = 0; i < 3; ++i) { p.w[i] = ctx->actor_bt[i]; p.w_per[i] = (long long)ctx->actor_bt_per[i]; }
+    p.bias[0] = (const float*)ctx->tab[AOM_T_ACTOR_B1][0]; p.bias[1] = (const float*)ctx->tab[AOM_T_ACTOR_B2][0];
+    p.bias[2] = (const float*)ctx->tab[AOM_T_ACTOR_BH][0];
+    p.actor_out = c.actor_out; p.act_slot = (const int*)ctx->tab[AOM_T_AGENT_ACT][0];
+    p.log_sig_min = c.log_sig_min; p.log_sig_max = c.log_sig_max; p.act_scale = c.pol_act_scale; p.act_bias = c.pol_act_bias;
+    p.eval_mode = eval_mode; p.step = ctx->step; p.k0 = ctx->k0; p.k1 = ctx->k1;
+    p.step_env = ctx->staggered ? ctx->step_env : nullptr;
+    p.action = ctx->action; p.action_mean = ctx->action_mean; p.lda = ctx->ldact;
+    actor_fused_launch(p, A, ctx->d_err, st);
+    KCHECK();
+    // the decision counters advance after every agent's CTAs have read them
+    if (ctx->staggered) {
+      step_env_advance_kernel<<<(E + 255) / 256, 256, 0, st>>>(ctx->step_env, ctx->first, E);
+      KCHECK();
+    }
+    ctx->step++;
+    return AOM_OK;
+  }
+  // hidden or head layers wider than two column tiles, or the SIMT path: gather, three GEMMs, sampling
   actor_gather_kernel<<<E, 256, 0, st>>>(ctx->state, ctx->ldst, (const int*)ctx->tab[AOM_T_AGENT_IDX][0], c.actor_in,
                                          ctx->ld_ain, E, A, ctx->aX);
   KCHECK();

@@ -1,5 +1,5 @@
 // Translation unit of the env-batched GEMMs: the tcgen05 kernel (gemm_tc.cuh), the SIMT kernels (gemm_kernels.cuh) and
-// the choice between them.
+// the choice between them; and the fused actor forward (actor_tc.cuh).
 #include <stdarg.h>
 #include <stdio.h>
 
@@ -7,6 +7,7 @@
 #include "dispatch.h"
 #include "gemm_host.h"
 #include "gemm_tc.cuh"
+#include "actor_tc.cuh"
 
 // Kernels launched with more dynamic shared memory than the default: f(kernel, bytes, its template arguments) for every
 // instantiation.  gemm_init sets the attribute of each and gemm_launch launches from the same list.
@@ -17,12 +18,24 @@ static void gemm_tc_each(F&& f) {     // tcgen05 GEMM: epilogue, column tile
   });
 }
 
+#define ATC_SMEM_MAX (227 * 1024)
+
 cudaError_t gemm_init() {
   cudaError_t ae = cudaSuccess;
   gemm_tc_each([&](auto kernel, size_t smem, auto...) {
     if (ae == cudaSuccess) ae = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   });
+  if (ae == cudaSuccess) ae = cudaFuncSetAttribute(actor_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATC_SMEM_MAX);
   return ae;
+}
+
+bool actor_fused_fits(int actor_in, int hidden, int heads) {
+  return hidden > 0 && hidden <= 2 * GTC_BN && heads > 0 && heads <= 2 * GTC_BN && ATC_SMEM_BYTES(AOM_LD(actor_in)) <= ATC_SMEM_MAX;
+}
+
+void actor_fused_launch(const ActorParams& p, int n_agents, int* err_word, cudaStream_t st) {
+  const dim3 grid((p.E + GTC_BM - 1) / GTC_BM, n_agents);
+  actor_fused_kernel<<<grid, ATC_THREADS, ATC_SMEM_BYTES(p.nkb_in * GTC_BK), st>>>(p, err_word);
 }
 
 static int report(char (&err)[512], int code, const char* fmt, ...) {

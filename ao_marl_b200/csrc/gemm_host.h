@@ -2,6 +2,7 @@
 // integrator epilogue, on the tcgen05 kernel (gemm_tc.cuh) or the SIMT ones (gemm_kernels.cuh).
 #pragma once
 #include <cuda_runtime.h>
+#include <stdint.h>
 
 struct GemmParams {
   const float* A; const float* B; float* C; const float* bias;
@@ -17,6 +18,29 @@ struct GemmParams {
   // epilogue 2: the integrator of epilogue 1 with one gain per row (environment): com += gain_env[row] * err
   const float* gain_env;
 };
+
+// The batched actor forward of all agents in one kernel (actor_fused_kernel, actor_tc.cuh): X[a][e][k] = state[e][idx[a][k]],
+// H1 = relu(W1 X + b1), H2 = relu(W2 H1 + b2), heads = WH H2 + bh, then the tanh-Gaussian actions of actor_sample_kernel.
+struct ActorParams {
+  const float* state; int ldst, E;
+  const int* idx; int actor_in;           // [A][actor_in] state column of each input, -1: none
+  int hidden, heads, ldh;                 // hidden units, 2 actor_out head columns and their leading dimension
+  int nkb_in, nkb_h;                      // k blocks of 16 of layer 1 (AOM_LD(actor_in)) and of layers 2, 3 (AOM_LD(hidden))
+  int nt_hidden, nt_heads;                // 128-column tiles of the hidden and the head layers
+  const float* w[3]; long long w_per[3];  // pre-tiled hi / lo weights (gtc_pretile_host) and their floats per agent
+  const float* bias[3];                   // [A][hidden], [A][hidden], [A][heads]
+  int actor_out; const int* act_slot;     // [A][actor_out] action column, -1: unmapped
+  float log_sig_min, log_sig_max, act_scale, act_bias;
+  int eval_mode; uint32_t step;
+  const uint32_t *k0, *k1, *step_env;     // [E] Philox keys; per-environment decision counters or null (`step` for all)
+  float *action, *action_mean; int lda;
+};
+
+// Whether actor_fused_kernel serves these shapes: hidden and head layers of at most two 128-column tiles, and the input
+// row within the shared memory next to the stages.
+bool actor_fused_fits(int actor_in, int hidden, int heads);
+// Launches actor_fused_kernel over all agents on st; the caller checks the launch (cudaGetLastError).
+void actor_fused_launch(const ActorParams& p, int n_agents, int* err_word, cudaStream_t st);
 
 // Sets the dynamic shared-memory size of every tcgen05 GEMM instantiation; once per context, before any launch.
 cudaError_t gemm_init();

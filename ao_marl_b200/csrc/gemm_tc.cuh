@@ -5,7 +5,9 @@
 // Same contract as gemm_tn_kernel (gemm_kernels.cuh): A = per-environment vectors [E][ld], B = shared
 // operator [rows][ld], both K-major with zero-padded leading dimensions.  Serves the screen extrusion
 // (A.z + B.noise, iterkolmo.py:255-288), the command-matrix reconstruction (rtcCompass.py:527-547), the
-// Btt projections (rlSupervisor.py:784-818, ao_env.py:482-505) and the actors (model_rpc.py:121-158).
+// Btt projections (rlSupervisor.py:784-818, ao_env.py:482-505) and the actors (model_rpc.py:121-158) wherever their
+// kernels do not: the actor forward runs in actor_fused_kernel (actor_tc.cuh, which shares the helpers below) and comes
+// here only for hidden or head layers wider than 256 columns.
 //
 // Precision: every float32 operand is split on the fly into two TF32 numbers, hi = the leading 11
 // significant bits, lo = x - hi (exact), and each product is three kind::tf32 MMAs

@@ -1,5 +1,7 @@
 // Small per-environment vector kernels around the GEMMs: delay line, modal action injection,
-// state assembly with history ring, per-agent reward, actor input gather and action sampling.
+// state assembly with history ring, per-agent reward, actor input gather and action sampling.  The gather and the
+// sampling serve the actor forward of wide actors (hidden or head layers beyond 256 columns) and the SIMT path; the
+// fused actor kernel (actor_tc.cuh) does both itself and leaves the decision counters to step_env_advance_kernel.
 // Reference call sites are cited per kernel (paths relative to the reference root).
 #pragma once
 #include <cuda_runtime.h>
@@ -128,6 +130,13 @@ __global__ void __launch_bounds__(256) actor_sample_kernel(const float* __restri
     __syncthreads();                                  // every thread has read the counter
     if (threadIdx.x == 0 && !first[e]) step_env[e] = step + 1;
   }
+}
+
+// The per-environment decision counters after the fused actor forward (actor_tc.cuh), whose CTAs of every agent read
+// them: one decision more, except for an environment whose first step after aom_reset_envs is pending.
+__global__ void step_env_advance_kernel(uint32_t* step_env, const int* first, int E) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < E && !first[e]) step_env[e] += 1u;
 }
 
 __global__ void pixel_noise_kernel(const float* lam, float* out, long long n, float noise, uint32_t k0,
