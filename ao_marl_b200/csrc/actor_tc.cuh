@@ -16,6 +16,10 @@
 //   warp 8     TMEM allocation; one lane issues the MMAs and commits stages and accumulators.
 //   warp 9     one lane issues the weight copies, running ahead of the loaders by up to ATC_STAGES stages.
 // Every mbarrier wait is bounded (gtc_mbar_wait): on expiry the error word is raised and the kernel traps.
+//
+// PE (per-environment controllers, aom_set_controller_env): the CTA runs tile blockIdx.x of the tile list
+// (ctrl_tiles_host.h): its rows are the environments tile_env[tile][0..128) (-1: padding, read as zero and not sampled),
+// and the weights and biases are those of the tile's policy slot.  Row by row the arithmetic is that of the uniform form.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -34,13 +38,26 @@
 #define ATC_THREADS ((GTC_LOADERS + 2) * 32)
 #define ATC_H2_COL 256u
 
-// grid (E tiles of 128, agents)
-__global__ void __launch_bounds__(ATC_THREADS, 1) actor_fused_kernel(const __grid_constant__ ActorParams p, int* err) {
+// Weights (pre-tiled planes) and biases of layer l: those of the tile's policy slot in the per-environment form
+template <bool PE>
+__device__ __forceinline__ const float* atc_w(const ActorArgs<PE>& p, int slot, int l) {
+  if constexpr (PE) return p.ws[slot][l]; else return p.w[l];
+}
+template <bool PE>
+__device__ __forceinline__ const float* atc_bias(const ActorArgs<PE>& p, int slot, int l) {
+  if constexpr (PE) return p.bs[slot][l]; else return p.bias[l];
+}
+
+// grid (E tiles of 128, agents), PE: (tiles of the tile list, agents)
+template <bool PE>
+__global__ void __launch_bounds__(ATC_THREADS, 1) actor_fused_kernel(const __grid_constant__ ActorArgs<PE> p, int* err) {
   extern __shared__ __align__(1024) uint8_t atc_smem[];
   const int tid = threadIdx.x, warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = tid & 31;
   const int a = blockIdx.y, m0 = blockIdx.x * GTC_BM;
   const int nkb1 = p.nkb_in, nkb2 = p.nkb_h;
   const int nst = nkb1 + 2 * nkb2;                            // stages of the three layers, one ring
+  int slot = 0;                                               // PE: the tile's policy slot
+  if constexpr (PE) slot = __ldg(p.tile_slot + blockIdx.x);
 
   uint8_t* ring = atc_smem;
   uint64_t* bars = reinterpret_cast<uint64_t*>(atc_smem + ATC_STAGES * ATC_STAGE_BYTES);
@@ -75,15 +92,19 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) actor_fused_kernel(const __gri
     {
       const int c = (tid >> 3) & 3;
       const int r0 = (tid >> 5) * 8 + (tid & 7);
+      int env_r[2];                                           // PE: the environments of rows r0, r0 + 64
+      if constexpr (PE)
+        for (int i = 0; i < 2; ++i) env_r[i] = __ldg(p.tile_env + (size_t)blockIdx.x * GTC_BM + r0 + 64 * i);
       float4 va[GTC_INFLIGHT][2];
       auto load_regs = [&](int kb, float4 (&x)[2]) {
         const int k = kb * GTC_BK + c * 4;
         const int s0 = idx_s[k], s1 = idx_s[k + 1], s2 = idx_s[k + 2], s3 = idx_s[k + 3];
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
-          const int e = m0 + r0 + 64 * i;
+          int e;
+          bool in;
+          if constexpr (PE) { e = env_r[i]; in = e >= 0; } else { e = m0 + r0 + 64 * i; in = e < p.E; }
           const float* srow = p.state + (size_t)e * p.ldst;
-          const bool in = e < p.E;
           x[i].x = (in && s0 >= 0) ? __ldg(srow + s0) : 0.f;
           x[i].y = (in && s1 >= 0) ? __ldg(srow + s1) : 0.f;
           x[i].z = (in && s2 >= 0) ? __ldg(srow + s2) : 0.f;
@@ -125,7 +146,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) actor_fused_kernel(const __gri
     const uint32_t lane_addr = tmem_base + ((uint32_t)(lq * 32) << 16);
 #pragma unroll 1
     for (int l = 1; l < 3; ++l) {
-      const float* __restrict__ bias = p.bias[l - 1] + (size_t)a * p.hidden;
+      const float* __restrict__ bias = atc_bias<PE>(p, slot, l - 1) + (size_t)a * p.hidden;
       const uint32_t src = lane_addr + (l == 1 ? 0u : ATC_H2_COL);
       gtc_mbar_wait(acc0 + 8 * (l - 1), 0u, err);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -171,7 +192,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) actor_fused_kernel(const __gri
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     float* hs = reinterpret_cast<float*>(ring);
     const int hp = p.ldh + 1;                                 // odd pitch: lanes (rows) on distinct banks
-    const float* __restrict__ bias_h = p.bias[2] + (size_t)a * p.heads;
+    const float* __restrict__ bias_h = atc_bias<PE>(p, slot, 2) + (size_t)a * p.heads;
     const int ncb = p.ldh / 16, cb_split = (ncb + 1) / 2;
 #pragma unroll 1
     for (int cb = half ? cb_split : 0; cb < (half ? ncb : cb_split); ++cb) {
@@ -195,8 +216,15 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) actor_fused_kernel(const __gri
     const int out = p.actor_out, nb = (out + 3) >> 2;
 #pragma unroll 1
     for (int t = tid; t < GTC_BM * nb; t += GTC_LOADERS * 32) {
-      const int rr = t / nb, jb = t - rr * nb, e = m0 + rr;
-      if (e >= p.E) continue;
+      const int rr = t / nb, jb = t - rr * nb;
+      int e;
+      if constexpr (PE) {
+        e = __ldg(p.tile_env + (size_t)blockIdx.x * GTC_BM + rr);
+        if (e < 0) continue;
+      } else {
+        e = m0 + rr;
+        if (e >= p.E) continue;
+      }
       const uint32_t step = p.step_env ? p.step_env[e] : p.step;
       const aom_u4 w = aom_philox((uint32_t)jb, step, AOM_TAG_ACTOR, (uint32_t)a, p.k0[e], p.k1[e]);
 #pragma unroll
@@ -260,7 +288,7 @@ __global__ void __launch_bounds__(ATC_THREADS, 1) actor_fused_kernel(const __gri
       asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(2u * (uint32_t)cols * GTC_BK * 4u) : "memory");
       const uint32_t dst = gtc_smem_u32(ring + (size_t)s * ATC_STAGE_BYTES + ATC_A_BYTES);
       for (int t = 0; t < nt; ++t) {
-        const float* src = p.w[l] + (size_t)a * p.w_per[l] + (size_t)(t * nkb + kb) * (2 * GTC_BN * GTC_BK);
+        const float* src = atc_w<PE>(p, slot, l) + (size_t)a * p.w_per[l] + (size_t)(t * nkb + kb) * (2 * GTC_BN * GTC_BK);
         const uint32_t n = (uint32_t)min(GTC_BN, cols - GTC_BN * t) * GTC_BK * 4u;
         const uint32_t d = dst + (uint32_t)(t * GTC_BTILE_BYTES(GTC_BN));
         asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"

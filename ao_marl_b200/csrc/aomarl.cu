@@ -22,6 +22,9 @@
 #include "pupil_sweep.cuh"
 #include "denoise_kernels.cuh"
 #include "denoise_tc_host.h"
+#include "ctrl_tiles_host.h"
+
+static_assert(AOM_MAX_POLICIES <= AOM_MAX_LAYERS, "the actor tables of every policy slot live in tab[table][slot]");
 
 static char g_create_error[512] = "";
 
@@ -41,9 +44,17 @@ struct aom_ctx {
   // planes per table, and the scratch of the main stream (the extrusion has its own on the side stream)
   OzOperator ozop[AOM_T_COUNT];
   OzScratch oz;
-  // actor weights as pre-split TF32 hi / lo planes in the tile order of gemm_tc_kernel (W1, W2, WH), floats per agent
-  float* actor_bt[3];
+  // actor weights of every policy slot as pre-split TF32 hi / lo planes in the tile order of gemm_tc_kernel (W1, W2, WH),
+  // floats per agent
+  float* actor_bt[AOM_MAX_POLICIES][3];
   size_t actor_bt_per[3];
+  // per-environment controllers (aom_set_controller_env), all null while every environment is on slot 0: the assignment
+  // (host and device [E]), the tile list of the per-environment actor kernel (ctrl_tiles_host.h), the environments on
+  // the integrator, the skip mask of ctrl_skip_kernel and the com rows aom_rl_control keeps for them
+  int32_t* ctrl_host;
+  int *ctrl_dev, *ctrl_tile_slot, *ctrl_tile_env, *ctrl_integ, *ctrl_skip;
+  float* ctrl_com;
+  int ctrl_ntiles, ctrl_ninteg;
   // sensor / rtc
   float *slopes_frame, *slopes, *err_v, *com, *com1, *volts, *com_before;
   float *bincube, *phase;
@@ -255,7 +266,11 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
   for (void* b : bufs) cudaFree(b);
   for (int t = 0; t < AOM_T_COUNT; ++t) oz_operator_free(ctx->ozop[t]);
   oz_scratch_free(ctx->oz);
-  for (int i = 0; i < 3; ++i) cudaFree(ctx->actor_bt[i]);
+  for (int s = 0; s < AOM_MAX_POLICIES; ++s)
+    for (int i = 0; i < 3; ++i) cudaFree(ctx->actor_bt[s][i]);
+  void* ctrl[] = {ctx->ctrl_dev, ctx->ctrl_tile_slot, ctx->ctrl_tile_env, ctx->ctrl_integ, ctx->ctrl_skip, ctx->ctrl_com};
+  for (void* b : ctrl) cudaFree(b);
+  free(ctx->ctrl_host);
   wfs_frame_destroy(ctx->wfs);
   for (int i = 0; i < AOM_WFS_TIMERS; ++i)
     for (int j = 0; j < 2; ++j)
@@ -330,7 +345,8 @@ extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* hos
   if (table == AOM_T_DENOISER_TC) memcpy(ctx->dn_prm, host, (size_t)DT_NPARAM * 4);   // float parameters travel as kernel arguments
   if (table == AOM_T_ACTOR_W1 || table == AOM_T_ACTOR_W2 || table == AOM_T_ACTOR_WH) {
     // the same weights pre-split into TF32 hi / lo planes in the tile order of gemm_tc_kernel: the actor GEMMs then take
-    // their B operand by one bulk copy per stage instead of global loads + split + st.shared in the loader warps
+    // their B operand by one bulk copy per stage instead of global loads + split + st.shared in the loader warps.  One
+    // copy per policy slot (index)
     const aom_config& c = ctx->cfg;
     const int i = table == AOM_T_ACTOR_W1 ? 0 : table == AOM_T_ACTOR_W2 ? 1 : 2;
     const int K = i == 0 ? c.actor_in : c.actor_hidden, ldb = AOM_LD(K);
@@ -340,9 +356,10 @@ extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* hos
     float* h = (float*)calloc(per * (size_t)c.n_agents, sizeof(float));
     if (!h) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
     gtc_pretile_host((const float*)host, c.n_agents, (long long)rows * ldb, ldb, rows, ldc, AOM_LD(K), h);
-    cudaFree(ctx->actor_bt[i]); ctx->actor_bt[i] = nullptr;
-    cudaError_t e = cudaMalloc((void**)&ctx->actor_bt[i], per * c.n_agents * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemcpy(ctx->actor_bt[i], h, per * c.n_agents * sizeof(float), cudaMemcpyHostToDevice);
+    float*& bt = ctx->actor_bt[index][i];
+    cudaFree(bt); bt = nullptr;
+    cudaError_t e = cudaMalloc((void**)&bt, per * c.n_agents * sizeof(float));
+    if (e == cudaSuccess) e = cudaMemcpy(bt, h, per * c.n_agents * sizeof(float), cudaMemcpyHostToDevice);
     free(h);
     if (e != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "pre-tiled actor weights: %s", cudaGetErrorString(e));
     ctx->actor_bt_per[i] = per;
@@ -656,6 +673,8 @@ static int clear_loop_state(aom_ctx* ctx, cudaStream_t st) {
   return AOM_OK;
 }
 
+static int stagger_begin(aom_ctx* ctx, cudaStream_t st);
+
 extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
   if (!ctx || !seeds) return fail(ctx, AOM_ERR_INVALID, "null argument");
   cudaStream_t st = (cudaStream_t)stream;
@@ -684,6 +703,10 @@ extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
     CU(cudaMemsetAsync(ctx->step_env, 0, E * sizeof(uint32_t), st));
     CU(cudaMemsetAsync(ctx->le_n, 0, 2 * E * sizeof(int), st));
     CU(cudaMemsetAsync(ctx->first, 0, E * sizeof(int), st));
+  }
+  if (ctx->ctrl_ninteg) {                                                // integrator environments freeze their counters
+    rc = stagger_begin(ctx, st);
+    if (rc) return rc;
   }
   return atmos_reset(ctx->atmos, st, ctx->err);
 }
@@ -970,6 +993,108 @@ extern "C" int aom_load_envs(aom_ctx* ctx, int n, const int32_t* envs, const voi
   rc = atmos_load(ctx->atmos, n, ctx->snap_envs, envs, h, (double*)(h + n), st, ctx->err);
   if (rc) return rc;
   CU(cudaStreamSynchronize(st));
+  return AOM_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// per-environment controllers
+
+// Whether policy slot s has its six actor tables (and the pre-split copies of its weights)
+static bool slot_ready(const aom_ctx* ctx, int s) {
+  for (int t = AOM_T_ACTOR_W1; t <= AOM_T_ACTOR_BH; ++t)
+    if (!ctx->tab[t][s]) return false;
+  return ctx->actor_bt[s][0] && ctx->actor_bt[s][1] && ctx->actor_bt[s][2];
+}
+
+static void ctrl_free(aom_ctx* ctx) {
+  int** dev[] = {&ctx->ctrl_dev, &ctx->ctrl_tile_slot, &ctx->ctrl_tile_env, &ctx->ctrl_integ, &ctx->ctrl_skip};
+  for (int** b : dev) { cudaFree(*b); *b = nullptr; }
+  cudaFree(ctx->ctrl_com); ctx->ctrl_com = nullptr;
+  free(ctx->ctrl_host); ctx->ctrl_host = nullptr;
+  ctx->ctrl_ntiles = ctx->ctrl_ninteg = 0;
+}
+
+extern "C" int aom_set_controller_env(aom_ctx* ctx, const int32_t* ctrl) {
+  if (!ctx) return AOM_ERR_INVALID;
+  const int E = ctx->cfg.n_env;
+  bool uniform = true;
+  for (int e = 0; ctrl && e < E; ++e) {
+    const int v = ctrl[e];
+    if (v < AOM_CTRL_INTEGRATOR || v >= AOM_MAX_POLICIES)
+      return fail(ctx, AOM_ERR_INVALID, "aom_set_controller_env: environment %d: controller %d is neither a policy slot in "
+                  "[0, %d) nor AOM_CTRL_INTEGRATOR", e, v, AOM_MAX_POLICIES);
+    if (v >= 0 && !slot_ready(ctx, v))
+      return fail(ctx, AOM_ERR_STATE, "aom_set_controller_env: environment %d: policy slot %d does not have its six actor "
+                  "tables (AOM_T_ACTOR_W1 .. AOM_T_ACTOR_BH at index %d)", e, v, v);
+    uniform = uniform && v == 0;
+  }
+  CU(cudaDeviceSynchronize());                       // a kernel in flight may still read the old tile list
+  ctrl_free(ctx);
+  if (uniform) return AOM_OK;
+  const int tmax = ctl_tiles_max(E);
+  int32_t* ts = (int32_t*)malloc((size_t)tmax * (1 + CTL_TILE) * sizeof(int32_t));
+  int32_t* integ = (int32_t*)malloc((size_t)E * sizeof(int32_t));
+  ctx->ctrl_host = (int32_t*)malloc((size_t)E * sizeof(int32_t));
+  if (!ts || !integ || !ctx->ctrl_host) {
+    free(ts); free(integ); ctrl_free(ctx);
+    return fail(ctx, AOM_ERR_INVALID, "out of host memory");
+  }
+  memcpy(ctx->ctrl_host, ctrl, (size_t)E * sizeof(int32_t));
+  int32_t* te = ts + tmax;
+  const int nt = ctl_build_tiles(ctrl, E, ts, te, integ, &ctx->ctrl_ninteg);
+  ctx->ctrl_ntiles = nt;
+  cudaError_t ce = dalloc(&ctx->ctrl_dev, (size_t)E);
+  if (ce == cudaSuccess) ce = dalloc(&ctx->ctrl_tile_slot, (size_t)tmax);
+  if (ce == cudaSuccess) ce = dalloc(&ctx->ctrl_tile_env, (size_t)tmax * CTL_TILE);
+  if (ce == cudaSuccess) ce = dalloc(&ctx->ctrl_integ, (size_t)E);
+  if (ce == cudaSuccess) ce = dalloc(&ctx->ctrl_skip, (size_t)E);
+  if (ce == cudaSuccess && ctx->ctrl_ninteg) ce = dalloc(&ctx->ctrl_com, (size_t)ctx->ctrl_ninteg * ctx->lda);
+  if (ce == cudaSuccess) ce = cudaMemcpy(ctx->ctrl_dev, ctrl, (size_t)E * sizeof(int32_t), cudaMemcpyHostToDevice);
+  if (ce == cudaSuccess && nt) ce = cudaMemcpy(ctx->ctrl_tile_slot, ts, (size_t)nt * sizeof(int32_t), cudaMemcpyHostToDevice);
+  if (ce == cudaSuccess && nt)
+    ce = cudaMemcpy(ctx->ctrl_tile_env, te, (size_t)nt * CTL_TILE * sizeof(int32_t), cudaMemcpyHostToDevice);
+  if (ce == cudaSuccess && ctx->ctrl_ninteg)
+    ce = cudaMemcpy(ctx->ctrl_integ, integ, (size_t)ctx->ctrl_ninteg * sizeof(int32_t), cudaMemcpyHostToDevice);
+  free(ts); free(integ);
+  if (ce != cudaSuccess) {
+    ctrl_free(ctx);
+    return fail(ctx, AOM_ERR_CUDA, "aom_set_controller_env: %s (the batch is back on slot 0)", cudaGetErrorString(ce));
+  }
+  if (ctx->ctrl_ninteg) {                            // integrator environments freeze their decision counters
+    int rc = stagger_begin(ctx, nullptr);
+    if (rc) return rc;
+    CU(cudaDeviceSynchronize());
+  }
+  return AOM_OK;
+}
+
+extern "C" int aom_get_controller_env(aom_ctx* ctx, int32_t* ctrl, int* per_env) {
+  if (!ctx) return AOM_ERR_INVALID;
+  if (per_env) *per_env = ctx->ctrl_host != nullptr;
+  for (int e = 0; ctrl && e < ctx->cfg.n_env; ++e) ctrl[e] = ctx->ctrl_host ? ctx->ctrl_host[e] : 0;
+  return AOM_OK;
+}
+
+// The skip mask of the environments on the integrator and those whose first step is pending, when some environment is
+// on the integrator; else the first-step flags (null when none is set)
+static const int* ctrl_skip(aom_ctx* ctx, cudaStream_t st, int* rc) {
+  const int E = ctx->cfg.n_env;
+  const int* first = ctx->first_any ? ctx->first : nullptr;
+  *rc = AOM_OK;
+  if (!ctx->ctrl_ninteg) return first;
+  ctrl_skip_kernel<<<(E + 255) / 256, 256, 0, st>>>(ctx->ctrl_dev, first, ctx->ctrl_skip, E);
+  ctx->launches++;
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) *rc = fail(ctx, AOM_ERR_CUDA, "ctrl_skip_kernel launch failed: %s", cudaGetErrorString(e));
+  return ctx->ctrl_skip;
+}
+
+// com rows of the environments on the integrator around aom_rl_control's two products (restore 0: save, 1: write back)
+static int ctrl_com_rows(aom_ctx* ctx, int restore, cudaStream_t st) {
+  if (!ctx->ctrl_ninteg) return AOM_OK;
+  env_rows_kernel<<<dim3((ctx->lda + 255) / 256, ctx->ctrl_ninteg), 256, 0, st>>>(ctx->com, ctx->ctrl_com, ctx->lda,
+                                                                                  ctx->ctrl_integ, ctx->ctrl_ninteg, restore);
+  KCHECK();
   return AOM_OK;
 }
 
@@ -1398,17 +1523,25 @@ extern "C" int aom_rl_control(aom_ctx* ctx, const float* daction, void* stream) 
   NEED(AOM_T_M2V, 0); NEED(AOM_T_FREEDOM, 0); NEED(AOM_T_ACTION_MAP, 0);
   const float* act = daction ? daction : ctx->action;
   if (!act) return fail(ctx, AOM_ERR_STATE, "no action buffer");
-  int rc = project_v2m(ctx, ctx->com, ctx->modes, st);
+  // environments on the integrator: m2v . v2m is not the identity, so their com rows are kept aside and written back
+  int rc = ctrl_com_rows(ctx, 0, st);
+  if (rc) return rc;
+  const int* skip = ctrl_skip(ctx, st, &rc);
+  if (rc) return rc;
+  rc = project_v2m(ctx, ctx->com, ctx->modes, st);
   if (rc) return rc;
   dim3 grid((c.action_dim + 127) / 128, c.n_env);
   inject_action_kernel<<<grid, 128, 0, st>>>(ctx->modes, ctx->ldm, act, ctx->ldact, (const int*)ctx->tab[AOM_T_ACTION_MAP][0],
                                              (const float*)ctx->tab[AOM_T_FREEDOM][0], c.action_dim, c.n_env,
-                                             c.env_act_scale, c.env_act_bias, ctx->first_any ? ctx->first : nullptr);
+                                             c.env_act_scale, c.env_act_bias, skip);
   KCHECK();
   if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_M2V].planes)
-    return launch_oz_product(ctx, AOM_T_M2V, ctx->modes, ctx->ldm, c.nmodes, ctx->com, ctx->lda, c.nactu, 0, nullptr, 0, st);
-  return launch_gemm(ctx, 0, ctx->modes, ctx->ldm, 0, (const float*)ctx->tab[AOM_T_M2V][0], ctx->ldm, 0, ctx->com, ctx->lda, 0,
+    rc = launch_oz_product(ctx, AOM_T_M2V, ctx->modes, ctx->ldm, c.nmodes, ctx->com, ctx->lda, c.nactu, 0, nullptr, 0, st);
+  else
+    rc = launch_gemm(ctx, 0, ctx->modes, ctx->ldm, 0, (const float*)ctx->tab[AOM_T_M2V][0], ctx->ldm, 0, ctx->com, ctx->lda, 0,
                      c.n_env, c.nactu, c.nmodes, nullptr, 0, 0, 1, st);
+  if (rc) return rc;
+  return ctrl_com_rows(ctx, 1, st);
 }
 
 extern "C" int aom_state_begin(aom_ctx* ctx, void* stream) {
@@ -1466,10 +1599,20 @@ extern "C" int aom_actor_forward(aom_ctx* ctx, int eval_mode, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   const aom_config& c = ctx->cfg;
   if (c.n_agents <= 0 || !ctx->state) return fail(ctx, AOM_ERR_STATE, "no agents / state configured");
-  NEED(AOM_T_AGENT_IDX, 0); NEED(AOM_T_AGENT_ACT, 0); NEED(AOM_T_ACTOR_W1, 0); NEED(AOM_T_ACTOR_B1, 0);
-  NEED(AOM_T_ACTOR_W2, 0); NEED(AOM_T_ACTOR_B2, 0); NEED(AOM_T_ACTOR_WH, 0); NEED(AOM_T_ACTOR_BH, 0);
+  NEED(AOM_T_AGENT_IDX, 0); NEED(AOM_T_AGENT_ACT, 0);
   const int E = c.n_env, A = c.n_agents;
-  if (ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT && actor_fused_fits(c.actor_in, c.actor_hidden, 2 * c.actor_out)) {
+  const bool fused = ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT && actor_fused_fits(c.actor_in, c.actor_hidden, 2 * c.actor_out);
+  if (ctx->ctrl_host) {
+    // per-environment controllers: the slots' tables were checked by aom_set_controller_env
+    if (!fused)
+      return fail(ctx, AOM_ERR_UNSUPPORTED, "per-environment controllers are implemented in the fused actor kernel only, "
+                  "which does not serve %s", ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_SIMT ? "the SIMT GEMM path" :
+                  "hidden or head layers wider than 256 columns");
+  } else {
+    NEED(AOM_T_ACTOR_W1, 0); NEED(AOM_T_ACTOR_B1, 0); NEED(AOM_T_ACTOR_W2, 0); NEED(AOM_T_ACTOR_B2, 0);
+    NEED(AOM_T_ACTOR_WH, 0); NEED(AOM_T_ACTOR_BH, 0);
+  }
+  if (fused) {
     ActorParams p;
     memset(&p, 0, sizeof(p));
     p.state = ctx->state; p.ldst = ctx->ldst; p.E = E;
@@ -1477,7 +1620,7 @@ extern "C" int aom_actor_forward(aom_ctx* ctx, int eval_mode, void* stream) {
     p.hidden = c.actor_hidden; p.heads = 2 * c.actor_out; p.ldh = ctx->ld_aho;
     p.nkb_in = ctx->ld_ain / 16; p.nkb_h = ctx->ld_ah / 16;
     p.nt_hidden = (ctx->ld_ah + 127) / 128; p.nt_heads = (ctx->ld_aho + 127) / 128;
-    for (int i = 0; i < 3; ++i) { p.w[i] = ctx->actor_bt[i]; p.w_per[i] = (long long)ctx->actor_bt_per[i]; }
+    for (int i = 0; i < 3; ++i) { p.w[i] = ctx->actor_bt[0][i]; p.w_per[i] = (long long)ctx->actor_bt_per[i]; }
     p.bias[0] = (const float*)ctx->tab[AOM_T_ACTOR_B1][0]; p.bias[1] = (const float*)ctx->tab[AOM_T_ACTOR_B2][0];
     p.bias[2] = (const float*)ctx->tab[AOM_T_ACTOR_BH][0];
     p.actor_out = c.actor_out; p.act_slot = (const int*)ctx->tab[AOM_T_AGENT_ACT][0];
@@ -1485,11 +1628,28 @@ extern "C" int aom_actor_forward(aom_ctx* ctx, int eval_mode, void* stream) {
     p.eval_mode = eval_mode; p.step = ctx->step; p.k0 = ctx->k0; p.k1 = ctx->k1;
     p.step_env = ctx->staggered ? ctx->step_env : nullptr;
     p.action = ctx->action; p.action_mean = ctx->action_mean; p.lda = ctx->ldact;
-    actor_fused_launch(p, A, ctx->d_err, st);
-    KCHECK();
-    // the decision counters advance after every agent's CTAs have read them
+    if (!ctx->ctrl_host) {
+      actor_fused_launch(p, A, ctx->d_err, st);
+      KCHECK();
+    } else if (ctx->ctrl_ntiles) {
+      ActorEnvParams q;
+      memset(&q, 0, sizeof(q));
+      static_cast<ActorParams&>(q) = p;
+      q.tile_slot = ctx->ctrl_tile_slot; q.tile_env = ctx->ctrl_tile_env;
+      for (int s = 0; s < AOM_MAX_POLICIES; ++s) {
+        for (int i = 0; i < 3; ++i) q.ws[s][i] = ctx->actor_bt[s][i];
+        q.bs[s][0] = (const float*)ctx->tab[AOM_T_ACTOR_B1][s]; q.bs[s][1] = (const float*)ctx->tab[AOM_T_ACTOR_B2][s];
+        q.bs[s][2] = (const float*)ctx->tab[AOM_T_ACTOR_BH][s];
+      }
+      actor_fused_env_launch(q, ctx->ctrl_ntiles, A, ctx->d_err, st);
+      KCHECK();
+    }
+    // the decision counters advance after every agent's CTAs have read them (not those of integrator environments)
     if (ctx->staggered) {
-      step_env_advance_kernel<<<(E + 255) / 256, 256, 0, st>>>(ctx->step_env, ctx->first, E);
+      int rc = AOM_OK;
+      const int* skip = ctx->ctrl_ninteg ? ctrl_skip(ctx, st, &rc) : ctx->first;
+      if (rc) return rc;
+      step_env_advance_kernel<<<(E + 255) / 256, 256, 0, st>>>(ctx->step_env, skip, E);
       KCHECK();
     }
     ctx->step++;
@@ -1502,17 +1662,17 @@ extern "C" int aom_actor_forward(aom_ctx* ctx, int eval_mode, void* stream) {
   int rc = launch_gemm(ctx, 0, ctx->aX, ctx->ld_ain, (long long)E * ctx->ld_ain, (const float*)ctx->tab[AOM_T_ACTOR_W1][0],
                        ctx->ld_ain, (long long)c.actor_hidden * ctx->ld_ain, ctx->aH1, ctx->ld_ah, (long long)E * ctx->ld_ah, E,
                        c.actor_hidden, c.actor_in, (const float*)ctx->tab[AOM_T_ACTOR_B1][0], c.actor_hidden, 1, A, st, nullptr, 0, false,
-                       ctx->actor_bt[0], (long long)ctx->actor_bt_per[0]);
+                       ctx->actor_bt[0][0], (long long)ctx->actor_bt_per[0]);
   if (rc) return rc;
   rc = launch_gemm(ctx, 0, ctx->aH1, ctx->ld_ah, (long long)E * ctx->ld_ah, (const float*)ctx->tab[AOM_T_ACTOR_W2][0], ctx->ld_ah,
                    (long long)c.actor_hidden * ctx->ld_ah, ctx->aH2, ctx->ld_ah, (long long)E * ctx->ld_ah, E, c.actor_hidden,
                    c.actor_hidden, (const float*)ctx->tab[AOM_T_ACTOR_B2][0], c.actor_hidden, 1, A, st, nullptr, 0, false,
-                   ctx->actor_bt[1], (long long)ctx->actor_bt_per[1]);
+                   ctx->actor_bt[0][1], (long long)ctx->actor_bt_per[1]);
   if (rc) return rc;
   rc = launch_gemm(ctx, 0, ctx->aH2, ctx->ld_ah, (long long)E * ctx->ld_ah, (const float*)ctx->tab[AOM_T_ACTOR_WH][0], ctx->ld_ah,
                    (long long)2 * c.actor_out * ctx->ld_ah, ctx->aHO, ctx->ld_aho, (long long)E * ctx->ld_aho, E, 2 * c.actor_out,
                    c.actor_hidden, (const float*)ctx->tab[AOM_T_ACTOR_BH][0], 2 * c.actor_out, 0, A, st, nullptr, 0, false,
-                   ctx->actor_bt[2], (long long)ctx->actor_bt_per[2]);
+                   ctx->actor_bt[0][2], (long long)ctx->actor_bt_per[2]);
   if (rc) return rc;
   actor_sample_kernel<<<E, 256, 0, st>>>(ctx->aHO, ctx->ld_aho, c.actor_out, (const int*)ctx->tab[AOM_T_AGENT_ACT][0], E, A,
                                          c.log_sig_min, c.log_sig_max, c.pol_act_scale, c.pol_act_bias, eval_mode, ctx->step,

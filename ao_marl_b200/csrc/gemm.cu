@@ -25,7 +25,9 @@ cudaError_t gemm_init() {
   gemm_tc_each([&](auto kernel, size_t smem, auto...) {
     if (ae == cudaSuccess) ae = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   });
-  if (ae == cudaSuccess) ae = cudaFuncSetAttribute(actor_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATC_SMEM_MAX);
+  each<false, true>([&](auto PE) {
+    if (ae == cudaSuccess) ae = cudaFuncSetAttribute(actor_fused_kernel<PE>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATC_SMEM_MAX);
+  });
   return ae;
 }
 
@@ -35,7 +37,12 @@ bool actor_fused_fits(int actor_in, int hidden, int heads) {
 
 void actor_fused_launch(const ActorParams& p, int n_agents, int* err_word, cudaStream_t st) {
   const dim3 grid((p.E + GTC_BM - 1) / GTC_BM, n_agents);
-  actor_fused_kernel<<<grid, ATC_THREADS, ATC_SMEM_BYTES(p.nkb_in * GTC_BK), st>>>(p, err_word);
+  actor_fused_kernel<false><<<grid, ATC_THREADS, ATC_SMEM_BYTES(p.nkb_in * GTC_BK), st>>>(p, err_word);
+}
+
+void actor_fused_env_launch(const ActorEnvParams& p, int n_tiles, int n_agents, int* err_word, cudaStream_t st) {
+  const dim3 grid(n_tiles, n_agents);
+  actor_fused_kernel<true><<<grid, ATC_THREADS, ATC_SMEM_BYTES(p.nkb_in * GTC_BK), st>>>(p, err_word);
 }
 
 static int report(char (&err)[512], int code, const char* fmt, ...) {

@@ -3,6 +3,8 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <type_traits>
+#include "../../include/aomarl.h"
 
 struct GemmParams {
   const float* A; const float* B; float* C; const float* bias;
@@ -36,11 +38,24 @@ struct ActorParams {
   float *action, *action_mean; int lda;
 };
 
+// The per-environment form (aom_set_controller_env): CTA (t, a) runs agent a of policy slot tile_slot[t] on the
+// environments tile_env[t][0..128) (-1: padding; ctrl_tiles_host.h).  Slot s's pre-tiled weights are ws[s][l], its biases
+// bs[s][l], both laid out per agent as w / bias of the uniform form.
+struct ActorEnvParams : ActorParams {
+  const int *tile_slot, *tile_env;
+  const float* ws[AOM_MAX_POLICIES][3];
+  const float* bs[AOM_MAX_POLICIES][3];
+};
+template <bool PE>
+using ActorArgs = std::conditional_t<PE, ActorEnvParams, ActorParams>;
+
 // Whether actor_fused_kernel serves these shapes: hidden and head layers of at most two 128-column tiles, and the input
 // row within the shared memory next to the stages.
 bool actor_fused_fits(int actor_in, int hidden, int heads);
 // Launches actor_fused_kernel over all agents on st; the caller checks the launch (cudaGetLastError).
 void actor_fused_launch(const ActorParams& p, int n_agents, int* err_word, cudaStream_t st);
+// The same over the n_tiles tiles of the per-environment form.
+void actor_fused_env_launch(const ActorEnvParams& p, int n_tiles, int n_agents, int* err_word, cudaStream_t st);
 
 // Sets the dynamic shared-memory size of every tcgen05 GEMM instantiation; once per context, before any launch.
 cudaError_t gemm_init();

@@ -139,6 +139,23 @@ __global__ void step_env_advance_kernel(uint32_t* step_env, const int* first, in
   if (e < E && !first[e]) step_env[e] += 1u;
 }
 
+// Per-environment controllers (aom_set_controller_env): skip[e] = 1 for an environment on the integrator (ctrl[e] < 0) or
+// one whose first step after aom_reset_envs is pending (first[e]; first may be null).  inject_action_kernel and
+// step_env_advance_kernel read it as their `first`: such an environment takes no action and keeps its decision counter.
+__global__ void ctrl_skip_kernel(const int* ctrl, const int* first, int* skip, int E) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < E) skip[e] = (ctrl[e] < 0 || (first && first[e])) ? 1 : 0;
+}
+
+// Rows envs[0..n) of buf [E][ld]: saved to rows [n][ld] (restore 0) or written back from it (restore 1).  grid (ld / 256, n)
+__global__ void env_rows_kernel(float* buf, float* rows, int ld, const int* envs, int n, int restore) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x, k = blockIdx.y;
+  if (i >= ld || k >= n) return;
+  float* b = buf + (size_t)envs[k] * ld + i;
+  float* r = rows + (size_t)k * ld + i;
+  if (restore) *b = *r; else *r = *b;
+}
+
 __global__ void pixel_noise_kernel(const float* lam, float* out, long long n, float noise, uint32_t k0,
                                    uint32_t k1, uint32_t frame, uint32_t wfs) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;

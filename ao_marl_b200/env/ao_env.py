@@ -87,6 +87,14 @@ class AoEnv:
         """Environments `dst` continue as copies of environments `src` (RlSupervisor.copy_envs)."""
         self.supervisor.copy_envs(src, dst)
 
+    def set_policies(self, slot, policies):
+        """Actors of policy slot `slot` (RlSupervisor.set_policies)."""
+        self.supervisor.set_policies(slot, policies)
+
+    def set_controllers(self, ctrl):
+        """Controller of every environment: [E] policy slots or -1 for the integrator (RlSupervisor.set_controllers)."""
+        self.supervisor.set_controllers(ctrl)
+
     def state(self):
         return self.sim.rows("STATE", self.state_size)
 

@@ -80,6 +80,14 @@ class BatchedTrainer(BatchedRollout):
     def _push(self, s0, a0, s2, r):
         import torch
         mem = self.learner.memory
+        ctrl = self.sim.controller_env
+        if ctrl is not None:
+            # per-environment controllers: the learner trains slot 0; integrator rows carry no action and the other
+            # slots' transitions are not the trained actor's
+            i = torch.as_tensor(np.flatnonzero(ctrl == 0), device=r.device)
+            if i.numel() == 0:
+                return
+            s0, a0, s2, r = s0[i], a0[i], s2[i], r[i]
         mem.push(self.states_per_agent(s0), self.actions_per_agent(a0), r.t().contiguous(),
                  self.states_per_agent(s2), torch.ones_like(r.t()))
 
@@ -119,6 +127,7 @@ class StepLearner:
         # transition of environment e is pushed only when the whole window lies after that step
         self._t = 0
         self._first = np.zeros(self.E, dtype=np.int64)
+        self._ctrl = np.zeros(self.E, dtype=np.int32)      # controllers of the last step (Simulator.controller_env)
 
     def reset_envs(self, envs, seeds):
         """Autoreset of the environments `envs` with `seeds` (Simulator.reset_envs): their next step returns their s0, and
@@ -150,6 +159,13 @@ class StepLearner:
         sim, rl, L = self.sim, self.rl, self.learner
         main = torch.cuda.current_stream()
         can_learn = learn and len(L.memory) > L.batch_size
+        # per-environment controllers: only slot 0 (the trained actor) pushes, and an environment whose controller
+        # changed restarts its window at the current state, so that no transition mixes two controllers
+        ctrl = sim.controller_env
+        ctrl = np.zeros(self.E, dtype=np.int32) if ctrl is None else ctrl
+        changed = ctrl != self._ctrl
+        self._first[changed] = np.maximum(self._first[changed], self._t)
+        self._ctrl = ctrl
         if can_learn and overlap:
             self.stream.wait_stream(main)
             with torch.cuda.stream(self.stream):
@@ -165,7 +181,7 @@ class StepLearner:
             main.wait_stream(self.stream)          # the replay is written below; the new actors are uploaded by the caller
         if self.mdp.check_update_possibility():
             s0, a0, s2 = self.mdp.credit_assignment()
-            ok = self._first <= self._t - self.mdp.depth - 1        # the oldest state of the window is the episode's
+            ok = (self._first <= self._t - self.mdp.depth - 1) & (ctrl == 0)   # the oldest state of the window is the episode's
             if not ok.all():
                 i = torch.as_tensor(np.flatnonzero(ok), device=r.device)
                 s0, a0, s2, r = s0[i], a0[i], s2[i], r[i]

@@ -60,6 +60,12 @@ class Roket(RlSupervisor):
             raise NotImplementedError("ROKET's loop filter has one gain for the whole batch: per-environment gains "
                                       "(set_gain with an [E] array) are not supported; set a scalar gain")
 
+    def _one_controller(self):
+        """The breakdown models one controller for the whole batch."""
+        if self.sim.controller_env is not None:
+            raise NotImplementedError("ROKET's breakdown models one controller for the whole batch: per-environment "
+                                      "controllers (set_controllers) are not supported; call set_controllers(None)")
+
     def reset_envs(self, envs, seeds):
         """Not available: the error-breakdown buffers ([N_total, E, .]) hold one run of the whole batch."""
         raise NotImplementedError("ROKET's breakdown buffers are whole-batch: use reset()")
@@ -78,6 +84,7 @@ class Roket(RlSupervisor):
         import torch
         assert N_total >= N_preloop
         self._common_gain()
+        self._one_controller()
         t, E = self.tables, self.n_env
         dev = "cuda"
         self.agent, self.include_tip_tilt = agent, include_tip_tilt
@@ -148,6 +155,7 @@ class Roket(RlSupervisor):
         corrected) command and evaluate the target."""
         import torch
         self._common_gain()
+        self._one_controller()
         i = self.iter_number
         if a is not None and i < self.n:
             act = torch.as_tensor(a, dtype=torch.float32, device="cuda")

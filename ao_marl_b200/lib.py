@@ -61,7 +61,7 @@ O = {name: i for i, name in enumerate(OPTIONS)}
 EXPORTS = ["aom_config_size", "aom_create", "aom_destroy", "aom_last_error", "aom_set_table", "aom_get_buffer",
            "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_reset_envs", "aom_env_state_bytes", "aom_save_envs", "aom_load_envs", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_set_wfs_noise", "aom_set_wfs_noise_env", "aom_get_condition", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
            "aom_comp_strehl", "aom_reset_strehl", "aom_do_control_geo", "aom_apply_control_geo", "aom_denoise", "aom_set_bincube", "aom_do_centroids", "aom_do_centroids_geom", "aom_do_control", "aom_set_command", "aom_apply_control",
-           "aom_set_gain", "aom_set_gain_env", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
+           "aom_set_gain", "aom_set_gain_env", "aom_set_controller_env", "aom_get_controller_env", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
            "aom_state_begin", "aom_state_end", "aom_reward", "aom_actor_forward", "aom_step", "aom_gemm_tn",
            "aom_pixel_noise"]
 
@@ -124,6 +124,8 @@ def load_library():
     lib.aom_apply_control.argtypes = [vp, i32, vp]
     lib.aom_set_gain.argtypes = [vp, f32]
     lib.aom_set_gain_env.argtypes = [vp, vp]
+    lib.aom_set_controller_env.argtypes = [vp, vp]
+    lib.aom_get_controller_env.argtypes = [vp, vp, ctypes.POINTER(i32)]
     lib.aom_set_loop.argtypes = [vp, i32]
     lib.aom_reset_dm.argtypes = [vp, vp]
     lib.aom_set_dm_volts.argtypes = [vp, vp, i32, vp]
@@ -685,6 +687,31 @@ class Simulator:
         a = None if g is None else self._env_array(g, "set_gain_env")
         self._check(self.lib.aom_set_gain_env(self._ctx, None if a is None else a.ctypes.data_as(ctypes.c_void_p)),
                     "aom_set_gain_env")
+
+    CTRL_INTEGRATOR = -1
+    MAX_POLICIES = 8
+
+    def set_controller_env(self, ctrl):
+        """Controller of every environment ([E] ints): a policy slot 0 .. MAX_POLICIES-1 (the `index` its actor tables
+        were uploaded at, e.g. RLLayout.upload_actors(sim, slot)) or CTRL_INTEGRATOR (-1) for the integrator alone; None
+        puts every environment back on slot 0.  A value out of range raises ValueError, a slot without its actor tables
+        RuntimeError; the assignment in force is unchanged then.  Persists through reset / reset_envs / load_envs."""
+        if ctrl is None:
+            self._check(self.lib.aom_set_controller_env(self._ctx, None), "aom_set_controller_env")
+            return
+        a = np.asarray(ctrl)
+        if a.shape != (self.n_env,) or not np.issubdtype(a.dtype, np.integer):
+            raise ValueError("set_controller_env: expected %d integers, got shape %s (%s)" % (self.n_env, a.shape, a.dtype))
+        a = np.ascontiguousarray(a, dtype=np.int32)
+        self._check(self.lib.aom_set_controller_env(self._ctx, a.ctypes.data_as(ctypes.c_void_p)), "aom_set_controller_env")
+
+    @property
+    def controller_env(self):
+        """int32 [E] controller of every environment (slot or CTRL_INTEGRATOR), or None while all are on slot 0."""
+        per_env, values = ctypes.c_int(), np.empty(self.n_env, np.int32)
+        self._check(self.lib.aom_get_controller_env(self._ctx, values.ctypes.data_as(ctypes.c_void_p), ctypes.byref(per_env)),
+                    "aom_get_controller_env")
+        return values if per_env.value else None
 
     def set_loop(self, closed):
         self._check(self.lib.aom_set_loop(self._ctx, int(bool(closed))), "aom_set_loop")

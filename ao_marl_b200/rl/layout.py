@@ -161,6 +161,11 @@ class RLLayout:
             sim.set_table("AGENT_REWARD", self.agent_reward)
             self.upload_actors(sim)
 
-    def upload_actors(self, sim):
-        for name, arr in pack_actors(self.policies, self.actor_in, self.hidden, self.actor_out).items():
-            sim.set_table(name, arr)
+    def upload_actors(self, sim, slot=0, policies=None):
+        """Upload the actors (this layout's policies, or `policies`, one GaussianPolicy per agent) into policy slot
+        `slot` of the simulator (Simulator.set_controller_env chooses the slot of each environment)."""
+        pols = self.policies if policies is None else policies
+        if len(pols) != self.n_agents:
+            raise ValueError("upload_actors: %d policies for %d agents" % (len(pols), self.n_agents))
+        for name, arr in pack_actors(pols, self.actor_in, self.hidden, self.actor_out).items():
+            sim.set_table(name, arr, index=slot)

@@ -350,9 +350,10 @@ class BatchedSAC:
                     ACTOR_W2=pad(self.actor.W[1], H), ACTOR_B2=self.actor.b[1].detach().cpu().numpy(),
                     ACTOR_WH=pad(self.head.W[0], H), ACTOR_BH=self.head.b[0].detach().cpu().numpy())
 
-    def upload_actors(self, sim):
+    def upload_actors(self, sim, slot=0):
+        """Upload the current actors into policy slot `slot` of the simulator."""
         for name, arr in self.pack_for_sim().items():
-            sim.set_table(name, np.ascontiguousarray(arr, dtype=np.float32))
+            sim.set_table(name, np.ascontiguousarray(arr, dtype=np.float32), index=slot)
 
     @classmethod
     def from_layout(cls, rl, device="cuda", seed=0, dist=None, memory_size=None):

@@ -141,6 +141,16 @@ class RlSupervisor:
         """Environments `dst` continue as copies of environments `src` (Simulator.copy_envs)."""
         self.sim.copy_envs(src, dst)
 
+    def set_policies(self, slot, policies):
+        """Upload `policies` (one GaussianPolicy per agent, packed with pack_actors) into policy slot `slot`; slot 0 holds
+        the actors every environment runs unless set_controllers assigns another slot."""
+        self.rl.upload_actors(self.sim, slot=slot, policies=policies)
+
+    def set_controllers(self, ctrl):
+        """Controller of every environment: [E] policy slots, or -1 for the integrator alone (Simulator.set_controller_env);
+        None: every environment on slot 0.  Persists through reset, reset_envs and load_envs."""
+        self.sim.set_controller_env(ctrl)
+
     def get_m_pupil(self):
         return self.config.p_geom._mpupil
 

@@ -22,6 +22,8 @@ extern "C" {
 #endif
 
 #define AOM_MAX_LAYERS 8
+#define AOM_MAX_POLICIES 8            /* policy slots: the index of the AOM_T_ACTOR_* tables (aom_set_controller_env) */
+#define AOM_CTRL_INTEGRATOR (-1)      /* aom_set_controller_env: the environment runs the integrator alone */
 #define AOM_WFS_TIMERS 64             /* sensor-kernel launches timed between two aom_wfs_time_ms calls */
 #define AOM_LD(n) (((n) + 15) & ~15)
 
@@ -109,6 +111,8 @@ typedef enum aom_table {
   AOM_T_AGENT_IDX,     /* int32 [n_agents][actor_in]  state index per actor input, -1 = pad (helper_states.py:286-317) */
   AOM_T_AGENT_ACT,     /* int32 [n_agents][actor_out] global action slot per actor output, -1 = pad (train_rpc.py:667-675) */
   AOM_T_AGENT_REWARD,  /* int32 [n_agents][2]  mode range [a0, a1) of the reward     (train_rpc.py:402-416)  */
+  /* the six actor tables: index = policy slot 0 .. AOM_MAX_POLICIES-1 (slot 0 is what every environment runs unless
+     aom_set_controller_env says otherwise); an upload into one slot leaves every other slot's weights as they are */
   AOM_T_ACTOR_W1,      /* float [n_agents][hidden][ld(actor_in)]                      (model_rpc.py:78-84)   */
   AOM_T_ACTOR_B1,      /* float [n_agents][hidden] */
   AOM_T_ACTOR_W2,      /* float [n_agents][hidden][ld(hidden)] */
@@ -476,6 +480,33 @@ int aom_actor_forward(aom_ctx* ctx, int eval_mode, void* stream);
  * does not depend on the actions, so a host-in-the-loop caller can run it while the actions travel over PCIe). */
 #define AOM_STEP_ATMOS_DONE 8
 int aom_step(aom_ctx* ctx, int mode, int eval_mode, void* stream);
+
+/* Per-environment controllers: which actor policy, or the integrator alone, drives each environment of the batch.
+ * ctrl_host: host int32 [E], a policy slot 0 .. AOM_MAX_POLICIES-1 (the index its six AOM_T_ACTOR_* tables were uploaded
+ * at) or AOM_CTRL_INTEGRATOR per environment; NULL returns the batch to the uniform state, every environment on slot 0.
+ * - Policy slot p, in aom_actor_forward and aom_step mode 0: the environment computes bit for bit what it computes in a
+ *   batch whose slot 0 holds p's weights (actions, action means and everything downstream), in eval and stochastic mode.
+ * - Integrator, in aom_step modes 0 and 1 and in direct calls of aom_actor_forward and aom_rl_control: the environment is
+ *   treated the way mode 2 treats every environment.  No actor forward and no rl_control: its rows of com, action and
+ *   action_mean are untouched and its decision counter does not advance; apply_control, reward, Strehl and the linear
+ *   half-step run as usual.  It computes bit for bit what a batch stepped with mode 2 computes.  Mode 2 is unchanged:
+ *   every environment is on the integrator.
+ * - Switching an environment's controller mid-episode: it continues with its own decision counter.  A -> integrator -> B
+ *   equals a uniform batch that ran A, then mode 2, then B with B uploaded into slot 0.
+ * - Decision counters: as integrator environments freeze theirs, the batch takes per-environment counters (as after
+ *   aom_reset_envs) as soon as an environment is put on the integrator, and again after every aom_reset while one is.
+ * - The assignment belongs to the batch's slots, not to the environments' records: it persists through aom_reset and
+ *   aom_reset_envs, aom_load_envs keeps the destination's controller, and the record (aom_env_head) does not carry it.
+ * - An assignment of slot 0 everywhere is the uniform state.  While another one is in force, the actor paths the fused
+ *   kernel does not serve (AOM_GEMM_SIMT, hidden or head layers wider than 256 columns) return AOM_ERR_UNSUPPORTED from
+ *   aom_actor_forward / aom_step mode 0.
+ * - Every value is checked before anything changes: AOM_ERR_INVALID for a value out of range, AOM_ERR_STATE for a slot
+ *   whose six actor tables are not all uploaded.  Waits for the device; not for the step path. */
+int aom_set_controller_env(aom_ctx* ctx, const int32_t* ctrl_host);
+/* Read back the assignment in force: ctrl_host (host int32 [E], may be NULL) each environment's slot or
+ * AOM_CTRL_INTEGRATOR; per_env (may be NULL) 1 while an assignment other than slot 0 everywhere is in force.  Answers
+ * from the host copy, never touches the device. */
+int aom_get_controller_env(aom_ctx* ctx, int32_t* ctrl_host, int* per_env);
 
 /* Generic device GEMM used by the path, exposed for the parity tests:
  * C[M][ldc] = A[M][lda] . B[N][ldb]^T (+ bias[N]) ; relu optional. */
