@@ -12,19 +12,14 @@
 #include "dalloc.h"
 #include "atmos_host.h"
 #include "gemm_host.h"
-#include "gemm_tc_host.h"
-#include "rtc_kernels.cuh"
+#include "rtc_host.h"
 #include "snapshot_kernels.cuh"
 #include "pupil_kernels.cuh"
 #include "wfs_frame_host.h"
-#include "extrude_i8_host.h"
 #include "geo_kernels.cuh"
 #include "pupil_sweep.cuh"
 #include "denoise_kernels.cuh"
 #include "denoise_tc_host.h"
-#include "ctrl_tiles_host.h"
-
-static_assert(AOM_MAX_POLICIES <= AOM_MAX_LAYERS, "the actor tables of every policy slot live in tab[table][slot]");
 
 static char g_create_error[512] = "";
 
@@ -40,23 +35,10 @@ struct aom_ctx {
   // the turbulence layers: screens, wind state, extrusion (atmos.cu)
   Atmos* atmos;
   uint32_t *k0, *k1;          // device [E] Philox keys (environment seeds)
-  // the integer contraction (extrude_i8.cuh) of the controller's operator products (cmat, v2m, m2v): operator digit
-  // planes per table, and the scratch of the main stream (the extrusion has its own on the side stream)
-  OzOperator ozop[AOM_T_COUNT];
-  OzScratch oz;
-  // actor weights of every policy slot as pre-split TF32 hi / lo planes in the tile order of gemm_tc_kernel (W1, W2, WH),
-  // floats per agent
-  float* actor_bt[AOM_MAX_POLICIES][3];
-  size_t actor_bt_per[3];
-  // per-environment controllers (aom_set_controller_env), all null while every environment is on slot 0: the assignment
-  // (host and device [E]), the tile list of the per-environment actor kernel (ctrl_tiles_host.h), the environments on
-  // the integrator, the skip mask of ctrl_skip_kernel and the com rows aom_rl_control keeps for them
-  int32_t* ctrl_host;
-  int *ctrl_dev, *ctrl_tile_slot, *ctrl_tile_env, *ctrl_integ, *ctrl_skip;
-  float* ctrl_com;
-  int ctrl_ntiles, ctrl_ninteg;
-  // sensor / rtc
-  float *slopes_frame, *slopes, *err_v, *com, *com1, *volts, *com_before;
+  // the controller: integrator, RL vectors, actors of every policy slot, per-environment controllers (rtc.cu)
+  Rtc* rtc;
+  // sensor
+  float *slopes_frame, *slopes;
   float *bincube, *phase;
   const float* cube_override;
   double* tar_mom;            // [2][E][5] pupil sums of the target phase (aom_comp_strehl): main target, geometric one
@@ -72,8 +54,7 @@ struct aom_ctx {
   uint32_t* sweep_mask;
   float* sweep_ttp;
   int sweep_nb;               // 128-pixel column blocks per pupil row
-  int lds, lda, ldm;
-  int closed;
+  int lds, lda;
   uint32_t frame;
   // the conditions [aom_condition][layer] (layer 0 for those of the sensor and the controller); the only copy of them
   // after aom_create, which clears their initial values in cfg
@@ -83,12 +64,8 @@ struct aom_ctx {
   float dn_prm[DT_NPARAM];    // float parameters of the tensor-core denoiser (head of AOM_T_DENOISER_TC)
   int tar_peak, geo_tar_peak; // whether the pending target sums hold the PSF core (AOM_TAR_PEAK)
   int* d_err;                 // device error word raised by bounded waits (gemm_tc.cuh)
-  // RL
-  float *modes, *modes_before, *modes_res, *state, *hist, *reward, *action, *action_mean, *strehl;
-  int ldst, ldact, hist_head;
-  uint32_t step;
-  float *aX, *aH1, *aH2, *aHO;
-  int ld_ain, ld_ah, ld_aho;
+  float* strehl;
+  uint32_t step;              // the batch's actor decisions (the exploration-noise counter)
   bool seeded;
   // staggered environments (aom_reset_envs): from the first partial reset until the next aom_reset every environment
   // counts its noise frames, actor decisions and long-exposure frames from its own reset, and an environment whose
@@ -173,7 +150,6 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   ctx->cond[AOM_COND_NPHOTONS][0].common = cfg->nphotons;
   ctx->cond[AOM_COND_GAIN][0].common = cfg->gain;
   ctx->cfg.noise = ctx->cfg.nphotons = ctx->cfg.gain = 0.f;
-  ctx->closed = 1;
   ctx->opt[AOM_OPT_WFS_PATH] = AOM_WFS_UMMA_WS;
   {
     // development overrides of the default kernel paths (see aom_set_option)
@@ -193,7 +169,6 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   const size_t E = cfg->n_env;
   ctx->lds = AOM_LD(cfg->nslopes);
   ctx->lda = AOM_LD(cfg->nactu);
-  ctx->ldm = AOM_LD(cfg->nmodes > 0 ? cfg->nmodes : 1);
   CU(dalloc(&ctx->k0, E));
   CU(dalloc(&ctx->k1, E));
   CU(dalloc(&ctx->d_err, 1));
@@ -202,41 +177,14 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   if (rc) return rc;
   CU(dalloc(&ctx->slopes_frame, E * ctx->lds));
   CU(dalloc(&ctx->slopes, E * ctx->lds));
-  CU(dalloc(&ctx->err_v, E * ctx->lda));
-  CU(dalloc(&ctx->com, E * ctx->lda));
-  CU(dalloc(&ctx->com1, E * ctx->lda));
-  CU(dalloc(&ctx->volts, E * ctx->lda));
-  CU(dalloc(&ctx->com_before, E * ctx->lda));
+  const RtcLinks rl = {&ctx->cond[AOM_COND_GAIN][0], ctx->tab, ctx->opt, ctx->k0, ctx->k1, ctx->d_err, &ctx->launches,
+                       ctx->num_sms};
+  rc = rtc_create(ctx->cfg, rl, &ctx->rtc, ctx->err);
+  if (rc) return rc;
   CU(dalloc(&ctx->strehl, E * 4));
   CU(dalloc(&ctx->tar_mom, E * 2 * PSW_MOM2));     // main target, then the geometric controller's
   CU(dalloc(&ctx->tar_acc, E * TAR_ACC));
   CU(cudaMalloc((void**)&ctx->dn_dbg, 32 * sizeof(long long)));
-  if (cfg->nmodes > 0) {
-    CU(dalloc(&ctx->modes, E * ctx->ldm));
-    CU(dalloc(&ctx->modes_before, E * ctx->ldm));
-    CU(dalloc(&ctx->modes_res, E * ctx->ldm));
-  }
-  if (cfg->state_dim > 0) {
-    ctx->ldst = AOM_LD(cfg->state_dim);
-    CU(dalloc(&ctx->state, E * ctx->ldst));
-    if (cfg->n_hist > 0) CU(dalloc(&ctx->hist, (size_t)cfg->n_hist * E * cfg->state_modes));
-  }
-  if (cfg->action_dim > 0) {
-    ctx->ldact = AOM_LD(cfg->action_dim);
-    CU(dalloc(&ctx->action, E * ctx->ldact));
-    CU(dalloc(&ctx->action_mean, E * ctx->ldact));
-  }
-  if (cfg->n_agents > 0) {
-    CU(dalloc(&ctx->reward, E * cfg->n_agents));
-    ctx->ld_ain = AOM_LD(cfg->actor_in);
-    ctx->ld_ah = AOM_LD(cfg->actor_hidden);
-    ctx->ld_aho = AOM_LD(2 * cfg->actor_out);
-    size_t A = cfg->n_agents;
-    CU(dalloc(&ctx->aX, A * E * ctx->ld_ain));
-    CU(dalloc(&ctx->aH1, A * E * ctx->ld_ah));
-    CU(dalloc(&ctx->aH2, A * E * ctx->ld_ah));
-    CU(dalloc(&ctx->aHO, A * E * ctx->ld_aho));
-  }
   float* screens[AOM_MAX_LAYERS] = {};
   for (int l = 0; l < cfg->n_layers; ++l) screens[l] = atmos_layer(ctx->atmos, l).screen;
   ctx->wfs = wfs_frame_create(ctx->cfg, screens, ctx->d_err, ctx->num_sms);
@@ -256,21 +204,13 @@ extern "C" void aom_destroy(aom_ctx* ctx) {
   for (int l = 0; l < AOM_MAX_LAYERS; ++l)
     for (int k = 0; k < AOM_COND_COUNT; ++k) { cudaFree(ctx->cond[k][l].dev); free(ctx->cond[k][l].host); }
   atmos_destroy(ctx->atmos);
-  void* bufs[] = {ctx->k0, ctx->k1, ctx->slopes_frame, ctx->slopes, ctx->err_v,
-                  ctx->com, ctx->com1, ctx->volts, ctx->com_before, ctx->bincube, ctx->phase, ctx->modes,
-                  ctx->modes_before, ctx->modes_res, ctx->state, ctx->hist, ctx->reward, ctx->action,
-                  ctx->action_mean, ctx->strehl, ctx->tar_mom, ctx->tar_acc, ctx->aX, ctx->aH1, ctx->aH2, ctx->aHO, ctx->d_err,
+  rtc_destroy(ctx->rtc);
+  void* bufs[] = {ctx->k0, ctx->k1, ctx->slopes_frame, ctx->slopes, ctx->bincube, ctx->phase, ctx->strehl, ctx->tar_mom,
+                  ctx->tar_acc, ctx->d_err,
                   ctx->geo_com, ctx->geo_volts, ctx->geo_b, ctx->geo_T, ctx->strehl_geo, ctx->geo_acc, ctx->geo_mom,
                   ctx->sweep_mask, ctx->sweep_ttp, ctx->rs_envs, ctx->rs_seeds, ctx->frame0, ctx->step_env,
                   ctx->le_n, ctx->first, ctx->snap_envs};
   for (void* b : bufs) cudaFree(b);
-  for (int t = 0; t < AOM_T_COUNT; ++t) oz_operator_free(ctx->ozop[t]);
-  oz_scratch_free(ctx->oz);
-  for (int s = 0; s < AOM_MAX_POLICIES; ++s)
-    for (int i = 0; i < 3; ++i) cudaFree(ctx->actor_bt[s][i]);
-  void* ctrl[] = {ctx->ctrl_dev, ctx->ctrl_tile_slot, ctx->ctrl_tile_env, ctx->ctrl_integ, ctx->ctrl_skip, ctx->ctrl_com};
-  for (void* b : ctrl) cudaFree(b);
-  free(ctx->ctrl_host);
   wfs_frame_destroy(ctx->wfs);
   for (int i = 0; i < AOM_WFS_TIMERS; ++i)
     for (int j = 0; j < 2; ++j)
@@ -327,15 +267,8 @@ extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* hos
     return fail(ctx, AOM_ERR_INVALID, "Dimension mismatch: table %d[%d] expects %zu bytes, got %zu", table, index, want, nbytes);
   // operators of the integer contraction first: a non-finite one is refused before anything changes
   int rc = atmos_set_table(ctx->atmos, table, index, host, ctx->err);
+  if (!rc) rc = rtc_set_table(ctx->rtc, table, index, host, ctx->err);
   if (rc) return rc;
-  if (table == AOM_T_CMAT || table == AOM_T_V2M || table == AOM_T_M2V) {
-    // digit planes of the controller operators for the exact integer products
-    const aom_config& c = ctx->cfg;
-    const int rows = table == AOM_T_V2M ? c.nmodes : c.nactu;
-    const int K = table == AOM_T_CMAT ? c.nslopes : table == AOM_T_V2M ? c.nactu : c.nmodes;
-    rc = oz_operator_upload(ctx->ozop[table], (const float*)host, rows, AOM_LD(K), K, ctx->err);
-    if (rc) return rc;
-  }
   if (ctx->tab[table][index]) { cudaFree(ctx->tab[table][index]); ctx->tab[table][index] = nullptr; }
   CU(cudaMalloc(&ctx->tab[table][index], nbytes ? nbytes : 4));
   CU(cudaMemcpy(ctx->tab[table][index], host, nbytes, cudaMemcpyHostToDevice));
@@ -343,27 +276,6 @@ extern "C" int aom_set_table(aom_ctx* ctx, int table, int index, const void* hos
   if (!wfs_frame_set_table(ctx->wfs, table, host, nbytes)) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
   if (table == AOM_T_MPUPIL || table == AOM_T_TT_PLANES) ctx->sweep_state = 0;
   if (table == AOM_T_DENOISER_TC) memcpy(ctx->dn_prm, host, (size_t)DT_NPARAM * 4);   // float parameters travel as kernel arguments
-  if (table == AOM_T_ACTOR_W1 || table == AOM_T_ACTOR_W2 || table == AOM_T_ACTOR_WH) {
-    // the same weights pre-split into TF32 hi / lo planes in the tile order of gemm_tc_kernel: the actor GEMMs then take
-    // their B operand by one bulk copy per stage instead of global loads + split + st.shared in the loader warps.  One
-    // copy per policy slot (index)
-    const aom_config& c = ctx->cfg;
-    const int i = table == AOM_T_ACTOR_W1 ? 0 : table == AOM_T_ACTOR_W2 ? 1 : 2;
-    const int K = i == 0 ? c.actor_in : c.actor_hidden, ldb = AOM_LD(K);
-    const int rows = i == 2 ? 2 * c.actor_out : c.actor_hidden;
-    const int ldc = AOM_LD(rows);                                   // the output's leading dimension fixes the n tiles
-    const size_t per = gtc_pretile_floats(ldc, AOM_LD(K));
-    float* h = (float*)calloc(per * (size_t)c.n_agents, sizeof(float));
-    if (!h) return fail(ctx, AOM_ERR_INVALID, "out of host memory");
-    gtc_pretile_host((const float*)host, c.n_agents, (long long)rows * ldb, ldb, rows, ldc, AOM_LD(K), h);
-    float*& bt = ctx->actor_bt[index][i];
-    cudaFree(bt); bt = nullptr;
-    cudaError_t e = cudaMalloc((void**)&bt, per * c.n_agents * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemcpy(bt, h, per * c.n_agents * sizeof(float), cudaMemcpyHostToDevice);
-    free(h);
-    if (e != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "pre-tiled actor weights: %s", cudaGetErrorString(e));
-    ctx->actor_bt_per[i] = per;
-  }
   return AOM_OK;
 }
 
@@ -467,6 +379,7 @@ extern "C" int aom_get_buffer(aom_ctx* ctx, int buffer, int index, void** dptr, 
   if (!ctx || !dptr || !count) return fail(ctx, AOM_ERR_INVALID, "null argument");
   const aom_config& c = ctx->cfg;
   const size_t E = c.n_env;
+  const RtcView v = rtc_view(ctx->rtc);
   void* p = nullptr;
   size_t n = 0;
   switch (buffer) {
@@ -483,21 +396,21 @@ extern "C" int aom_get_buffer(aom_ctx* ctx, int buffer, int index, void** dptr, 
       if (index < 0 || index >= c.n_layers) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
       p = atmos_layer(ctx->atmos, index).count; n = E; break;
     case AOM_B_SLOPES: p = ctx->slopes; n = E * ctx->lds; break;
-    case AOM_B_ERR: p = ctx->err_v; n = E * ctx->lda; break;
-    case AOM_B_COM: p = ctx->com; n = E * ctx->lda; break;
-    case AOM_B_VOLTS: p = ctx->volts; n = E * ctx->lda; break;
+    case AOM_B_ERR: p = v.err; n = E * v.lda; break;
+    case AOM_B_COM: p = v.com; n = E * v.lda; break;
+    case AOM_B_VOLTS: p = v.volts; n = E * v.lda; break;
     case AOM_B_BINCUBE:
       if (!ctx->bincube) CU(dalloc(&ctx->bincube, E * c.nvalid * 256));
       p = ctx->bincube; n = E * c.nvalid * 256; break;
     case AOM_B_PHASE:
       if (!ctx->phase) CU(dalloc(&ctx->phase, E * c.n * c.n));
       p = ctx->phase; n = E * c.n * c.n; break;
-    case AOM_B_MODES: p = ctx->modes; n = E * ctx->ldm; break;
-    case AOM_B_RES_MODES: p = ctx->modes_res; n = E * ctx->ldm; break;
-    case AOM_B_STATE: p = ctx->state; n = E * ctx->ldst; break;
-    case AOM_B_REWARD: p = ctx->reward; n = E * c.n_agents; break;
-    case AOM_B_ACTION: p = ctx->action; n = E * ctx->ldact; break;
-    case AOM_B_ACTION_MEAN: p = ctx->action_mean; n = E * ctx->ldact; break;
+    case AOM_B_MODES: p = v.modes; n = E * v.ldm; break;
+    case AOM_B_RES_MODES: p = v.modes_res; n = E * v.ldm; break;
+    case AOM_B_STATE: p = v.state; n = E * v.ldst; break;
+    case AOM_B_REWARD: p = v.reward; n = E * c.n_agents; break;
+    case AOM_B_ACTION: p = v.action; n = E * v.ldact; break;
+    case AOM_B_ACTION_MEAN: p = v.action_mean; n = E * v.ldact; break;
     case AOM_B_STREHL: p = ctx->strehl; n = E * 4; break;
     case AOM_B_GEO_COM: case AOM_B_GEO_VOLTS: case AOM_B_STREHL_GEO: case AOM_B_GEO_PROJ: {
       int rc = geo_prepare(ctx);
@@ -515,50 +428,16 @@ extern "C" int aom_get_buffer(aom_ctx* ctx, int buffer, int index, void** dptr, 
 }
 
 // ---------------------------------------------------------------------------------------------
-static int launch_gemm(aom_ctx* ctx, int epi, const float* A, int lda, long long sA, const float* B, int ldb,
-                       long long sB, float* C, int ldc, long long sC, int M, int N, int K, const float* bias,
-                       long long sBias, int relu, int batch, cudaStream_t st, float* com = nullptr, int ldcom = 0,
-                       bool exact = false, const float* Bt = nullptr, long long sBt = 0) {
-  GemmParams p;
-  memset(&p, 0, sizeof(p));
-  p.A = A; p.B = B; p.C = C; p.bias = bias;
-  p.lda = lda; p.ldb = ldb; p.ldc = ldc; p.M = M; p.N = N; p.K = K;
-  p.sA = sA; p.sB = sB; p.sC = sC; p.sBias = sBias; p.relu = relu;
-  p.com = com; p.ldcom = ldcom; p.gain = ctx->cond[AOM_COND_GAIN][0].common; p.closed = ctx->closed;
-  p.Bt = Bt; p.sBt = sBt;
-  const float* gain_env = ctx->cond[AOM_COND_GAIN][0].dev;
-  if (epi == 1 && gain_env) { epi = 2; p.gain_env = gain_env; }   // integrator with one gain per environment
-  int rc = gemm_launch(p, epi, batch, exact, ctx->opt[AOM_OPT_GEMM_PATH], ctx->num_sms, ctx->d_err, st, ctx->err);
-  if (rc) return rc;
-  KCHECK();
-  return AOM_OK;
-}
-
-// out[E][ldo] = X[E][ldx] . OP^T with the operator's digit planes (table id `op`): exact integer accumulation, one
-// rounding to float32 -- the oracle's float64 evaluation of the controller products (oracle/loop.py)
-static int launch_oz_product(aom_ctx* ctx, int op, const float* X, int ldx, int K, float* out, int ldo, int N, int integrator,
-                             float* com, int ldcom, cudaStream_t st) {
-  const aom_config& c = ctx->cfg;
-  const OzOperator& P = ctx->ozop[op];
-  const int MT = (c.n_env + OZ_BM - 1) / OZ_BM;
-  CU(oz_scratch_reserve(ctx->oz, MT, P.kb, c.n_env, st));
-  OzSliceParams sl;
-  sl.X = X; sl.ld = ldx; sl.K = K; sl.E = c.n_env; sl.KB = P.kb; sl.Zs = ctx->oz.zs; sl.ev = ctx->oz.ev;
-  OzGemmParams m;
-  memset(&m, 0, sizeof(m));
-  m.Zs = ctx->oz.zs; m.ABs = P.planes; m.ev = ctx->oz.ev; m.ea = P.ea; m.out = out; m.ldo = ldo;
-  m.E = c.n_env; m.N = N; m.KB = P.kb; m.com = com; m.ldcom = ldcom; m.closed = ctx->closed; m.err = ctx->d_err;
-  m.gain = ctx->cond[AOM_COND_GAIN][0].common; m.gain_env = integrator ? ctx->cond[AOM_COND_GAIN][0].dev : nullptr;
-  cudaError_t le = oz_product_launch(sl, m, integrator, MT, P.nt, st);
-  if (le != cudaSuccess) return fail(ctx, AOM_ERR_CUDA, "oz_product_launch: %s", cudaGetErrorString(le));
-  ctx->launches += 2;
-  return AOM_OK;
-}
-
 extern "C" int aom_gemm_tn(aom_ctx* ctx, const float* A, int lda, const float* B, int ldb, float* C, int ldc,
                            int M, int N, int K, const float* bias, int relu, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
-  return launch_gemm(ctx, 0, A, lda, 0, B, ldb, 0, C, ldc, 0, M, N, K, bias, 0, relu, 1, (cudaStream_t)stream);
+  GemmParams p;
+  memset(&p, 0, sizeof(p));
+  p.A = A; p.lda = lda; p.B = B; p.ldb = ldb; p.C = C; p.ldc = ldc; p.M = M; p.N = N; p.K = K; p.bias = bias; p.relu = relu;
+  int rc = gemm_launch(p, 0, 1, false, ctx->opt[AOM_OPT_GEMM_PATH], ctx->num_sms, ctx->d_err, (cudaStream_t)stream, ctx->err);
+  if (rc) return rc;
+  KCHECK();
+  return AOM_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -649,16 +528,8 @@ static int clear_loop_state(aom_ctx* ctx, cudaStream_t st) {
   const size_t E = c.n_env;
   CU(cudaMemsetAsync(ctx->slopes, 0, E * ctx->lds * 4, st));
   CU(cudaMemsetAsync(ctx->slopes_frame, 0, E * ctx->lds * 4, st));
-  CU(cudaMemsetAsync(ctx->err_v, 0, E * ctx->lda * 4, st));
-  CU(cudaMemsetAsync(ctx->com, 0, E * ctx->lda * 4, st));
-  CU(cudaMemsetAsync(ctx->com1, 0, E * ctx->lda * 4, st));
-  CU(cudaMemsetAsync(ctx->volts, 0, E * ctx->lda * 4, st));
-  CU(cudaMemsetAsync(ctx->com_before, 0, E * ctx->lda * 4, st));
-  if (ctx->modes_res) CU(cudaMemsetAsync(ctx->modes_res, 0, E * ctx->ldm * 4, st));
-  if (ctx->hist) CU(cudaMemsetAsync(ctx->hist, 0, (size_t)c.n_hist * E * c.state_modes * 4, st));
-  if (ctx->state) CU(cudaMemsetAsync(ctx->state, 0, E * ctx->ldst * 4, st));
-  if (ctx->action) CU(cudaMemsetAsync(ctx->action, 0, E * ctx->ldact * 4, st));
-  ctx->hist_head = 0;
+  int rc = rtc_clear(ctx->rtc, st, ctx->err);
+  if (rc) return rc;
   ctx->cube_override = nullptr;
   ctx->tar_n = 0;
   CU(cudaMemsetAsync(ctx->tar_acc, 0, E * TAR_ACC * sizeof(float), st));
@@ -704,7 +575,7 @@ extern "C" int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream) {
     CU(cudaMemsetAsync(ctx->le_n, 0, 2 * E * sizeof(int), st));
     CU(cudaMemsetAsync(ctx->first, 0, E * sizeof(int), st));
   }
-  if (ctx->ctrl_ninteg) {                                                // integrator environments freeze their counters
+  if (rtc_integrators(ctx->rtc)) {                                       // integrator environments freeze their counters
     rc = stagger_begin(ctx, st);
     if (rc) return rc;
   }
@@ -762,14 +633,15 @@ struct EnvRow {
 static int env_rows(const aom_ctx* ctx, EnvRow* out) {
   const aom_config& c = ctx->cfg;
   const long long E = c.n_env;
+  const RtcView v = rtc_view(ctx->rtc);
   int n = 0;
   auto add = [&](void* b, long long ld, int clear = 1, int slots = 1, long long slot_stride = 0, int ring = 0) {
     if (b) out[n++] = EnvRow{b, ld, slot_stride, slots, ring, clear};
   };
-  add(ctx->slopes, ctx->lds); add(ctx->slopes_frame, ctx->lds); add(ctx->err_v, ctx->lda); add(ctx->com, ctx->lda);
-  add(ctx->com1, ctx->lda); add(ctx->volts, ctx->lda); add(ctx->com_before, ctx->lda); add(ctx->modes_res, ctx->ldm);
-  add(ctx->state, ctx->ldst); add(ctx->action, ctx->ldact); add(ctx->tar_acc, TAR_ACC); add(ctx->strehl, 4);
-  add(ctx->hist, c.state_modes, 1, c.n_hist, E * c.state_modes, 1);      // every slot of the ring
+  add(ctx->slopes, ctx->lds); add(ctx->slopes_frame, ctx->lds); add(v.err, v.lda); add(v.com, v.lda);
+  add(v.com1, v.lda); add(v.volts, v.lda); add(v.com_before, v.lda); add(v.modes_res, v.ldm);
+  add(v.state, v.ldst); add(v.action, v.ldact); add(ctx->tar_acc, TAR_ACC); add(ctx->strehl, 4);
+  add(v.hist, c.state_modes, 1, c.n_hist, E * c.state_modes, 1);         // every slot of the ring
   add(ctx->geo_com, ctx->lda); add(ctx->geo_volts, ctx->lda); add(ctx->geo_acc, TAR_ACC); add(ctx->strehl_geo, 4);
   for (int l = 0; l < c.n_layers; ++l) {
     const AtmosLayer a = atmos_layer(ctx->atmos, l);
@@ -877,7 +749,7 @@ static void snap_params(aom_ctx* ctx, SnapParams& P, int n, void* rec) {
   memset(&P, 0, sizeof(P));
   const size_t bytes = snap_layout(ctx, P);
   P.envs = ctx->snap_envs; P.rec = (unsigned char*)rec; P.bytes = (long long)bytes;
-  P.E = c.n_env; P.hist_head = ctx->hist_head;
+  P.E = c.n_env; P.hist_head = rtc_view(ctx->rtc).hist_head;
   P.magic = AOM_ENV_MAGIC; P.rec_bytes = (uint32_t)bytes; P.fingerprint = config_fingerprint(c); P.n_layers = c.n_layers;
   P.frame = ctx->frame; P.step = ctx->step; P.le_c[0] = ctx->tar_n; P.le_c[1] = ctx->geo_tar_n;
   if (ctx->staggered) { P.frame0 = ctx->frame0; P.step_env = ctx->step_env; P.le_n = ctx->le_n; P.first = ctx->first; }
@@ -999,102 +871,19 @@ extern "C" int aom_load_envs(aom_ctx* ctx, int n, const int32_t* envs, const voi
 // ---------------------------------------------------------------------------------------------
 // per-environment controllers
 
-// Whether policy slot s has its six actor tables (and the pre-split copies of its weights)
-static bool slot_ready(const aom_ctx* ctx, int s) {
-  for (int t = AOM_T_ACTOR_W1; t <= AOM_T_ACTOR_BH; ++t)
-    if (!ctx->tab[t][s]) return false;
-  return ctx->actor_bt[s][0] && ctx->actor_bt[s][1] && ctx->actor_bt[s][2];
-}
-
-static void ctrl_free(aom_ctx* ctx) {
-  int** dev[] = {&ctx->ctrl_dev, &ctx->ctrl_tile_slot, &ctx->ctrl_tile_env, &ctx->ctrl_integ, &ctx->ctrl_skip};
-  for (int** b : dev) { cudaFree(*b); *b = nullptr; }
-  cudaFree(ctx->ctrl_com); ctx->ctrl_com = nullptr;
-  free(ctx->ctrl_host); ctx->ctrl_host = nullptr;
-  ctx->ctrl_ntiles = ctx->ctrl_ninteg = 0;
-}
-
 extern "C" int aom_set_controller_env(aom_ctx* ctx, const int32_t* ctrl) {
   if (!ctx) return AOM_ERR_INVALID;
-  const int E = ctx->cfg.n_env;
-  bool uniform = true;
-  for (int e = 0; ctrl && e < E; ++e) {
-    const int v = ctrl[e];
-    if (v < AOM_CTRL_INTEGRATOR || v >= AOM_MAX_POLICIES)
-      return fail(ctx, AOM_ERR_INVALID, "aom_set_controller_env: environment %d: controller %d is neither a policy slot in "
-                  "[0, %d) nor AOM_CTRL_INTEGRATOR", e, v, AOM_MAX_POLICIES);
-    if (v >= 0 && !slot_ready(ctx, v))
-      return fail(ctx, AOM_ERR_STATE, "aom_set_controller_env: environment %d: policy slot %d does not have its six actor "
-                  "tables (AOM_T_ACTOR_W1 .. AOM_T_ACTOR_BH at index %d)", e, v, v);
-    uniform = uniform && v == 0;
-  }
-  CU(cudaDeviceSynchronize());                       // a kernel in flight may still read the old tile list
-  ctrl_free(ctx);
-  if (uniform) return AOM_OK;
-  const int tmax = ctl_tiles_max(E);
-  int32_t* ts = (int32_t*)malloc((size_t)tmax * (1 + CTL_TILE) * sizeof(int32_t));
-  int32_t* integ = (int32_t*)malloc((size_t)E * sizeof(int32_t));
-  ctx->ctrl_host = (int32_t*)malloc((size_t)E * sizeof(int32_t));
-  if (!ts || !integ || !ctx->ctrl_host) {
-    free(ts); free(integ); ctrl_free(ctx);
-    return fail(ctx, AOM_ERR_INVALID, "out of host memory");
-  }
-  memcpy(ctx->ctrl_host, ctrl, (size_t)E * sizeof(int32_t));
-  int32_t* te = ts + tmax;
-  const int nt = ctl_build_tiles(ctrl, E, ts, te, integ, &ctx->ctrl_ninteg);
-  ctx->ctrl_ntiles = nt;
-  cudaError_t ce = dalloc(&ctx->ctrl_dev, (size_t)E);
-  if (ce == cudaSuccess) ce = dalloc(&ctx->ctrl_tile_slot, (size_t)tmax);
-  if (ce == cudaSuccess) ce = dalloc(&ctx->ctrl_tile_env, (size_t)tmax * CTL_TILE);
-  if (ce == cudaSuccess) ce = dalloc(&ctx->ctrl_integ, (size_t)E);
-  if (ce == cudaSuccess) ce = dalloc(&ctx->ctrl_skip, (size_t)E);
-  if (ce == cudaSuccess && ctx->ctrl_ninteg) ce = dalloc(&ctx->ctrl_com, (size_t)ctx->ctrl_ninteg * ctx->lda);
-  if (ce == cudaSuccess) ce = cudaMemcpy(ctx->ctrl_dev, ctrl, (size_t)E * sizeof(int32_t), cudaMemcpyHostToDevice);
-  if (ce == cudaSuccess && nt) ce = cudaMemcpy(ctx->ctrl_tile_slot, ts, (size_t)nt * sizeof(int32_t), cudaMemcpyHostToDevice);
-  if (ce == cudaSuccess && nt)
-    ce = cudaMemcpy(ctx->ctrl_tile_env, te, (size_t)nt * CTL_TILE * sizeof(int32_t), cudaMemcpyHostToDevice);
-  if (ce == cudaSuccess && ctx->ctrl_ninteg)
-    ce = cudaMemcpy(ctx->ctrl_integ, integ, (size_t)ctx->ctrl_ninteg * sizeof(int32_t), cudaMemcpyHostToDevice);
-  free(ts); free(integ);
-  if (ce != cudaSuccess) {
-    ctrl_free(ctx);
-    return fail(ctx, AOM_ERR_CUDA, "aom_set_controller_env: %s (the batch is back on slot 0)", cudaGetErrorString(ce));
-  }
-  if (ctx->ctrl_ninteg) {                            // integrator environments freeze their decision counters
-    int rc = stagger_begin(ctx, nullptr);
-    if (rc) return rc;
-    CU(cudaDeviceSynchronize());
-  }
+  int rc = rtc_set_controller(ctx->rtc, ctrl, ctx->err);
+  if (rc || !rtc_integrators(ctx->rtc)) return rc;
+  rc = stagger_begin(ctx, nullptr);                  // integrator environments freeze their decision counters
+  if (rc) return rc;
+  CU(cudaDeviceSynchronize());
   return AOM_OK;
 }
 
 extern "C" int aom_get_controller_env(aom_ctx* ctx, int32_t* ctrl, int* per_env) {
   if (!ctx) return AOM_ERR_INVALID;
-  if (per_env) *per_env = ctx->ctrl_host != nullptr;
-  for (int e = 0; ctrl && e < ctx->cfg.n_env; ++e) ctrl[e] = ctx->ctrl_host ? ctx->ctrl_host[e] : 0;
-  return AOM_OK;
-}
-
-// The skip mask of the environments on the integrator and those whose first step is pending, when some environment is
-// on the integrator; else the first-step flags (null when none is set)
-static const int* ctrl_skip(aom_ctx* ctx, cudaStream_t st, int* rc) {
-  const int E = ctx->cfg.n_env;
-  const int* first = ctx->first_any ? ctx->first : nullptr;
-  *rc = AOM_OK;
-  if (!ctx->ctrl_ninteg) return first;
-  ctrl_skip_kernel<<<(E + 255) / 256, 256, 0, st>>>(ctx->ctrl_dev, first, ctx->ctrl_skip, E);
-  ctx->launches++;
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) *rc = fail(ctx, AOM_ERR_CUDA, "ctrl_skip_kernel launch failed: %s", cudaGetErrorString(e));
-  return ctx->ctrl_skip;
-}
-
-// com rows of the environments on the integrator around aom_rl_control's two products (restore 0: save, 1: write back)
-static int ctrl_com_rows(aom_ctx* ctx, int restore, cudaStream_t st) {
-  if (!ctx->ctrl_ninteg) return AOM_OK;
-  env_rows_kernel<<<dim3((ctx->lda + 255) / 256, ctx->ctrl_ninteg), 256, 0, st>>>(ctx->com, ctx->ctrl_com, ctx->lda,
-                                                                                  ctx->ctrl_integ, ctx->ctrl_ninteg, restore);
-  KCHECK();
+  rtc_get_controller(ctx->rtc, ctrl, per_env);
   return AOM_OK;
 }
 
@@ -1116,7 +905,7 @@ static int fill_wfs_params(aom_ctx* ctx, WfsParams& p, int flags, float noise) {
   p.sub_x0 = (const int*)ctx->tab[AOM_T_SUB_X0][0];
   p.sub_y0 = (const int*)ctx->tab[AOM_T_SUB_Y0][0];
   p.flux = (const float*)ctx->tab[AOM_T_FLUX][0];
-  p.volts = ctx->volts; p.ldv = ctx->lda;
+  p.volts = rtc_view(ctx->rtc).volts; p.ldv = ctx->lda;
   p.stamp1d = (const float*)ctx->tab[AOM_T_STAMP1D][0]; p.ss = c.stamp_size;
   p.act_map = (const int*)ctx->tab[AOM_T_ACT_MAP][0];
   p.grid_n = c.pzt_grid_n; p.pitch = c.pzt_pitch; p.i1_0 = c.pzt_i1_0; p.j1_0 = c.pzt_j1_0;
@@ -1300,8 +1089,14 @@ extern "C" int aom_do_control_geo(aom_ctx* ctx, void* stream) {
   // exact float32 FFMA accumulation: the tip-tilt entries of b are 100x the piezo ones and the product cancels to
   // ~1e-3 of its largest terms; the tensor core's truncated accumulator left 3 % errors in the commands (measured,
   // profiles/dev/geo_probe.py).  The reference inverts and multiplies in double (sutra_controller_geo).
-  return launch_gemm(ctx, 0, ctx->geo_b, ctx->lda, 0, (const float*)ctx->tab[AOM_T_GEO_PROJ][0], ctx->lda, 0, ctx->geo_com,
-                     ctx->lda, 0, c.n_env, c.nactu, c.nactu, nullptr, 0, 0, 1, st, nullptr, 0, true);
+  GemmParams g;
+  memset(&g, 0, sizeof(g));
+  g.A = ctx->geo_b; g.lda = ctx->lda; g.B = (const float*)ctx->tab[AOM_T_GEO_PROJ][0]; g.ldb = ctx->lda;
+  g.C = ctx->geo_com; g.ldc = ctx->lda; g.M = c.n_env; g.N = c.nactu; g.K = c.nactu;
+  rc = gemm_launch(g, 0, 1, true, ctx->opt[AOM_OPT_GEMM_PATH], ctx->num_sms, ctx->d_err, st, ctx->err);
+  if (rc) return rc;
+  KCHECK();
+  return AOM_OK;
 }
 
 extern "C" int aom_apply_control_geo(aom_ctx* ctx, void* stream) {
@@ -1399,44 +1194,21 @@ extern "C" int aom_do_centroids(aom_ctx* ctx, void* stream) {
 }
 
 extern "C" int aom_do_control(aom_ctx* ctx, void* stream) {
-  if (!ctx) return AOM_ERR_INVALID;
-  const aom_config& c = ctx->cfg;
-  NEED(AOM_T_CMAT, 0);
-  if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_CMAT].planes)
-    return launch_oz_product(ctx, AOM_T_CMAT, ctx->slopes, ctx->lds, c.nslopes, ctx->err_v, ctx->lda, c.nactu, 1, ctx->com,
-                             ctx->lda, (cudaStream_t)stream);
-  return launch_gemm(ctx, 1, ctx->slopes, ctx->lds, 0, (const float*)ctx->tab[AOM_T_CMAT][0], ctx->lds, 0, ctx->err_v,
-                     ctx->lda, 0, c.n_env, c.nactu, c.nslopes, nullptr, 0, 0, 1, (cudaStream_t)stream, ctx->com, ctx->lda);
+  return ctx ? rtc_do_control(ctx->rtc, ctx->slopes, (cudaStream_t)stream, ctx->err) : AOM_ERR_INVALID;
 }
 
 extern "C" int aom_set_command(aom_ctx* ctx, const float* dcom, int ld, void* stream) {
   if (!ctx || !dcom) return fail(ctx, AOM_ERR_INVALID, "null argument");
-  const aom_config& c = ctx->cfg;
-  if (ld < c.nactu) return fail(ctx, AOM_ERR_INVALID, "Dimension mismatch");
-  dim3 grid((ctx->lda + 255) / 256, c.n_env);
-  copy_rows_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(dcom, ld, ctx->com, ctx->lda, c.nactu, c.n_env);
-  KCHECK();
-  return AOM_OK;
+  return rtc_set_rows(ctx->rtc, AOM_B_COM, dcom, ld, (cudaStream_t)stream, ctx->err);
 }
 
 extern "C" int aom_set_dm_volts(aom_ctx* ctx, const float* dvolts, int ld, void* stream) {
   if (!ctx || !dvolts) return fail(ctx, AOM_ERR_INVALID, "null argument");
-  const aom_config& c = ctx->cfg;
-  if (ld < c.nactu) return fail(ctx, AOM_ERR_INVALID, "Dimension mismatch");
-  dim3 grid((ctx->lda + 255) / 256, c.n_env);
-  copy_rows_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(dvolts, ld, ctx->volts, ctx->lda, c.nactu, c.n_env);
-  KCHECK();
-  return AOM_OK;
+  return rtc_set_rows(ctx->rtc, AOM_B_VOLTS, dvolts, ld, (cudaStream_t)stream, ctx->err);
 }
 
 extern "C" int aom_apply_control(aom_ctx* ctx, int comp_voltage, void* stream) {
-  if (!ctx) return AOM_ERR_INVALID;
-  const aom_config& c = ctx->cfg;
-  size_t total = (size_t)c.n_env * ctx->lda;
-  apply_control_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ctx->com, ctx->com1, ctx->volts,
-                                                                                         ctx->lda, total, c.delay, comp_voltage);
-  KCHECK();
-  return AOM_OK;
+  return ctx ? rtc_apply_control(ctx->rtc, comp_voltage, (cudaStream_t)stream, ctx->err) : AOM_ERR_INVALID;
 }
 
 extern "C" int aom_set_option(aom_ctx* ctx, int option, int value) {
@@ -1485,7 +1257,7 @@ extern "C" int aom_set_wfs_noise_env(aom_ctx* ctx, const float* noise_host, cons
 
 extern "C" int aom_set_loop(aom_ctx* ctx, int closed) {
   if (!ctx) return AOM_ERR_INVALID;
-  ctx->closed = closed ? 1 : 0;
+  rtc_set_loop(ctx->rtc, closed);
   return AOM_OK;
 }
 
@@ -1501,54 +1273,20 @@ extern "C" int aom_set_layer_amp(aom_ctx* ctx, int layer, const float* amp_host)
 }
 
 extern "C" int aom_reset_dm(aom_ctx* ctx, void* stream) {
-  if (!ctx) return AOM_ERR_INVALID;
-  CU(cudaMemsetAsync(ctx->volts, 0, (size_t)ctx->cfg.n_env * ctx->lda * 4, (cudaStream_t)stream));
-  return AOM_OK;
+  return ctx ? rtc_reset_dm(ctx->rtc, (cudaStream_t)stream, ctx->err) : AOM_ERR_INVALID;
 }
 
-// ---------------------------------------------------------------------------------------------
-static int project_v2m(aom_ctx* ctx, const float* v, float* out, cudaStream_t st) {
-  const aom_config& c = ctx->cfg;
-  NEED(AOM_T_V2M, 0);
-  if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_V2M].planes)
-    return launch_oz_product(ctx, AOM_T_V2M, v, ctx->lda, c.nactu, out, ctx->ldm, c.nmodes, 0, nullptr, 0, st);
-  return launch_gemm(ctx, 0, v, ctx->lda, 0, (const float*)ctx->tab[AOM_T_V2M][0], ctx->lda, 0, out, ctx->ldm, 0, c.n_env,
-                     c.nmodes, c.nactu, nullptr, 0, 0, 1, st);
+// The counters of this context that the controller's half-steps read
+static RtcCounters counters(const aom_ctx* ctx) {
+  return RtcCounters{ctx->step, ctx->staggered ? ctx->step_env : nullptr, ctx->first, ctx->first_any};
 }
 
 extern "C" int aom_rl_control(aom_ctx* ctx, const float* daction, void* stream) {
-  if (!ctx) return AOM_ERR_INVALID;
-  cudaStream_t st = (cudaStream_t)stream;
-  const aom_config& c = ctx->cfg;
-  NEED(AOM_T_M2V, 0); NEED(AOM_T_FREEDOM, 0); NEED(AOM_T_ACTION_MAP, 0);
-  const float* act = daction ? daction : ctx->action;
-  if (!act) return fail(ctx, AOM_ERR_STATE, "no action buffer");
-  // environments on the integrator: m2v . v2m is not the identity, so their com rows are kept aside and written back
-  int rc = ctrl_com_rows(ctx, 0, st);
-  if (rc) return rc;
-  const int* skip = ctrl_skip(ctx, st, &rc);
-  if (rc) return rc;
-  rc = project_v2m(ctx, ctx->com, ctx->modes, st);
-  if (rc) return rc;
-  dim3 grid((c.action_dim + 127) / 128, c.n_env);
-  inject_action_kernel<<<grid, 128, 0, st>>>(ctx->modes, ctx->ldm, act, ctx->ldact, (const int*)ctx->tab[AOM_T_ACTION_MAP][0],
-                                             (const float*)ctx->tab[AOM_T_FREEDOM][0], c.action_dim, c.n_env,
-                                             c.env_act_scale, c.env_act_bias, skip);
-  KCHECK();
-  if (ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_TCGEN05 && ctx->ozop[AOM_T_M2V].planes)
-    rc = launch_oz_product(ctx, AOM_T_M2V, ctx->modes, ctx->ldm, c.nmodes, ctx->com, ctx->lda, c.nactu, 0, nullptr, 0, st);
-  else
-    rc = launch_gemm(ctx, 0, ctx->modes, ctx->ldm, 0, (const float*)ctx->tab[AOM_T_M2V][0], ctx->ldm, 0, ctx->com, ctx->lda, 0,
-                     c.n_env, c.nactu, c.nmodes, nullptr, 0, 0, 1, st);
-  if (rc) return rc;
-  return ctrl_com_rows(ctx, 1, st);
+  return ctx ? rtc_rl_control(ctx->rtc, daction, counters(ctx), (cudaStream_t)stream, ctx->err) : AOM_ERR_INVALID;
 }
 
 extern "C" int aom_state_begin(aom_ctx* ctx, void* stream) {
-  if (!ctx) return AOM_ERR_INVALID;
-  CU(cudaMemcpyAsync(ctx->com_before, ctx->com, (size_t)ctx->cfg.n_env * ctx->lda * 4, cudaMemcpyDeviceToDevice,
-                     (cudaStream_t)stream));
-  return AOM_OK;
+  return ctx ? rtc_state_begin(ctx->rtc, (cudaStream_t)stream, ctx->err) : AOM_ERR_INVALID;
 }
 
 // The linear half-step of environments restarted by aom_reset_envs is done: their next rl half-step is an ordinary one.
@@ -1561,124 +1299,18 @@ static int end_first_steps(aom_ctx* ctx, cudaStream_t st) {
 
 extern "C" int aom_state_end(aom_ctx* ctx, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
-  cudaStream_t st = (cudaStream_t)stream;
-  const aom_config& c = ctx->cfg;
-  if (!ctx->state) return fail(ctx, AOM_ERR_STATE, "state_dim is 0 in this configuration");
-  NEED(AOM_T_STATE_MAP, 0); NEED(AOM_T_NORM_DM_MEAN, 0); NEED(AOM_T_NORM_DM_STD, 0);
-  NEED(AOM_T_NORM_RES_MEAN, 0); NEED(AOM_T_NORM_RES_STD, 0);
-  int rc = project_v2m(ctx, ctx->com_before, ctx->modes_before, st);
-  if (rc) return rc;
-  rc = project_v2m(ctx, ctx->err_v, ctx->modes_res, st);
-  if (rc) return rc;
-  dim3 grid((c.state_modes + 127) / 128, c.n_env);
-  build_state_kernel<<<grid, 128, 0, st>>>(ctx->state, ctx->ldst, ctx->hist, c.n_hist, ctx->hist_head, ctx->modes_before,
-                                           ctx->modes_res, ctx->ldm, (const int*)ctx->tab[AOM_T_STATE_MAP][0], c.state_modes,
-                                           (const float*)ctx->tab[AOM_T_NORM_DM_MEAN][0], (const float*)ctx->tab[AOM_T_NORM_DM_STD][0],
-                                           (const float*)ctx->tab[AOM_T_NORM_RES_MEAN][0], (const float*)ctx->tab[AOM_T_NORM_RES_STD][0],
-                                           c.n_env);
-  KCHECK();
-  if (c.n_hist > 0) ctx->hist_head = (ctx->hist_head + 1) % c.n_hist;
-  return end_first_steps(ctx, st);
+  int rc = rtc_state_end(ctx->rtc, (cudaStream_t)stream, ctx->err);
+  return rc ? rc : end_first_steps(ctx, (cudaStream_t)stream);
 }
 
 extern "C" int aom_reward(aom_ctx* ctx, float factor, void* stream) {
-  if (!ctx) return AOM_ERR_INVALID;
-  const aom_config& c = ctx->cfg;
-  if (!ctx->reward) return fail(ctx, AOM_ERR_STATE, "n_agents is 0 in this configuration");
-  NEED(AOM_T_AGENT_REWARD, 0);
-  long long threads = (long long)c.n_env * c.n_agents * 32;
-  reward_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(ctx->modes_res, ctx->ldm,
-                                                                                     (const int*)ctx->tab[AOM_T_AGENT_REWARD][0],
-                                                                                     c.n_agents, c.n_env, factor, ctx->reward);
-  KCHECK();
-  return AOM_OK;
+  return ctx ? rtc_reward(ctx->rtc, factor, (cudaStream_t)stream, ctx->err) : AOM_ERR_INVALID;
 }
 
 extern "C" int aom_actor_forward(aom_ctx* ctx, int eval_mode, void* stream) {
   if (!ctx) return AOM_ERR_INVALID;
-  cudaStream_t st = (cudaStream_t)stream;
-  const aom_config& c = ctx->cfg;
-  if (c.n_agents <= 0 || !ctx->state) return fail(ctx, AOM_ERR_STATE, "no agents / state configured");
-  NEED(AOM_T_AGENT_IDX, 0); NEED(AOM_T_AGENT_ACT, 0);
-  const int E = c.n_env, A = c.n_agents;
-  const bool fused = ctx->opt[AOM_OPT_GEMM_PATH] != AOM_GEMM_SIMT && actor_fused_fits(c.actor_in, c.actor_hidden, 2 * c.actor_out);
-  if (ctx->ctrl_host) {
-    // per-environment controllers: the slots' tables were checked by aom_set_controller_env
-    if (!fused)
-      return fail(ctx, AOM_ERR_UNSUPPORTED, "per-environment controllers are implemented in the fused actor kernel only, "
-                  "which does not serve %s", ctx->opt[AOM_OPT_GEMM_PATH] == AOM_GEMM_SIMT ? "the SIMT GEMM path" :
-                  "hidden or head layers wider than 256 columns");
-  } else {
-    NEED(AOM_T_ACTOR_W1, 0); NEED(AOM_T_ACTOR_B1, 0); NEED(AOM_T_ACTOR_W2, 0); NEED(AOM_T_ACTOR_B2, 0);
-    NEED(AOM_T_ACTOR_WH, 0); NEED(AOM_T_ACTOR_BH, 0);
-  }
-  if (fused) {
-    ActorParams p;
-    memset(&p, 0, sizeof(p));
-    p.state = ctx->state; p.ldst = ctx->ldst; p.E = E;
-    p.idx = (const int*)ctx->tab[AOM_T_AGENT_IDX][0]; p.actor_in = c.actor_in;
-    p.hidden = c.actor_hidden; p.heads = 2 * c.actor_out; p.ldh = ctx->ld_aho;
-    p.nkb_in = ctx->ld_ain / 16; p.nkb_h = ctx->ld_ah / 16;
-    p.nt_hidden = (ctx->ld_ah + 127) / 128; p.nt_heads = (ctx->ld_aho + 127) / 128;
-    for (int i = 0; i < 3; ++i) { p.w[i] = ctx->actor_bt[0][i]; p.w_per[i] = (long long)ctx->actor_bt_per[i]; }
-    p.bias[0] = (const float*)ctx->tab[AOM_T_ACTOR_B1][0]; p.bias[1] = (const float*)ctx->tab[AOM_T_ACTOR_B2][0];
-    p.bias[2] = (const float*)ctx->tab[AOM_T_ACTOR_BH][0];
-    p.actor_out = c.actor_out; p.act_slot = (const int*)ctx->tab[AOM_T_AGENT_ACT][0];
-    p.log_sig_min = c.log_sig_min; p.log_sig_max = c.log_sig_max; p.act_scale = c.pol_act_scale; p.act_bias = c.pol_act_bias;
-    p.eval_mode = eval_mode; p.step = ctx->step; p.k0 = ctx->k0; p.k1 = ctx->k1;
-    p.step_env = ctx->staggered ? ctx->step_env : nullptr;
-    p.action = ctx->action; p.action_mean = ctx->action_mean; p.lda = ctx->ldact;
-    if (!ctx->ctrl_host) {
-      actor_fused_launch(p, A, ctx->d_err, st);
-      KCHECK();
-    } else if (ctx->ctrl_ntiles) {
-      ActorEnvParams q;
-      memset(&q, 0, sizeof(q));
-      static_cast<ActorParams&>(q) = p;
-      q.tile_slot = ctx->ctrl_tile_slot; q.tile_env = ctx->ctrl_tile_env;
-      for (int s = 0; s < AOM_MAX_POLICIES; ++s) {
-        for (int i = 0; i < 3; ++i) q.ws[s][i] = ctx->actor_bt[s][i];
-        q.bs[s][0] = (const float*)ctx->tab[AOM_T_ACTOR_B1][s]; q.bs[s][1] = (const float*)ctx->tab[AOM_T_ACTOR_B2][s];
-        q.bs[s][2] = (const float*)ctx->tab[AOM_T_ACTOR_BH][s];
-      }
-      actor_fused_env_launch(q, ctx->ctrl_ntiles, A, ctx->d_err, st);
-      KCHECK();
-    }
-    // the decision counters advance after every agent's CTAs have read them (not those of integrator environments)
-    if (ctx->staggered) {
-      int rc = AOM_OK;
-      const int* skip = ctx->ctrl_ninteg ? ctrl_skip(ctx, st, &rc) : ctx->first;
-      if (rc) return rc;
-      step_env_advance_kernel<<<(E + 255) / 256, 256, 0, st>>>(ctx->step_env, skip, E);
-      KCHECK();
-    }
-    ctx->step++;
-    return AOM_OK;
-  }
-  // hidden or head layers wider than two column tiles, or the SIMT path: gather, three GEMMs, sampling
-  actor_gather_kernel<<<E, 256, 0, st>>>(ctx->state, ctx->ldst, (const int*)ctx->tab[AOM_T_AGENT_IDX][0], c.actor_in,
-                                         ctx->ld_ain, E, A, ctx->aX);
-  KCHECK();
-  int rc = launch_gemm(ctx, 0, ctx->aX, ctx->ld_ain, (long long)E * ctx->ld_ain, (const float*)ctx->tab[AOM_T_ACTOR_W1][0],
-                       ctx->ld_ain, (long long)c.actor_hidden * ctx->ld_ain, ctx->aH1, ctx->ld_ah, (long long)E * ctx->ld_ah, E,
-                       c.actor_hidden, c.actor_in, (const float*)ctx->tab[AOM_T_ACTOR_B1][0], c.actor_hidden, 1, A, st, nullptr, 0, false,
-                       ctx->actor_bt[0][0], (long long)ctx->actor_bt_per[0]);
+  int rc = rtc_actor_forward(ctx->rtc, eval_mode, counters(ctx), (cudaStream_t)stream, ctx->err);
   if (rc) return rc;
-  rc = launch_gemm(ctx, 0, ctx->aH1, ctx->ld_ah, (long long)E * ctx->ld_ah, (const float*)ctx->tab[AOM_T_ACTOR_W2][0], ctx->ld_ah,
-                   (long long)c.actor_hidden * ctx->ld_ah, ctx->aH2, ctx->ld_ah, (long long)E * ctx->ld_ah, E, c.actor_hidden,
-                   c.actor_hidden, (const float*)ctx->tab[AOM_T_ACTOR_B2][0], c.actor_hidden, 1, A, st, nullptr, 0, false,
-                   ctx->actor_bt[0][1], (long long)ctx->actor_bt_per[1]);
-  if (rc) return rc;
-  rc = launch_gemm(ctx, 0, ctx->aH2, ctx->ld_ah, (long long)E * ctx->ld_ah, (const float*)ctx->tab[AOM_T_ACTOR_WH][0], ctx->ld_ah,
-                   (long long)2 * c.actor_out * ctx->ld_ah, ctx->aHO, ctx->ld_aho, (long long)E * ctx->ld_aho, E, 2 * c.actor_out,
-                   c.actor_hidden, (const float*)ctx->tab[AOM_T_ACTOR_BH][0], 2 * c.actor_out, 0, A, st, nullptr, 0, false,
-                   ctx->actor_bt[0][2], (long long)ctx->actor_bt_per[2]);
-  if (rc) return rc;
-  actor_sample_kernel<<<E, 256, 0, st>>>(ctx->aHO, ctx->ld_aho, c.actor_out, (const int*)ctx->tab[AOM_T_AGENT_ACT][0], E, A,
-                                         c.log_sig_min, c.log_sig_max, c.pol_act_scale, c.pol_act_bias, eval_mode, ctx->step,
-                                         ctx->k0, ctx->k1, ctx->action, ctx->action_mean, ctx->ldact,
-                                         ctx->staggered ? ctx->step_env : nullptr, ctx->first);
-  KCHECK();
   ctx->step++;      // one decision per call: the exploration-noise counter (oracle/rng.py TAG_ACTOR)
   return AOM_OK;
 }
@@ -1714,7 +1346,8 @@ extern "C" int aom_step(aom_ctx* ctx, int mode, int eval_mode, void* stream) {
   if (strehl == 1) { rc = aom_comp_strehl(ctx, 3, (float)nm * 1e-3f, 1, stream); if (rc) return rc; }
   rc = aom_apply_control(ctx, 1, stream); if (rc) return rc;
   if (strehl >= 2) { rc = aom_comp_strehl(ctx, 3, (float)nm * 1e-3f, 1, stream); if (rc) return rc; }
-  if (ctx->reward) { rc = aom_reward(ctx, ctx->cfg.reward_factor, stream); if (rc) return rc; }
+  const RtcView v = rtc_view(ctx->rtc);
+  if (v.reward) { rc = aom_reward(ctx, ctx->cfg.reward_factor, stream); if (rc) return rc; }
   // linear half-step: AoEnv.linear_step -> RlSupervisor.next_part_one (rlSupervisor.py:1015-1051)
   rc = aom_state_begin(ctx, stream); if (rc) return rc;
   if (fork) CU(cudaStreamWaitEvent(st, ctx->ev_join, 0));
@@ -1736,7 +1369,7 @@ extern "C" int aom_step(aom_ctx* ctx, int mode, int eval_mode, void* stream) {
   if (denoise) { rc = aom_denoise(ctx, nullptr, nullptr, 0, stream); if (rc) return rc; }
   rc = aom_do_centroids(ctx, stream); if (rc) return rc;
   rc = aom_do_control(ctx, stream); if (rc) return rc;
-  if (ctx->state) { rc = aom_state_end(ctx, stream); if (rc) return rc; }
+  if (v.state) { rc = aom_state_end(ctx, stream); if (rc) return rc; }
   else { rc = end_first_steps(ctx, st); if (rc) return rc; }
   if (geo && fork) CU(cudaStreamWaitEvent(st, ctx->ev_geo, 0));
   return AOM_OK;

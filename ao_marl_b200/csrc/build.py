@@ -8,8 +8,8 @@ from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB = os.path.join(HERE, "libaomarl.so")
-SOURCES = ["aomarl.cu", "atmos.cu", "gemm.cu", "wfs_frame.cu", "wfs_umma.cu", "extrude_i8.cu", "denoise_tc.cu"]
-HEADERS = ["atmos_kernels.cuh", "atmos_host.h", "env_cond.h", "dalloc.h", "gemm_kernels.cuh", "gemm_tc.cuh", "actor_tc.cuh", "gemm_host.h", "gemm_tc_host.h", "rtc_kernels.cuh", "snapshot_kernels.cuh", "wfs_kernels.cuh", "wfs_params.cuh", "wind_host.h",
+SOURCES = ["aomarl.cu", "atmos.cu", "rtc.cu", "gemm.cu", "wfs_frame.cu", "wfs_umma.cu", "extrude_i8.cu", "denoise_tc.cu"]
+HEADERS = ["atmos_kernels.cuh", "atmos_host.h", "env_cond.h", "dalloc.h", "gemm_kernels.cuh", "gemm_tc.cuh", "actor_tc.cuh", "gemm_host.h", "gemm_tc_host.h", "rtc_host.h", "rtc_kernels.cuh", "snapshot_kernels.cuh", "wfs_kernels.cuh", "wfs_params.cuh", "wind_host.h",
            "wfs_frame_host.h", "pupil_kernels.cuh", "device_common.cuh", "wfs_mma.cuh", "wfs_lattice_host.h", "ctrl_tiles_host.h", "wfs_tma.cuh", "wfs_umma.cuh", "wfs_umma_ws.cuh", "wfs_umma_host.h", "extrude_i8.cuh", "extrude_i8_digits.h", "extrude_i8_host.h", "geo_kernels.cuh",
            "pupil_sweep.cuh", "denoise_kernels.cuh", "denoise_tc.cuh", "denoise_tc_host.h", "fft16.cuh", "twiddles.cuh", "rng.cuh", "dispatch.h", "../../include/aomarl.h"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]

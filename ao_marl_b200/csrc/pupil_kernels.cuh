@@ -4,6 +4,7 @@
 // and the pupil sweep (pupil_sweep.cuh) restate the same arithmetic in their own layouts.
 #pragma once
 #include <cuda_runtime.h>
+#include "rng.cuh"
 #include "wfs_params.cuh"
 
 // Atmosphere part of the phase (microns) of pixel (x, y) of the mpupil frame for environment e: bilinear sample of every
@@ -213,4 +214,12 @@ __global__ void cog_kernel(const float* cube, float* slopes, int lds, int nvalid
     slopes[(size_t)e * lds + k] = (gx - cog_offset) * pixsize;
     slopes[(size_t)e * lds + nvalid + k] = (gy - cog_offset) * pixsize;
   }
+}
+
+// Photon and read noise of n detector pixels of mean lam (aom_pixel_noise): the sensor kernels' draw, one counter per pixel
+__global__ void pixel_noise_kernel(const float* lam, float* out, long long n, float noise, uint32_t k0,
+                                   uint32_t k1, uint32_t frame, uint32_t wfs) {
+  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  out[i] = aom_pixel_noise(lam[i], noise, (uint32_t)i, frame, wfs, k0, k1);
 }

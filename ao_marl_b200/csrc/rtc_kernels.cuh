@@ -156,69 +156,9 @@ __global__ void env_rows_kernel(float* buf, float* rows, int ld, const int* envs
   if (restore) *b = *r; else *r = *b;
 }
 
-__global__ void pixel_noise_kernel(const float* lam, float* out, long long n, float noise, uint32_t k0,
-                                   uint32_t k1, uint32_t frame, uint32_t wfs) {
-  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  out[i] = aom_pixel_noise(lam[i], noise, (uint32_t)i, frame, wfs, k0, k1);
-}
-
 __global__ void copy_rows_kernel(const float* src, int lds_, float* dst, int ldd, int n, int E) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   int e = blockIdx.y;
   if (i >= ldd || e >= E) return;
   dst[(size_t)e * ldd + i] = (i < n) ? src[(size_t)e * lds_ + i] : 0.f;
-}
-
-// ---------------------------------------------------------------------------------------------
-// aom_reset_envs: restart listed environments while the others run on.
-#define RESET_MAX_BUFS (17 + 4 * AOM_MAX_LAYERS)    // controller, state and Strehl rows + screen and ring state per layer
-struct ResetEnvsParams {
-  // per-environment buffers whose rows are zeroed: word (s * slot_stride + e * ld + i), s < slots, i < ld
-  uint32_t* buf[RESET_MAX_BUFS];
-  long long ld[RESET_MAX_BUFS], slot_stride[RESET_MAX_BUFS];
-  int slots[RESET_MAX_BUFS];
-  int nbuf;
-  const int* envs;              // [K] environments to restart
-  const uint32_t* seeds;        // [2][K] low, high words of their new seeds
-  int K, E;
-  uint32_t *k0, *k1;            // [E] Philox keys
-  uint32_t* frame0;             // [E] noise frame of the environment's first sensor frame
-  uint32_t* step_env;           // [E] actor decision counters
-  int* le_n;                    // [2][E] long-exposure counts (main target, geometric target)
-  int* first;                   // [E] first step pending
-  uint32_t frame;
-};
-
-// grid (K, nbuf + 1): block (k, b < nbuf) zeroes the rows of buffer b of environment envs[k]; block (k, nbuf) sets its
-// keys and counters.
-__global__ void __launch_bounds__(256) reset_envs_kernel(const __grid_constant__ ResetEnvsParams P) {
-  const int k = blockIdx.x, b = blockIdx.y, e = P.envs[k];
-  if (b < P.nbuf) {
-    uint32_t* base = P.buf[b] + (size_t)e * P.ld[b];
-    for (int s = 0; s < P.slots[b]; ++s)
-      for (long long i = threadIdx.x; i < P.ld[b]; i += blockDim.x) base[s * P.slot_stride[b] + i] = 0u;
-    return;
-  }
-  if (threadIdx.x == 0) {
-    P.k0[e] = P.seeds[k];
-    P.k1[e] = P.seeds[P.K + k];
-    P.frame0[e] = P.frame;
-    P.step_env[e] = 0u;
-    P.le_n[e] = 0;
-    P.le_n[P.E + e] = 0;
-    P.first[e] = 1;
-  }
-}
-
-// The per-environment counters when the batch stops running in lockstep: every environment at the batch's counts.
-__global__ void stagger_counters_kernel(uint32_t* frame0, uint32_t* step_env, int* le_n, int* first, int E, uint32_t step,
-                                        int n_main, int n_geo) {
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= E) return;
-  frame0[e] = 0u;
-  step_env[e] = step;
-  le_n[e] = n_main;
-  le_n[E + e] = n_geo;
-  first[e] = 0;
 }

@@ -8,11 +8,68 @@
 // (unpack) the head.  The command history is stored in logical order, oldest slot first: slot s of the record is
 // physical slot (s + hist_head) % n_hist of the context.  Counters are stored relative to the environment's reset and
 // rebased onto the context's global counters on unpack.
+//
+// Next to them the other per-environment bookkeeping: the restart of listed environments (aom_reset_envs), whose rows
+// are those of the same enumeration, and the per-environment counters of a batch that leaves lockstep.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "../../include/aomarl.h"
 
+// aom_reset_envs: restart listed environments while the others run on.
+#define RESET_MAX_BUFS (17 + 4 * AOM_MAX_LAYERS)    // controller, state and Strehl rows + screen and ring state per layer
+struct ResetEnvsParams {
+  // per-environment buffers whose rows are zeroed: word (s * slot_stride + e * ld + i), s < slots, i < ld
+  uint32_t* buf[RESET_MAX_BUFS];
+  long long ld[RESET_MAX_BUFS], slot_stride[RESET_MAX_BUFS];
+  int slots[RESET_MAX_BUFS];
+  int nbuf;
+  const int* envs;              // [K] environments to restart
+  const uint32_t* seeds;        // [2][K] low, high words of their new seeds
+  int K, E;
+  uint32_t *k0, *k1;            // [E] Philox keys
+  uint32_t* frame0;             // [E] noise frame of the environment's first sensor frame
+  uint32_t* step_env;           // [E] actor decision counters
+  int* le_n;                    // [2][E] long-exposure counts (main target, geometric target)
+  int* first;                   // [E] first step pending
+  uint32_t frame;
+};
+
+// grid (K, nbuf + 1): block (k, b < nbuf) zeroes the rows of buffer b of environment envs[k]; block (k, nbuf) sets its
+// keys and counters.
+__global__ void __launch_bounds__(256) reset_envs_kernel(const __grid_constant__ ResetEnvsParams P) {
+  const int k = blockIdx.x, b = blockIdx.y, e = P.envs[k];
+  if (b < P.nbuf) {
+    uint32_t* base = P.buf[b] + (size_t)e * P.ld[b];
+    for (int s = 0; s < P.slots[b]; ++s)
+      for (long long i = threadIdx.x; i < P.ld[b]; i += blockDim.x) base[s * P.slot_stride[b] + i] = 0u;
+    return;
+  }
+  if (threadIdx.x == 0) {
+    P.k0[e] = P.seeds[k];
+    P.k1[e] = P.seeds[P.K + k];
+    P.frame0[e] = P.frame;
+    P.step_env[e] = 0u;
+    P.le_n[e] = 0;
+    P.le_n[P.E + e] = 0;
+    P.first[e] = 1;
+  }
+}
+
+// The per-environment counters when the batch stops running in lockstep: every environment at the batch's counts.
+__global__ void stagger_counters_kernel(uint32_t* frame0, uint32_t* step_env, int* le_n, int* first, int E, uint32_t step,
+                                        int n_main, int n_geo) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= E) return;
+  frame0[e] = 0u;
+  step_env[e] = step;
+  le_n[e] = n_main;
+  le_n[E + e] = n_geo;
+  first[e] = 0;
+}
+
+// ---------------------------------------------------------------------------------------------
+// aom_save_envs / aom_load_envs
 #define SNAP_MAX_SEGS (RESET_MAX_BUFS + 4)    // rows aom_reset_envs clears + keys and pending target sums
 #define SNAP_CHUNK_WORDS 8192                 // 32 KB of a slot per block
 #define SNAP_THREADS 256
