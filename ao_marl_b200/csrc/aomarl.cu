@@ -135,7 +135,7 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   if (cfg->stamp_size > 64) return fail(nullptr, AOM_ERR_UNSUPPORTED, "actuator stamp larger than 64 pixels");
   if (cfg->pzt_pitch > 0 && (cfg->stamp_size + 15 + cfg->pzt_pitch - 1) / cfg->pzt_pitch + 1 > WFS_NG_MAX)
     return fail(nullptr, AOM_ERR_UNSUPPORTED, "actuator pitch too small for the %d-cell neighbourhood", WFS_NG_MAX);
-  if (cfg->delay != 0 && cfg->delay != 1) return fail(nullptr, AOM_ERR_UNSUPPORTED, "controller delay must be 0 or 1 frame");
+  if (cfg->delay < 0 || cfg->delay > 2) return fail(nullptr, AOM_ERR_UNSUPPORTED, "controller delay must be 0, 1 or 2 frames");
 
   ctx = (aom_ctx*)calloc(1, sizeof(aom_ctx));
   if (!ctx) return fail(nullptr, AOM_ERR_INVALID, "out of host memory");
@@ -149,7 +149,9 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   ctx->cond[AOM_COND_NOISE][0].common = cfg->noise;
   ctx->cond[AOM_COND_NPHOTONS][0].common = cfg->nphotons;
   ctx->cond[AOM_COND_GAIN][0].common = cfg->gain;
+  ctx->cond[AOM_COND_DELAY][0].common = (float)cfg->delay;
   ctx->cfg.noise = ctx->cfg.nphotons = ctx->cfg.gain = 0.f;
+  ctx->cfg.delay = 0;
   ctx->opt[AOM_OPT_WFS_PATH] = AOM_WFS_UMMA_WS;
   {
     // development overrides of the default kernel paths (see aom_set_option)
@@ -177,7 +179,7 @@ extern "C" int aom_create(const aom_config* cfg, aom_ctx** out) {
   if (rc) return rc;
   CU(dalloc(&ctx->slopes_frame, E * ctx->lds));
   CU(dalloc(&ctx->slopes, E * ctx->lds));
-  const RtcLinks rl = {&ctx->cond[AOM_COND_GAIN][0], ctx->tab, ctx->opt, ctx->k0, ctx->k1, ctx->d_err, &ctx->launches,
+  const RtcLinks rl = {&ctx->cond[AOM_COND_GAIN][0], &ctx->cond[AOM_COND_DELAY][0], ctx->tab, ctx->opt, ctx->k0, ctx->k1, ctx->d_err, &ctx->launches,
                        ctx->num_sms};
   rc = rtc_create(ctx->cfg, rl, &ctx->rtc, ctx->err);
   if (rc) return rc;
@@ -442,7 +444,17 @@ extern "C" int aom_gemm_tn(aom_ctx* ctx, const float* A, int lda, const float* B
 
 // ---------------------------------------------------------------------------------------------
 // the conditions (aom_condition)
-static const char* const cond_names[AOM_COND_COUNT] = {"amplitude", "wind x", "wind y", "sensor noise", "photon count", "gain"};
+static const char* const cond_names[AOM_COND_COUNT] = {"amplitude", "wind x", "wind y", "sensor noise", "photon count", "gain",
+                                                       "", "delay"};
+static_assert(AOM_COND_COUNT == 8, "cond_names and cond_layers list every condition");
+
+// Whether value v is allowed for condition k: finite, photon counts > 0, delays in [0, 2] frames
+static const char* cond_refusal(int k, float v) {
+  if (!isfinite(v)) return "is not finite";
+  if (k == AOM_COND_NPHOTONS && !(v > 0.f)) return "must be > 0";
+  if (k == AOM_COND_DELAY && !(v >= 0.f && v <= 2.f)) return "must be in [0, 2] frames";
+  return nullptr;
+}
 
 // One change of condition (k, l): env false sets the common value *v; env true sets the per-environment values v[E]
 // (host), or with v null returns to the common value.
@@ -452,7 +464,7 @@ struct CondSet {
   const float* v;
 };
 
-// The one setter of the conditions.  Checks every value of the n changes first (finite; photon counts > 0), then
+// The one setter of the conditions.  Checks every value of the n changes first (cond_refusal), then
 // allocates the arrays of those that become per-environment, all or none: a refused call changes nothing.  Waits for the
 // device when per-environment values change (a kernel in flight may still read the old ones).
 static int set_conditions(aom_ctx* ctx, int n, const CondSet* s) {
@@ -464,12 +476,12 @@ static int set_conditions(aom_ctx* ctx, int n, const CondSet* s) {
     if (c.l < 0 || c.l >= cond_layers(c.k, ctx->cfg.n_layers)) return fail(ctx, AOM_ERR_INVALID, "layer index out of range");
     env = env || c.env;
     for (int e = 0; e < (!c.v ? 0 : c.env ? E : 1); ++e) {
-      const float v = c.v[e];
-      if (isfinite(v) && (c.k != AOM_COND_NPHOTONS || v > 0.f)) continue;
+      const char* why = cond_refusal(c.k, c.v[e]);
+      if (!why) continue;
       char where[32] = "", who[32] = "";
       if (c.k <= AOM_COND_WIND_Y) snprintf(where, sizeof(where), "layer %d: ", c.l);
       if (c.env) snprintf(who, sizeof(who), " of environment %d", e);
-      return fail(ctx, AOM_ERR_INVALID, "%s%s%s %s", where, cond_names[c.k], who, isfinite(v) ? "must be > 0" : "is not finite");
+      return fail(ctx, AOM_ERR_INVALID, "%s%s%s %s", where, cond_names[c.k], who, why);
     }
   }
   if (env) CU(cudaDeviceSynchronize());
@@ -500,7 +512,7 @@ static int set_conditions(aom_ctx* ctx, int n, const CondSet* s) {
 
 extern "C" int aom_get_condition(aom_ctx* ctx, int cond, int layer, float* common, float* values_host, int* per_env) {
   if (!ctx) return AOM_ERR_INVALID;
-  if (cond < 0 || cond >= AOM_COND_COUNT) return fail(ctx, AOM_ERR_INVALID, "unknown condition %d", cond);
+  if (cond < 0 || cond >= AOM_COND_COUNT || !cond_layers(cond, 1)) return fail(ctx, AOM_ERR_INVALID, "unknown condition %d", cond);
   if (layer < 0 || layer >= cond_layers(cond, ctx->cfg.n_layers)) return fail(ctx, AOM_ERR_INVALID, "%s: layer %d out of range", cond_names[cond], layer);
   const EnvCond& C = ctx->cond[cond][layer];
   if (common) *common = C.common;
@@ -639,7 +651,7 @@ static int env_rows(const aom_ctx* ctx, EnvRow* out) {
     if (b) out[n++] = EnvRow{b, ld, slot_stride, slots, ring, clear};
   };
   add(ctx->slopes, ctx->lds); add(ctx->slopes_frame, ctx->lds); add(v.err, v.lda); add(v.com, v.lda);
-  add(v.com1, v.lda); add(v.volts, v.lda); add(v.com_before, v.lda); add(v.modes_res, v.ldm);
+  add(v.com1, v.lda); add(v.com2, v.lda); add(v.volts, v.lda); add(v.com_before, v.lda); add(v.modes_res, v.ldm);
   add(v.state, v.ldst); add(v.action, v.ldact); add(ctx->tar_acc, TAR_ACC); add(ctx->strehl, 4);
   add(v.hist, c.state_modes, 1, c.n_hist, E * c.state_modes, 1);         // every slot of the ring
   add(ctx->geo_com, ctx->lda); add(ctx->geo_volts, ctx->lda); add(ctx->geo_acc, TAR_ACC); add(ctx->strehl_geo, 4);
@@ -1242,6 +1254,16 @@ extern "C" int aom_set_gain(aom_ctx* ctx, float gain) {
 
 extern "C" int aom_set_gain_env(aom_ctx* ctx, const float* gain_host) {
   const CondSet s = {AOM_COND_GAIN, 0, true, gain_host};
+  return set_conditions(ctx, 1, &s);
+}
+
+extern "C" int aom_set_delay(aom_ctx* ctx, float delay) {
+  const CondSet s = {AOM_COND_DELAY, 0, false, &delay};
+  return set_conditions(ctx, 1, &s);
+}
+
+extern "C" int aom_set_delay_env(aom_ctx* ctx, const float* delay_host) {
+  const CondSet s = {AOM_COND_DELAY, 0, true, delay_host};
   return set_conditions(ctx, 1, &s);
 }
 

@@ -1,7 +1,7 @@
 // Host side of the controller: the integrator and the modal projections (extrude_i8.cuh, or the GEMMs of gemm.cu), the
 // RL vectors around them (rtc_kernels.cuh), the actor forward (actor_tc.cuh, or gather, three GEMMs and sampling for
-// wide actors) and the per-environment controllers.  The gain, keys and tables stay the context's and are read through
-// RtcLinks.
+// wide actors) and the per-environment controllers.  The gain, delay, keys and tables stay the context's and are read
+// through RtcLinks.
 #include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -37,7 +37,7 @@ struct Rtc {
   int *ctrl_dev, *ctrl_tile_slot, *ctrl_tile_env, *ctrl_integ, *ctrl_skip;
   float* ctrl_com;
   int ctrl_ntiles, ctrl_ninteg;
-  float *err_v, *com, *com1, *volts, *com_before;
+  float *err_v, *com, *com1, *com2, *volts, *com_before;
   float *modes, *modes_before, *modes_res, *state, *hist, *reward, *action, *action_mean;
   int lda, ldm, ldst, ldact, hist_head;
   float *aX, *aH1, *aH2, *aHO;   // the wide actors' inputs, hidden layers and heads [A][E][ld]
@@ -86,7 +86,7 @@ int rtc_create(const aom_config& c, const RtcLinks& links, Rtc** out, char (&err
   const size_t E = c.n_env;
   r->lda = AOM_LD(c.nactu);
   r->ldm = AOM_LD(c.nmodes > 0 ? c.nmodes : 1);
-  float** rows[] = {&r->err_v, &r->com, &r->com1, &r->volts, &r->com_before};
+  float** rows[] = {&r->err_v, &r->com, &r->com1, &r->com2, &r->volts, &r->com_before};
   for (float** b : rows) CU(dalloc(b, E * r->lda));
   for (float** b : {&r->modes, &r->modes_before, &r->modes_res})
     if (c.nmodes > 0) CU(dalloc(b, E * r->ldm));
@@ -124,7 +124,7 @@ static void ctrl_free(Rtc* r) {
 
 void rtc_destroy(Rtc* r) {
   if (!r) return;
-  void* bufs[] = {r->err_v, r->com, r->com1, r->volts, r->com_before, r->modes, r->modes_before, r->modes_res, r->state,
+  void* bufs[] = {r->err_v, r->com, r->com1, r->com2, r->volts, r->com_before, r->modes, r->modes_before, r->modes_res, r->state,
                   r->hist, r->reward, r->action, r->action_mean, r->aX, r->aH1, r->aH2, r->aHO};
   for (void* b : bufs) cudaFree(b);
   for (OzOperator& o : r->op) oz_operator_free(o);
@@ -136,8 +136,8 @@ void rtc_destroy(Rtc* r) {
 }
 
 RtcView rtc_view(const Rtc* r) {
-  return RtcView{r->err_v, r->com, r->com1, r->volts, r->com_before, r->modes, r->modes_res, r->state, r->hist, r->reward,
-                 r->action, r->action_mean, r->lda, r->ldm, r->ldst, r->ldact, r->hist_head};
+  return RtcView{r->err_v, r->com, r->com1, r->com2, r->volts, r->com_before, r->modes, r->modes_res, r->state, r->hist,
+                 r->reward, r->action, r->action_mean, r->lda, r->ldm, r->ldst, r->ldact, r->hist_head};
 }
 
 // Operator o (OP_*): its table, the K columns of its input rows and the N of its output rows, and their leading dimensions
@@ -184,7 +184,7 @@ int rtc_set_table(Rtc* r, int table, int index, const void* host, char (&err)[51
 int rtc_clear(Rtc* r, cudaStream_t st, char (&err)[512]) {
   const aom_config& c = r->cfg;
   const size_t E = c.n_env;
-  float* rows[] = {r->err_v, r->com, r->com1, r->volts, r->com_before};
+  float* rows[] = {r->err_v, r->com, r->com1, r->com2, r->volts, r->com_before};
   for (float* b : rows) CU(cudaMemsetAsync(b, 0, E * r->lda * 4, st));
   if (r->modes_res) CU(cudaMemsetAsync(r->modes_res, 0, E * r->ldm * 4, st));
   if (r->hist) CU(cudaMemsetAsync(r->hist, 0, (size_t)c.n_hist * E * c.state_modes * 4, st));
@@ -337,8 +337,9 @@ int rtc_set_rows(Rtc* r, int buffer, const float* src, int ld, cudaStream_t st, 
 
 int rtc_apply_control(Rtc* r, int comp_voltage, cudaStream_t st, char (&err)[512]) {
   const size_t total = (size_t)r->cfg.n_env * r->lda;
-  apply_control_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(r->com, r->com1, r->volts, r->lda, total,
-                                                                         r->cfg.delay, comp_voltage);
+  const EnvCond& delay = *r->in.delay;
+  delay_line_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(r->com, r->com1, r->com2, r->volts, r->lda, total,
+                                                                      delay.common, delay.dev, comp_voltage);
   KCHECK();
   return AOM_OK;
 }

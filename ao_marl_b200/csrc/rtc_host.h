@@ -13,6 +13,7 @@ struct Rtc;
 // What the controller reads from its context on every call; each pointer stays valid for the context's life.
 struct RtcLinks {
   const EnvCond* gain;                     // the integrator gain of the conditions store
+  const EnvCond* delay;                    // the controller delay (frames) of the conditions store
   void* const (*tab)[AOM_MAX_LAYERS];      // the device tables [aom_table][index]
   const int* opt;                          // the options [aom_option]: GEMM path
   const uint32_t* k0;                      // Philox keys [E]
@@ -32,10 +33,10 @@ struct RtcCounters {
   bool first_any;
 };
 
-// The controller's device buffers, [E] rows each (hist: [n_hist][E][state_modes], slot hist_head the oldest); null when
-// the configuration has none.
+// The controller's device buffers, [E] rows each (hist: [n_hist][E][state_modes], slot hist_head the oldest; com1 /
+// com2 the commands of the last two aom_apply_control calls before this one); null when the configuration has none.
 struct RtcView {
-  float *err, *com, *com1, *volts, *com_before;
+  float *err, *com, *com1, *com2, *volts, *com_before;
   float *modes, *modes_res, *state, *hist, *reward, *action, *action_mean;
   int lda, ldm, ldst, ldact, hist_head;
 };
@@ -65,6 +66,7 @@ bool rtc_integrators(const Rtc* r);
 int rtc_do_control(Rtc* r, const float* slopes, cudaStream_t st, char (&err)[512]);
 // Rows of com (buffer AOM_B_COM, aom_set_command) or volts (AOM_B_VOLTS, aom_set_dm_volts) from src [E][ld]
 int rtc_set_rows(Rtc* r, int buffer, const float* src, int ld, cudaStream_t st, char (&err)[512]);
+// The delay line with each environment's delay (the store's array, else its common value)
 int rtc_apply_control(Rtc* r, int comp_voltage, cudaStream_t st, char (&err)[512]);
 int rtc_reset_dm(Rtc* r, cudaStream_t st, char (&err)[512]);
 

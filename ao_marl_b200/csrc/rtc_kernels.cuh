@@ -7,16 +7,25 @@
 #include <cuda_runtime.h>
 #include "rng.cuh"
 
-// RtcCompass.apply_control -> sutra comp_voltage (rtcCompass.py:573-582): volt = com (delay 0) or the
-// command stored at the previous call (delay 1); then the delay line shifts.
-__global__ void apply_control_kernel(const float* com, float* com1, float* volts, int ld, size_t total,
-                                     int delay, int comp_voltage) {
+// RtcCompass.apply_control -> sutra comp_voltage (rtcCompass.py:573-582), volts = a com + b com1 + c com2 with the
+// weights of sutra's set_delay for a delay d in [0, 2] frames: k = floor(d), f = d - k; an integer delay copies row k
+// (a non-finite row of another age stays out of volts), a fractional one is fmaf(f, c_(k+1), (1 - f) c_k).  Then the
+// line shifts for every delay.  delay_env [E] (or null: `delay` for every environment).
+__global__ void delay_line_kernel(const float* com, float* com1, float* com2, float* volts, int ld, size_t total,
+                                  float delay, const float* delay_env, int comp_voltage) {
   size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
   if (i >= total) return;
   if (!comp_voltage) return;          // "directly apply the current voltage vector": volts unchanged
-  float c = com[i];
-  volts[i] = delay ? com1[i] : c;
-  com1[i] = c;
+  const float d = delay_env ? delay_env[(unsigned)i / (unsigned)ld] : delay;
+  const int k = (int)d;
+  const float f = d - (float)k;
+  const float c0 = com[i], c1 = com1[i];
+  float v;
+  if (f == 0.f) v = k == 0 ? c0 : k == 1 ? c1 : com2[i];
+  else v = k == 0 ? fmaf(f, c1, (1.f - f) * c0) : fmaf(f, com2[i], (1.f - f) * c1);
+  volts[i] = v;
+  com2[i] = c1;
+  com1[i] = c0;
 }
 
 // RlSupervisor.correction_modal_basis step 2 (rlSupervisor.py:799-813):

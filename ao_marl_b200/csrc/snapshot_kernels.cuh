@@ -17,7 +17,7 @@
 #include "../../include/aomarl.h"
 
 // aom_reset_envs: restart listed environments while the others run on.
-#define RESET_MAX_BUFS (17 + 4 * AOM_MAX_LAYERS)    // controller, state and Strehl rows + screen and ring state per layer
+#define RESET_MAX_BUFS (18 + 4 * AOM_MAX_LAYERS)    // controller, state and Strehl rows + screen and ring state per layer
 struct ResetEnvsParams {
   // per-environment buffers whose rows are zeroed: word (s * slot_stride + e * ld + i), s < slots, i < ld
   uint32_t* buf[RESET_MAX_BUFS];
@@ -106,8 +106,11 @@ struct SnapParams {
   float cond_c[AOM_COND_COUNT][AOM_MAX_LAYERS];
 };
 
-// Layers of condition k in a context of L layers, and its field of layer l in a record head
-__host__ __device__ __forceinline__ int cond_layers(int k, int L) { return k <= AOM_COND_WIND_Y ? L : 1; }
+// Layers of condition k in a context of L layers (none for the unassigned value between AOM_COND_GAIN and
+// AOM_COND_DELAY), and its field of layer l in a record head
+__host__ __device__ __forceinline__ int cond_layers(int k, int L) {
+  return k <= AOM_COND_WIND_Y ? L : k <= AOM_COND_GAIN || k == AOM_COND_DELAY ? 1 : 0;
+}
 
 __host__ __device__ __forceinline__ float& head_cond(aom_env_head& h, int k, int l) {
   switch (k) {
@@ -116,6 +119,7 @@ __host__ __device__ __forceinline__ float& head_cond(aom_env_head& h, int k, int
     case AOM_COND_WIND_Y: return h.wind[l][1];
     case AOM_COND_NOISE: return h.noise;
     case AOM_COND_NPHOTONS: return h.nphotons;
+    case AOM_COND_DELAY: return h.delay;
     default: return h.gain;
   }
 }

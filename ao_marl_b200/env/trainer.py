@@ -56,7 +56,11 @@ class BatchedTrainer(BatchedRollout):
     `DelayedMDP` exactly as the reference: oldest state/action of the window, newest next state, current reward,
     mask = 1 because episodes are time-limited, train_rpc.py:755); after the episode the learner runs
     `updates_per_episode` batched SAC updates (gradients all-reduced over the process group when there is one)
-    and the new actors are uploaded into the simulator's tables."""
+    and the new actors are uploaded into the simulator's tables.
+
+    The window depth comes from env_rl["delayed_assignment"], a knob of its own as in the reference: it does not follow
+    the controller delay (Simulator.set_delay / set_delay_env), and one depth serves every environment of the batch
+    whatever their delays."""
 
     def __init__(self, env, learner, seed=1234, updates_per_episode=1000):
         super().__init__(env, seed=seed)
@@ -107,7 +111,9 @@ class StepLearner:
     agent per env-step on a second stream (the reference runs updates_per_episode_rpc = 1000 updates per 1000-step
     episode per agent, GlobalConfig.py:63, train_rpc.py:759-781, 1084-1133), gradients all-reduced over the process
     group when there is one.  Transitions go to the learner's device replay with the credit assignment window of
-    `DelayedMDP` (oldest state / action, newest next state, current reward; train_rpc.py:734-757)."""
+    `DelayedMDP` (oldest state / action, newest next state, current reward; train_rpc.py:734-757).  Its depth is
+    env_rl["delayed_assignment"] (or `depth`), set by the user as in the reference and independent of the controller
+    delay: per-environment delays (Simulator.set_delay_env) share the batch's one window."""
 
     def __init__(self, sim, rl, learner, depth=None):
         import torch

@@ -32,7 +32,7 @@ How each contributor is measured on this simulator (the arithmetic of the refere
 
 Loop filter.  On this simulator the breakdown of frame i sees the command c[i] that already contains the error of the
 frame's measurement, and that measurement saw the turbulence of frame i through the mirrors of command c[i-d],
-d = controller delay + 1 (apply_control's delay line):   c[i] = c[i-1] + g (-R s[i]),  s[i] = D (c[i-d] - B[i]) + ...
+d = controller delay + 1 (apply_control's delay line; the batch's common delay of 0, 1 or 2 frames):   c[i] = c[i-1] + g (-R s[i]),  s[i] = D (c[i-d] - B[i]) + ...
 Writing every part of -R s[i] separately gives, exactly,
     x[i]  = x[i-1]  - g gamma R D x[i-d]  + g b[i]                                (noise, non linearity, aliasing, tomography)
     bp[i] = bp[i-1] - g gamma R D bp[i-d] - (B[i] - B[i-1]) + g gamma R D (B[i] - B[i-d])        (bandwidth)
@@ -60,6 +60,17 @@ class Roket(RlSupervisor):
             raise NotImplementedError("ROKET's loop filter has one gain for the whole batch: per-environment gains "
                                       "(set_gain with an [E] array) are not supported; set a scalar gain")
 
+    def _common_delay(self):
+        """The loop filter of the breakdown uses one whole-frame delay for the whole batch: the common one of the store."""
+        if self.sim.delay_env is not None:
+            raise NotImplementedError("ROKET's loop filter has one delay for the whole batch: per-environment delays "
+                                      "(set_delay with an [E] array) are not supported; set a scalar delay")
+        d = self.sim.delay
+        if d != int(d):
+            raise NotImplementedError("ROKET's loop filter delays commands by whole frames: a fractional delay (%g) is not "
+                                      "supported; set a delay of 0, 1 or 2" % d)
+        return int(d)
+
     def _one_controller(self):
         """The breakdown models one controller for the whole batch."""
         if self.sim.controller_env is not None:
@@ -85,6 +96,7 @@ class Roket(RlSupervisor):
         assert N_total >= N_preloop
         self._common_gain()
         self._one_controller()
+        d = self._common_delay()
         t, E = self.tables, self.n_env
         dev = "cuda"
         self.agent, self.include_tip_tilt = agent, include_tip_tilt
@@ -117,7 +129,7 @@ class Roket(RlSupervisor):
         self.RD = self.cmat @ self.D
         self.g = float(self.config.p_controllers[0].gain)
         self.gRD = self.g * self.gamma * self.RD
-        self.delay = int(round(float(self.config.p_controllers[0].delay))) + 1
+        self.delay = d + 1
         nm = self.P.shape[0]
         keep = torch.ones(nm, dtype=torch.bool, device=dev)
         if self.nfiltered > 0:
@@ -156,6 +168,7 @@ class Roket(RlSupervisor):
         import torch
         self._common_gain()
         self._one_controller()
+        self.delay = self._common_delay() + 1
         i = self.iter_number
         if a is not None and i < self.n:
             act = torch.as_tensor(a, dtype=torch.float32, device="cuda")

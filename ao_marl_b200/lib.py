@@ -51,17 +51,18 @@ B = {name: i for i, name in enumerate(BUFFERS)}
 ENV_HEAD = np.dtype([("magic", "<u4"), ("bytes", "<u4"), ("fingerprint", "<u8"), ("frame", "<u4"), ("step", "<u4"),
                      ("le_n", "<i4", 2), ("first", "<i4"), ("n_layers", "<i4"), ("acc", "<f8", (MAX_LAYERS, 2)),
                      ("wind", "<f4", (MAX_LAYERS, 2)), ("amp", "<f4", MAX_LAYERS), ("noise", "<f4"), ("nphotons", "<f4"),
-                     ("gain", "<f4"), ("reserved", "<u4")])
+                     ("gain", "<f4"), ("reserved", "<u4"), ("delay", "<f4"), ("pad", "<u4")])
 _INT_BUFFERS = {"RING_OX", "RING_OY", "EXT_COUNT"}
-CONDITIONS = ["AMP", "WIND_X", "WIND_Y", "NOISE", "NPHOTONS", "GAIN"]
-COND = {name: i for i, name in enumerate(CONDITIONS)}
+CONDITIONS = ["AMP", "WIND_X", "WIND_Y", "NOISE", "NPHOTONS", "GAIN", "DELAY"]
+COND = {name: i for i, name in enumerate(CONDITIONS[:-1])}
+COND["DELAY"] = 7                    # aom_condition leaves 6 unassigned (AOM_COND_COUNT of builds without the delay)
 OPTIONS = ["WFS_PATH", "GEMM_PATH", "TIME_WFS", "GEO", "DENOISE", "PUPIL_PATH", "KEEP_IMAGE", "STREHL", "STREHL_LAMBDA_NM", "EXTRUDE_PATH", "STREHL_PEAK", "PSF_NFFT", "DENOISE_PATH"]
 O = {name: i for i, name in enumerate(OPTIONS)}
 
 EXPORTS = ["aom_config_size", "aom_create", "aom_destroy", "aom_last_error", "aom_set_table", "aom_get_buffer",
            "aom_device_count_launches", "aom_set_option", "aom_check_device", "aom_reset", "aom_reset_envs", "aom_env_state_bytes", "aom_save_envs", "aom_load_envs", "aom_move_atmos", "aom_set_layer", "aom_set_layer_amp", "aom_set_layer_wind", "aom_comp_wfs_image", "aom_set_wfs_noise", "aom_set_wfs_noise_env", "aom_get_condition", "aom_wfs_kernel", "aom_wfs_time_ms", "aom_raytrace_wfs",
            "aom_comp_strehl", "aom_reset_strehl", "aom_do_control_geo", "aom_apply_control_geo", "aom_denoise", "aom_set_bincube", "aom_do_centroids", "aom_do_centroids_geom", "aom_do_control", "aom_set_command", "aom_apply_control",
-           "aom_set_gain", "aom_set_gain_env", "aom_set_controller_env", "aom_get_controller_env", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
+           "aom_set_gain", "aom_set_gain_env", "aom_set_delay", "aom_set_delay_env", "aom_set_controller_env", "aom_get_controller_env", "aom_set_loop", "aom_reset_dm", "aom_set_dm_volts", "aom_rl_control",
            "aom_state_begin", "aom_state_end", "aom_reward", "aom_actor_forward", "aom_step", "aom_gemm_tn",
            "aom_pixel_noise"]
 
@@ -124,6 +125,8 @@ def load_library():
     lib.aom_apply_control.argtypes = [vp, i32, vp]
     lib.aom_set_gain.argtypes = [vp, f32]
     lib.aom_set_gain_env.argtypes = [vp, vp]
+    lib.aom_set_delay.argtypes = [vp, f32]
+    lib.aom_set_delay_env.argtypes = [vp, vp]
     lib.aom_set_controller_env.argtypes = [vp, vp]
     lib.aom_get_controller_env.argtypes = [vp, vp, ctypes.POINTER(i32)]
     lib.aom_set_loop.argtypes = [vp, i32]
@@ -231,10 +234,12 @@ class Simulator:
         cfg.tt_dim, cfg.tt_off = t.tt_dim, t.tt_off
         cfg.nactu, cfg.nslopes = t.nactu, t.nslopes
         cfg.nmodes = int(t.Btt.shape[1]) if getattr(t, "Btt", None) is not None else 0
-        cfg.gain, cfg.delay = t.gain, int(round(t.delay))
+        # the context starts with the whole frames of the delay; a fractional one is set right after aom_create
+        delay = float(t.delay)
+        if not 0.0 <= delay <= 2.0:
+            raise NotImplementedError("controller delay must be in [0, 2] frames, got %r" % delay)
+        cfg.gain, cfg.delay = t.gain, int(np.floor(delay))
         cfg.reward_factor = 1000.0
-        if float(t.delay) not in (0.0, 1.0):
-            raise NotImplementedError("controller delay must be 0 or 1 frame")
         if rl is not None:
             rl.fill_config(cfg)
         self.cfg = cfg
@@ -247,6 +252,8 @@ class Simulator:
                 self._ctx = ctypes.c_void_p()
             raise (ValueError if rc == -1 else RuntimeError)("aom_create: " + msg)
         self._stream = stream
+        if delay != cfg.delay:
+            self.set_delay(delay)
         self._views = {}
         # focal-plane grid of the target image (p_geom._ipupil, geom_init: 2^ceil(log2(pupdiam) + 1)) for the PSF core
         try:
@@ -311,6 +318,9 @@ class Simulator:
     wfs_noise_env = property(lambda self: self._condition("NOISE")[1])
     wfs_nphotons_env = property(lambda self: self._condition("NPHOTONS")[1])
     gain_env = property(lambda self: self._condition("GAIN")[1])
+    # controller delay in frames: the common value, and per-environment float32 [E] or None
+    delay = property(lambda self: self._condition("DELAY")[0])
+    delay_env = property(lambda self: self._condition("DELAY")[1])
 
     def launches(self):
         n = ctypes.c_uint64()
@@ -441,8 +451,8 @@ class Simulator:
         """Load the records `snap` ([n, env_state_bytes()] uint8, CPU or CUDA; from save_envs of this context or of one with
         the same configuration and tables) into the slots `envs` (aom_load_envs).  From then on each of those
         environments computes bit for bit what the saved one would have computed; the others are unaffected.  Conditions
-        carried by a record (amplitude, wind, sensor noise, photon count, gain) that differ from those in force become
-        per-environment values."""
+        carried by a record (amplitude, wind, sensor noise, photon count, gain, delay) that differ from those in force
+        become per-environment values."""
         torch = self.torch
         envs = self._env_list(envs, "load_envs")
         if not isinstance(snap, torch.Tensor) or snap.dtype != torch.uint8:
@@ -687,6 +697,22 @@ class Simulator:
         a = None if g is None else self._env_array(g, "set_gain_env")
         self._check(self.lib.aom_set_gain_env(self._ctx, None if a is None else a.ctypes.data_as(ctypes.c_void_p)),
                     "aom_set_gain_env")
+
+    def set_delay(self, d):
+        """Controller delay in frames, any real value in [0, 2]: a scalar sets the common delay (per-environment delays stay
+        in force, as aom_set_delay); an [E] array one delay per environment (set_delay_env).  A fractional delay blends
+        two commands of the delay line as sutra's set_delay: 1.5 gives the mean of the last two before this frame's."""
+        if np.ndim(d) == 0:
+            self._check(self.lib.aom_set_delay(self._ctx, float(d)), "aom_set_delay")
+        else:
+            self.set_delay_env(d)
+
+    def set_delay_env(self, d):
+        """One controller delay per environment ([E] in [0, 2]; a scalar broadcasts); None: back to the common delay.  The
+        delay line keeps every environment's last three commands, so a change takes effect at the next apply_control."""
+        a = None if d is None else self._env_array(d, "set_delay_env")
+        self._check(self.lib.aom_set_delay_env(self._ctx, None if a is None else a.ctypes.data_as(ctypes.c_void_p)),
+                    "aom_set_delay_env")
 
     CTRL_INTEGRATOR = -1
     MAX_POLICIES = 8

@@ -247,7 +247,8 @@ class DmB200(_Base):
 
 
 class _Controller:
-    """Stand-in for ``rtc._rtc.d_control[i]`` (ao_env.py:957, train_rpc.py:84 read .gain / call .set_gain)."""
+    """Stand-in for ``rtc._rtc.d_control[i]`` (ao_env.py:957, train_rpc.py:84 read .gain / call .set_gain; sutra's
+    controller also has .delay / set_delay)."""
 
     def __init__(self, sim, ctype):
         self._sim = sim
@@ -267,6 +268,21 @@ class _Controller:
             self._sim.set_gain_env(None)
         else:
             self._sim.set_gain_env(g)
+
+    @property
+    def delay(self):
+        """The controller delay in frames in force: the common one, or the float32 [E] per-environment delays."""
+        d = self._sim.delay_env
+        return self._sim.delay if d is None else d
+
+    def set_delay(self, d):
+        """A scalar in [0, 2] sets the delay of every environment (and drops per-environment delays); an [E] array one
+        delay per environment."""
+        if np.ndim(d) == 0:
+            self._sim.set_delay(float(d))
+            self._sim.set_delay_env(None)
+        else:
+            self._sim.set_delay_env(d)
 
 
 class _RtcHandle:

@@ -71,7 +71,8 @@ typedef struct aom_config {
   /* controller (rtc_init.py:451-513) */
   int32_t nactu, nslopes, nmodes;
   float gain;
-  int32_t delay;                        /* 0 or 1 frames of command latency (p_controller.delay) */
+  int32_t delay;                        /* 0, 1 or 2 frames of command latency (p_controller.delay): the initial common
+                                           value of AOM_COND_DELAY (aom_set_delay takes fractional ones) */
   /* RL layer (ao_env.py, train_rpc.py) */
   int32_t n_hist;                       /* number_of_previous_dm */
   int32_t state_modes;                  /* modes kept per state block (all modes when windowed, else the action range) */
@@ -240,8 +241,8 @@ int aom_reset(aom_ctx* ctx, const int64_t* seeds, void* stream);
  * distinct, 0 <= e < E) with seeds[0..n) (host int64) while the others run on.
  * - Each listed environment gets at once what aom_reset gives it: screens regenerated from its new seed (2N start-up
  *   extrusions per layer with its current amplitude and the sign of its current x wind, common or per-environment), ring
- *   origins, extrusion counters and wind accumulators at 0, and its rows of slopes, err, com, com1, volts, com_before,
- *   residual modes, every history slot, state, Strehl accumulators / figures and geometric controller buffers cleared.
+ *   origins, extrusion counters and wind accumulators at 0, and its rows of slopes, err, com, com1, com2, volts,
+ *   com_before, residual modes, every history slot, state, Strehl accumulators / figures and geometric controller buffers cleared.
  *   Set the new episode's conditions (aom_set_layer_amp / aom_set_layer_wind) before the call.
  * - Its next aom_step acts as the linear step that follows an aom_reset: its rl half-step is ignored (no action is
  *   injected, com stays 0, no Strehl is accumulated, reward 0) and the state it leaves is the s0 of a fresh episode
@@ -265,16 +266,16 @@ int aom_reset_envs(aom_ctx* ctx, int n, const int32_t* envs, const int64_t* seed
  *   record: bit-exactness needs the same tables in both contexts.
  * - A record is aom_env_state_bytes long (a multiple of 16): the head below, then the environment's rows of the state
  *   aom_reset_envs clears (screens in physical order with their ring origins and extrusion counts; slopes, err, com,
- *   com1, volts, com_before, residual modes, state, action, Strehl figures and accumulators, the geometric controller's
+ *   com1, com2, volts, com_before, residual modes, state, action, Strehl figures and accumulators, the geometric controller's
  *   rows when they are allocated), the command history in logical order (oldest first), the Philox keys and the pending
  *   target sums of both targets (AOM_TAR_TRACE / AOM_TAR_PUBLISH), each row padded to 16 bytes.
  * - aom_load_envs rebases the counters onto the context's own (noise frame, actor decisions, long-exposure counts and the
  *   first-step-pending flag of aom_reset_envs) and the history onto its ring head: the batch becomes staggered as after
  *   aom_reset_envs.  Loaded wind accumulators or winds that differ from the batch's common state put the batch into the
- *   per-environment wind state (aom_set_layer_wind); loaded amplitudes, sensor noise, photon counts and gains that
- *   differ from those in force create the per-environment arrays (aom_set_layer_amp, aom_set_wfs_noise_env,
- *   aom_set_gain_env) with every other environment's value kept.  The uniform kernels return as they do otherwise, at
- *   the latest at the next aom_reset.
+ *   per-environment wind state (aom_set_layer_wind); loaded amplitudes, sensor noise, photon counts, gains and delays
+ *   that differ from those in force create the per-environment arrays (aom_set_layer_amp, aom_set_wfs_noise_env,
+ *   aom_set_gain_env, aom_set_delay_env) with every other environment's value kept.  The uniform kernels return as
+ *   they do otherwise, at the latest at the next aom_reset.
  * - Errors: AOM_ERR_INVALID for n < 0, a slot out of range or listed twice, a null buffer, or (load) a record whose
  *   magic, size or fingerprint does not match this context -- nothing changes then.  AOM_ERR_STATE before the first
  *   aom_reset.  AOM_ERR_UNSUPPORTED (load) when a loaded wind state puts a pupil footprint off a screen.  As after
@@ -286,7 +287,7 @@ typedef struct aom_env_head {
   uint32_t magic;                   /* AOM_ENV_MAGIC */
   uint32_t bytes;                   /* record size (aom_env_state_bytes of the saving context) */
   uint64_t fingerprint;             /* FNV-1a of aom_config without n_env and the values setters change (deltax, deltay,
-                                       amp, gain, noise, nphotons) */
+                                       amp, gain, delay, noise, nphotons) */
   uint32_t frame;                   /* noise frames since the environment's reset */
   uint32_t step;                    /* actor decisions since its reset */
   int32_t le_n[2];                  /* long-exposure counts: main target, geometric target */
@@ -297,6 +298,8 @@ typedef struct aom_env_head {
   float amp[AOM_MAX_LAYERS];        /* innovation amplitude */
   float noise, nphotons, gain;      /* sensor noise, photons per subaperture and frame, integrator gain */
   uint32_t reserved;
+  float delay;                      /* controller delay, frames */
+  uint32_t pad;
 } aom_env_head;
 /* Size in bytes of one environment's record under the context's current allocation. */
 int aom_env_state_bytes(aom_ctx* ctx, size_t* bytes);
@@ -364,9 +367,9 @@ int aom_set_wfs_noise(aom_ctx* ctx, float noise, float nphotons);
  * Waits for the device; not for the step path. */
 int aom_set_wfs_noise_env(aom_ctx* ctx, const float* noise_host, const float* nphotons_host);
 
-/* Per-episode conditions: each is one common value or one value per environment of the batch.  The setters above and
- * aom_set_gain / aom_set_gain_env change them (every value must be finite, photon counts > 0); aom_load_envs merges
- * those of loaded records.  The values of aom_config are only their initial common values. */
+/* Per-episode conditions: each is one common value or one value per environment of the batch.  The setters above,
+ * aom_set_gain / aom_set_gain_env and aom_set_delay / aom_set_delay_env change them (every value must be finite, photon
+ * counts > 0, delays in [0, 2]); aom_load_envs merges those of loaded records.  The values of aom_config are only their initial common values. */
 typedef enum aom_condition {
   AOM_COND_AMP = 0,    /* innovation amplitude of a layer (aom_set_layer, aom_set_layer_amp) */
   AOM_COND_WIND_X,     /* wind step of a layer, pixels / frame (aom_set_layer, aom_set_layer_wind) */
@@ -374,6 +377,9 @@ typedef enum aom_condition {
   AOM_COND_NOISE,      /* sensor noise (aom_set_wfs_noise, aom_set_wfs_noise_env); layer 0 */
   AOM_COND_NPHOTONS,   /* photons per subaperture and frame; layer 0 */
   AOM_COND_GAIN,       /* integrator gain (aom_set_gain, aom_set_gain_env); layer 0 */
+  /* 6 is not a condition: it was AOM_COND_COUNT in builds without the delay, and callers built against those headers
+     may still pass it as their out-of-range value */
+  AOM_COND_DELAY = 7,  /* controller delay in frames, [0, 2] (aom_set_delay, aom_set_delay_env); layer 0 */
   AOM_COND_COUNT
 } aom_condition;
 /* Read back one condition (layer: that of AOM_COND_AMP / WIND_X / WIND_Y, 0 for the others).  Any output may be NULL.
@@ -446,6 +452,13 @@ int aom_do_centroids_geom(aom_ctx* ctx, int flags, float alpha, void* stream);
  * default tcgen05 path writes NaN to every output of that row; the SIMT path may give +-Inf instead. */
 int aom_do_control(aom_ctx* ctx, void* stream);
 int aom_set_command(aom_ctx* ctx, const float* dcom, int ld, void* stream);
+/* The delay line (sutra comp_voltage, a com + b com1 + c com2): c0 = com (this call's command), c1 = com1 and c2 = com2
+ * (those of the two calls before).  An environment with delay d in [0, 2], k = floor(d), f = d - k, gets
+ *   volts = c_k                                  when f == 0 (a copy: a non-finite row of another age stays out of volts)
+ *   volts = fmaf(f, c_(k+1), (1 - f) * c_k)     otherwise (float32, this expression)
+ * and then the line shifts for every environment and every delay, com2 <- com1, com1 <- com, so that a delay changed
+ * mid-episode reads a history that is already right.  d = 1.5 gives (com1 + com2) / 2, as sutra's set_delay weights.
+ * comp_voltage == 0: nothing happens (volts and the line unchanged).  One kernel launch. */
 int aom_apply_control(aom_ctx* ctx, int comp_voltage, void* stream);
 int aom_set_gain(aom_ctx* ctx, float gain);     /* common gain (finite); per-environment gains (aom_set_gain_env) stay in force */
 /* RtcCompass.set_gain per environment (the reference tunes the integrator gain per parameter file, params.py): gain of
@@ -453,6 +466,21 @@ int aom_set_gain(aom_ctx* ctx, float gain);     /* common gain (finite); per-env
  * com += g[e] err in all three controller paths.  Persists through aom_reset / aom_reset_envs.  AOM_ERR_INVALID for a
  * non-finite entry.  Waits for the device; not for the step path. */
 int aom_set_gain_env(aom_ctx* ctx, const float* gain_host);
+/* RtcCompass.set_delay (sutra set_delay; the reference's parameter files differ in p_controller.delay): common delay of
+ * every environment's controller in frames, any real value in [0, 2] (aom_apply_control says how a fractional one
+ * blends two commands).  It starts as aom_config.delay; per-environment delays (aom_set_delay_env) stay in force.
+ * AOM_ERR_INVALID for a non-finite value or one outside [0, 2]. */
+int aom_set_delay(aom_ctx* ctx, float delay);
+/* The same per environment (one loop latency per environment of the batch): host float [E] (NULL: back to the common
+ * delay of aom_config.delay / aom_set_delay).
+ * - Every environment computes bit for bit what it computes in a batch whose common delay is its value, in
+ *   aom_apply_control and in every mode of aom_step.
+ * - The delay line holds the last three commands of every environment whatever its delay, so a change mid-episode (of
+ *   one environment or of all) takes effect at the next aom_apply_control with the history already in place.
+ * - Persists through aom_reset / aom_reset_envs; aom_load_envs merges the delays of loaded records.
+ * - AOM_ERR_INVALID for a non-finite entry or one outside [0, 2]; nothing changes then.  Waits for the device; not for
+ *   the step path. */
+int aom_set_delay_env(aom_ctx* ctx, const float* delay_host);
 int aom_set_loop(aom_ctx* ctx, int closed);       /* rtc.open_loop / close_loop (rtcCompass.py:116-142) */
 int aom_reset_dm(aom_ctx* ctx, void* stream);     /* DmCompass.reset_dm */
 int aom_set_dm_volts(aom_ctx* ctx, const float* dvolts, int ld, void* stream); /* DmCompass.set_command */
